@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload unary_b64|pairwise_b64|pairwise_w4_b64|...]
   python bench.py --impl reference ...      # the reference's own implementation, same workload
+  python bench.py ... --dump-outputs DIR    # also write the results of the last timed step as DIR/*.npy
 
 A "step" is one pass of the whole path (column join -> tables -> DP -> backtracking -> instance
 grouping -> result packing) over one batch of synthetic Cityscapes-shaped frames per GPU.  Frames are
@@ -50,6 +51,8 @@ ROWS, COLS = 1024, 2048
 RECORD_WORDS_PER_ROW = 32   # prefix records: one 128-byte row per image row and column (common.cuh kRecBWords)
 OPS_PER_CELL = {"unary": 103, "pairwise": 128}  # SURVEY.md 8d minimal op budget
 NCU_SOURCE = "profiles/r2d_*.txt"
+DUMP_BYTES = 64 * 2**20 - 2**16   # --dump-outputs: at most 64 MB, .npy headers included
+DUMP_SEED = 0x5717E1
 # dram__bytes_read.sum + dram__bytes_write.sum per launch, from the `ncu --set full` captures summarised in
 # profiles/r2d_{unary,pairwise}.txt (width 8; unary launches carry 32 frames, pairwise launches 64; no capture for
 # width 4).  "tables" = join_columns + (frame_tables) + column_tables + object_lut kernels.
@@ -297,6 +300,33 @@ def narrow_inputs(disp, seg):
     return d16, s16
 
 
+def dump_outputs(out_dir, sections, instances, offsets):
+    """What the timed path delivers for its last batch (isx_fetch_batch_results), as float32 .npy files so that two
+    builds can be compared output for output: the stixels of every column of every frame, top to bottom, one file
+    per Section field (section_<field>.npy), stixels_per_column.npy [frames][C], and the instance records, one file
+    per field (instance_<field>.npy) with instances_per_frame.npy.  Every value is an integer below 2**24 or a
+    float32, so float32 holds it exactly.  When the whole batch does not fit in DUMP_BYTES, frames are taken in a
+    seeded random order until the next one would not fit; frames.npy lists the frames written, in batch order."""
+    S = sections.shape[2]
+    term = sections["type"] == -1
+    lengths = np.where(term.any(axis=2), term.argmax(axis=2), S)
+    inst_counts = np.diff(offsets)
+    frame_bytes = (lengths.sum(axis=1) * len(sections.dtype.names) + lengths.shape[1]) * 4 + \
+        inst_counts * len(instances.dtype.names) * 4 + 8
+    order = np.random.default_rng(DUMP_SEED).permutation(len(sections))
+    k = int(np.searchsorted(np.cumsum(frame_bytes[order]), DUMP_BYTES, side="right"))
+    frames = np.sort(order[:k])
+    used = np.arange(S)[None, None, :] < lengths[frames][:, :, None]
+    stixels = sections[frames][used]
+    inst = np.concatenate([instances[offsets[f]:offsets[f + 1]] for f in frames]) if k else instances[:0]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {f"section_{n}": stixels[n] for n in sections.dtype.names}
+    arrays.update({f"instance_{n}": inst[n] for n in instances.dtype.names})
+    arrays.update(stixels_per_column=lengths[frames], instances_per_frame=inst_counts[frames], frames=frames)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def time_device(env, st, step, steps, stream):
     """`steps` device-resident batches between two CUDA events on the library's stream, max over ranks (ms)."""
     import torch
@@ -313,7 +343,7 @@ def time_device(env, st, step, steps, stream):
     return env.max_over_ranks(local), local
 
 
-def measure(env, name, wl, steps, warmup, primary, extras=True):
+def measure(env, name, wl, steps, warmup, primary, extras=True, dump_dir=None):
     """One workload on this rank's GPU: the same dict on every rank (rank 0 prints it)."""
     import torch
     from instance_stixels_b200 import api, synth
@@ -351,6 +381,8 @@ def measure(env, name, wl, steps, warmup, primary, extras=True):
     units_eval, units_total = units1[0] - units0[0], units1[1] - units0[1]
     stages = st.stage_times(reset=True)
     st.set_profiling(False)
+    if dump_dir:   # before the e2e runs below overwrite the results of the timed steps
+        dump_outputs(dump_dir, *st.FetchBatchResults(B))
 
     # ---- e2e: host buffers through the public batch API, copies inside the timed region ----
     # One host thread, one context, the streaming form of the batch call: isx_submit_batch_host enqueues a batch
@@ -572,7 +604,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="only --workload: no other configurations, latency or no-prune runs")
     ap.add_argument("--extra-workloads", default="pairwise_b64,pairwise_w4_b64,pairwise_stream_b256")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of --workload computed as DIR/<name>.npy (float32, at most "
+                         "64 MB; with several ranks DIR/rank<k>/)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of --impl ours")
     wl = WORKLOADS[args.workload]
     env = Env()
 
@@ -605,7 +644,11 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", env.local))
 
     t_start = time.perf_counter()
-    main_res = measure(env, args.workload, wl, args.steps, args.warmup, primary=True, extras=not args.no_extra)
+    dump_dir = args.dump_outputs
+    if dump_dir and env.world > 1:
+        dump_dir = os.path.join(dump_dir, f"rank{env.rank}")
+    main_res = measure(env, args.workload, wl, args.steps, args.warmup, primary=True, extras=not args.no_extra,
+                       dump_dir=dump_dir)
     others = {}
     if not args.no_extra:
         for name in [n for n in args.extra_workloads.split(",") if n and n != args.workload]:

@@ -1,6 +1,8 @@
 """Comparison helpers shared by the parity tests and tools/gpu_parity_report.py."""
 from __future__ import annotations
 
+import hashlib
+
 import numpy as np
 
 from instance_stixels_b200 import _lib as L
@@ -90,6 +92,31 @@ def compare_instances(ours: np.ndarray, ref: np.ndarray) -> dict:
     keys_r = {(int(r["column"]), int(r["index"])) for r in ref}
     return dict(n_ours=len(ours), n_ref=len(ref), same_keys=keys_o == keys_r, clusters_ours=len(so),
                 clusters_ref=len(sr), same_partition=(so == sr and po.get(None, set()) == pr.get(None, set())))
+
+
+def sections_digest(sections: np.ndarray) -> str:
+    """SHA-256 of the column lengths and the stixels of a [C][200] Section array: equal digests mean identical
+    boundaries, types and classes and bit-identical floats on every column (the terminators are not included)."""
+    n = column_lengths(sections)
+    used = np.arange(sections.shape[1])[None, :] < n[:, None]
+    h = hashlib.sha256(n.astype(np.int32).tobytes())
+    h.update(np.ascontiguousarray(sections[used]).tobytes())
+    return h.hexdigest()
+
+
+def partition_digest(instances: np.ndarray) -> str:
+    """SHA-256 of the instance stixels and their partition up to label permutation: equal digests mean what
+    compare_instances calls same_keys and same_partition."""
+    groups = partition_of(instances)
+    keys = sorted((int(r["column"]), int(r["index"])) for r in instances)
+    clusters = sorted(sorted(v) for k, v in groups.items() if k is not None)
+    noise = sorted(groups.get(None, ()))
+    return hashlib.sha256(repr((keys, clusters, noise)).encode()).hexdigest()
+
+
+def array_digest(a: np.ndarray) -> str:
+    """SHA-256 of the bytes of an array (bit-exact comparison of a stored table)."""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def bit_equal(a: np.ndarray, b: np.ndarray) -> float:

@@ -1,46 +1,52 @@
 """Parity at BASELINE.json's size ON THE FRAMES THE BENCH TIMES: all 64 frames of unary_b64, pairwise_b64 and
-pairwise_w4_b64 (1024 x 2048) through the batched host entry point against the reference CUDA build
-(oracle/_ref), frame by frame.  Bar (north star): boundaries / types / classes / instance partitions identical on
-every column, costs / disparities / instance means within 1e-4 relative on every column.
+pairwise_w4_b64 (1024 x 2048) through the batched host entry point against what the reference CUDA build computed
+for them, frame by frame (per-frame digests in tests/golden/reference_build/digests.json, see
+tools/make_reference_build_golden.py).  Bar: boundaries / types / classes / instance partitions identical on every
+column and every float field of every stixel bit-identical.
 
 Plus a seeded fuzz of the two pruning DP kernels against the exhaustive ones (full cost / argmin tables) over random
 small shapes, weights and horizons."""
+import json
 import os
-import sys
 
 import numpy as np
 import pytest
 
 import parity
 from instance_stixels_b200 import _lib as L, api, synth
-from oracle import refbind
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "tools"))
+DIGESTS = os.path.join(ROOT, "tests", "golden", "reference_build", "digests.json")
+FULL_ROWS, FULL_COLS = 1024, 2048
+# the bench's workloads (bench.py WORKLOADS): mode, column_step
+BENCH_WORKLOADS = {"unary_b64": ("unary", 8), "pairwise_b64": ("pairwise", 8), "pairwise_w4_b64": ("pairwise", 4)}
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.skipif(not refbind.available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("workload", ["unary_b64", "pairwise_b64", "pairwise_w4_b64"])
+@pytest.mark.parametrize("workload", list(BENCH_WORKLOADS))
 def test_all_bench_frames_against_reference_cuda_build(workload):
-    import fullsize_parity
-    rep = fullsize_parity.run_workload(workload, frames=64)
-    assert rep["columns"] == 64 * (2048 // rep["column_step"])
-    # stixel boundaries, types and classes: identical on EVERY column of every frame (no ties to document)
-    assert rep["columns_exact"] == rep["columns"], rep["differing_columns"]
-    assert rep["stixels_ours"] == rep["stixels_ref"]
-    # DP costs, stixel disparities, instance means: within 1e-4 relative (north-star tolerance) on every column
-    assert rep["columns_close_1e4"] == rep["columns"], rep["field_bit_mismatches"]
+    mode, step = BENCH_WORKLOADS[workload]
+    with open(DIGESTS) as f:
+        want = json.load(f)["fullsize"][workload]
+    pre = synth.preset(mode, FULL_ROWS, FULL_COLS, step)
+    disp, seg, roads = synth.make_batch(64, rows=FULL_ROWS, cols=FULL_COLS, column_step=step)
+    st = api.make_stixels(pre, max_batch=64)
+    sec, inst, offs = st.ComputeBatch(mode == "pairwise", disp, seg, roads)
+    ev, tot = st.dp_units()
+    st.Finish()
+    assert sec.shape[:2] == (64, FULL_COLS // step)
+    assert [int(parity.column_lengths(s).sum()) for s in sec] == want["stixels"]
+    # stixel boundaries, types and classes identical and every float field of every stixel bit-identical, on EVERY
+    # column of every frame (profiles/r2_fullsize_parity.json: 2.8 million stixels, no differing bit).  The kernels
+    # spell every float operation in the order of the reference's SASS.
+    differing = [f for f in range(64) if parity.sections_digest(sec[f]) != want["sections"][f]]
+    assert not differing, differing
     # instance ids up to label permutation (same candidates AND same partition), frame by frame
-    assert rep["frames_same_keys"] == 64 and rep["frames_same_partition"] == 64
-    # ... and in fact bit-identical: every float field of every stixel (profiles/r2_fullsize_parity.json: 2.8 million
-    # stixels, no differing bit).  The kernels spell every float operation in the order of the reference's SASS.
-    assert rep["columns_bitwise"] == rep["columns"], rep["field_bit_mismatches"]
-    for f, m in rep["field_bit_mismatches"].items():
-        assert m["stixels"] == 0, (f, m)
+    differing = [f for f in range(64) if parity.partition_digest(inst[offs[f]:offs[f + 1]]) != want["instances"][f]]
+    assert not differing, differing
     if workload == "unary_b64":
-        assert rep["dp_units_evaluated_frac"] < 0.5
+        assert ev / tot < 0.5
 
 
 def _fuzz_case(rng, mode):
