@@ -15,7 +15,7 @@
 // Not kept: OpenCV, rapidjson and HDF5 (apps/loaders.h reads the PNG, the three camera numbers and an .npy copy of
 // the "nlogprobs" dataset; tools/h5_to_npy.py converts), the TensorRT path (argument 11 is refused), readdir order
 // (frames are processed in sorted order).  Rows >= 1024 are refused like the reference does (:129-134) unless
-// ISX_ALLOW_1024=1: the library itself handles 1024 rows.
+// ISX_ALLOW_1024=1: the library itself handles frames of up to ISX_MAX_ROWS (2047) rows.
 #include <dirent.h>
 #include <sys/stat.h>
 
@@ -123,8 +123,10 @@ Disparity load_disparity(const std::string& path, int max_dis) {
         throw std::invalid_argument("ERROR: Image height has to be equal or bigger than maximum disparity.");
     const char* allow = std::getenv("ISX_ALLOW_1024");
     const bool allow_1024 = allow && std::atoi(allow) != 0;
-    if (png.rows > 1024 || (png.rows == 1024 && !allow_1024))
+    if (png.rows >= 1024 && !allow_1024)
         throw std::invalid_argument("ERROR: Maximum image height has to be less than 1024.");
+    if (png.rows > ISX_MAX_ROWS)
+        throw std::invalid_argument("ERROR: Maximum image height is " + std::to_string(ISX_MAX_ROWS) + ".");
     Disparity d;
     d.rows = png.rows;
     d.cols = png.cols;

@@ -50,6 +50,12 @@ typedef enum isx_status {
 #define ISX_DOWNSAMPLE_FACTOR 8
 #define ISX_INSTANCE_CLASSES 8      /* Cityscapes trainIds 11..18 (Stixels.cu:47) */
 #define ISX_FIRST_INSTANCE_CLASS 11 /* StixelsKernels.cu:926 */
+/* Tallest frame isx_initialize accepts.  The reference stops at 1024 rows (one
+ * thread per row in one block); its tile DP does not need that, and up to 2047
+ * rows the reference's padded sizes (rows_power2 = 2048,
+ * rows_power2_segmentation = 256) and so the segmentation layout stay the same.
+ * Taller frames are refused with ISX_ERR_UNSUPPORTED. */
+#define ISX_MAX_ROWS 2047
 
 /* Same members, defaults and "-1 == unset" sentinels as `StixelConfig`
  * (types.h:30-141).  isx_config_init() writes the reference's defaults. */
@@ -165,7 +171,8 @@ int isx_set_model_parameters(isx_handle h, int column_step, int median_join, flo
                              float range_objects_z, int width_margin); /* :439-446 */
 /* Stixels::Initialize (Stixels.cu:43-248): allocations + LUT precompute.
  * `max_batch` >= 1 is the number of frames one batched call may carry (the
- * reference has no batching; its Initialize is max_batch == 1). */
+ * reference has no batching; its Initialize is max_batch == 1).  Frames of
+ * more than ISX_MAX_ROWS rows are refused with ISX_ERR_UNSUPPORTED. */
 int isx_initialize(isx_handle h, int max_batch);
 /* Stixels::Finish (Stixels.cu:250-283). */
 int isx_finish(isx_handle h);

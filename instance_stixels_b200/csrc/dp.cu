@@ -388,7 +388,7 @@ __device__ __forceinline__ void store_best(float4 *p, const Best &b) {
   __stcg(p, make_float4(b.gs, b.o, __int_as_float(b.vb_gs), __int_as_float(b.vb_o)));
 }
 
-template <bool PAIRWISE, bool HAS_INVALID, int WARPS>
+template <bool PAIRWISE, bool HAS_INVALID, int WARPS, int HP>
 __global__ void __launch_bounds__(WARPS * 32, WARPS == kDpWarps ? (PAIRWISE ? ISX_PAIRWISE_CTAS : ISX_UNARY_CTAS) : 2)
 dp_kernel(const uint32_t *__restrict__ records_b,
           const float *__restrict__ object_lut, const float *__restrict__ stat, float *__restrict__ pm_out,
@@ -400,7 +400,7 @@ dp_kernel(const uint32_t *__restrict__ records_b,
   const int tid = threadIdx.x, lane = tid & 31;
   const int gcol = blockIdx.x;  // frame * C + column
   const int H = p.rows, C = p.realcols;
-  constexpr int Hp = kRecStride;  // == p.rec_stride; a constant so that the A-side word offsets are immediates
+  constexpr int Hp = HP;  // == p.rec_stride; a constant so that the A-side word offsets are immediates
   const int f = gcol / C;
   const int vhor = vhor_arr[f];
   const float inf = inf_f();
@@ -728,13 +728,18 @@ dp_kernel(const uint32_t *__restrict__ records_b,
 //      the result of at most 37 additions (32 chunk carries + 5 Kogge-Stone / Blelloch levels) of partial sums whose
 //      magnitude is at most rows * cmax (cmax = largest |per-row cost| of the model): |error| <= 2 * 37 * 2^-24 *
 //      rows * cmax, plus one rounding each for the bound's own rows * lb product and its scaling by dw.
-//      kDataErr = 2^-17 = 128 * 2^-24 covers 2 * 37 + 6 roundings;
+//      kDataErr = 2^-17 = 128 * 2^-24 covers 2 * 37 + 6 roundings.  Frames of up to 2047 rows have up to 64 chunk
+//      carries, 69 additions: kDataErrTall = 2^-16 = 256 * 2^-24 covers 2 * 69 + 6 = 144 roundings;
 //  (b) the order of the final operations (the cell: one FFMA on the data term and the prior, then one on the class
 //      sum; the bound: FMUL, FADD, FFMA): each rounding is relative 2^-24 of a value no larger than
 //      |X| + |dw * data_lb| + |prior_lb|; kRelErr = 2^-20 leaves a factor 16 over the <= 4 roundings involved.
-// Nothing else is hand-picked: the bound holds for any rows, max_dis and non-negative weights.
+// Nothing else is hand-picked: with the data slack of its record stride, the bound holds for any rows up to
+// kMaxRows, any max_dis and non-negative weights.
 constexpr float kDataErr = 7.62939453125e-06f;     // 2^-17
+constexpr float kDataErrTall = 1.52587890625e-05f; // 2^-16
 constexpr float kRelErr = 9.5367431640625e-07f;    // 2^-20
+template <int HP>
+__device__ __forceinline__ constexpr float data_err() { return HP > kRecStride ? kDataErrTall : kDataErr; }
 __device__ __forceinline__ float prune_bound(float x, float dneg, float prior, float data_slack) {
   if (!(x < inf_f())) return x;   // +inf (no finite candidate in the chunk) stays +inf; NaN never prunes
   const float mag = fadd(fadd(fabsf(x), fabsf(dneg)), fabsf(prior));
@@ -757,7 +762,7 @@ struct PruneLayout {
   }
 };
 
-template <bool HAS_INVALID, int WARPS>
+template <bool HAS_INVALID, int WARPS, int HP>
 __global__ void __launch_bounds__(WARPS * 32, WARPS == kDpWarps ? ISX_PRUNED_CTAS : 2)
 dp_unary_pruned_kernel(const uint32_t *__restrict__ records_b,
                        const float *__restrict__ object_lut, const float *__restrict__ ground,
@@ -769,7 +774,7 @@ dp_unary_pruned_kernel(const uint32_t *__restrict__ records_b,
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int gcol = blockIdx.x;  // frame * C + column
   const int H = p.rows, C = p.realcols;
-  constexpr int Hp = kRecStride;
+  constexpr int Hp = HP;  // == p.rec_stride
   const int f = gcol / C;
   const int vhor = vhor_arr[f];
   const float inf = inf_f();
@@ -871,9 +876,9 @@ dp_unary_pruned_kernel(const uint32_t *__restrict__ records_b,
     const float nmaxf = (float)(vTmaxc + 1);
     const float dneg_o = fmul(c.dw, fmul(nmaxf, fminf(lb_o, 0.0f)));
     const float dneg_gs = fmul(c.dw, fmul(nmaxf, fminf(vTc < vhor ? lb_g : lb_s, 0.0f)));
-    // slack of the data terms (prune_slack below): dw * kDataErr * rows * largest per-row cost
-    const float dslack_o = fmul(c.dw, fmul(fmul(nmaxf, cmax_o), kDataErr));
-    const float dslack_gs = fmul(c.dw, fmul(fmul(nmaxf, vTc < vhor ? cmax_g : cmax_s), kDataErr));
+    // slack of the data terms (prune_bound above): dw * data_err<HP>() * rows * largest per-row cost
+    const float dslack_o = fmul(c.dw, fmul(fmul(nmaxf, cmax_o), data_err<HP>()));
+    const float dslack_gs = fmul(c.dw, fmul(fmul(nmaxf, vTc < vhor ? cmax_g : cmax_s), data_err<HP>()));
 
     Best carried{inf, inf, 0, 0};
     int buf = 0;
@@ -1043,7 +1048,7 @@ __device__ __forceinline__ float object_prior_floor(const RowInfo &q, bool groun
   return fmul(m, pw);
 }
 
-template <bool HAS_INVALID, int WARPS>
+template <bool HAS_INVALID, int WARPS, int HP>
 __global__ void __launch_bounds__(WARPS * 32, WARPS == 1 ? ISX_WALK_WARPS_PER_SM : WARPS == kDpWarps ? ISX_WALK_CTAS : 2)
 dp_pairwise_walk_kernel(const uint32_t *__restrict__ records_b,
                         const float *__restrict__ object_lut, const float *__restrict__ stat,
@@ -1057,7 +1062,7 @@ dp_pairwise_walk_kernel(const uint32_t *__restrict__ records_b,
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int gcol = blockIdx.x;
   const int H = p.rows, C = p.realcols;
-  constexpr int Hp = kRecStride;
+  constexpr int Hp = HP;  // == p.rec_stride
   const int f = gcol / C;
   const int vhor = vhor_arr[f];
   const float inf = inf_f();
@@ -1149,8 +1154,8 @@ dp_pairwise_walk_kernel(const uint32_t *__restrict__ records_b,
     const float nmaxf = (float)(vTmaxc + 1);
     const float dneg_o = fmul(c.dw, fmul(nmaxf, fminf(lb_o, 0.0f)));
     const float dneg_gs = fmul(c.dw, fmul(nmaxf, fminf(vTc < vhor ? lb_g : lb_s, 0.0f)));
-    const float dslack_o = fmul(c.dw, fmul(fmul(nmaxf, cmax_o), kDataErr));
-    const float dslack_gs = fmul(c.dw, fmul(fmul(nmaxf, vTc < vhor ? cmax_g : cmax_s), kDataErr));
+    const float dslack_o = fmul(c.dw, fmul(fmul(nmaxf, cmax_o), data_err<HP>()));
+    const float dslack_gs = fmul(c.dw, fmul(fmul(nmaxf, vTc < vhor ? cmax_g : cmax_s), data_err<HP>()));
     const float nicA = fmul((float)(int)A[kRecOff], c.iw);   // iw * O(vT + 1)
     (void)dneg_gs;
 
@@ -1438,15 +1443,15 @@ size_t dp_smem_bytes(const KParams &p, bool pairwise) {
   return DpLayout(p.rows, p.max_dis, pairwise).total;
 }
 
-template <bool PAIRWISE, bool HAS_INVALID, int WARPS>
+template <bool PAIRWISE, bool HAS_INVALID, int WARPS, int HP>
 static void launch_dp_warps(const KParams &p, const BatchBuffers &b, int ncolumns, size_t smem, cudaStream_t s) {
   static SmemOptIn optin;
-  opt_in_smem(dp_kernel<PAIRWISE, HAS_INVALID, WARPS>, optin);
-  dp_kernel<PAIRWISE, HAS_INVALID, WARPS><<<ncolumns, WARPS * 32, smem, s>>>(
+  opt_in_smem(dp_kernel<PAIRWISE, HAS_INVALID, WARPS, HP>, optin);
+  dp_kernel<PAIRWISE, HAS_INVALID, WARPS, HP><<<ncolumns, WARPS * 32, smem, s>>>(
       b.records_b, b.object_lut, b.stat, b.pm, b.vhor, b.object_disparity_range, b.inverse_height, b.dp, p);
 }
 
-template <bool PAIRWISE, bool HAS_INVALID>
+template <bool PAIRWISE, bool HAS_INVALID, int HP>
 static void launch_dp_variant(const KParams &p, const BatchBuffers &b, int ncolumns, size_t smem, cudaStream_t s) {
   const int sms = device_sm_count();
   bool latency = ncolumns < 2 * sms;
@@ -1454,20 +1459,20 @@ static void launch_dp_variant(const KParams &p, const BatchBuffers &b, int ncolu
     if (std::atoi(e) == kDpWarps) latency = false;
     if (std::atoi(e) == kDpWarpsLatency) latency = true;
   }
-  if (latency) launch_dp_warps<PAIRWISE, HAS_INVALID, kDpWarpsLatency>(p, b, ncolumns, smem, s);
-  else launch_dp_warps<PAIRWISE, HAS_INVALID, kDpWarps>(p, b, ncolumns, smem, s);
+  if (latency) launch_dp_warps<PAIRWISE, HAS_INVALID, kDpWarpsLatency, HP>(p, b, ncolumns, smem, s);
+  else launch_dp_warps<PAIRWISE, HAS_INVALID, kDpWarps, HP>(p, b, ncolumns, smem, s);
 }
 
-template <bool HAS_INVALID, int WARPS>
+template <bool HAS_INVALID, int WARPS, int HP>
 static void launch_unary_pruned_warps(const KParams &p, const BatchBuffers &b, int ncolumns, cudaStream_t s) {
   const size_t smem = PruneLayout(p.rows, WARPS).total;
   static SmemOptIn optin;
-  opt_in_smem(dp_unary_pruned_kernel<HAS_INVALID, WARPS>, optin);
-  dp_unary_pruned_kernel<HAS_INVALID, WARPS><<<ncolumns, WARPS * 32, smem, s>>>(
+  opt_in_smem(dp_unary_pruned_kernel<HAS_INVALID, WARPS, HP>, optin);
+  dp_unary_pruned_kernel<HAS_INVALID, WARPS, HP><<<ncolumns, WARPS * 32, smem, s>>>(
       b.records_b, b.object_lut, b.ground, b.vhor, b.inverse_height, b.dp, b.dp_units, b.col_flags, p);
 }
 
-template <bool HAS_INVALID>
+template <bool HAS_INVALID, int HP>
 static void launch_unary_pruned(const KParams &p, const BatchBuffers &b, int ncolumns, cudaStream_t s) {
   const int sms = device_sm_count();
   bool latency = ncolumns < 2 * sms;
@@ -1475,21 +1480,21 @@ static void launch_unary_pruned(const KParams &p, const BatchBuffers &b, int nco
     if (std::atoi(e) == kDpWarps) latency = false;
     if (std::atoi(e) == kDpWarpsLatency) latency = true;
   }
-  if (latency) launch_unary_pruned_warps<HAS_INVALID, kDpWarpsLatency>(p, b, ncolumns, s);
-  else launch_unary_pruned_warps<HAS_INVALID, kDpWarps>(p, b, ncolumns, s);
+  if (latency) launch_unary_pruned_warps<HAS_INVALID, kDpWarpsLatency, HP>(p, b, ncolumns, s);
+  else launch_unary_pruned_warps<HAS_INVALID, kDpWarps, HP>(p, b, ncolumns, s);
 }
 
-template <bool HAS_INVALID, int WARPS>
+template <bool HAS_INVALID, int WARPS, int HP>
 static void launch_pairwise_walk_warps(const KParams &p, const BatchBuffers &b, int ncolumns, cudaStream_t s) {
   const size_t smem = WalkLayout(p.rows, p.max_dis, WARPS).total;
   static SmemOptIn optin;
-  opt_in_smem(dp_pairwise_walk_kernel<HAS_INVALID, WARPS>, optin);
-  dp_pairwise_walk_kernel<HAS_INVALID, WARPS><<<ncolumns, WARPS * 32, smem, s>>>(
+  opt_in_smem(dp_pairwise_walk_kernel<HAS_INVALID, WARPS, HP>, optin);
+  dp_pairwise_walk_kernel<HAS_INVALID, WARPS, HP><<<ncolumns, WARPS * 32, smem, s>>>(
       b.records_b, b.object_lut, b.stat, b.ground, b.pm, b.qrows, b.vhor, b.object_disparity_range, b.dp,
       b.dp_units, b.col_flags, p);
 }
 
-template <bool HAS_INVALID>
+template <bool HAS_INVALID, int HP>
 static void launch_pairwise_walk(const KParams &p, const BatchBuffers &b, int ncolumns, cudaStream_t s) {
   const int sms = device_sm_count();
   bool latency = ncolumns < 2 * sms;
@@ -1501,9 +1506,9 @@ static void launch_pairwise_walk(const KParams &p, const BatchBuffers &b, int nc
   // carried minima see every chunk it evaluated); ISX_WALK_WARPS=4 keeps the 4-warp CTA per column for A/B runs
   int tw = 1;
   if (const char *e = std::getenv("ISX_WALK_WARPS")) tw = std::atoi(e);
-  if (latency) launch_pairwise_walk_warps<HAS_INVALID, kDpWarpsLatency>(p, b, ncolumns, s);
-  else if (tw == kDpWarps) launch_pairwise_walk_warps<HAS_INVALID, kDpWarps>(p, b, ncolumns, s);
-  else launch_pairwise_walk_warps<HAS_INVALID, 1>(p, b, ncolumns, s);
+  if (latency) launch_pairwise_walk_warps<HAS_INVALID, kDpWarpsLatency, HP>(p, b, ncolumns, s);
+  else if (tw == kDpWarps) launch_pairwise_walk_warps<HAS_INVALID, kDpWarps, HP>(p, b, ncolumns, s);
+  else launch_pairwise_walk_warps<HAS_INVALID, 1, HP>(p, b, ncolumns, s);
 }
 
 // Which pairwise kernel runs: the tile-major walk (ISX_PAIRWISE_WALK=1) or the chunk-major exhaustive one.
@@ -1521,7 +1526,9 @@ bool pairwise_walk_used(int ncolumns, bool have_qrows) {
   return pairwise_walk_enabled() && have_qrows && (ncolumns >= 16 * sm_count || forced);
 }
 
-void launch_dp(const KParams &p, const BatchBuffers &b, int nframes, bool pairwise, cudaStream_t s) {
+// HP: the record stride (kRecStride, or kRecStrideTall for frames of more than kShortRows rows)
+template <int HP>
+static void launch_dp_rows(const KParams &p, const BatchBuffers &b, int nframes, bool pairwise, cudaStream_t s) {
   const int ncolumns = nframes * p.realcols;
   const size_t smem = dp_smem_bytes(p, pairwise);
   const bool has_invalid = p.invalid_disparity >= 0.0f;  // ComputeMean's two modes (StixelsKernels.cu:47-60)
@@ -1529,19 +1536,24 @@ void launch_dp(const KParams &p, const BatchBuffers &b, int nframes, bool pairwi
   const char *ex = std::getenv("ISX_UNARY_EXHAUSTIVE");
   const bool exhaustive = ex && std::atoi(ex) != 0;
   if (pairwise && pairwise_walk_used(ncolumns, b.qrows != nullptr)) {
-    if (has_invalid) launch_pairwise_walk<true>(p, b, ncolumns, s);
-    else launch_pairwise_walk<false>(p, b, ncolumns, s);
+    if (has_invalid) launch_pairwise_walk<true, HP>(p, b, ncolumns, s);
+    else launch_pairwise_walk<false, HP>(p, b, ncolumns, s);
   } else if (pairwise) {
-    if (has_invalid) launch_dp_variant<true, true>(p, b, ncolumns, smem, s);
-    else launch_dp_variant<true, false>(p, b, ncolumns, smem, s);
+    if (has_invalid) launch_dp_variant<true, true, HP>(p, b, ncolumns, smem, s);
+    else launch_dp_variant<true, false, HP>(p, b, ncolumns, smem, s);
   } else if (!exhaustive) {
-    if (has_invalid) launch_unary_pruned<true>(p, b, ncolumns, s);
-    else launch_unary_pruned<false>(p, b, ncolumns, s);
+    if (has_invalid) launch_unary_pruned<true, HP>(p, b, ncolumns, s);
+    else launch_unary_pruned<false, HP>(p, b, ncolumns, s);
   } else {
-    if (has_invalid) launch_dp_variant<false, true>(p, b, ncolumns, smem, s);
-    else launch_dp_variant<false, false>(p, b, ncolumns, smem, s);
+    if (has_invalid) launch_dp_variant<false, true, HP>(p, b, ncolumns, smem, s);
+    else launch_dp_variant<false, false, HP>(p, b, ncolumns, smem, s);
   }
   g_launch_count++;
+}
+
+void launch_dp(const KParams &p, const BatchBuffers &b, int nframes, bool pairwise, cudaStream_t s) {
+  if (p.rec_stride == kRecStrideTall) launch_dp_rows<kRecStrideTall>(p, b, nframes, pairwise, s);
+  else launch_dp_rows<kRecStride>(p, b, nframes, pairwise, s);
 }
 
 }  // namespace isx

@@ -65,7 +65,7 @@ __global__ void frame_tables_kernel(const float *__restrict__ ground, const int 
 }
 
 // ---------------------------------------------------------------------------
-// Blelloch-order exclusive prefix sum of e[0..H) (H <= 1024), one warp.
+// Blelloch-order exclusive prefix sum of e[0..H) (H <= 1024, TALL: H <= 2047), one warp.
 //
 // The reference scans in place with the classic work-efficient tree
 // (StixelsKernels.h:73-103): block sums are pairwise trees U(.), and ps[i]
@@ -74,19 +74,31 @@ __global__ void frame_tables_kernel(const float *__restrict__ ground, const int 
 // A butterfly (shfl_xor) reproduces U(.) of every aligned block; the value a
 // lane receives at level b while its bit b is set is exactly the U(left
 // sibling) the down-sweep adds.  Levels 0-4 live inside a 32-row chunk,
-// levels 5-9 across the (<= 32) chunk totals.
+// levels 5-9 across the (<= 32) chunk totals.  A taller tree only adds top
+// levels that pass 0 to the left, so ps[i] does not depend on the padded size:
+// TALL frames have a second group of 32 chunk totals (chunks 32-63), whose
+// prefixes start from level 10, 0 + U(rows 0..1023).
 // ---------------------------------------------------------------------------
+template <bool TALL>
 __device__ void blelloch_prefix_warp(const float *e, int H, float *ps) {
   const unsigned full = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const int nchunks = (H + 31) >> 5;
   float total_k = 0.0f;  // lane k: U(chunk k)
+  float total2_k = 0.0f;  // TALL, lane k: U(chunk 32 + k)
   for (int k = 0; k < nchunks; k++) {
     const int v = (k << 5) + lane;
     float x = v < H ? e[v] : 0.0f;
 #pragma unroll
     for (int b = 0; b < 5; b++) x = fadd(x, __shfl_xor_sync(full, x, 1 << b));
-    if (lane == k) total_k = x;
+    if constexpr (TALL) {
+      if (lane == (k & 31)) {
+        if (k < 32) total_k = x;
+        else total2_k = x;
+      }
+    } else {
+      if (lane == k) total_k = x;
+    }
   }
   float y = total_k, left[5];
 #pragma unroll
@@ -99,6 +111,20 @@ __device__ void blelloch_prefix_warp(const float *e, int H, float *ps) {
 #pragma unroll
   for (int b = 4; b >= 0; b--)
     if ((lane >> b) & 1) hi = fadd(hi, left[b]);
+  float hi2 = 0.0f;  // TALL, lane k: prefix of chunk 32 + k's first row
+  if constexpr (TALL) {
+    float y2 = total2_k, left2[5];
+#pragma unroll
+    for (int b = 0; b < 5; b++) {
+      const float o = __shfl_xor_sync(full, y2, 1 << b);
+      left2[b] = o;
+      y2 = fadd(y2, o);
+    }
+    hi2 = fadd(0.0f, y);  // level 10: the root of the first 1024 rows
+#pragma unroll
+    for (int b = 4; b >= 0; b--)
+      if ((lane >> b) & 1) hi2 = fadd(hi2, left2[b]);
+  }
   const int kmax = H >> 5;  // chunk index of row H itself
   for (int k = 0; k <= kmax; k++) {
     const int v = (k << 5) + lane;
@@ -110,8 +136,14 @@ __device__ void blelloch_prefix_warp(const float *e, int H, float *ps) {
       lo[b] = o;
       x = fadd(x, o);
     }
-    // k == 32 only for H == 1024, lane 0: the root total.
-    float pre = (k < 32) ? __shfl_sync(full, hi, k & 31) : y;
+    float pre;
+    if constexpr (TALL) {
+      // H <= 2047: row H lies in chunk 63 or below, there is no root total to store
+      pre = __shfl_sync(full, k < 32 ? hi : hi2, k & 31);
+    } else {
+      // k == 32 only for H == 1024, lane 0: the root total.
+      pre = (k < 32) ? __shfl_sync(full, hi, k & 31) : y;
+    }
 #pragma unroll
     for (int b = 4; b >= 0; b--)
       if ((lane >> b) & 1) pre = fadd(pre, lo[b]);
@@ -146,6 +178,7 @@ constexpr int kTabThreads = 256;
 // Every array is scanned in place (a scan reads e[v] and writes ps[v] from the same lane; a 1/8-resolution channel
 // value is recovered as ps[q + 1] - ps[q], exact in integers), and the sums of the instance means themselves are
 // 32-bit (only their squares need 64): 50 KB per CTA at 1024 rows, so that FOUR CTAs share an SM (r1/r2a: 71 KB, three).
+// Frames taller than 1024 rows need up to 100 KB (2047 rows): two CTAs per SM.
 struct TabSmem {
   int Hp, nq;
   size_t off_e[4], off_seg, off_i64, off_i32, total;
@@ -162,8 +195,18 @@ struct TabSmem {
   }
 };
 
-constexpr int kMeanRowLimit = 1 << 20;  // |instance mean of a row|: 1024 rows of them cannot wrap an int32 sum
+// Integer guards of the table build, so that no int32 prefix sum can wrap (TALL: up to 2047 rows, 256 entries of a
+// 1/8-resolution channel):
+//   kMeanRowLimit: |instance mean of a row|; 1024 rows (TALL: 2047) of them stay below 2^30;
+//   kClassLimit:   a class value; P_c(v) = 8 * ps[q] + seg[q] * r over <= 129 (TALL: 256) entries stays below 2^31;
+//   kSqOffLimit:   each squared offset; their sum per entry is <= 2 * kSqOffLimit = kClassLimit.
+template <bool TALL> struct TabLimits {
+  static constexpr int kMeanRowLimit = TALL ? 1 << 19 : 1 << 20;
+  static constexpr int kClassLimit = TALL ? 1 << 19 : 1 << 20;
+  static constexpr int kSqOffLimit = TALL ? 1 << 18 : 1 << 19;
+};
 
+template <bool TALL>
 __global__ void __launch_bounds__(kTabThreads, 4)
 column_tables_kernel(const float *__restrict__ joined, const int32_t *__restrict__ segmentation,
                      const float *__restrict__ ground, const int *__restrict__ vhor_arr,
@@ -192,6 +235,7 @@ column_tables_kernel(const float *__restrict__ joined, const int32_t *__restrict
   const float invalid = p.invalid_disparity;
   const int K = p.n_classes;  // 19; channel K = y offsets, K+1 = x offsets
   const bool has_oy = K < p.n_channels, has_ox = K + 1 < p.n_channels;
+  constexpr int kMeanRowLimit = TabLimits<TALL>::kMeanRowLimit;
 
   // ---- 1/8-resolution channels: the 19 classes, and as a 20th the sum of the two squared offsets (:411-416; the
   //      DP only ever uses the sum, ComputeNonInstanceOffsetCost :62-70).  Warp = channel, lane = entry: the loads of
@@ -204,14 +248,15 @@ column_tables_kernel(const float *__restrict__ joined, const int32_t *__restrict
       int v = 0;
       if (c < K) {
         if (c < p.n_channels && q < p.hs2) v = __ldg(seg_col + (size_t)c * p.hs2 + q);
-        negative_class_value |= v < 0 || v > (1 << 20);   // the int32 prefix sums over <= 1032 rows cannot wrap
+        negative_class_value |= v < 0 || v > TabLimits<TALL>::kClassLimit;   // the int32 prefix sums cannot wrap
       } else {
         int oy = 0, ox = 0;
         if (q < p.hs2 && has_oy) oy = __ldg(seg_col + (size_t)K * p.hs2 + q);
         if (q < p.hs2 && has_ox) ox = __ldg(seg_col + (size_t)(K + 1) * p.hs2 + q);
         oy = oy * oy;
         ox = ox * ox;
-        negative_class_value |= oy < 0 || oy > (1 << 19) || ox < 0 || ox > (1 << 19);   // their sum: likewise
+        negative_class_value |= oy < 0 || oy > TabLimits<TALL>::kSqOffLimit || ox < 0 ||
+                                ox > TabLimits<TALL>::kSqOffLimit;   // their sum: likewise
         v = oy + ox;
       }
       seg_ps[c * segld + q] = v;
@@ -287,7 +332,7 @@ column_tables_kernel(const float *__restrict__ joined, const int32_t *__restrict
 
   // ---- prefix sums, in place: warps 0-3 float (Blelloch order), 4-5 int64, 6-7 int32; then all: 1/8-res ints ----
   if (warp < 4) {
-    blelloch_prefix_warp(e_disp + warp * L.Hp, H, e_disp + warp * L.Hp);
+    blelloch_prefix_warp<TALL>(e_disp + warp * L.Hp, H, e_disp + warp * L.Hp);
   } else if (warp < 6) {
     exact_prefix_warp<long long>(ps_i64 + (warp - 4) * L.Hp, H, ps_i64 + (warp - 4) * L.Hp);
   } else {
@@ -373,10 +418,13 @@ __device__ __forceinline__ void stg_lo_hi(unsigned lo, unsigned hi, float v) {
                : "memory");
 }
 
+// MAXH: the largest frame height of the instantiation (1024, or 2048 for frames of up to 2047 rows: up to 64 chunk
+// carries per LUT row)
+template <int MAXH>
 __global__ void __launch_bounds__(kLutThreads)
 object_lut_kernel(const float *__restrict__ joined, const float *__restrict__ cost_t,
                   float *__restrict__ object_lut, KParams p) {
-  __shared__ __align__(16) uint8_t dis_s[1024 + 32];
+  __shared__ __align__(16) uint8_t dis_s[MAXH + 32];
   __shared__ float tile[kLutWarps][32][33];
   const int H = p.rows, C = p.realcols, D = p.max_dis;
   const int Dp = (D + 31) & ~31;
@@ -472,17 +520,25 @@ static size_t padded_smem(size_t need, size_t static_bytes) {
   return want > need ? want : need;
 }
 
-void launch_column_tables(const KParams &p, const BatchBuffers &b, int nframes, cudaStream_t s) {
+template <bool TALL>
+static void launch_column_tables_rows(const KParams &p, const BatchBuffers &b, int nframes, cudaStream_t s) {
+  constexpr int kLutMaxH = TALL ? 2048 : 1024;
   dim3 grid(p.realcols, nframes);
   const size_t smem = padded_smem(tab_smem_bytes(p), 0);
   static SmemOptIn optin, optin_lut;
-  opt_in_smem(column_tables_kernel, optin);
-  opt_in_smem(object_lut_kernel, optin_lut);
-  column_tables_kernel<<<grid, kTabThreads, smem, s>>>(b.joined, b.segmentation, b.ground, b.vhor, b.records_b,
-                                                        b.error_flag, b.col_flags, p);
+  opt_in_smem(column_tables_kernel<TALL>, optin);
+  opt_in_smem(object_lut_kernel<kLutMaxH>, optin_lut);
+  column_tables_kernel<TALL><<<grid, kTabThreads, smem, s>>>(b.joined, b.segmentation, b.ground, b.vhor, b.records_b,
+                                                              b.error_flag, b.col_flags, p);
   dim3 lgrid(p.realcols, (p.max_dis + 32 * kLutWarps - 1) / (32 * kLutWarps), nframes);
-  object_lut_kernel<<<lgrid, kLutThreads, padded_smem(0, sizeof(float) * kLutWarps * 32 * 33 + 1056), s>>>(b.joined, b.obj_cost_lut_t, b.object_lut, p);
+  object_lut_kernel<kLutMaxH><<<lgrid, kLutThreads, padded_smem(0, sizeof(float) * kLutWarps * 32 * 33 + kLutMaxH + 32), s>>>(
+      b.joined, b.obj_cost_lut_t, b.object_lut, p);
   g_launch_count += 2;
+}
+
+void launch_column_tables(const KParams &p, const BatchBuffers &b, int nframes, cudaStream_t s) {
+  if (p.rows > kShortRows) launch_column_tables_rows<true>(p, b, nframes, s);
+  else launch_column_tables_rows<false>(p, b, nframes, s);
 }
 
 }  // namespace isx
