@@ -251,6 +251,12 @@ public:
         unpack(p.n, p.roads.data(), p.sections.data(), frames, instances);
     }
 
+    // Frames [first, first + n) of the last batch into the caller's device buffers (isx_export_batch_device):
+    // packed frame-ordered Sections, offsets, instance labels and Get3DVertices, asynchronous on isx_stream().
+    void ExportBatchDevice(int first, int n, const isx_device_results& out) {
+        check(isx_export_batch_device(h_, first, n, &out));
+    }
+
     isx_handle handle() { return h_; }  // for the other C entry points
 
 private:

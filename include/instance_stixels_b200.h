@@ -389,6 +389,30 @@ int isx_rasterize_batch_device(isx_handle h, int first, int n, uint8_t *d_label_
                                float *d_disparity);
 
 /* ------------------------------------------------------------------------
+ * Device results: the stixels of frames [first, first + n) of the last batch (or of the last isx_compute: first = 0,
+ * n = 1) in the caller's DEVICE buffers, for consumers on the GPU (a tracker, a BEV grid, a second network).
+ * Frame-ordered CSR: the used Sections of frame f (0 = `first`) at [frame_offsets[f], frame_offsets[f+1]), column 0
+ * first, each column top to bottom (the order of isx_wait_batch_packed and of Stixels::Get3DVertices); column c of
+ * frame f starts at column_offsets[f*realcols + c], column_offsets[n*realcols] = frame_offsets[n].  Per stixel:
+ *   labels[i]     the DBSCAN label of the stixels GetInstanceStixels lists (-1 = noise), -2 for every other stixel
+ *   vertices[i]   [4][3] what Stixels::Get3DVertices computes for the stixel, bit for bit (needs camera_center_x/y)
+ * frame_errors[f] = the frame's error bits (1: a column reached MAX_STIXELS_PER_COLUMN, 2: instance offsets out of
+ * range).  `capacity` counts stixels (entries of sections / labels / vertices): a frame's stixels are written only if
+ * frame_offsets[f+1] <= capacity, nothing past it; offsets and errors are always complete.  No atomics: the same
+ * bytes on every call.  Asynchronous on isx_stream().
+ * ------------------------------------------------------------------------ */
+typedef struct isx_device_results { /* device pointers; NULL = not written (frame_offsets is required) */
+  isx_section *sections;            /* [capacity], 16-byte aligned */
+  int32_t *frame_offsets;           /* [n+1] */
+  int32_t *column_offsets;          /* [n*realcols+1] */
+  int32_t *labels;                  /* [capacity] */
+  float *vertices;                  /* [capacity][4][3] */
+  int32_t *frame_errors;            /* [n] */
+  int32_t capacity, reserved;
+} isx_device_results;               /* 56 bytes */
+int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_results *out);
+
+/* ------------------------------------------------------------------------
  * Road estimation (SURVEY.md 8f rank 1): the step in front of the stixel path.
  * Replaces `class RoadEstimation` (InstanceStixels/include/InstanceStixels/RoadEstimation.h:31-93,
  * src/RoadEstimation.cu:24-193, src/RoadEstimationKernels.cu:25-60) including its one third-party

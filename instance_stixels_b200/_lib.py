@@ -36,6 +36,8 @@ EXPORTS = [
     "isx_set_segmentation_from_cnn_device", "isx_flip_and_pad_batch_device",
     # result images (SURVEY.md 8f rank 3)
     "isx_rasterize_batch_device",
+    # device results
+    "isx_export_batch_device",
     # road estimation (SURVEY.md 8f rank 1)
     "isx_road_create", "isx_road_destroy", "isx_road_initialize", "isx_road_finish", "isx_road_is_initialized",
     "isx_road_compute_host", "isx_road_compute_device", "isx_road_compute_batch_device", "isx_road_last_error",
@@ -79,6 +81,13 @@ class RoadEstimate(C.Structure):
     """isx_road_estimate: what RoadEstimation::Compute leaves in its getters (RoadEstimation.h:46-50)."""
     _fields_ = [("ok", C.c_int32), ("horizon_point", C.c_int32), ("pitch", C.c_float), ("camera_height", C.c_float),
                 ("slope", C.c_float), ("rho", C.c_float), ("theta", C.c_float)]
+
+
+class DeviceResults(C.Structure):
+    """isx_device_results: device pointers the export writes (None = not written; frame_offsets is required)."""
+    _fields_ = [("sections", C.c_void_p), ("frame_offsets", C.c_void_p), ("column_offsets", C.c_void_p),
+                ("labels", C.c_void_p), ("vertices", C.c_void_p), ("frame_errors", C.c_void_p),
+                ("capacity", C.c_int32), ("reserved", C.c_int32)]
 
 
 # numpy views of isx_section (== Section, types.h:186-194) and isx_instance
@@ -177,6 +186,7 @@ def _declare(lib):
     lib.isx_set_segmentation_from_cnn_device.argtypes = [H, C.c_void_p, i, i]
     lib.isx_flip_and_pad_batch_device.argtypes = [H, i, C.c_void_p, i, i, C.c_void_p]
     lib.isx_rasterize_batch_device.argtypes = [H, i, i, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.isx_export_batch_device.argtypes = [H, i, i, C.POINTER(DeviceResults)]
     lib.isx_road_create.argtypes = [C.POINTER(H), i]
     lib.isx_road_destroy.argtypes = [H]
     lib.isx_road_destroy.restype = None

@@ -8,7 +8,8 @@ the CUDA library; nothing here computes.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Sequence
+from dataclasses import dataclass
+from typing import Any, Optional, Sequence
 
 import numpy as np
 
@@ -53,11 +54,63 @@ class StixelsData:
             setattr(self, n, getattr(meta, n))
 
 
+@dataclass
+class DeviceStixels:
+    """Torch tensors of Stixels.ComputeBatchTensors (the isx_device_results layout).  `sections` is the int32
+    [capacity, 8] view of the Sections; frame f owns rows [frame_offsets[f], frame_offsets[f+1]); `vertices` is
+    [capacity, 4, 3] or None."""
+    sections: Any
+    frame_offsets: Any
+    column_offsets: Any
+    labels: Any
+    vertices: Any
+    frame_errors: Any
+
+    # typed columns of `sections` (isx_section)
+    @property
+    def type(self):
+        return self.sections[:, 0]
+
+    @property
+    def vB(self):
+        return self.sections[:, 1]
+
+    @property
+    def vT(self):
+        return self.sections[:, 2]
+
+    @property
+    def disparity(self):
+        return self.sections[:, 3].view(self._f32())
+
+    @property
+    def semantic_class(self):
+        return self.sections[:, 4]
+
+    @property
+    def cost(self):
+        return self.sections[:, 5].view(self._f32())
+
+    @property
+    def instance_meanx(self):
+        return self.sections[:, 6].view(self._f32())
+
+    @property
+    def instance_meany(self):
+        return self.sections[:, 7].view(self._f32())
+
+    @staticmethod
+    def _f32():
+        import torch
+        return torch.float32
+
+
 class Stixels:
     def __init__(self, device: int = 0):
         self._lib = L.load()
         self._h = C.c_void_p()
         self._check(self._lib.isx_create(C.byref(self._h), device), None)
+        self._device = device
         self._pairwise = False
 
     # -- plumbing ---------------------------------------------------------
@@ -130,6 +183,73 @@ class Stixels:
         the device (clustering_visualization.py:118-142, 397-409); pointers may be 0."""
         self._check(self._lib.isx_rasterize_batch_device(self._h, first, n, d_label_ids or None,
                                                          d_instance_ids or None, d_disparity or None))
+
+    def ExportBatchDevice(self, first: int, n: int, frame_offsets: int, sections: int = 0, column_offsets: int = 0,
+                          labels: int = 0, vertices: int = 0, frame_errors: int = 0, capacity: int = 0):
+        """Stixels of frames [first, first+n) of the last batch into caller device buffers (raw pointers, 0 = not
+        written): frame-ordered CSR Sections, offsets, instance labels (-2 outside GetInstanceStixels) and
+        Get3DVertices per stixel; `capacity` counts stixels.  Asynchronous on stream()."""
+        out = L.DeviceResults(sections or None, frame_offsets or None, column_offsets or None, labels or None,
+                              vertices or None, frame_errors or None, capacity, 0)
+        self._check(self._lib.isx_export_batch_device(self._h, first, n, C.byref(out)))
+
+    def ComputeBatchTensors(self, pairwise: bool, disparity, roads: Sequence[dict], segmentation=None, cnn=None,
+                            vertices: bool = False, capacity: Optional[int] = None) -> "DeviceStixels":
+        """CUDA torch tensors in, torch tensors out, no host synchronisation: `disparity` float32 [n][rows][cols]
+        and either `segmentation` int32 in the library layout [n][realcols][21][rows_power2_segmentation] or `cnn`
+        float32 [n][21][rows/8][cols/8] (run through FlipAndPadBatchDevice).  The library's stream waits for the
+        current torch stream, and the current torch stream waits for the results.  `capacity` (stixels) defaults
+        to the worst case n * realcols * 200."""
+        import torch
+        n = len(roads)
+        if (segmentation is None) == (cnn is None):
+            raise InvalidArgument("pass exactly one of segmentation= and cnn=")
+        if not (disparity.is_cuda and disparity.dtype == torch.float32 and disparity.is_contiguous()):
+            raise InvalidArgument("disparity must be a contiguous float32 CUDA tensor")
+        inputs = [disparity]
+        dev = disparity.device
+        if dev.index != self._device:
+            raise InvalidArgument(f"the tensors are on {dev}, the handle computes on cuda:{self._device}")
+        C_ = self.GetRealCols()
+        if cnn is not None:
+            if not (cnn.device == dev and cnn.dtype == torch.float32 and cnn.is_contiguous() and cnn.dim() == 4
+                    and cnn.shape[0] == n):
+                raise InvalidArgument("cnn must be a contiguous float32 tensor [n][21][rows/8][cols/8] on the handle's device")
+            inputs.append(cnn)
+            segmentation = torch.empty(n * self.segmentation_elems(), dtype=torch.int32, device=dev)
+        elif not (segmentation.device == dev and segmentation.dtype == torch.int32 and segmentation.is_contiguous()
+                  and segmentation.numel() == n * self.segmentation_elems()):
+            raise InvalidArgument("segmentation must be a contiguous int32 tensor in the library layout on the handle's device")
+        inputs.append(segmentation)
+        if disparity.numel() != n * self._frame_pixels():
+            raise InvalidArgument("disparity must hold n frames of rows*cols")
+        cap = n * C_ * self.GetMaxSections() if capacity is None else int(capacity)
+        out = DeviceStixels(
+            sections=torch.empty((cap, 8), dtype=torch.int32, device=dev),
+            frame_offsets=torch.empty(n + 1, dtype=torch.int32, device=dev),
+            column_offsets=torch.empty(n * C_ + 1, dtype=torch.int32, device=dev),
+            labels=torch.empty(cap, dtype=torch.int32, device=dev),
+            vertices=torch.empty((cap, 4, 3), dtype=torch.float32, device=dev) if vertices else None,
+            frame_errors=torch.empty(n, dtype=torch.int32, device=dev))
+        current = torch.cuda.current_stream(dev)
+        ext = torch.cuda.ExternalStream(self.stream(), device=dev)
+        # the inputs and the outputs allocated above are ready on the current stream
+        ready = torch.cuda.Event()
+        ready.record(current)
+        ext.wait_event(ready)
+        for t in inputs:
+            t.record_stream(ext)   # read on the library's stream: not reused before that work is done
+        if cnn is not None:
+            self.FlipAndPadBatchDevice(n, cnn.data_ptr(), cnn.shape[2], cnn.shape[3], segmentation.data_ptr())
+        self.ComputeBatchDevice(pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), roads)
+        self.ExportBatchDevice(0, n, out.frame_offsets.data_ptr(), sections=out.sections.data_ptr(),
+                               column_offsets=out.column_offsets.data_ptr(), labels=out.labels.data_ptr(),
+                               vertices=out.vertices.data_ptr() if vertices else 0,
+                               frame_errors=out.frame_errors.data_ptr(), capacity=cap)
+        done = torch.cuda.Event()
+        done.record(ext)
+        current.wait_event(done)
+        return out
 
     def SetRoadParameters(self, vhor: int, camera_tilt: float, camera_height: float, alpha_ground: float):
         self._check(self._lib.isx_set_road_parameters(self._h, vhor, camera_tilt, camera_height, alpha_ground))

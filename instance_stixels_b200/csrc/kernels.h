@@ -89,6 +89,26 @@ struct PackArgs {
   isx_packed_frame *h_frames;    // [n]
 };
 void launch_pack(const KParams &p, const PackArgs &a, int nframes, cudaStream_t s);
+// Device export of a computed batch (export.cu): frames [0, n) of the arrays below, into the caller's buffers.
+struct ExportArgs {
+  const isx_section *sections;   // [n][C][200] padded device results
+  const int *n_sections;         // [n][C]
+  const isx_instance *inst;      // [n][inst_cap]
+  const int *inst_count;         // [n]
+  int inst_cap;
+  const isx_packed_frame *frames;  // [n] descriptors the packing wrote (mapped host memory): the error words
+  int *col_local;                // [n][C] scratch: column offsets relative to the frame
+  int realcols, rows, column_step;
+  float focal, bf, camera_center_x, camera_center_y;   // bf = baseline * focal
+  isx_device_results out;
+};
+constexpr int kExportFramesPerLaunch = 128;
+struct ExportFrames {              // per-frame road scalars of one launch: alpha_ground and the flipped horizon row
+  float alpha_ground[kExportFramesPerLaunch];
+  int vhor[kExportFramesPerLaunch];
+};
+void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_ground, const int *vhor,
+                           cudaStream_t s);
 // u16 disparity / i16 segmentation staging -> the float / int32 layouts of the path (ingest.cu)
 void launch_widen_inputs(const KParams &p, const uint16_t *disp16, float scale, const int16_t *seg16, float *disp,
                          int32_t *seg, int nframes, cudaStream_t s);
