@@ -26,10 +26,12 @@ public:
     RoadEstimation(const RoadEstimation&) = delete;
     RoadEstimation& operator=(const RoadEstimation&) = delete;
 
+    // Extension: `max_batch` frames per batched call (Stixels::ComputeBatchDevice with road estimation).
     void Initialize(const float camera_center_y, const float baseline, const float focal, const int rows,
-                    const int cols, const int max_dis, const float road_vdisparity_threshold = 0.2f) {
+                    const int cols, const int max_dis, const float road_vdisparity_threshold = 0.2f,
+                    int max_batch = 1) {
         check(isx_road_initialize(h_, camera_center_y, baseline, focal, rows, cols, max_dis,
-                                  road_vdisparity_threshold, 1));
+                                  road_vdisparity_threshold, max_batch));
     }
     void Finish() { check(isx_road_finish(h_)); }
 
@@ -49,6 +51,8 @@ public:
     float GetSlope() { return est_.slope; }
     int GetHorizonPoint() { return est_.horizon_point; }
     bool IsInitialized() { return isx_road_is_initialized(h_) != 0; }
+
+    isx_road_handle handle() { return h_; }  // for the other C entry points
 
 private:
     // the reference only overwrites its members when a line was accepted (RoadEstimation.cu:123-133)

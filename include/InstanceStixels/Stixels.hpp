@@ -23,6 +23,7 @@
 #include <vector>
 
 #include "../instance_stixels_b200.h"
+#include "RoadEstimation.h"
 #include "configuration.h"
 #include "types.h"
 #include "util.h"
@@ -249,6 +250,23 @@ public:
         check(isx_wait_batch_host(h_, inst_.data(), (int)inst_.size(), offs_.data()));
         waited_++;
         unpack(p.n, p.roads.data(), p.sections.data(), frames, instances);
+    }
+
+    // n frames resident on the device (isx_compute_batch_device): results stay there for ExportBatchDevice /
+    // isx_fetch_batch_results; asynchronous on isx_stream().
+    void ComputeBatchDevice(bool pairwise, int n, const pixel_t* d_disparity, const int32_t* d_segmentation,
+                            const Road* roads) {
+        check(isx_compute_batch_device(h_, pairwise ? 1 : 0, n, d_disparity, d_segmentation, roads));
+    }
+    // The same with the road of every frame estimated on the device by `road` from the frame's own disparity
+    // (isx_compute_batch_device_road): a frame without an accepted line keeps the last accepted estimate, before the
+    // first one `fallback` is used; fallback == nullptr continues from the previous call on `road`.  d_estimates /
+    // d_roads: optional device arrays [n].  No host round trip between road estimation and stixels.
+    void ComputeBatchDevice(bool pairwise, int n, const pixel_t* d_disparity, const int32_t* d_segmentation,
+                            RoadEstimation& road, const Road* fallback, isx_road_estimate* d_estimates = nullptr,
+                            Road* d_roads = nullptr) {
+        check(isx_compute_batch_device_road(h_, road.handle(), pairwise ? 1 : 0, n, d_disparity, d_segmentation,
+                                            fallback, d_estimates, d_roads));
     }
 
     // Frames [first, first + n) of the last batch into the caller's device buffers (isx_export_batch_device):

@@ -448,6 +448,29 @@ int isx_road_compute_host(isx_road_handle h, const float *disparity, size_t n_pi
 int isx_road_compute_device(isx_road_handle h, const float *d_disparity, isx_road_estimate *out);
 /* Extension: n frames [n][rows][cols] resident on the device, one estimate per frame. */
 int isx_road_compute_batch_device(isx_road_handle h, int n, const float *d_disparity, isx_road_estimate *out);
+
+/* Like isx_compute_batch_device, but each frame's road parameters are estimated on the device from its own
+ * disparity image, with `road` (RoadEstimation::Compute(pixel_t*) per frame), in stream order on isx_stream().
+ * A frame whose estimation fails (ok == 0) uses the last accepted estimate in frame order, as the getters of
+ * RoadEstimation keep it (RoadEstimation.cu:123-133).  Before any estimate has been accepted, it uses `fallback`.
+ * fallback != NULL: reset that state to *fallback.  NULL: continue from the state the previous call on `road` left
+ * (only this entry point reads or writes that state).
+ * d_estimates [n] (optional, device): what isx_road_compute_batch_device would return for each frame.
+ * d_roads [n] (optional, device): the road each frame was computed with.  Returns after enqueueing: the caller's
+ * thread never waits, and every accessor of the last batch (isx_export_batch_device, isx_fetch_batch_results,
+ * isx_rasterize_batch_device, isx_flush, isx_synchronize) works as after isx_compute_batch_device.
+ * The line is selected on the device as the argmax of (votes, -accumulator index) over the local maxima above the
+ * vote threshold whose pitch is in range -- the line the host walk of isx_road_compute_* accepts -- so the
+ * estimates are bit-identical to isx_road_compute_batch_device; unlike that walk it has no cap on the number of
+ * candidate lines (isx_road_compute_* return ISX_ERR_CAPACITY beyond 65536).  The ground tables of the frames are
+ * computed on the host in stream order (a host function per chunk, cached per road).
+ * `road` must be initialised on h's device with h's rows, cols and max_dis, and n must not exceed either handle's
+ * max_batch; refusals (ISX_ERR_INVALID_ARGUMENT, ISX_ERR_CAPACITY for sizes) enqueue nothing.  The first call on a
+ * road handle builds its table of per-cell estimates on the host (numangle x numrho cells) and must pass a
+ * `fallback`.  `road` must not be used from another thread during the call. */
+int isx_compute_batch_device_road(isx_handle h, isx_road_handle road, int pairwise, int n,
+                                  const float *d_disparity, const int32_t *d_segmentation,
+                                  const isx_road *fallback, isx_road_estimate *d_estimates, isx_road *d_roads);
 const char *isx_road_last_error(isx_road_handle h);
 /* Intermediates of the last call, frame `frame` of it (tests): 0 = v-disparity int32 [rows][max_dis],
  * 1 = binary image uint8 [rows][max_dis], 2 = Hough accumulator int32 [numangle+2][numrho+2]. */

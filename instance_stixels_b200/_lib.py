@@ -42,6 +42,8 @@ EXPORTS = [
     "isx_road_create", "isx_road_destroy", "isx_road_initialize", "isx_road_finish", "isx_road_is_initialized",
     "isx_road_compute_host", "isx_road_compute_device", "isx_road_compute_batch_device", "isx_road_last_error",
     "isx_road_tensor_bytes", "isx_road_read_tensor",
+    # device batches with road estimation in stream order
+    "isx_compute_batch_device_road",
 ]
 
 
@@ -201,6 +203,8 @@ def _declare(lib):
     lib.isx_road_tensor_bytes.argtypes = [H, i]
     lib.isx_road_tensor_bytes.restype = C.c_size_t
     lib.isx_road_read_tensor.argtypes = [H, i, i, C.c_void_p, C.c_size_t]
+    lib.isx_compute_batch_device_road.argtypes = [H, H, i, i, C.c_void_p, C.c_void_p, C.POINTER(Road), C.c_void_p,
+                                                  C.c_void_p]
 
 
 def load():

@@ -54,17 +54,50 @@ class StixelsData:
             setattr(self, n, getattr(meta, n))
 
 
+def _f32():
+    import torch
+    return torch.float32
+
+
+@dataclass
+class DeviceRoadEstimates:
+    """isx_road_estimate records on the device: `data` is the int32 [n, 7] tensor, the properties are its columns."""
+    data: Any
+
+    ok = property(lambda self: self.data[:, 0])
+    horizon_point = property(lambda self: self.data[:, 1])
+    pitch = property(lambda self: self.data[:, 2].view(_f32()))
+    camera_height = property(lambda self: self.data[:, 3].view(_f32()))
+    slope = property(lambda self: self.data[:, 4].view(_f32()))
+    rho = property(lambda self: self.data[:, 5].view(_f32()))
+    theta = property(lambda self: self.data[:, 6].view(_f32()))
+
+
+@dataclass
+class DeviceRoads:
+    """isx_road records on the device (the SetRoadParameters arguments of every frame): `data` is int32 [n, 4]."""
+    data: Any
+
+    vhor = property(lambda self: self.data[:, 0])
+    camera_tilt = property(lambda self: self.data[:, 1].view(_f32()))
+    camera_height = property(lambda self: self.data[:, 2].view(_f32()))
+    alpha_ground = property(lambda self: self.data[:, 3].view(_f32()))
+
+
 @dataclass
 class DeviceStixels:
     """Torch tensors of Stixels.ComputeBatchTensors (the isx_device_results layout).  `sections` is the int32
     [capacity, 8] view of the Sections; frame f owns rows [frame_offsets[f], frame_offsets[f+1]); `vertices` is
-    [capacity, 4, 3] or None."""
+    [capacity, 4, 3] or None.  With road estimation on the device (road=), `road_estimates` holds what the
+    estimation returned for every frame and `roads` the road every frame was computed with."""
     sections: Any
     frame_offsets: Any
     column_offsets: Any
     labels: Any
     vertices: Any
     frame_errors: Any
+    road_estimates: Optional[DeviceRoadEstimates] = None
+    roads: Optional[DeviceRoads] = None
 
     # typed columns of `sections` (isx_section)
     @property
@@ -193,19 +226,29 @@ class Stixels:
                               vertices or None, frame_errors or None, capacity, 0)
         self._check(self._lib.isx_export_batch_device(self._h, first, n, C.byref(out)))
 
-    def ComputeBatchTensors(self, pairwise: bool, disparity, roads: Sequence[dict], segmentation=None, cnn=None,
-                            vertices: bool = False, capacity: Optional[int] = None) -> "DeviceStixels":
+    def ComputeBatchTensors(self, pairwise: bool, disparity, roads: Optional[Sequence[dict]] = None,
+                            segmentation=None, cnn=None, vertices: bool = False, capacity: Optional[int] = None,
+                            road: Optional["RoadEstimation"] = None, fallback: Optional[dict] = None) -> "DeviceStixels":
         """CUDA torch tensors in, torch tensors out, no host synchronisation: `disparity` float32 [n][rows][cols]
         and either `segmentation` int32 in the library layout [n][realcols][21][rows_power2_segmentation] or `cnn`
         float32 [n][21][rows/8][cols/8] (run through FlipAndPadBatchDevice).  The library's stream waits for the
         current torch stream, and the current torch stream waits for the results.  `capacity` (stixels) defaults
-        to the worst case n * realcols * 200."""
+        to the worst case n * realcols * 200.
+        The road of every frame: either `roads` (one dict per frame) or `road`, a RoadEstimation that estimates it
+        on the device from the frame's disparity (ComputeBatchDeviceRoad; `fallback` as there).  With `road`, the
+        result also carries `road_estimates` and `roads`."""
         import torch
-        n = len(roads)
+        if (roads is None) == (road is None):
+            raise InvalidArgument("pass exactly one of roads= and road=")
+        if fallback is not None and road is None:
+            raise InvalidArgument("fallback= goes with road=")
         if (segmentation is None) == (cnn is None):
             raise InvalidArgument("pass exactly one of segmentation= and cnn=")
         if not (disparity.is_cuda and disparity.dtype == torch.float32 and disparity.is_contiguous()):
             raise InvalidArgument("disparity must be a contiguous float32 CUDA tensor")
+        n = len(roads) if roads is not None else disparity.numel() // self._frame_pixels()
+        if n < 1:
+            raise InvalidArgument("disparity must hold n >= 1 frames of rows*cols")
         inputs = [disparity]
         dev = disparity.device
         if dev.index != self._device:
@@ -231,6 +274,9 @@ class Stixels:
             labels=torch.empty(cap, dtype=torch.int32, device=dev),
             vertices=torch.empty((cap, 4, 3), dtype=torch.float32, device=dev) if vertices else None,
             frame_errors=torch.empty(n, dtype=torch.int32, device=dev))
+        if road is not None:
+            out.road_estimates = DeviceRoadEstimates(torch.empty((n, 7), dtype=torch.int32, device=dev))
+            out.roads = DeviceRoads(torch.empty((n, 4), dtype=torch.int32, device=dev))
         current = torch.cuda.current_stream(dev)
         ext = torch.cuda.ExternalStream(self.stream(), device=dev)
         # the inputs and the outputs allocated above are ready on the current stream
@@ -241,7 +287,11 @@ class Stixels:
             t.record_stream(ext)   # read on the library's stream: not reused before that work is done
         if cnn is not None:
             self.FlipAndPadBatchDevice(n, cnn.data_ptr(), cnn.shape[2], cnn.shape[3], segmentation.data_ptr())
-        self.ComputeBatchDevice(pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), roads)
+        if road is None:
+            self.ComputeBatchDevice(pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), roads)
+        else:
+            self.ComputeBatchDeviceRoad(road, pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), fallback,
+                                        out.road_estimates.data.data_ptr(), out.roads.data.data_ptr())
         self.ExportBatchDevice(0, n, out.frame_offsets.data_ptr(), sections=out.sections.data_ptr(),
                                column_offsets=out.column_offsets.data_ptr(), labels=out.labels.data_ptr(),
                                vertices=out.vertices.data_ptr() if vertices else 0,
@@ -440,6 +490,18 @@ class Stixels:
         self._check(self._lib.isx_compute_batch_device(self._h, int(pairwise), n, d_disparity, d_segmentation,
                                                        _roads(roads)))
 
+    def ComputeBatchDeviceRoad(self, road: "RoadEstimation", pairwise: bool, n: int, d_disparity: int,
+                               d_segmentation: int, fallback: Optional[dict] = None, d_estimates: int = 0,
+                               d_roads: int = 0):
+        """ComputeBatchDevice with the road of every frame estimated on the device by `road` (a RoadEstimation
+        initialised with the same rows, cols and max_dis), in stream order: asynchronous, no host round trip.  A frame
+        without an accepted line keeps the last accepted estimate; before the first, `fallback` (a road dict) is
+        used.  fallback=None continues from the state the previous call on `road` left.  d_estimates [n] /
+        d_roads [n] (device pointers, 0 = not written) receive the estimates and the roads used."""
+        fb = C.byref(_roads([fallback])[0]) if fallback is not None else None
+        self._check(self._lib.isx_compute_batch_device_road(self._h, road.handle(), int(pairwise), n, d_disparity,
+                                                            d_segmentation, fb, d_estimates or None, d_roads or None))
+
     def Flush(self):
         """Order the results of every enqueued batch before later work on stream(); asynchronous."""
         self._check(self._lib.isx_flush(self._h))
@@ -550,6 +612,10 @@ class RoadEstimation:
         self._check(self._lib.isx_road_compute_batch_device(self._h, n, d_disparity, est))
         return [dict(ok=bool(e.ok), vhor=e.horizon_point, camera_tilt=e.pitch, camera_height=e.camera_height,
                      alpha_ground=e.slope, rho=e.rho, theta=e.theta) for e in est]
+
+    def handle(self):
+        """The isx_road_handle, for the C entry points (isx_compute_batch_device_road)."""
+        return self._h
 
     def GetCameraHeight(self) -> float:
         return self._est.camera_height

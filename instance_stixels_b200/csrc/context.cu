@@ -148,7 +148,12 @@ struct isx_context {
   unsigned long long dp_units_total = 0;              // 32 x 32-cell units of all DP launches so far
   int host_slot = 0;                                  // input slot / chunk set of the next host chunk (alternates across batches)
 
+  // ground tables per road; also read by the host functions of isx_compute_batch_device_road (a driver thread)
   std::map<isx::RoadKey, std::vector<float>> road_cache;
+  std::mutex road_cache_mutex;
+  isx_road *h_stage_roads = nullptr;  // [kStageSlots][chunk] pinned: the device-estimated roads of a staged chunk
+  isx_road *d_batch_roads = nullptr;  // [max_batch] roads of the last isx_compute_batch_device_road batch
+  bool last_roads_device = false;     // ... which the export reads instead of last_roads
   isx_road single_road{0, 0.f, 0.f, 0.f};
   bool single_has_road = false;
   int last_batch = 0;          // frames of the last batch (results valid for these)
@@ -270,7 +275,9 @@ static void fill_kparams(isx_context *c) {
   k.prune_pairwise = (e2 && std::atoi(e2) == 0) ? 0 : 1;
 }
 
-static const float *road_tables(isx_context *c, const isx_road &r) {
+// The ground tables [3][H] of road `r` into `dst`.
+static void copy_road_tables(isx_context *c, const isx_road &r, float *dst) {
+  std::lock_guard<std::mutex> lock(c->road_cache_mutex);
   RoadKey key{r.vhor, r.camera_tilt, r.camera_height, r.alpha_ground};
   auto it = c->road_cache.find(key);
   if (it == c->road_cache.end()) {
@@ -279,7 +286,21 @@ static const float *road_tables(isx_context *c, const isx_road &r) {
     c->model.ground_tables(r, t.data());
     it = c->road_cache.emplace(key, std::move(t)).first;
   }
-  return it->second.data();
+  std::memcpy(dst, it->second.data(), sizeof(float) * 3 * c->model.rows);
+}
+
+// The staged road tables of `n` frames -> the next slot of the road ring, on `st`.  Returns the slot or an error.
+static int send_road_tables(isx_context *c, int stage, int n, cudaStream_t st) {
+  const int H = c->kp.rows;
+  const float *hg = c->h_ground + (size_t)stage * c->chunk * 3 * H;
+  const int *hv = c->h_vhor + (size_t)stage * c->chunk;
+  const int rslot = (int)(c->road_next++ % kRoadSlots);
+  const isx_context::RoadSlot &rd = c->roads[rslot];
+  ISX_TRY(c, cudaStreamWaitEvent(st, rd.ev_free, 0));
+  ISX_TRY(c, cudaMemcpyAsync(rd.ground, hg, sizeof(float) * 3 * H * n, cudaMemcpyHostToDevice, st));
+  ISX_TRY(c, cudaMemcpyAsync(rd.vhor, hv, sizeof(int) * n, cudaMemcpyHostToDevice, st));
+  ISX_TRY(c, cudaEventRecord(c->ev_stage_done[stage], st));
+  return rslot;
 }
 
 // Enqueue the kernel sequence for `n` frames whose inputs are at d_disp/d_seg.
@@ -300,16 +321,44 @@ static int stage_road_tables(isx_context *c, const isx_road *roads, int n, cudaS
   float *hg = c->h_ground + (size_t)stage * c->chunk * 3 * H;
   int *hv = c->h_vhor + (size_t)stage * c->chunk;
   for (int i = 0; i < n; i++) {
-    std::memcpy(hg + (size_t)i * 3 * H, road_tables(c, roads[i]), sizeof(float) * 3 * H);
+    copy_road_tables(c, roads[i], hg + (size_t)i * 3 * H);
     hv[i] = H - roads[i].vhor - 1;  // Stixels.cu:377
   }
-  const int rslot = (int)(c->road_next++ % kRoadSlots);
-  const isx_context::RoadSlot &rd = c->roads[rslot];
-  ISX_TRY(c, cudaStreamWaitEvent(st, rd.ev_free, 0));
-  ISX_TRY(c, cudaMemcpyAsync(rd.ground, hg, sizeof(float) * 3 * H * n, cudaMemcpyHostToDevice, st));
-  ISX_TRY(c, cudaMemcpyAsync(rd.vhor, hv, sizeof(int) * n, cudaMemcpyHostToDevice, st));
-  ISX_TRY(c, cudaEventRecord(c->ev_stage_done[stage], st));
-  return rslot;
+  return send_road_tables(c, stage, n, st);
+}
+
+// Roads estimated on the device (isx_compute_batch_device_road) are not known when the chunk is enqueued.  The ground
+// tables stay host-computed all the same -- HostModel::ground_tables must equal the reference bit for bit, and the
+// glibc erff it uses is not correctly rounded, so no device erff matches it -- but in stream order on `st`: the roads
+// of the chunk go to pinned memory, a host function fills the staging buffer from them (no CUDA calls; the ground
+// tables of a road are cached, and video frames mostly keep their road), and the usual copy takes it to the road ring.
+// The reuse of the staging buffer is ordered on the stream too, so the calling thread never waits.
+struct StageFill {
+  isx_context *c;
+  int stage, n;
+};
+
+static void CUDART_CB fill_stage_from_roads(void *arg) {
+  const StageFill p = *static_cast<StageFill *>(arg);
+  delete static_cast<StageFill *>(arg);
+  isx_context *c = p.c;
+  const int H = c->kp.rows;
+  const isx_road *roads = c->h_stage_roads + (size_t)p.stage * c->chunk;
+  float *hg = c->h_ground + (size_t)p.stage * c->chunk * 3 * H;
+  int *hv = c->h_vhor + (size_t)p.stage * c->chunk;
+  for (int i = 0; i < p.n; i++) {
+    copy_road_tables(c, roads[i], hg + (size_t)i * 3 * H);
+    hv[i] = H - roads[i].vhor - 1;  // Stixels.cu:377
+  }
+}
+
+static int stage_device_road_tables(isx_context *c, const isx_road *d_roads, int n, cudaStream_t st) {
+  const int stage = (int)(c->stage_next++ % kStageSlots);
+  ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_stage_done[stage], 0));
+  ISX_TRY(c, cudaMemcpyAsync(c->h_stage_roads + (size_t)stage * c->chunk, d_roads, sizeof(isx_road) * n,
+                             cudaMemcpyDeviceToHost, st));
+  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{c, stage, n}));
+  return send_road_tables(c, stage, n, st);
 }
 
 // `road_slot` >= 0: the caller has already copied the road tables of the chunk into that slot of the ring (host
@@ -757,6 +806,8 @@ int isx_initialize(isx_handle h, int max_batch) {
 
   ISX_TRY(h, cudaMallocHost(&h->h_ground, sizeof(float) * kStageSlots * ch * 3 * H));
   ISX_TRY(h, cudaMallocHost(&h->h_vhor, sizeof(int) * kStageSlots * ch));
+  ISX_TRY(h, cudaMallocHost(&h->h_stage_roads, sizeof(isx_road) * kStageSlots * ch));
+  ISX_TRY(h, dev_alloc(h, &h->d_batch_roads, MB));
   for (int i = 0; i < kStageSlots; i++) ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_stage_done[i], cudaEventDisableTiming));
   h->stage_next = 0;
   h->road_cache.clear();
@@ -776,6 +827,10 @@ int isx_finish(isx_handle h) {
   h->allocations.clear();
   cudaFreeHost(h->h_ground);
   cudaFreeHost(h->h_vhor);
+  cudaFreeHost(h->h_stage_roads);
+  h->h_stage_roads = nullptr;
+  h->d_batch_roads = nullptr;
+  h->last_roads_device = false;
   for (int i = 0; i < kStageSlots; i++) {
     if (h->ev_stage_done[i]) cudaEventDestroy(h->ev_stage_done[i]);
     h->ev_stage_done[i] = nullptr;
@@ -982,6 +1037,7 @@ int isx_compute(isx_handle h, int pairwise, isx_section *sections, isx_frame_met
   if (int rc = join_emit_stream(h)) return rc;
   h->last_batch = 1;
   h->last_roads.assign(1, h->single_road);
+  h->last_roads_device = false;
   if (int rc = wait_last_emission(h)) return rc;
   if (int rc = deliver(h, h->rs[h->cur], 1, sections, nullptr, 0, nullptr, direct)) return rc;
   if (meta) {
@@ -1043,6 +1099,46 @@ int isx_compute_batch_device(isx_handle h, int pairwise, int n, const float *d_d
   h->emit_join_pending = true;  // joined lazily: isx_flush / isx_synchronize / any result access
   h->last_batch = n;
   h->last_roads.assign(roads, roads + n);
+  h->last_roads_device = false;
+  return ISX_OK;
+}
+
+int isx_compute_batch_device_road(isx_handle h, isx_road_handle road, int pairwise, int n, const float *d_disparity,
+                                  const int32_t *d_segmentation, const isx_road *fallback,
+                                  isx_road_estimate *d_estimates, isx_road *d_roads) {
+  if (int rc = check_ready(h)) return rc;
+  if (int rc = no_batches_in_flight(h)) return rc;
+  if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
+  if (!road || !d_disparity || !d_segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
+  std::string msg;
+  if (int rc = road_check_batch(road, h->device, h->kp.rows, h->kp.cols, h->kp.max_dis, n, fallback != nullptr, msg))
+    return fail(h, rc, msg);
+  if (int rc = road_enqueue_batch(road, h->s_tables, n, d_disparity, fallback, d_estimates, d_roads, h->d_batch_roads,
+                                  msg))
+    return fail(h, rc, msg);
+  const size_t hw = (size_t)h->kp.rows * h->kp.cols, se = seg_elems(h);
+  int slot = h->host_slot;
+  if (int rc = begin_batch(h)) return rc;
+  const int chunk = pairwise ? h->chunk : h->chunk_unary;
+  h->last_launch_frames = chunk;
+  // the batch's results replace the last ones from here on: the export reads the device roads
+  h->last_batch = n;
+  h->last_roads.clear();
+  h->last_roads_device = true;
+  for (int first = 0; first < n; first += chunk) {
+    const int cn = (n - first) < chunk ? (n - first) : chunk;
+    const int road_slot = stage_device_road_tables(h, h->d_batch_roads + first, cn, h->s_tables);
+    if (road_slot < 0) return road_slot;
+    h->results_stay_on_device = true;
+    const int erc = enqueue_chunk(h, pairwise != 0, first, cn, d_disparity + first * hw, d_segmentation + first * se,
+                                  nullptr, slot, road_slot);
+    h->results_stay_on_device = false;
+    if (erc) return erc;
+    ISX_TRY(h, cudaEventRecord(h->ev_in_free[slot], h->s_tables));
+    slot ^= 1;
+  }
+  h->host_slot = slot;
+  h->emit_join_pending = true;
   return ISX_OK;
 }
 
@@ -1171,6 +1267,7 @@ static int enqueue_host_batch(isx_handle h, int pairwise, int n, const HostInput
   h->host_slot = slot;
   h->last_batch = n;
   h->last_roads.assign(roads, roads + n);
+  h->last_roads_device = false;
   return ISX_OK;
 }
 
@@ -1372,9 +1469,10 @@ int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_res
   a.camera_center_x = m.camera_center_x;
   a.camera_center_y = m.camera_center_y;
   a.out = *out;
+  a.roads = h->last_roads_device ? h->d_batch_roads + first : nullptr;
   std::vector<float> alpha((size_t)n);
   std::vector<int> vhor((size_t)n);
-  for (int f = 0; f < n; f++) {
+  for (int f = 0; f < n && !a.roads; f++) {
     alpha[f] = h->last_roads[first + f].alpha_ground;
     vhor[f] = h->kp.rows - h->last_roads[first + f].vhor - 1;   // isx_frame_meta.vhor (Stixels.cu:377)
   }

@@ -127,8 +127,8 @@ export_stixels_kernel(ExportArgs a, ExportFrames fr, int f0) {
     for (int col = tid; col < C; col += kExportThreads) o.column_offsets[(size_t)f * C + col] = base + loc[col];
   if (tid == 0 && o.frame_errors) o.frame_errors[f] = a.frames[f].error;
   if (!fits) return;
-  const float alpha = fr.alpha_ground[blockIdx.x];
-  const int vhor = fr.vhor[blockIdx.x];
+  const float alpha = a.roads ? a.roads[f].alpha_ground : fr.alpha_ground[blockIdx.x];
+  const int vhor = a.roads ? a.rows - a.roads[f].vhor - 1 : fr.vhor[blockIdx.x];   // flipped (Stixels.cu:377)
   for (int col = warp; col < C; col += kExportWarps) {
     const int n = ns[col], dst0 = base + loc[col];
     const isx_section *src = a.sections + ((size_t)f * C + col) * kMaxSections;
@@ -172,13 +172,14 @@ void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_
   export_frame_scan_kernel<<<1, kFrameScanThreads, 0, s>>>(a.out.frame_offsets, a.out.column_offsets, nframes,
                                                            a.realcols);
   g_launch_count += 2;
-  // the road scalars of the frames travel as kernel parameters, kExportFramesPerLaunch frames per launch
+  // the road scalars of the frames travel as kernel parameters, kExportFramesPerLaunch frames per launch (unless they
+  // are in device memory, a.roads)
   for (int f0 = 0; f0 < nframes; f0 += kExportFramesPerLaunch) {
     const int gn = nframes - f0 < kExportFramesPerLaunch ? nframes - f0 : kExportFramesPerLaunch;
     ExportFrames fr;
     for (int i = 0; i < gn; i++) {
-      fr.alpha_ground[i] = alpha_ground[f0 + i];
-      fr.vhor[i] = vhor[f0 + i];
+      fr.alpha_ground[i] = a.roads ? 0.0f : alpha_ground[f0 + i];
+      fr.vhor[i] = a.roads ? 0 : vhor[f0 + i];
     }
     export_stixels_kernel<<<gn, kExportThreads, 0, s>>>(a, fr, f0);
     g_launch_count++;

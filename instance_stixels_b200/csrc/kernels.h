@@ -4,6 +4,7 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <string>
 
 #include "../../include/instance_stixels_b200.h"
 #include "common.cuh"
@@ -100,6 +101,9 @@ struct ExportArgs {
   int *col_local;                // [n][C] scratch: column offsets relative to the frame
   int realcols, rows, column_step;
   float focal, bf, camera_center_x, camera_center_y;   // bf = baseline * focal
+  // [n] roads of the frames in device memory (batches whose roads were estimated on the device), or null: the road
+  // scalars then travel as kernel parameters (ExportFrames)
+  const isx_road *roads;
   isx_device_results out;
 };
 constexpr int kExportFramesPerLaunch = 128;
@@ -109,6 +113,14 @@ struct ExportFrames {              // per-frame road scalars of one launch: alph
 };
 void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_ground, const int *vhor,
                            cudaStream_t s);
+// Road estimation in front of a device batch (road.cu, isx_compute_batch_device_road): the checks (nothing enqueued),
+// then the Hough kernels, the device line selection and the keep-last rule on the road handle's stream, ordered after
+// and before `caller`.  d_roads [n]: the road every frame is computed with.  0 or an isx_status, text in `msg`.
+int road_check_batch(isx_road_handle road, int device, int rows, int cols, int max_dis, int n, bool has_fallback,
+                     std::string &msg);
+int road_enqueue_batch(isx_road_handle road, cudaStream_t caller, int n, const float *d_disparity,
+                       const isx_road *fallback, isx_road_estimate *d_estimates, isx_road *d_roads_out,
+                       isx_road *d_roads, std::string &msg);
 // u16 disparity / i16 segmentation staging -> the float / int32 layouts of the path (ingest.cu)
 void launch_widen_inputs(const KParams &p, const uint16_t *disp16, float scale, const int16_t *seg16, float *disp,
                          int32_t *seg, int nframes, cudaStream_t s);
