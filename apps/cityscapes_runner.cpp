@@ -43,8 +43,11 @@ struct Options {
     bool pairwise = false;
     StixelConfig config;  // everything that does not depend on the frame
     // extensions (not in the reference's CLI): --batch B frames per batched call, --gpus G GPUs of this box
+    // and --road-on-device (below)
     int batch = 1, gpus = 1;
     int replicate = 1;   // --replicate K (measurement only): the timed call streams the loaded frames K times
+    // --road-on-device (with --batch / --gpus): the road of every frame is estimated inside the timed pool call
+    bool road_on_device = false;
 };
 
 bool parse_options(int argc, char** argv, Options* o) {
@@ -52,6 +55,10 @@ bool parse_options(int argc, char** argv, Options* o) {
     std::vector<char*> pos;
     for (int i = 0; i < argc; i++) {
         const std::string a(argv[i]);
+        if (a == "--road-on-device") {
+            o->road_on_device = true;
+            continue;
+        }
         if ((a == "--batch" || a == "--gpus" || a == "--replicate") && i + 1 < argc) {
             (a == "--batch" ? o->batch : a == "--gpus" ? o->gpus : o->replicate) = std::max(1, std::atoi(argv[++i]));
             continue;
@@ -257,6 +264,10 @@ bool segmentation_fits(const isx_apps::NpyInt32& seg, int rows, int cols, int co
 // frames, three in flight) from pinned host buffers.  The .stixels files are the same bytes as the one-frame loop
 // writes; the timed region is the pool call (host buffers in -> Sections and instance maps out), after one
 // discarded warm-up call like the reference's first frame.
+// --road-on-device: no road is estimated while loading.  The pool call estimates every frame's road on the device
+// inside its pipeline (isx_pool_compute_host_road), so road estimation is inside the timed region as in the
+// reference's loop.  Frames whose estimate failed or is all zeros are reported and skipped after the call, like the
+// one-frame loop skips them; they were computed with the camera's nominal road, whose results are discarded.
 struct LoadedFrame {
     std::string base;
     int rows = 0, cols = 0;
@@ -277,6 +288,18 @@ struct Pinned {
     Pinned(const Pinned&) = delete;
     Pinned& operator=(const Pinned&) = delete;
 };
+
+// RoadEstimation's accepted estimate of all zeros, which the reference's loop refuses (apps/run_cityscapes.cu:401-405)
+bool invalid_road(const Stixels::Road& r) {
+    return r.camera_tilt == 0 && r.camera_height == 0 && r.vhor == 0 && r.alpha_ground == 0;
+}
+
+// The road a frame whose estimate fails is computed with under --road-on-device: horizon at the principal point, no
+// pitch, a car's camera height.  Its results are discarded; it only has to be a plausible road.
+Stixels::Road nominal_road(const isx_apps::Camera& cam) {
+    const float height = 1.2f;
+    return Stixels::Road{(int)cam.center_y, 0.0f, height, cam.baseline / height};
+}
 
 int run_batched(const Options& opt) {
     const std::vector<std::string> bases = list_frames(opt.dataset + "/disparities");
@@ -304,23 +327,26 @@ int run_batched(const Options& opt) {
                 }
                 isx_apps::NpyInt32 s = load_segmentation(opt.dataset + "/probs/" + base + "_probs");
                 if (!segmentation_fits(s, d.rows, d.cols, opt.config.column_step)) continue;
-                if (group.empty()) {
-                    if (road.IsInitialized()) road.Finish();
-                    road.Initialize(cam.center_y, cam.baseline, cam.focal, d.rows, d.cols, opt.config.max_dis);
-                }
-                if (!road.Compute(d.values)) {
-                    std::printf("Road estimation failed.\n");
-                    continue;
-                }
                 LoadedFrame f;
                 f.base = base;
                 f.rows = d.rows;
                 f.cols = d.cols;
                 f.cam = cam;
-                f.road = Stixels::Road{road.GetHorizonPoint(), road.GetPitch(), road.GetCameraHeight(), road.GetSlope()};
-                if (f.road.camera_tilt == 0 && f.road.camera_height == 0 && f.road.vhor == 0 && f.road.alpha_ground == 0) {
-                    std::printf("Invalid road estimation.\n");
-                    continue;
+                if (!opt.road_on_device) {
+                    if (group.empty()) {
+                        if (road.IsInitialized()) road.Finish();
+                        road.Initialize(cam.center_y, cam.baseline, cam.focal, d.rows, d.cols, opt.config.max_dis);
+                    }
+                    if (!road.Compute(d.values)) {
+                        std::printf("Road estimation failed.\n");
+                        continue;
+                    }
+                    f.road = Stixels::Road{road.GetHorizonPoint(), road.GetPitch(), road.GetCameraHeight(),
+                                           road.GetSlope()};
+                    if (invalid_road(f.road)) {
+                        std::printf("Invalid road estimation.\n");
+                        continue;
+                    }
                 }
                 f.slot = group.size();
                 group.push_back(f);
@@ -357,9 +383,18 @@ int run_batched(const Options& opt) {
         std::vector<isx_instance> records;   // the reference builds its std::map after the timed region too (:430)
         std::vector<int32_t> offsets;
         const int warm = std::min(n, opt.batch * opt.gpus);
-        pool.ComputeBatch(opt.pairwise, warm, h_disp.p, h_seg.p, roads.data(), sections.p, &records, &offsets);  // warm-up
+        const Stixels::Road fallback = nominal_road(group[0].cam);
+        std::vector<isx_road_estimate> estimates;
+        if (opt.road_on_device)   // warm-up
+            pool.ComputeBatch(opt.pairwise, warm, h_disp.p, h_seg.p, fallback, &estimates, sections.p, &records, &offsets);
+        else
+            pool.ComputeBatch(opt.pairwise, warm, h_disp.p, h_seg.p, roads.data(), sections.p, &records, &offsets);
         const auto t0 = std::chrono::steady_clock::now();
-        pool.ComputeBatch(opt.pairwise, n, h_disp.p, h_seg.p, roads.data(), sections.p, &records, &offsets);
+        if (opt.road_on_device)
+            pool.ComputeBatch(opt.pairwise, n, h_disp.p, h_seg.p, fallback, &estimates, sections.p, &records, &offsets,
+                              &roads);
+        else
+            pool.ComputeBatch(opt.pairwise, n, h_disp.p, h_seg.p, roads.data(), sections.p, &records, &offsets);
         const auto t1 = std::chrono::steady_clock::now();
         const double ms = (double)std::chrono::duration_cast<std::chrono::microseconds>(t1 - t0).count() * 1e-3;
         std::cout << "Done. Time elapsed (s): " << ms * 1e-3 << " for " << n << " frames on " << pool.Size()
@@ -373,7 +408,20 @@ int run_batched(const Options& opt) {
         total_frames += (size_t)n;
         const size_t per = per_frame;
         for (int f = 0; f < loaded; f++) {
-            const LoadedFrame& lf = group[(size_t)f];
+            LoadedFrame& lf = group[(size_t)f];
+            if (opt.road_on_device) {
+                if (!estimates[(size_t)f].ok) {
+                    std::cout << lf.base << ": ";
+                    std::printf("Road estimation failed.\n");
+                    continue;
+                }
+                lf.road = roads[(size_t)f];   // the frame's own estimate (the pool's per-frame rule)
+                if (invalid_road(lf.road)) {
+                    std::cout << lf.base << ": ";
+                    std::printf("Invalid road estimation.\n");
+                    continue;
+                }
+            }
             Stixels::SaveStixels(sections.p + (size_t)f * per, StixelsPool::MapOf(records, offsets, f), lf.road.alpha_ground,
                                  lf.rows - 1 - lf.road.vhor, pool.GetRealCols(), pool.GetMaxSections(),
                                  (opt.dataset + "/stixels/" + lf.base + ".stixels").c_str());
@@ -391,6 +439,10 @@ int run_batched(const Options& opt) {
 int main(int argc, char* argv[]) {
     Options opt;
     if (!parse_options(argc, argv, &opt)) return -1;
+    if (opt.road_on_device && opt.batch <= 1 && opt.gpus <= 1) {
+        std::cerr << "--road-on-device applies to the batched mode: give --batch B (B > 1) or --gpus G (G > 1).\n";
+        return -1;
+    }
     if (opt.batch > 1 || opt.gpus > 1) return run_batched(opt);
     Pipeline pipeline(opt);
     std::vector<double> frame_ms;

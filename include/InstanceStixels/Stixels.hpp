@@ -12,6 +12,7 @@
 
 #include <stdint.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 #include <fstream>
@@ -238,9 +239,26 @@ public:
         Pending& p = pending_[submitted_ % 3];
         p.n = n;
         p.roads.assign(roads, roads + n);
+        p.roads_out = nullptr;
         p.sections.resize((size_t)n * GetRealCols() * GetMaxSections());
         check(isx_submit_batch_host(h_, pairwise ? 1 : 0, n, disparity, segmentation, roads,
                                     reinterpret_cast<isx_section*>(p.sections.data())));
+        submitted_++;
+    }
+    // The same with the road of every frame estimated on the device by `road` inside the batch's pipeline
+    // (isx_submit_batch_host_road): a frame without an accepted line keeps the last accepted estimate, before the
+    // first one `fallback` is used; fallback == nullptr continues from the previous batch submitted with `road`.
+    // `estimates` / `roads_out`: optional host arrays [n], filled when WaitBatch for this batch returns (which also
+    // gives every StixelsData the road its frame was computed with).
+    void SubmitBatch(bool pairwise, int n, const pixel_t* disparity, const int32_t* segmentation, RoadEstimation& road,
+                     const Road* fallback, isx_road_estimate* estimates = nullptr, Road* roads_out = nullptr) {
+        Pending& p = pending_[submitted_ % 3];
+        p.n = n;
+        p.roads.assign((size_t)n, Road{0, 0.f, 0.f, 0.f});   // written by the device, read after the wait
+        p.roads_out = roads_out;
+        p.sections.resize((size_t)n * GetRealCols() * GetMaxSections());
+        check(isx_submit_batch_host_road(h_, road.handle(), pairwise ? 1 : 0, n, disparity, segmentation, fallback,
+                                         estimates, p.roads.data(), reinterpret_cast<isx_section*>(p.sections.data())));
         submitted_++;
     }
     void WaitBatch(std::vector<StixelsData>& frames, std::vector<InstanceMap>* instances = nullptr) {
@@ -249,6 +267,8 @@ public:
         offs_.resize((size_t)p.n + 1);
         check(isx_wait_batch_host(h_, inst_.data(), (int)inst_.size(), offs_.data()));
         waited_++;
+        if (p.roads_out) std::copy(p.roads.begin(), p.roads.end(), p.roads_out);
+        p.roads_out = nullptr;
         unpack(p.n, p.roads.data(), p.sections.data(), frames, instances);
     }
 
@@ -284,6 +304,7 @@ private:
     struct Pending {
         int n = 0;
         std::vector<Road> roads;
+        Road* roads_out = nullptr;   // the caller's copy of `roads` (estimated roads)
         std::vector<Section> sections;
     } pending_[3];
     unsigned long long submitted_ = 0, waited_ = 0;
@@ -394,6 +415,32 @@ public:
         if (isx_pool_compute_host(p_, pairwise ? 1 : 0, n, disparity, segmentation, roads,
                                   reinterpret_cast<isx_section*>(sections), records ? scratch_.get() : nullptr,
                                   records ? (int)scratch_cap_ : 0, offsets ? offsets->data() : nullptr) != ISX_OK) {
+            std::cerr << "instance_stixels_b200: " << isx_pool_last_error(p_) << std::endl;
+            std::exit(1);
+        }
+        if (records) records->assign(scratch_.get(), scratch_.get() + (*offsets)[(size_t)n]);
+    }
+    // The same with the road of every frame estimated on the device inside the pipeline
+    // (isx_pool_compute_host_road).  The rule is per frame: a frame whose estimate is accepted is computed with it,
+    // every other frame with `fallback`.  `estimates` / `roads` (optional) receive n entries: what the estimation
+    // returned and the road each frame was computed with.
+    void ComputeBatch(bool pairwise, int n, const pixel_t* disparity, const int32_t* segmentation, const Road& fallback,
+                      std::vector<isx_road_estimate>* estimates, Section* sections, std::vector<isx_instance>* records,
+                      std::vector<int32_t>* offsets, std::vector<Road>* roads = nullptr) {
+        const size_t per = (size_t)GetRealCols() * GetMaxSections();
+        if (records && scratch_cap_ < (size_t)n * per) {
+            scratch_.reset(new isx_instance[(size_t)n * per]);
+            scratch_cap_ = (size_t)n * per;
+        }
+        std::vector<int32_t> local_offsets;
+        if (records && !offsets) offsets = &local_offsets;
+        if (offsets) offsets->resize((size_t)n + 1);
+        if (estimates) estimates->resize((size_t)n);
+        if (roads) roads->resize((size_t)n);
+        if (isx_pool_compute_host_road(p_, pairwise ? 1 : 0, n, disparity, segmentation, &fallback,
+                                       estimates ? estimates->data() : nullptr, roads ? roads->data() : nullptr,
+                                       reinterpret_cast<isx_section*>(sections), records ? scratch_.get() : nullptr,
+                                       records ? (int)scratch_cap_ : 0, offsets ? offsets->data() : nullptr) != ISX_OK) {
             std::cerr << "instance_stixels_b200: " << isx_pool_last_error(p_) << std::endl;
             std::exit(1);
         }

@@ -346,6 +346,11 @@ int isx_get_stage_times(isx_handle h, double *ms, long *chunks, int n_stages, in
  * grouping begin | emission end).  Returns the number of chunks written (or a negative status); call it before
  * isx_get_stage_times, which consumes the same events. */
 int isx_get_chunk_trace(isx_handle h, double *ms, int max_chunks);
+/* Host time of the host functions that fill the ground tables of chunks whose roads are estimated on the device
+ * (isx_compute_batch_device_road, isx_submit_batch_host_road), counted for the chunks enqueued while profiling was
+ * enabled: *ms in total, *calls = number of chunks (either may be NULL).  Synchronises the handle's stream first;
+ * reset != 0 clears both. */
+int isx_get_road_fill_time(isx_handle h, double *ms, long *calls, int reset);
 /* Frames per kernel launch of the last batch (batches are cut into chunks: 32 frames in unary mode, 64 in pairwise
  * mode, ISX_CHUNK overrides). */
 /* DP work since isx_initialize in units of 32 x 32 cells: `total` = every (tile, chunk) pair of every column,
@@ -472,6 +477,38 @@ int isx_compute_batch_device_road(isx_handle h, isx_road_handle road, int pairwi
                                   const float *d_disparity, const int32_t *d_segmentation,
                                   const isx_road *fallback, isx_road_estimate *d_estimates, isx_road *d_roads);
 const char *isx_road_last_error(isx_road_handle h);
+
+/* Like isx_submit_batch_host / isx_submit_batch_host_u16 (same inputs, layouts and in-flight rules; the results are
+ * collected with isx_wait_batch_host or isx_wait_batch_packed), but each frame's road parameters are estimated on the
+ * device from its own disparity image, with `road`, inside the batch's pipeline -- the road rules of
+ * isx_compute_batch_device_road: a frame whose estimate is accepted is computed with it, a frame whose estimate
+ * fails keeps the last accepted road in frame order, and before any accepted estimate a frame uses `fallback`.
+ * fallback == NULL continues from the state the previous call on `road` left, including the previous SUBMITTED batch
+ * (a stream of batches behaves like one long batch).  `estimates` / `roads_out` (optional, host, [n]): what the
+ * estimation returned for every frame and the road each frame was computed with; both are filled when the wait for
+ * this batch returns.  After that wait the accessors of the last batch (isx_export_batch_device) use these roads.
+ * The u16 form estimates from the widened image (u16 * disparity_scale).
+ * Refusals enqueue and copy nothing: `road` uninitialised, on another device or of other rows / cols / max_dis
+ * (ISX_ERR_INVALID_ARGUMENT); road max_batch below the chunk the batch is cut into (min(n, isx_chunk_frames of
+ * the mode)) or batch sizes as for isx_submit_batch_host (ISX_ERR_CAPACITY); no fallback on a never-seeded road
+ * handle and null inputs (ISX_ERR_INVALID_ARGUMENT); a fourth batch in flight (ISX_ERR_CAPACITY).  `road` must not
+ * be used by another handle or thread while batches that use it are in flight. */
+int isx_submit_batch_host_road(isx_handle h, isx_road_handle road, int pairwise, int n, const float *disparity,
+                               const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
+                               isx_road *roads_out, isx_section *sections);
+int isx_submit_batch_host_u16_road(isx_handle h, isx_road_handle road, int pairwise, int n, const uint16_t *disparity,
+                                   float disparity_scale, const int16_t *segmentation, const isx_road *fallback,
+                                   isx_road_estimate *estimates, isx_road *roads_out, isx_section *sections);
+/* isx_pool_compute_host with the road of every frame estimated on the device inside the pipeline (every worker owns
+ * a road handle on its GPU, initialised from the pool's isx_config on the first call).  The rule is PER FRAME, not
+ * keep-last: a frame whose estimate is accepted is computed with it, every other frame with `fallback`, which is
+ * required.  (Frames are sharded over the workers and idle workers take sub-batches from other blocks, so the last
+ * accepted frame before a frame need not have been computed on the same GPU before it: a keep-last rule would make
+ * the results depend on the schedule.)  `estimates` / `roads_out` (optional, host, [n]) as above. */
+int isx_pool_compute_host_road(isx_pool_handle p, int pairwise, int n, const float *disparity,
+                               const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
+                               isx_road *roads_out, isx_section *sections, isx_instance *instances,
+                               int instances_capacity, int32_t *instance_offsets);
 /* Intermediates of the last call, frame `frame` of it (tests): 0 = v-disparity int32 [rows][max_dis],
  * 1 = binary image uint8 [rows][max_dis], 2 = Hough accumulator int32 [numangle+2][numrho+2]. */
 size_t isx_road_tensor_bytes(isx_road_handle h, int tensor);

@@ -44,6 +44,9 @@ EXPORTS = [
     "isx_road_tensor_bytes", "isx_road_read_tensor",
     # device batches with road estimation in stream order
     "isx_compute_batch_device_road",
+    # host batches and the frame pool with road estimation inside the pipeline
+    "isx_submit_batch_host_road", "isx_submit_batch_host_u16_road", "isx_pool_compute_host_road",
+    "isx_get_road_fill_time",
 ]
 
 
@@ -205,6 +208,13 @@ def _declare(lib):
     lib.isx_road_read_tensor.argtypes = [H, i, i, C.c_void_p, C.c_size_t]
     lib.isx_compute_batch_device_road.argtypes = [H, H, i, i, C.c_void_p, C.c_void_p, C.POINTER(Road), C.c_void_p,
                                                   C.c_void_p]
+    lib.isx_submit_batch_host_road.argtypes = [H, H, i, i, C.c_void_p, C.c_void_p, C.POINTER(Road), C.c_void_p,
+                                               C.c_void_p, C.c_void_p]
+    lib.isx_submit_batch_host_u16_road.argtypes = [H, H, i, i, C.c_void_p, f, C.c_void_p, C.POINTER(Road), C.c_void_p,
+                                                   C.c_void_p, C.c_void_p]
+    lib.isx_get_road_fill_time.argtypes = [H, C.POINTER(C.c_double), C.POINTER(C.c_long), i]
+    lib.isx_pool_compute_host_road.argtypes = [H, i, i, C.c_void_p, C.c_void_p, C.POINTER(Road), C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_void_p, i, C.c_void_p]
 
 
 def load():

@@ -397,6 +397,53 @@ class Stixels:
         self._in_flight = getattr(self, "_in_flight", [])
         self._in_flight.append((n, disparity, segmentation, sections_out))
 
+    def _road_outputs(self, n, estimates, roads_out):
+        est = (L.RoadEstimate * n)() if estimates is None else estimates
+        rds = (L.Road * n)() if roads_out is None else roads_out
+        if len(est) < n or len(rds) < n:
+            raise InvalidArgument("estimates / roads_out must hold n entries")
+        return est, rds
+
+    def SubmitBatchRoad(self, road: "RoadEstimation", pairwise: bool, disparity: np.ndarray,
+                        segmentation: np.ndarray, fallback: Optional[dict], sections_out: Optional[np.ndarray],
+                        estimates=None, roads_out=None):
+        """SubmitBatch with the road of every frame estimated on the device by `road` inside the pipeline
+        (isx_submit_batch_host_road), with the rules of ComputeBatchDeviceRoad: a failing frame keeps the last
+        accepted estimate, before the first one `fallback` (a road dict) is used; fallback=None continues from the
+        state the previous call on `road` left, submitted batches included.  Returns (estimates, roads): arrays of
+        n RoadEstimate / Road records (`estimates` / `roads_out` if given), filled when WaitBatch or WaitBatchPacked
+        for this batch returns."""
+        n = disparity.shape[0]
+        if disparity.dtype != np.float32 or segmentation.dtype != np.int32 or \
+                not disparity.flags.c_contiguous or not segmentation.flags.c_contiguous:
+            raise InvalidArgument("SubmitBatchRoad needs C-contiguous float32 / int32 arrays (no hidden copies)")
+        est, rds = self._road_outputs(n, estimates, roads_out)
+        fb = C.byref(_roads([fallback])[0]) if fallback is not None else None
+        self._check(self._lib.isx_submit_batch_host_road(
+            self._h, road.handle(), int(pairwise), n, disparity.ctypes.data, segmentation.ctypes.data, fb, est, rds,
+            sections_out.ctypes.data if sections_out is not None else None))
+        self._in_flight = getattr(self, "_in_flight", [])
+        self._in_flight.append((n, disparity, segmentation, sections_out, est, rds))
+        return est, rds
+
+    def SubmitBatchU16Road(self, road: "RoadEstimation", pairwise: bool, disparity_u16: np.ndarray,
+                           disparity_scale: float, segmentation_i16: np.ndarray, fallback: Optional[dict],
+                           sections_out: Optional[np.ndarray], estimates=None, roads_out=None):
+        """SubmitBatchRoad with narrow host inputs (see SubmitBatchU16): the road is estimated from the widened
+        image, u16 * disparity_scale."""
+        n = disparity_u16.shape[0]
+        if disparity_u16.dtype != np.uint16 or segmentation_i16.dtype != np.int16 or \
+                not disparity_u16.flags.c_contiguous or not segmentation_i16.flags.c_contiguous:
+            raise InvalidArgument("SubmitBatchU16Road needs C-contiguous uint16 / int16 arrays (no hidden copies)")
+        est, rds = self._road_outputs(n, estimates, roads_out)
+        fb = C.byref(_roads([fallback])[0]) if fallback is not None else None
+        self._check(self._lib.isx_submit_batch_host_u16_road(
+            self._h, road.handle(), int(pairwise), n, disparity_u16.ctypes.data, disparity_scale,
+            segmentation_i16.ctypes.data, fb, est, rds, sections_out.ctypes.data if sections_out is not None else None))
+        self._in_flight = getattr(self, "_in_flight", [])
+        self._in_flight.append((n, disparity_u16, segmentation_i16, sections_out, est, rds))
+        return est, rds
+
     def narrow_segmentation_elems(self) -> int:
         return self._lib.isx_narrow_segmentation_elems(self._h)
 
@@ -442,11 +489,14 @@ class Stixels:
         (sections [total], counts [n][C], instances [total], frames [n] of PACKED_FRAME_DTYPE)."""
         if not getattr(self, "_in_flight", None):
             raise InvalidArgument("no submitted batch is in flight")
-        self._in_flight.pop(0)
+        # the entry keeps the batch's buffers alive until the wait has returned: the library writes the estimates
+        # and roads of SubmitBatchRoad into them during the wait
+        entry = self._in_flight.pop(0)
         ps, pc, pi, pf = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p()
         n = C.c_int(0)
         self._check(self._lib.isx_wait_batch_packed(self._h, C.byref(ps), C.byref(pc), C.byref(pi), C.byref(pf),
                                                     C.byref(n)))
+        del entry
         n = n.value
         C_ = self.GetRealCols()
 
@@ -466,10 +516,12 @@ class Stixels:
         """Wait for the oldest submitted batch; returns (sections, instances, offsets) like ComputeBatch."""
         if not getattr(self, "_in_flight", None):
             raise InvalidArgument("no submitted batch is in flight")
-        n, _, _, sections_out = self._in_flight.pop(0)
+        entry = self._in_flight.pop(0)   # alive until the wait has returned (see WaitBatchPacked)
+        n, sections_out = entry[0], entry[3]
         inst, offs, cap = self._instance_buffers(n) if want_instances else (None, None, 0)
         self._check(self._lib.isx_wait_batch_host(self._h, inst.ctypes.data if want_instances else None, cap,
                                                   offs.ctypes.data if want_instances else None))
+        del entry
         if not want_instances:
             return sections_out, np.zeros(0, dtype=L.INSTANCE_DTYPE), np.zeros(n + 1, dtype=np.int32)
         return sections_out, inst[:offs[n]].copy(), offs.copy()
@@ -693,6 +745,29 @@ class StixelsPool:
         if rc != L.ISX_OK:
             raise StixelsError(f"isx_pool_compute_host: {self._lib.isx_pool_last_error(self._p).decode()} ({rc})")
         return sections_out, inst[:offs[n]].copy(), offs
+
+    def ComputeBatchRoad(self, pairwise: bool, disparity: np.ndarray, segmentation: np.ndarray, fallback: dict,
+                         sections_out: Optional[np.ndarray] = None):
+        """ComputeBatch with the road of every frame estimated on the device inside the pipeline
+        (isx_pool_compute_host_road).  Per frame: its own accepted estimate, else `fallback` (required).
+        Returns (sections, instances, offsets, estimates, roads); estimates / roads are arrays of n RoadEstimate /
+        Road records."""
+        disparity = np.ascontiguousarray(disparity, dtype=np.float32)
+        segmentation = np.ascontiguousarray(segmentation, dtype=np.int32)
+        n = disparity.shape[0]
+        if sections_out is None:
+            sections_out = np.zeros((n, self.GetRealCols(), 200), dtype=L.SECTION_DTYPE)
+        inst = np.empty(self._inst_cap * n, dtype=L.INSTANCE_DTYPE)
+        offs = np.zeros(n + 1, dtype=np.int32)
+        est, rds = (L.RoadEstimate * n)(), (L.Road * n)()
+        fb = _roads([fallback])[0]
+        rc = self._lib.isx_pool_compute_host_road(self._p, int(pairwise), n, disparity.ctypes.data,
+                                                  segmentation.ctypes.data, C.byref(fb), est, rds,
+                                                  sections_out.ctypes.data, inst.ctypes.data, inst.size,
+                                                  offs.ctypes.data)
+        if rc != L.ISX_OK:
+            raise StixelsError(f"isx_pool_compute_host_road: {self._lib.isx_pool_last_error(self._p).decode()} ({rc})")
+        return sections_out, inst[:offs[n]].copy(), offs, est, rds
 
     def frames_by_worker(self):
         """Frames every worker processed in the last ComputeBatch (its block, less or plus what was taken over)."""

@@ -10,6 +10,8 @@
 // overlap on three streams; there is no per-frame cudaMalloc, handle
 // construction or device-wide synchronisation.
 #include <algorithm>
+#include <atomic>
+#include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -117,6 +119,9 @@ struct isx_context {
     int *h_counts = nullptr, *m_counts = nullptr;               // [max_batch][C] stixels per column
     isx_packed_frame *h_frames = nullptr, *m_frames = nullptr;  // [max_batch]
     int sections_cap = 0, inst_cap = 0;           // entries of the packed arrays
+    // batches with estimated roads (isx_submit_batch_host_road), allocated on first use: mapped pinned [max_batch]
+    isx_road_estimate *h_est = nullptr, *m_est = nullptr;   // what the estimation returned for every frame
+    isx_road *h_roads = nullptr, *m_roads = nullptr;        // the road every frame was computed with
   } rs[isx::kResultSets];
   int cur = 0;                                    // result set of the batch being enqueued / of the last batch
   int *d_raster_table = nullptr;                  // [max_batch][C][200] instance id per stixel (rasteriser)
@@ -139,6 +144,8 @@ struct isx_context {
   int batch_n[isx::kResultSets] = {};                     // frames of the batch in flight with that ticket, 0 = none
   int batch_set[isx::kResultSets] = {};                   // its result set
   isx_section *batch_sections[isx::kResultSets] = {};     // the caller's padded array the wait expands into
+  isx_road_estimate *batch_est[isx::kResultSets] = {};    // the caller's arrays the wait fills (estimated roads)
+  isx_road *batch_roads[isx::kResultSets] = {};
   bool batch_direct[isx::kResultSets] = {};               // ... or that the device has already filled (mapped memory)
   isx_section *direct_sections = nullptr;               // device address of the caller's array for the batch being enqueued
   bool results_stay_on_device = false;                  // set while a device batch is enqueued
@@ -153,7 +160,13 @@ struct isx_context {
   std::mutex road_cache_mutex;
   isx_road *h_stage_roads = nullptr;  // [kStageSlots][chunk] pinned: the device-estimated roads of a staged chunk
   isx_road *d_batch_roads = nullptr;  // [max_batch] roads of the last isx_compute_batch_device_road batch
-  bool last_roads_device = false;     // ... which the export reads instead of last_roads
+  bool last_roads_device = false;     // the roads of the last batch were estimated on the device: the export reads
+  const isx_road *last_roads_dev = nullptr;   // them here (d_batch_roads or rs[cur].m_roads) instead of last_roads
+  // device addresses of the pinned staging (h_ground, h_vhor, h_stage_roads), taken on the first host batch with
+  // estimated roads: its road step writes the roads there and pull_tables_kernel reads the tables from there
+  float *m_ground = nullptr;
+  int *m_vhor = nullptr;
+  isx_road *m_stage_roads = nullptr;
   isx_road single_road{0, 0.f, 0.f, 0.f};
   bool single_has_road = false;
   int last_batch = 0;          // frames of the last batch (results valid for these)
@@ -170,6 +183,8 @@ struct isx_context {
   size_t prof_h2d_used = 0;
   double stage_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   long stage_launches[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  // host time of the ground-table host functions of batches with estimated roads (a driver thread writes it)
+  std::atomic<long long> host_fill_ns{0}, host_fill_calls{0};
 };
 
 namespace isx {
@@ -336,12 +351,14 @@ static int stage_road_tables(isx_context *c, const isx_road *roads, int n, cudaS
 struct StageFill {
   isx_context *c;
   int stage, n;
+  bool timed;   // isx_set_profiling at enqueue time: the host function's time goes to isx_get_road_fill_time
 };
 
 static void CUDART_CB fill_stage_from_roads(void *arg) {
   const StageFill p = *static_cast<StageFill *>(arg);
   delete static_cast<StageFill *>(arg);
   isx_context *c = p.c;
+  const auto t0 = std::chrono::steady_clock::now();
   const int H = c->kp.rows;
   const isx_road *roads = c->h_stage_roads + (size_t)p.stage * c->chunk;
   float *hg = c->h_ground + (size_t)p.stage * c->chunk * 3 * H;
@@ -350,6 +367,10 @@ static void CUDART_CB fill_stage_from_roads(void *arg) {
     copy_road_tables(c, roads[i], hg + (size_t)i * 3 * H);
     hv[i] = H - roads[i].vhor - 1;  // Stixels.cu:377
   }
+  if (p.timed) {
+    c->host_fill_ns += std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count();
+    c->host_fill_calls++;
+  }
 }
 
 static int stage_device_road_tables(isx_context *c, const isx_road *d_roads, int n, cudaStream_t st) {
@@ -357,8 +378,43 @@ static int stage_device_road_tables(isx_context *c, const isx_road *d_roads, int
   ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_stage_done[stage], 0));
   ISX_TRY(c, cudaMemcpyAsync(c->h_stage_roads + (size_t)stage * c->chunk, d_roads, sizeof(isx_road) * n,
                              cudaMemcpyDeviceToHost, st));
-  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{c, stage, n}));
+  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{c, stage, n, c->profiling}));
   return send_road_tables(c, stage, n, st);
+}
+
+// Host batches with estimated roads (isx_submit_batch_host_road): the road step of a chunk runs on s_tables once the
+// chunk's images have arrived.  Its tables cannot travel in front of the images, and a copy on s_tables would queue
+// on the copy engine behind the next chunk's images (DESIGN.md 3, 6).  So nothing here is a copy: resolve_kernel writes
+// the chunk's roads straight into the mapped staging slot, the host function fills the slot's tables from them, and
+// pull_tables_kernel moves the tables into the road ring with loads of the SMs.  Everything is ordered on s_tables, the
+// copy stream never waits for any of it, and the calling thread does not wait either.  Returns the ring slot or an
+// error.
+struct HostRoad {
+  isx_road_handle road = nullptr;
+  const isx_road *fallback = nullptr;   // the seed: given to the road step of the first chunk of the call only
+  bool carry = true;                    // false: the frame pool's per-frame rule
+};
+
+static int stage_estimated_road_tables(isx_context *c, const HostRoad &hr, const isx_road *fallback, int n,
+                                       const float *d_disp, isx_road_estimate *m_est, isx_road *m_roads) {
+  const int H = c->kp.rows;
+  cudaStream_t st = c->s_tables;
+  const int stage = (int)(c->stage_next++ % kStageSlots);
+  // the staging slot is free once the pull that last read it is done (the road stream is ordered behind st)
+  ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_stage_done[stage], 0));
+  std::string msg;
+  if (int rc = road_enqueue_batch(hr.road, st, n, d_disp, fallback, m_est, m_roads,
+                                  c->m_stage_roads + (size_t)stage * c->chunk, msg, hr.carry))
+    return fail(c, rc, msg);
+  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{c, stage, n, c->profiling}));
+  const int rslot = (int)(c->road_next++ % kRoadSlots);
+  const isx_context::RoadSlot &rd = c->roads[rslot];
+  ISX_TRY(c, cudaStreamWaitEvent(st, rd.ev_free, 0));
+  launch_pull_road_tables(c->m_ground + (size_t)stage * c->chunk * 3 * H, rd.ground, (size_t)n * 3 * H,
+                          c->m_vhor + (size_t)stage * c->chunk, rd.vhor, n, st);
+  ISX_TRY(c, cudaGetLastError());
+  ISX_TRY(c, cudaEventRecord(c->ev_stage_done[stage], st));
+  return rslot;
 }
 
 // `road_slot` >= 0: the caller has already copied the road tables of the chunk into that slot of the ring (host
@@ -512,6 +568,28 @@ static int alloc_result_set(isx_context *c, int i) {
   ISX_TRY(c, cudaHostGetDevicePointer(&R.m_frames, R.h_frames, 0));
   std::memset(R.h_frames, 0, sizeof(isx_packed_frame) * MB);
   R.allocated = true;
+  return ISX_OK;
+}
+
+// The estimates and roads of a batch with estimated roads (mapped pinned, written by resolve_kernel), and the device
+// addresses of the staging its road steps write and read.
+static int alloc_road_results(isx_context *c, int i) {
+  isx_context::ResultSet &R = c->rs[i];
+  const size_t MB = c->max_batch;
+  const unsigned flags = cudaHostAllocMapped | cudaHostAllocPortable;
+  if (!R.h_est) {
+    ISX_TRY(c, cudaHostAlloc(&R.h_est, sizeof(isx_road_estimate) * MB, flags));
+    ISX_TRY(c, cudaHostGetDevicePointer(&R.m_est, R.h_est, 0));
+  }
+  if (!R.h_roads) {
+    ISX_TRY(c, cudaHostAlloc(&R.h_roads, sizeof(isx_road) * MB, flags));
+    ISX_TRY(c, cudaHostGetDevicePointer(&R.m_roads, R.h_roads, 0));
+  }
+  if (!c->m_ground) {
+    ISX_TRY(c, cudaHostGetDevicePointer(&c->m_ground, c->h_ground, 0));
+    ISX_TRY(c, cudaHostGetDevicePointer(&c->m_vhor, c->h_vhor, 0));
+    ISX_TRY(c, cudaHostGetDevicePointer(&c->m_stage_roads, c->h_stage_roads, 0));
+  }
   return ISX_OK;
 }
 
@@ -831,6 +909,10 @@ int isx_finish(isx_handle h) {
   h->h_stage_roads = nullptr;
   h->d_batch_roads = nullptr;
   h->last_roads_device = false;
+  h->last_roads_dev = nullptr;
+  h->m_ground = nullptr;
+  h->m_vhor = nullptr;
+  h->m_stage_roads = nullptr;
   for (int i = 0; i < kStageSlots; i++) {
     if (h->ev_stage_done[i]) cudaEventDestroy(h->ev_stage_done[i]);
     h->ev_stage_done[i] = nullptr;
@@ -847,10 +929,14 @@ int isx_finish(isx_handle h) {
       cudaFreeHost(R.h_counts);
       cudaFreeHost(R.h_frames);
     }
+    if (R.h_est) cudaFreeHost(R.h_est);
+    if (R.h_roads) cudaFreeHost(R.h_roads);
     R = isx_context::ResultSet();
     if (h->ev_batch_done[i]) cudaEventDestroy(h->ev_batch_done[i]);
     h->ev_batch_done[i] = nullptr;
     h->batch_sections[i] = nullptr;
+    h->batch_est[i] = nullptr;
+    h->batch_roads[i] = nullptr;
     h->batch_n[i] = 0;
   }
   for (int i = 0; i < 2; i++) {
@@ -1125,6 +1211,7 @@ int isx_compute_batch_device_road(isx_handle h, isx_road_handle road, int pairwi
   h->last_batch = n;
   h->last_roads.clear();
   h->last_roads_device = true;
+  h->last_roads_dev = h->d_batch_roads;
   for (int first = 0; first < n; first += chunk) {
     const int cn = (n - first) < chunk ? (n - first) : chunk;
     const int road_slot = stage_device_road_tables(h, h->d_batch_roads + first, cn, h->s_tables);
@@ -1195,8 +1282,9 @@ static int ensure_narrow_staging(isx_handle h) {
 // chunks behind).
 // `caller_waits`: a synchronous call -- the kernels of the last chunk run with nothing beside them while the caller
 // waits, so the tail goes in quarter pieces like the head.
+// `hr`: estimate the roads on the device instead (then `roads` is null): the chunk's road step runs behind its images.
 static int enqueue_host_batch(isx_handle h, int pairwise, int n, const HostInputs &in, const isx_road *roads,
-                              bool caller_waits) {
+                              bool caller_waits, const HostRoad *hr = nullptr) {
   const size_t hw = (size_t)h->kp.rows * h->kp.cols, se = seg_elems(h), se16 = narrow_seg_elems(h);
   if (in.narrow()) {
     if (hw % 8 != 0) return fail(h, ISX_ERR_UNSUPPORTED, "the uint16 disparity path needs rows*cols to be a multiple of 8");
@@ -1232,8 +1320,11 @@ static int enqueue_host_batch(isx_handle h, int pairwise, int n, const HostInput
       cudaEventRecord(h->prof_h2d[h->prof_h2d_used++], h->s_h2d);
     };
     mark_h2d();
-    const int road_slot = stage_road_tables(h, roads + first, cn, h->s_h2d);
-    if (road_slot < 0) return road_slot;
+    int road_slot = -1;
+    if (!hr) {
+      road_slot = stage_road_tables(h, roads + first, cn, h->s_h2d);
+      if (road_slot < 0) return road_slot;
+    }
     if (in.narrow()) {
       ISX_TRY(h, cudaMemcpyAsync(h->d_in_disp16[slot], in.disparity16 + first * hw, sizeof(uint16_t) * hw * cn,
                                  cudaMemcpyHostToDevice, h->s_h2d));
@@ -1258,16 +1349,28 @@ static int enqueue_host_batch(isx_handle h, int pairwise, int n, const HostInput
     if (in.narrow())
       launch_widen_inputs(h->kp, h->d_in_disp16[slot], in.scale, h->d_in_seg16[slot], h->d_in_disp[slot],
                           h->d_in_seg[slot], cn, h->s_tables);
-    if (int rc = enqueue_chunk(h, pairwise != 0, first, cn, h->d_in_disp[slot], h->d_in_seg[slot], roads + first,
-                               slot, road_slot))
+    if (hr) {
+      const isx_context::ResultSet &R = h->rs[h->cur];
+      road_slot = stage_estimated_road_tables(h, *hr, first == 0 ? hr->fallback : nullptr, cn, h->d_in_disp[slot],
+                                              R.m_est + first, R.m_roads + first);
+      if (road_slot < 0) return road_slot;
+    }
+    if (int rc = enqueue_chunk(h, pairwise != 0, first, cn, h->d_in_disp[slot], h->d_in_seg[slot],
+                               hr ? nullptr : roads + first, slot, road_slot))
       return rc;
     ISX_TRY(h, cudaEventRecord(h->ev_in_free[slot], h->s_tables));   // the inputs are read by the table build only
     slot ^= 1;
   }
   h->host_slot = slot;
   h->last_batch = n;
-  h->last_roads.assign(roads, roads + n);
-  h->last_roads_device = false;
+  if (hr) {
+    h->last_roads.clear();
+    h->last_roads_device = true;
+    h->last_roads_dev = h->rs[h->cur].m_roads;
+  } else {
+    h->last_roads.assign(roads, roads + n);
+    h->last_roads_device = false;
+  }
   return ISX_OK;
 }
 
@@ -1318,10 +1421,19 @@ int isx_compute_batch_host_u16(isx_handle h, int pairwise, int n, const uint16_t
 size_t isx_narrow_segmentation_elems(isx_handle h) { return (h && h->initialized) ? narrow_seg_elems(h) : 0; }
 
 static int submit_batch_host(isx_handle h, int pairwise, int n, const HostInputs &in, const isx_road *roads,
-                             isx_section *sections) {
+                             isx_section *sections, const HostRoad *hr = nullptr, isx_road_estimate *estimates = nullptr,
+                             isx_road *roads_out = nullptr) {
   if (int rc = check_ready(h)) return rc;
   if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
-  if (!roads) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
+  if (!roads && !hr) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
+  if (hr) {
+    // the road step runs per chunk: the road handle must hold the largest chunk the batch is cut into
+    const int chunk = pairwise ? h->chunk : h->chunk_unary;
+    std::string msg;
+    if (int rc = road_check_batch(hr->road, h->device, h->kp.rows, h->kp.cols, h->kp.max_dis, n < chunk ? n : chunk,
+                                  hr->fallback != nullptr, msg))
+      return fail(h, rc, msg);
+  }
   if (h->submitted - h->waited >= (unsigned long long)(kResultSets - 1))
     return fail(h, ISX_ERR_CAPACITY, "three batches are already in flight: call isx_wait_batch_host first");
   int next = 0;
@@ -1332,12 +1444,15 @@ static int submit_batch_host(isx_handle h, int pairwise, int n, const HostInputs
     while (busy[next]) next++;
   }
   if (int rc = alloc_result_set(h, next)) return rc;
+  if (hr) {
+    if (int rc = alloc_road_results(h, next)) return rc;
+  }
   for (int i = 0; i < kResultSets; i++)
     if (!h->ev_batch_done[i]) ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_batch_done[i], cudaEventDisableTiming));
   h->cur = next;
   h->direct_sections = device_view_of(sections);
   const bool direct = h->direct_sections != nullptr;
-  const int erc = enqueue_host_batch(h, pairwise, n, in, roads, /*caller_waits=*/false);
+  const int erc = enqueue_host_batch(h, pairwise, n, in, roads, /*caller_waits=*/false, hr);
   h->direct_sections = nullptr;
   if (erc) return erc;
   const int par = (int)(h->submitted % kResultSets);
@@ -1346,6 +1461,8 @@ static int submit_batch_host(isx_handle h, int pairwise, int n, const HostInputs
   h->batch_n[par] = n;
   h->batch_set[par] = h->cur;
   h->batch_sections[par] = sections;
+  h->batch_est[par] = hr ? estimates : nullptr;
+  h->batch_roads[par] = hr ? roads_out : nullptr;
   h->submitted++;
   h->emit_join_pending = true;  // isx_stream() itself has not been ordered behind the emission stream
   return ISX_OK;
@@ -1370,6 +1487,33 @@ int isx_submit_batch_host_u16(isx_handle h, int pairwise, int n, const uint16_t 
   return submit_batch_host(h, pairwise, n, in, roads, sections);
 }
 
+int isx_submit_batch_host_road(isx_handle h, isx_road_handle road, int pairwise, int n, const float *disparity,
+                               const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
+                               isx_road *roads_out, isx_section *sections) {
+  if (!road || !disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
+  HostInputs in;
+  in.disparity = disparity;
+  in.segmentation = segmentation;
+  HostRoad hr;
+  hr.road = road;
+  hr.fallback = fallback;
+  return submit_batch_host(h, pairwise, n, in, nullptr, sections, &hr, estimates, roads_out);
+}
+
+int isx_submit_batch_host_u16_road(isx_handle h, isx_road_handle road, int pairwise, int n, const uint16_t *disparity,
+                                   float disparity_scale, const int16_t *segmentation, const isx_road *fallback,
+                                   isx_road_estimate *estimates, isx_road *roads_out, isx_section *sections) {
+  if (!road || !disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
+  HostInputs in;
+  in.disparity16 = disparity;
+  in.scale = disparity_scale;
+  in.segmentation16 = segmentation;
+  HostRoad hr;
+  hr.road = road;
+  hr.fallback = fallback;
+  return submit_batch_host(h, pairwise, n, in, nullptr, sections, &hr, estimates, roads_out);
+}
+
 int isx_reserve_in_flight(isx_handle h, int batches) {
   if (int rc = check_ready(h)) return rc;
   if (batches < 1 || batches > kResultSets - 1)
@@ -1388,6 +1532,12 @@ static int wait_oldest(isx_handle h) {
   ISX_TRY(h, cudaEventSynchronize(h->ev_batch_done[par]));
   h->last_waited_set = h->batch_set[par];
   h->waited++;
+  const isx_context::ResultSet &R = h->rs[h->batch_set[par]];
+  const size_t n = (size_t)h->batch_n[par];
+  if (h->batch_est[par]) std::memcpy(h->batch_est[par], R.h_est, sizeof(isx_road_estimate) * n);
+  if (h->batch_roads[par]) std::memcpy(h->batch_roads[par], R.h_roads, sizeof(isx_road) * n);
+  h->batch_est[par] = nullptr;
+  h->batch_roads[par] = nullptr;
   return par;
 }
 
@@ -1469,7 +1619,7 @@ int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_res
   a.camera_center_x = m.camera_center_x;
   a.camera_center_y = m.camera_center_y;
   a.out = *out;
-  a.roads = h->last_roads_device ? h->d_batch_roads + first : nullptr;
+  a.roads = h->last_roads_device ? h->last_roads_dev + first : nullptr;
   std::vector<float> alpha((size_t)n);
   std::vector<int> vhor((size_t)n);
   for (int f = 0; f < n && !a.roads; f++) {
@@ -1606,6 +1756,18 @@ int isx_get_stage_times(isx_handle h, double *ms, long *chunks, int n_stages, in
   return ISX_OK;
 }
 
+int isx_get_road_fill_time(isx_handle h, double *ms, long *calls, int reset) {
+  if (int rc = check_ready(h)) return rc;
+  ISX_TRY(h, cudaStreamSynchronize(h->s_tables));
+  if (ms) *ms = (double)h->host_fill_ns.load() * 1e-6;
+  if (calls) *calls = (long)h->host_fill_calls.load();
+  if (reset) {
+    h->host_fill_ns = 0;
+    h->host_fill_calls = 0;
+  }
+  return ISX_OK;
+}
+
 // Developer trace of the host-batch pipeline (profiling enabled): per profiled chunk 11 time stamps in ms relative
 // to the first one -- input copy begin | end (copy stream); join | frame tables | column tables | tables end (table
 // stream); DP begin | DP end (compute stream); emission begin | grouping begin | emission end (emission stream).
@@ -1645,3 +1807,25 @@ int isx_chunk_frames(isx_handle h) { return (h && h->initialized) ? h->last_laun
 int isx_instance_capacity(isx_handle h) { return (h && h->initialized) ? h->inst_cap : 0; }
 
 }  // extern "C"
+
+namespace isx {
+
+// For the frame pool (pool.cu): isx_submit_batch_host_road with the per-frame rule (carry == false: a frame's own
+// estimate, else `fallback`, never another frame's), and the largest chunk a batch of h is cut into.
+int pool_submit_batch_host_road(isx_handle h, isx_road_handle road, int pairwise, int n, const float *disparity,
+                                const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
+                                isx_road *roads_out, isx_section *sections) {
+  if (!road || !disparity || !segmentation || !fallback) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
+  HostInputs in;
+  in.disparity = disparity;
+  in.segmentation = segmentation;
+  HostRoad hr;
+  hr.road = road;
+  hr.fallback = fallback;
+  hr.carry = false;
+  return submit_batch_host(h, pairwise, n, in, nullptr, sections, &hr, estimates, roads_out);
+}
+
+int largest_chunk(isx_handle h) { return (h && h->initialized) ? std::max(h->chunk, h->chunk_unary) : 0; }
+
+}  // namespace isx

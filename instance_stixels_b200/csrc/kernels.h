@@ -113,14 +113,19 @@ struct ExportFrames {              // per-frame road scalars of one launch: alph
 };
 void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_ground, const int *vhor,
                            cudaStream_t s);
-// Road estimation in front of a device batch (road.cu, isx_compute_batch_device_road): the checks (nothing enqueued),
-// then the Hough kernels, the device line selection and the keep-last rule on the road handle's stream, ordered after
-// and before `caller`.  d_roads [n]: the road every frame is computed with.  0 or an isx_status, text in `msg`.
+// Road estimation in front of a device batch (road.cu, isx_compute_batch_device_road) or of a chunk of a host batch
+// (isx_submit_batch_host_road): the checks (nothing enqueued), then the Hough kernels, the device line selection and
+// the keep-last rule on the road handle's stream, ordered after and before `caller`.  d_roads [n]: the road every
+// frame is computed with.  carry == false: the frame pool's per-frame rule (own estimate, else the seed).  0 or an
+// isx_status, text in `msg`.
 int road_check_batch(isx_road_handle road, int device, int rows, int cols, int max_dis, int n, bool has_fallback,
                      std::string &msg);
 int road_enqueue_batch(isx_road_handle road, cudaStream_t caller, int n, const float *d_disparity,
                        const isx_road *fallback, isx_road_estimate *d_estimates, isx_road *d_roads_out,
-                       isx_road *d_roads, std::string &msg);
+                       isx_road *d_roads, std::string &msg, bool carry = true);
+// [ground_floats] + [n] ints from mapped pinned memory into device memory, a kernel on `s` (road.cu)
+void launch_pull_road_tables(const float *src_ground, float *dst_ground, size_t ground_floats, const int *src_vhor,
+                             int *dst_vhor, int n, cudaStream_t s);
 // u16 disparity / i16 segmentation staging -> the float / int32 layouts of the path (ingest.cu)
 void launch_widen_inputs(const KParams &p, const uint16_t *disp16, float scale, const int16_t *seg16, float *disp,
                          int32_t *seg, int nframes, cudaStream_t s);

@@ -11,6 +11,11 @@
 // call takes as long as the slowest of them.  Frames are independent, so there is no collective: every sub-batch
 // writes its frames' Sections into the caller's array at their place; the instance records are concatenated in frame
 // order when all workers are done.
+//
+// isx_pool_compute_host_road estimates the road of every frame on the device inside the same pipeline (the road step of
+// isx_submit_batch_host_road): every worker owns a road handle on its GPU, created on the first such call.  A frame is
+// computed with its OWN accepted estimate, else with the caller's fallback -- never with another frame's: which frames
+// a worker sees, and in which order, depends on the schedule, so a keep-last rule would make the results depend on it.
 #include <algorithm>
 #include <condition_variable>
 #include <deque>
@@ -23,6 +28,14 @@
 
 #include "../../include/instance_stixels_b200.h"
 
+namespace isx {
+// context.cu
+int pool_submit_batch_host_road(isx_handle h, isx_road_handle road, int pairwise, int n, const float *disparity,
+                                const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
+                                isx_road *roads_out, isx_section *sections);
+int largest_chunk(isx_handle h);
+}  // namespace isx
+
 namespace {
 
 // One call's frames: per worker the part of its block nobody has taken yet.
@@ -31,6 +44,10 @@ struct Job {
   const float *disparity = nullptr;
   const int32_t *segmentation = nullptr;
   const isx_road *roads = nullptr;
+  // road estimation on the device (isx_pool_compute_host_road): `roads` is null, these are set
+  const isx_road *fallback = nullptr;
+  isx_road_estimate *estimates = nullptr;
+  isx_road *roads_out = nullptr;
   isx_section *sections = nullptr;
   bool want_instances = false;
   std::mutex m;
@@ -46,6 +63,7 @@ struct Piece {
 
 struct Worker {
   isx_handle h = nullptr;
+  isx_road_handle road = nullptr;    // created by the first isx_pool_compute_host_road
   int device = 0, index = 0;
   std::thread thread;
   std::mutex m;
@@ -64,6 +82,7 @@ struct Worker {
 
 struct isx_pool {
   std::vector<Worker *> workers;
+  isx_config cfg;                    // for the road handles of the workers
   int max_batch = 0;
   size_t hw = 0, seg_elems = 0, sec_per_frame = 0;
   int realcols = 0, inst_cap = 0;
@@ -128,9 +147,14 @@ void run_job(isx_pool *p, Worker *w) {
       int f0 = 0, cn = 0;
       more = claim(j, w->index, mb, &f0, &cn);
       if (!more) break;
-      const int rc = isx_submit_batch_host(w->h, j.pairwise, cn, j.disparity + (size_t)f0 * p->hw,
-                                           j.segmentation + (size_t)f0 * p->seg_elems, j.roads + f0,
-                                           j.sections ? j.sections + (size_t)f0 * p->sec_per_frame : nullptr);
+      isx_section *sec = j.sections ? j.sections + (size_t)f0 * p->sec_per_frame : nullptr;
+      const int rc = j.roads ? isx_submit_batch_host(w->h, j.pairwise, cn, j.disparity + (size_t)f0 * p->hw,
+                                                     j.segmentation + (size_t)f0 * p->seg_elems, j.roads + f0, sec)
+                             : isx::pool_submit_batch_host_road(
+                                   w->h, w->road, j.pairwise, cn, j.disparity + (size_t)f0 * p->hw,
+                                   j.segmentation + (size_t)f0 * p->seg_elems, j.fallback,
+                                   j.estimates ? j.estimates + f0 : nullptr, j.roads_out ? j.roads_out + f0 : nullptr,
+                                   sec);
       if (rc != ISX_OK) {
         w->rc = rc;
         w->error = isx_last_error(w->h);
@@ -185,6 +209,7 @@ int isx_pool_create(isx_pool_handle *out, const int *devices, int n_devices, con
     return pool_fail(nullptr, ISX_ERR_INVALID_ARGUMENT, "isx_pool_create: bad argument");
   isx_pool *p = new isx_pool();
   p->max_batch = max_batch;
+  p->cfg = *cfg;
   for (int i = 0; i < n_devices; i++) {
     Worker *w = new Worker();
     w->device = devices[i];
@@ -226,6 +251,7 @@ int isx_pool_destroy(isx_pool_handle p) {
     w->cv.notify_all();
     if (w->thread.joinable()) w->thread.join();
     isx_destroy(w->h);
+    isx_road_destroy(w->road);
     delete w;
   }
   delete p;
@@ -244,20 +270,17 @@ int isx_pool_frames_by_worker(isx_pool_handle p, int *frames, int capacity) {
   return n;
 }
 
-int isx_pool_compute_host(isx_pool_handle p, int pairwise, int n, const float *disparity,
-                          const int32_t *segmentation, const isx_road *roads, isx_section *sections,
-                          isx_instance *instances, int instances_capacity, int32_t *instance_offsets) {
-  if (!p) return pool_fail(nullptr, ISX_ERR_INVALID_ARGUMENT, "null pool");
-  if (n < 1 || !disparity || !segmentation || !roads) return pool_fail(p, ISX_ERR_INVALID_ARGUMENT, "bad argument");
-  const int G = (int)p->workers.size();
-  Job job;
-  job.pairwise = pairwise;
+}  // extern "C"
+
+namespace {
+
+// One call: the frames of `job` (inputs and road arguments set) through all workers.
+int pool_run(isx_pool *p, Job &job, int n, isx_section *sections, isx_instance *instances, int instances_capacity,
+             int32_t *instance_offsets) {
   job.n = n;
-  job.disparity = disparity;
-  job.segmentation = segmentation;
-  job.roads = roads;
   job.sections = sections;
   job.want_instances = instances != nullptr || instance_offsets != nullptr;
+  const int G = (int)p->workers.size();
   job.lo.resize((size_t)G);
   job.hi.resize((size_t)G);
   // worker g owns frames [n * g / G, n * (g + 1) / G): contiguous blocks (SURVEY.md 8e)
@@ -308,6 +331,56 @@ int isx_pool_compute_host(isx_pool_handle p, int pairwise, int n, const float *d
     if (instance_offsets) instance_offsets[n] = total;
   }
   return ISX_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int isx_pool_compute_host(isx_pool_handle p, int pairwise, int n, const float *disparity,
+                          const int32_t *segmentation, const isx_road *roads, isx_section *sections,
+                          isx_instance *instances, int instances_capacity, int32_t *instance_offsets) {
+  if (!p) return pool_fail(nullptr, ISX_ERR_INVALID_ARGUMENT, "null pool");
+  if (n < 1 || !disparity || !segmentation || !roads) return pool_fail(p, ISX_ERR_INVALID_ARGUMENT, "bad argument");
+  Job job;
+  job.pairwise = pairwise;
+  job.disparity = disparity;
+  job.segmentation = segmentation;
+  job.roads = roads;
+  return pool_run(p, job, n, sections, instances, instances_capacity, instance_offsets);
+}
+
+int isx_pool_compute_host_road(isx_pool_handle p, int pairwise, int n, const float *disparity,
+                               const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
+                               isx_road *roads_out, isx_section *sections, isx_instance *instances,
+                               int instances_capacity, int32_t *instance_offsets) {
+  if (!p) return pool_fail(nullptr, ISX_ERR_INVALID_ARGUMENT, "null pool");
+  if (n < 1 || !disparity || !segmentation || !fallback)
+    return pool_fail(p, ISX_ERR_INVALID_ARGUMENT, "bad argument (the fallback road is required)");
+  for (Worker *w : p->workers) {
+    if (w->road) continue;
+    // one road handle per worker, on its GPU, for the largest chunk its context cuts a sub-batch into
+    const isx_config &c = p->cfg;
+    int rc = isx_road_create(&w->road, w->device);
+    if (rc == ISX_OK)
+      rc = isx_road_initialize(w->road, c.camera_center_y, c.baseline, c.focal, (int)c.rows, (int)c.cols, c.max_dis,
+                               c.road_vdisparity_threshold, isx::largest_chunk(w->h));
+    if (rc != ISX_OK) {
+      const std::string msg = std::string("isx_pool_compute_host_road, device ") + std::to_string(w->device) + ": " +
+                              isx_road_last_error(w->road);
+      isx_road_destroy(w->road);
+      w->road = nullptr;
+      return pool_fail(p, rc, msg);
+    }
+  }
+  Job job;
+  job.pairwise = pairwise;
+  job.disparity = disparity;
+  job.segmentation = segmentation;
+  job.fallback = fallback;
+  job.estimates = estimates;
+  job.roads_out = roads_out;
+  return pool_run(p, job, n, sections, instances, instances_capacity, instance_offsets);
 }
 
 }  // extern "C"

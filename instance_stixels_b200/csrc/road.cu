@@ -19,7 +19,10 @@
 //                       vote threshold and the pitch range -- the first line the host's ordered walk accepts.  Whether
 //                       a cell's pitch is in range, and its camera properties, depend on the cell alone: a table
 //                       built once per handle on the host with the very code of the host walk (cell_estimate).
-//   resolve_kernel    : cells -> estimates, and the reference's keep-last rule across the frames of the batch.
+//   resolve_kernel    : cells -> estimates, and the reference's keep-last rule across the frames of the batch (or, for
+//                       the frame pool, every frame on its own: its estimate or the seed).
+//   pull_tables_kernel: host batches with estimated roads -- the staged ground tables of a chunk from mapped pinned
+//                       memory into the road ring, read by the SMs, so that no copy queues on the copy engine.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -166,13 +169,15 @@ select_kernel(const int *__restrict__ accum, const isx_road_estimate *__restrict
 // One thread walks the frames in order: the estimate of every frame (zeros when no line was accepted, like road_run)
 // and the road it is computed with -- its own estimate, else the last accepted one (RoadEstimation.cu:123-133 only
 // overwrites the getters on success), else the seed.  *state = the cell behind the last accepted estimate, -1 = seed.
+// carry == 0: no frame inherits from another (the frame pool's per-frame rule): its own estimate, else the seed.
 __global__ void resolve_kernel(const unsigned long long *__restrict__ sel, const isx_road_estimate *__restrict__ cells,
-                               int *__restrict__ state, int reset, isx_road seed, int n,
+                               int *__restrict__ state, int reset, int carry, isx_road seed, int n,
                                isx_road_estimate *__restrict__ estimates, isx_road *__restrict__ roads_out,
                                isx_road *__restrict__ roads) {
   if (threadIdx.x != 0) return;
   int cur = reset ? -1 : *state;
   for (int f = 0; f < n; f++) {
+    if (!carry) cur = -1;
     const unsigned long long key = sel[f];
     isx_road_estimate e = {0, 0, 0.f, 0.f, 0.f, 0.f, 0.f};
     if (key) {
@@ -189,6 +194,17 @@ __global__ void resolve_kernel(const unsigned long long *__restrict__ sel, const
     roads[f] = r;
   }
   *state = cur;
+}
+
+// [n][3][H] ground tables + [n] horizon rows: mapped pinned staging -> a slot of the road ring (under a MB per 64-frame
+// chunk of 1024 rows).  The loads cross the host link as reads of the SMs, beside whatever the copy engine is doing.
+__global__ void __launch_bounds__(256)
+pull_tables_kernel(const float *__restrict__ src_ground, float *__restrict__ dst_ground, size_t n_ground,
+                   const int *__restrict__ src_vhor, int *__restrict__ dst_vhor, int n) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_ground; i += stride) dst_ground[i] = src_ground[i];
+  if (blockIdx.x == 0)
+    for (int i = threadIdx.x; i < n; i += blockDim.x) dst_vhor[i] = src_vhor[i];
 }
 
 }  // namespace
@@ -487,7 +503,7 @@ int road_check_batch(isx_road_handle h, int device, int rows, int cols, int max_
 // frame is computed with.  Checked by road_check_batch before.
 int road_enqueue_batch(isx_road_handle h, cudaStream_t caller, int n, const float *d_disparity,
                        const isx_road *fallback, isx_road_estimate *d_estimates, isx_road *d_roads_out,
-                       isx_road *d_roads, std::string &msg) {
+                       isx_road *d_roads, std::string &msg, bool carry) {
   auto cuda = [&](cudaError_t e, const char *what) -> int {
     if (e == cudaSuccess) return ISX_OK;
     msg = std::string(what) + ": " + cudaGetErrorString(e);
@@ -523,8 +539,8 @@ int road_enqueue_batch(isx_road_handle h, cudaStream_t caller, int n, const floa
       h->d_points, h->d_counters + B, h->d_tab, h->d_tab + h->numangle, h->d_accum, h->numangle, h->numrho, total);
   select_kernel<<<dim3((h->numangle * h->numrho + 255) / 256, n), 256, 0, s>>>(h->d_accum, h->d_cells, h->d_sel,
                                                                                h->numangle, h->numrho, kHoughThreshold);
-  resolve_kernel<<<1, 32, 0, s>>>(h->d_sel, h->d_cells, h->d_state, fallback ? 1 : 0, h->seed, n, d_estimates,
-                                  d_roads_out, d_roads);
+  resolve_kernel<<<1, 32, 0, s>>>(h->d_sel, h->d_cells, h->d_state, fallback ? 1 : 0, carry ? 1 : 0, h->seed, n,
+                                  d_estimates, d_roads_out, d_roads);
   g_launch_count += 5;
   ROAD_ENQ(cudaGetLastError());
   ROAD_ENQ(cudaEventRecord(h->ev_done, s));
@@ -532,6 +548,14 @@ int road_enqueue_batch(isx_road_handle h, cudaStream_t caller, int n, const floa
 #undef ROAD_ENQ
   h->last_n = n;
   return ISX_OK;
+}
+
+void launch_pull_road_tables(const float *src_ground, float *dst_ground, size_t ground_floats, const int *src_vhor,
+                             int *dst_vhor, int n, cudaStream_t s) {
+  const int blocks = (int)std::min<size_t>((ground_floats + 255) / 256, 512);
+  pull_tables_kernel<<<blocks < 1 ? 1 : blocks, 256, 0, s>>>(src_ground, dst_ground, ground_floats, src_vhor, dst_vhor,
+                                                            n);
+  g_launch_count++;
 }
 
 }  // namespace isx

@@ -3,7 +3,7 @@
 "It took an average of ... fps" line beside bench.py's e2e number.  ISX_ALLOW_1024=1 lifts the reference's
 rows < 1024 guard of the loader (apps/run_cityscapes.cu:129-134) for the BASELINE size.
 
-  python tools/runner_bench.py [--frames 128] [--mode unary|pairwise] [--batch 64] [--gpus 1]
+  python tools/runner_bench.py [--frames 128] [--mode unary|pairwise] [--batch 64] [--gpus 1] [--road-on-device]
 """
 import argparse, json, os, re, subprocess, sys, tempfile, time
 import numpy as np
@@ -19,6 +19,7 @@ ap.add_argument("--replicate", type=int, default=10, help="the timed call stream
 ap.add_argument("--mode", default="unary")
 ap.add_argument("--batch", type=int, default=64)
 ap.add_argument("--gpus", type=int, default=1)
+ap.add_argument("--road-on-device", action="store_true", help="estimate the roads inside the timed pool call")
 a = ap.parse_args()
 rows, cols = 1024, 2048
 d = tempfile.mkdtemp(prefix="isx_ds_")
@@ -38,13 +39,14 @@ pre = synth.preset(a.mode, rows, cols, 8)
 pairwise = int(a.mode == "pairwise")
 args = [os.path.join(ROOT, "apps", "cityscapes_runner"), d, "128", repr(pre["segmentation_weight"]), repr(pre["instance_weight"]),
         repr(pre["disparity_weight"]), str(pairwise), "8", repr(pre["eps"]), str(pre["min_pts"]), str(pre["size_filter"]),
-        "--batch", str(a.batch), "--gpus", str(a.gpus), "--replicate", str(a.replicate)]
+        "--batch", str(a.batch), "--gpus", str(a.gpus), "--replicate", str(a.replicate)] + \
+       (["--road-on-device"] if a.road_on_device else [])
 env = dict(os.environ, ISX_ALLOW_1024="1")
 p = subprocess.run(args, capture_output=True, text=True, env=env)
 line = [l for l in p.stdout.splitlines() if l.startswith("It took an average")]
 done = [l for l in p.stdout.splitlines() if l.startswith("Done.")]
 m = re.search(r"([0-9.]+) milliseconds, ([0-9.]+) fps", line[0]) if line else None
-print(json.dumps(dict(mode=a.mode, frames=a.frames, replicate=a.replicate, batch=a.batch, gpus=a.gpus, runner_fps=float(m.group(2)) if m else None,
+print(json.dumps(dict(mode=a.mode, road_on_device=a.road_on_device, frames=a.frames, replicate=a.replicate, batch=a.batch, gpus=a.gpus, runner_fps=float(m.group(2)) if m else None,
                       runner_ms_per_frame=float(m.group(1)) if m else None, done_line=done[-1] if done else None,
                       stixels_files=len(os.listdir(os.path.join(d, "stixels"))), rc=p.returncode, stderr=p.stderr[-300:])))
 subprocess.run(["rm", "-rf", d])
