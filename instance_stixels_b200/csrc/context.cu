@@ -147,8 +147,6 @@ struct isx_context {
   isx_road_estimate *batch_est[isx::kResultSets] = {};    // the caller's arrays the wait fills (estimated roads)
   isx_road *batch_roads[isx::kResultSets] = {};
   bool batch_direct[isx::kResultSets] = {};               // ... or that the device has already filled (mapped memory)
-  isx_section *direct_sections = nullptr;               // device address of the caller's array for the batch being enqueued
-  bool results_stay_on_device = false;                  // set while a device batch is enqueued
   int last_waited_set = -1;                           // result set of the batch waited for last (isx_wait_batch_packed)
   unsigned long long submitted = 0, waited = 0;       // tickets: batches [waited, submitted) are in flight
   unsigned long long dp_units_pairwise = 0;           // ... of which in pairwise mode (never pruned)
@@ -160,8 +158,9 @@ struct isx_context {
   std::mutex road_cache_mutex;
   isx_road *h_stage_roads = nullptr;  // [kStageSlots][chunk] pinned: the device-estimated roads of a staged chunk
   isx_road *d_batch_roads = nullptr;  // [max_batch] roads of the last isx_compute_batch_device_road batch
-  bool last_roads_device = false;     // the roads of the last batch were estimated on the device: the export reads
-  const isx_road *last_roads_dev = nullptr;   // them here (d_batch_roads or rs[cur].m_roads) instead of last_roads
+  // the roads of the last batch were estimated on the device: the export reads them here (d_batch_roads or
+  // rs[cur].m_roads) instead of last_roads
+  const isx_road *last_roads_dev = nullptr;
   // device addresses of the pinned staging (h_ground, h_vhor, h_stage_roads), taken on the first host batch with
   // estimated roads: its road step writes the roads there and pull_tables_kernel reads the tables from there
   float *m_ground = nullptr;
@@ -290,6 +289,50 @@ static void fill_kparams(isx_context *c) {
   k.prune_pairwise = (e2 && std::atoi(e2) == 0) ? 0 : 1;
 }
 
+// Per-chunk road estimation of a host batch (isx_submit_batch_host_road, the frame pool).
+struct HostRoad {
+  isx_road_handle road = nullptr;
+  const isx_road *fallback = nullptr;   // the seed: given to the road step of the first chunk of the call only
+  bool carry = true;                    // false: the frame pool's per-frame rule
+};
+
+// Host inputs of one batch: the reference's types (float disparity, int32 segmentation with its padding), or the
+// narrow forms of the isx_*_u16 entry points.
+struct HostInputs {
+  const float *disparity = nullptr;
+  const int32_t *segmentation = nullptr;
+  const uint16_t *disparity16 = nullptr;
+  float scale = 0.0f;
+  const int16_t *segmentation16 = nullptr;
+  HostInputs() = default;
+  HostInputs(const float *d, const int32_t *s) : disparity(d), segmentation(s) {}
+  HostInputs(const uint16_t *d, float sc, const int16_t *s) : disparity16(d), scale(sc), segmentation16(s) {}
+  bool narrow() const { return disparity16 != nullptr; }
+};
+
+// Where the results of a batch go besides its result set rs[cur].
+struct ResultDest {
+  // device batches leave their results on the device: only the counts and descriptors cross the host link, a later
+  // fetch reads the padded device arrays (the frames are flagged like overflows)
+  bool stay_on_device = false;
+  isx_section *direct_sections = nullptr;   // device address of the caller's pinned Section array (device_view_of)
+};
+
+// One batch of enqueue_batch.
+struct Batch {
+  // inputs: [n] frames in device memory, or (d_disparity null) in host memory, copied chunk by chunk
+  const float *d_disparity = nullptr;
+  const int32_t *d_segmentation = nullptr;
+  HostInputs host;
+  // roads: given on the host (`roads`), or estimated on the device into d_roads [n] -- for the whole batch before
+  // the chunk loop, or (estimate.road set) per chunk, with what the road step returned in d_estimates [n]
+  const isx_road *roads = nullptr;
+  isx_road *d_roads = nullptr;
+  HostRoad estimate;
+  isx_road_estimate *d_estimates = nullptr;
+  ResultDest out;
+};
+
 // The ground tables [3][H] of road `r` into `dst`.
 static void copy_road_tables(isx_context *c, const isx_road &r, float *dst) {
   std::lock_guard<std::mutex> lock(c->road_cache_mutex);
@@ -302,6 +345,17 @@ static void copy_road_tables(isx_context *c, const isx_road &r, float *dst) {
     it = c->road_cache.emplace(key, std::move(t)).first;
   }
   std::memcpy(dst, it->second.data(), sizeof(float) * 3 * c->model.rows);
+}
+
+// The ground tables and flipped horizon rows of `n` roads into staging buffer `stage`.
+static void fill_stage(isx_context *c, int stage, const isx_road *roads, int n) {
+  const int H = c->kp.rows;
+  float *hg = c->h_ground + (size_t)stage * c->chunk * 3 * H;
+  int *hv = c->h_vhor + (size_t)stage * c->chunk;
+  for (int i = 0; i < n; i++) {
+    copy_road_tables(c, roads[i], hg + (size_t)i * 3 * H);
+    hv[i] = H - roads[i].vhor - 1;  // Stixels.cu:377
+  }
 }
 
 // The staged road tables of `n` frames -> the next slot of the road ring, on `st`.  Returns the slot or an error.
@@ -318,27 +372,14 @@ static int send_road_tables(isx_context *c, int stage, int n, cudaStream_t st) {
   return rslot;
 }
 
-// Enqueue the kernel sequence for `n` frames whose inputs are at d_disp/d_seg.
-// `slot` selects the pinned ground-table staging half and the ChunkSet; results
-// land at frame offset `first` of the per-batch result arrays.
-//
-// Three streams: join -> tables -> LUT on s_tables, the DP on s_compute; backtracking, candidate
-// collection, grouping and packing (short, latency-bound launches) on s_emit, so
-// that they overlap the next chunk's DP.
-// The per-frame road tables of a chunk (Stixels.cu:463-493: three blocking copies per frame in the reference) go
-// through a pinned staging buffer to the next slot of the road ring on stream `st`, behind the emission that last read
-// that slot (kRoadSlots chunks ago).  Returns the slot (>= 0) or an error (< 0).
+// Roads given on the host: the per-frame road tables of a chunk (Stixels.cu:463-493: three blocking copies per frame
+// in the reference) go through a pinned staging buffer to the next slot of the road ring on stream `st`, behind the
+// emission that last read that slot (kRoadSlots chunks ago).  Returns the slot (>= 0) or an error (< 0).
 static int stage_road_tables(isx_context *c, const isx_road *roads, int n, cudaStream_t st) {
-  const int H = c->kp.rows;
   const int stage = (int)(c->stage_next++ % kStageSlots);
   // the copy that read this staging buffer kStageSlots chunks ago must be done (a never-recorded event is complete)
   ISX_TRY(c, cudaEventSynchronize(c->ev_stage_done[stage]));
-  float *hg = c->h_ground + (size_t)stage * c->chunk * 3 * H;
-  int *hv = c->h_vhor + (size_t)stage * c->chunk;
-  for (int i = 0; i < n; i++) {
-    copy_road_tables(c, roads[i], hg + (size_t)i * 3 * H);
-    hv[i] = H - roads[i].vhor - 1;  // Stixels.cu:377
-  }
+  fill_stage(c, stage, roads, n);
   return send_road_tables(c, stage, n, st);
 }
 
@@ -359,14 +400,7 @@ static void CUDART_CB fill_stage_from_roads(void *arg) {
   delete static_cast<StageFill *>(arg);
   isx_context *c = p.c;
   const auto t0 = std::chrono::steady_clock::now();
-  const int H = c->kp.rows;
-  const isx_road *roads = c->h_stage_roads + (size_t)p.stage * c->chunk;
-  float *hg = c->h_ground + (size_t)p.stage * c->chunk * 3 * H;
-  int *hv = c->h_vhor + (size_t)p.stage * c->chunk;
-  for (int i = 0; i < p.n; i++) {
-    copy_road_tables(c, roads[i], hg + (size_t)i * 3 * H);
-    hv[i] = H - roads[i].vhor - 1;  // Stixels.cu:377
-  }
+  fill_stage(c, p.stage, c->h_stage_roads + (size_t)p.stage * c->chunk, p.n);
   if (p.timed) {
     c->host_fill_ns += std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count();
     c->host_fill_calls++;
@@ -389,22 +423,16 @@ static int stage_device_road_tables(isx_context *c, const isx_road *d_roads, int
 // pull_tables_kernel moves the tables into the road ring with loads of the SMs.  Everything is ordered on s_tables, the
 // copy stream never waits for any of it, and the calling thread does not wait either.  Returns the ring slot or an
 // error.
-struct HostRoad {
-  isx_road_handle road = nullptr;
-  const isx_road *fallback = nullptr;   // the seed: given to the road step of the first chunk of the call only
-  bool carry = true;                    // false: the frame pool's per-frame rule
-};
-
-static int stage_estimated_road_tables(isx_context *c, const HostRoad &hr, const isx_road *fallback, int n,
-                                       const float *d_disp, isx_road_estimate *m_est, isx_road *m_roads) {
+static int stage_estimated_road_tables(isx_context *c, const Batch &b, int first, int n, const float *d_disp) {
   const int H = c->kp.rows;
   cudaStream_t st = c->s_tables;
   const int stage = (int)(c->stage_next++ % kStageSlots);
   // the staging slot is free once the pull that last read it is done (the road stream is ordered behind st)
   ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_stage_done[stage], 0));
   std::string msg;
-  if (int rc = road_enqueue_batch(hr.road, st, n, d_disp, fallback, m_est, m_roads,
-                                  c->m_stage_roads + (size_t)stage * c->chunk, msg, hr.carry))
+  if (int rc = road_enqueue_batch(b.estimate.road, st, n, d_disp, first == 0 ? b.estimate.fallback : nullptr,
+                                  b.d_estimates + first, b.d_roads + first, c->m_stage_roads + (size_t)stage * c->chunk,
+                                  msg, b.estimate.carry))
     return fail(c, rc, msg);
   ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{c, stage, n, c->profiling}));
   const int rslot = (int)(c->road_next++ % kRoadSlots);
@@ -417,15 +445,42 @@ static int stage_estimated_road_tables(isx_context *c, const HostRoad &hr, const
   return rslot;
 }
 
-// `road_slot` >= 0: the caller has already copied the road tables of the chunk into that slot of the ring (host
-// batches send them on the copy stream IN FRONT of the chunk's images: as a copy on the compute stream they would
-// queue on the copy engine behind the next chunk's images -- several milliseconds of an idle GPU per chunk, measured
-// with isx_get_chunk_trace).
-static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const float *d_disp,
-                         const int32_t *d_seg, const isx_road *roads, int slot, int road_slot = -1) {
+// The intermediates of the chunk in set `slot` with its road tables in slot `road_slot` of the road ring.
+static BatchBuffers chunk_buffers(const isx_context *c, int slot, int road_slot) {
+  const isx_context::ChunkSet &cs = c->sets[slot];
+  const isx_context::RoadSlot &rd = c->roads[road_slot];
+  BatchBuffers b = c->buf;
+  b.ground = rd.ground; b.vhor = rd.vhor; b.stat = cs.stat;
+  b.records_b = cs.records_b; b.dp = cs.dp; b.pm = cs.pm;
+  b.joined = cs.joined; b.object_lut = cs.object_lut; b.col_flags = cs.col_flags;
+  b.error_flag = cs.err;
+  return b;
+}
+
+// Profiling (isx_set_profiling): records the next event of `pool` on `st`, creating it on first use.
+static void record_prof_event(isx_context *c, std::vector<cudaEvent_t> &pool, size_t &used, cudaStream_t st) {
+  if (!c->profiling) return;
+  if (used >= pool.size()) {
+    cudaEvent_t e;
+    cudaEventCreate(&e);
+    pool.push_back(e);
+  }
+  cudaEventRecord(pool[used++], st);
+}
+
+// Enqueue the kernel sequence for `n` frames whose inputs are at d_disp/d_seg.  `slot` selects the ChunkSet; results
+// land at frame offset `first` of result set rs[cur], and in `out`.
+//
+// Three streams: join -> tables -> LUT on s_tables, the DP on s_compute; backtracking, candidate collection, grouping
+// and packing (short, latency-bound launches) on s_emit, so that they overlap the next chunk's DP.
+// `road_slot` >= 0: the caller has already staged the road tables of the chunk into that slot of the ring (host
+// batches send given roads on the copy stream IN FRONT of the chunk's images: as a copy on the compute stream they
+// would queue on the copy engine behind the next chunk's images -- several milliseconds of an idle GPU per chunk,
+// measured with isx_get_chunk_trace).  Otherwise the given `roads` are staged here, behind the waits for the set.
+static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const float *d_disp, const int32_t *d_seg,
+                         const isx_road *roads, int slot, int road_slot, const ResultDest &out) {
   const KParams &kp = c->kp;
   const int H = kp.rows, C = kp.realcols;
-  const isx_context::ChunkSet &cs = c->sets[slot];
   cudaStream_t st = c->s_tables, s = c->s_compute, se = c->s_emit;
   // the emission of the chunk that used this set two chunks ago must be done with it (it follows that chunk's DP)
   ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_emit_done[slot], 0));
@@ -435,29 +490,16 @@ static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const 
     road_slot = stage_road_tables(c, roads, n, st);
     if (road_slot < 0) return road_slot;
   }
-  const isx_context::RoadSlot &rd = c->roads[road_slot];
-  ISX_TRY(c, cudaMemsetAsync(cs.err, 0, sizeof(int) * n, st));  // the error words of THIS chunk's frames
+  BatchBuffers b = chunk_buffers(c, slot, road_slot);
+  ISX_TRY(c, cudaMemsetAsync(b.error_flag, 0, sizeof(int) * n, st));  // the error words of THIS chunk's frames
   isx_context::ResultSet &R = c->rs[c->cur];
-  BatchBuffers b = c->buf;
-  b.ground = rd.ground; b.vhor = rd.vhor; b.stat = cs.stat;
-  b.records_b = cs.records_b; b.dp = cs.dp; b.pm = cs.pm;
-  b.joined = cs.joined; b.object_lut = cs.object_lut; b.col_flags = cs.col_flags;
-  b.error_flag = cs.err;
   b.disparity = d_disp;
   b.segmentation = d_seg;
   b.sections = R.d_sections + (size_t)first * C * kMaxSections;
   b.n_sections = R.d_nsections + (size_t)first * C;
   // profiling events per chunk: 0 join | 1 frame tables | 2 column tables + LUT | 3 end (s_tables); 4 dp | 5 dp end
   //                             (s_compute); 6 backtrack + collect | 7 grouping + pack | 8 end (s_emit)
-  auto mark = [&](cudaStream_t st) {
-    if (!c->profiling) return;
-    if (c->prof_used >= c->prof_events.size()) {
-      cudaEvent_t e;
-      cudaEventCreate(&e);
-      c->prof_events.push_back(e);
-    }
-    cudaEventRecord(c->prof_events[c->prof_used++], st);
-  };
+  auto mark = [&](cudaStream_t st) { record_prof_event(c, c->prof_events, c->prof_used, st); };
   mark(st);
   launch_join_columns(kp, b, n, st);
   mark(st);
@@ -488,20 +530,18 @@ static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const 
     PackArgs a;
     a.sections = b.sections; a.n_sections = b.n_sections;
     a.cand_count = b.cand_count; a.cand_idx = b.cand_idx; a.cand_label = b.cand_label;
-    a.err = cs.err; a.col_offset = b.pack_offset;
+    a.err = b.error_flag; a.col_offset = b.pack_offset;
     a.inst_out = R.d_inst + (size_t)first * c->inst_cap; a.inst_count_out = R.d_inst_count + first;
     a.inst_cap = c->inst_cap; a.cursors = R.d_cursors;
-    a.h_padded = c->direct_sections ? c->direct_sections + (size_t)first * C * kMaxSections : nullptr;
-    // a device batch leaves its results on the device (isx_compute_batch_device): only the counts and descriptors
-    // cross the host link, a later fetch reads the padded device arrays (the frames are flagged like overflows)
-    a.h_sections = R.m_sections; a.h_sections_cap = c->results_stay_on_device ? 0 : R.sections_cap;
-    a.h_inst = R.m_inst; a.h_inst_cap = c->results_stay_on_device ? 0 : R.inst_cap;
+    a.h_padded = out.direct_sections ? out.direct_sections + (size_t)first * C * kMaxSections : nullptr;
+    a.h_sections = R.m_sections; a.h_sections_cap = out.stay_on_device ? 0 : R.sections_cap;
+    a.h_inst = R.m_inst; a.h_inst_cap = out.stay_on_device ? 0 : R.inst_cap;
     a.h_counts = R.m_counts + (size_t)first * C; a.h_frames = R.m_frames + first;
     launch_pack(kp, a, n, se);
   }
   mark(se);
   ISX_TRY(c, cudaEventRecord(c->ev_emit_done[slot], se));
-  ISX_TRY(c, cudaEventRecord(rd.ev_free, se));
+  ISX_TRY(c, cudaEventRecord(c->roads[road_slot].ev_free, se));
   ISX_TRY(c, cudaGetLastError());
   c->last_chunk_first = first;
   c->last_chunk_n = n;
@@ -609,6 +649,117 @@ static int check_ready(isx_context *c) {
   if (!c->initialized) return fail(c, ISX_ERR_NOT_INITIALIZED, "Initialize() has not been called");
   cudaError_t e = cudaSetDevice(c->device);
   if (e != cudaSuccess) return fail(c, ISX_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+  return ISX_OK;
+}
+
+static size_t narrow_seg_elems(const isx_context *c) {
+  const size_t used = (size_t)(c->kp.rows + kDownsample - 1) / kDownsample;
+  return (size_t)c->kp.realcols * c->kp.n_channels * (used < (size_t)c->kp.hs2 ? used : (size_t)c->kp.hs2);
+}
+
+static int ensure_narrow_staging(isx_handle h) {
+  if (h->d_in_disp16[0]) return ISX_OK;
+  const size_t hw = (size_t)h->kp.rows * h->kp.cols, ch = h->chunk;
+  for (int i = 0; i < 2; i++) {
+    ISX_TRY(h, dev_alloc(h, &h->d_in_disp16[i], ch * hw));
+    ISX_TRY(h, dev_alloc(h, &h->d_in_seg16[i], ch * narrow_seg_elems(h)));
+  }
+  return ISX_OK;
+}
+
+// The chunks of one batch into result set rs[cur], kernels on s_tables / s_compute / s_emit; a host batch's input
+// copies run on s_h2d and its results reach host memory through pack_results_kernel (no D2H copies).  Blocks the
+// caller only for the reuse of an input slot (two chunks behind).
+// `caller_waits`: a synchronous host call -- the kernels of the last chunk run with nothing beside them while the
+// caller waits, so the tail goes in quarter pieces like the head.
+static int enqueue_batch(isx_handle h, int pairwise, int n, const Batch &b, bool caller_waits) {
+  const HostInputs &in = b.host;
+  const bool host = b.d_disparity == nullptr;
+  const size_t hw = (size_t)h->kp.rows * h->kp.cols, se = seg_elems(h), se16 = narrow_seg_elems(h);
+  if (in.narrow()) {
+    if (hw % 8 != 0) return fail(h, ISX_ERR_UNSUPPORTED, "the uint16 disparity path needs rows*cols to be a multiple of 8");
+    if (int rc = ensure_narrow_staging(h)) return rc;
+  }
+  if (int rc = begin_batch(h)) return rc;
+  // The slots keep alternating across batches, so that the first copy of a pipelined batch only waits for the
+  // second-to-last chunk of the batch before it.
+  int slot = h->host_slot;
+  int cn = 0;
+  const int chunk = pairwise ? h->chunk : h->chunk_unary;
+  h->last_launch_frames = chunk;
+  const bool pipeline_idle = h->submitted == h->waited;
+  for (int first = 0; first < n; first += cn) {
+    cn = (n - first) < chunk ? (n - first) : chunk;
+    // Where each road source is staged is part of its timing: given roads go in front of a host chunk's images (on
+    // the copy stream) or, for device inputs, into enqueue_chunk behind its waits; estimated roads go on s_tables
+    // once the chunk's inputs are there.
+    int road_slot = -1;
+    const float *d_disp;
+    const int32_t *d_seg;
+    if (host) {
+      // Nothing is running: no kernel hides the input copies, so the first `chunk` frames go in quarter pieces and
+      // the kernels of a piece run under the copy of the next (a synchronous 64-frame pairwise call: copy 13 ms +
+      // tables and DP of the last piece instead of copy + tables and DP of all 64 frames); likewise the last `chunk`
+      // frames of a call whose caller waits.  The shorter launches cost the DP a few per cent -- in between, and once
+      // the pipeline of a streaming caller is filled, launches are whole chunks.
+      const bool head = pipeline_idle && first < chunk, tail = caller_waits && n - first <= chunk;
+      if ((head || tail) && chunk >= 32) cn = cn < chunk / 4 ? cn : chunk / 4;
+      // H2D of this chunk on the copy stream, once the table build that last read this input slot is done (a
+      // device-side wait: the host thread runs ahead)
+      ISX_TRY(h, cudaStreamWaitEvent(h->s_h2d, h->ev_in_free[slot], 0));
+      record_prof_event(h, h->prof_h2d, h->prof_h2d_used, h->s_h2d);
+      if (b.roads) {
+        road_slot = stage_road_tables(h, b.roads + first, cn, h->s_h2d);
+        if (road_slot < 0) return road_slot;
+      }
+      if (in.narrow()) {
+        ISX_TRY(h, cudaMemcpyAsync(h->d_in_disp16[slot], in.disparity16 + first * hw, sizeof(uint16_t) * hw * cn,
+                                   cudaMemcpyHostToDevice, h->s_h2d));
+        ISX_TRY(h, cudaMemcpyAsync(h->d_in_seg16[slot], in.segmentation16 + first * se16, sizeof(int16_t) * se16 * cn,
+                                   cudaMemcpyHostToDevice, h->s_h2d));
+      } else {
+        ISX_TRY(h, cudaMemcpyAsync(h->d_in_disp[slot], in.disparity + first * hw, sizeof(float) * hw * cn,
+                                   cudaMemcpyHostToDevice, h->s_h2d));
+        // Only the first rows/8 entries of every [rows_power2_segmentation] channel row are ever read
+        // (StixelsKernels.cu:393-405, 462-468 index v/8 with v < rows); the zero padding of FlipAndPad does not
+        // travel: a 2-D copy of the used part, the rest of the staging buffer stays zero from isx_initialize.
+        const size_t hs2 = (size_t)h->kp.hs2;
+        size_t used = (size_t)(h->kp.rows + kDownsample - 1) / kDownsample;
+        used = used < hs2 ? used : hs2;
+        ISX_TRY(h, cudaMemcpy2DAsync(h->d_in_seg[slot], hs2 * sizeof(int32_t), in.segmentation + first * se,
+                                     hs2 * sizeof(int32_t), used * sizeof(int32_t), (se / hs2) * cn,
+                                     cudaMemcpyHostToDevice, h->s_h2d));
+      }
+      record_prof_event(h, h->prof_h2d, h->prof_h2d_used, h->s_h2d);
+      ISX_TRY(h, cudaEventRecord(h->ev_in_ready[slot], h->s_h2d));
+      ISX_TRY(h, cudaStreamWaitEvent(h->s_tables, h->ev_in_ready[slot], 0));
+      if (in.narrow())
+        launch_widen_inputs(h->kp, h->d_in_disp16[slot], in.scale, h->d_in_seg16[slot], h->d_in_disp[slot],
+                            h->d_in_seg[slot], cn, h->s_tables);
+      d_disp = h->d_in_disp[slot];
+      d_seg = h->d_in_seg[slot];
+    } else {
+      d_disp = b.d_disparity + first * hw;
+      d_seg = b.d_segmentation + first * se;
+    }
+    if (!b.roads) {
+      road_slot = b.estimate.road ? stage_estimated_road_tables(h, b, first, cn, d_disp)
+                                  : stage_device_road_tables(h, b.d_roads + first, cn, h->s_tables);
+      if (road_slot < 0) return road_slot;
+    }
+    if (int rc = enqueue_chunk(h, pairwise != 0, first, cn, d_disp, d_seg, b.roads ? b.roads + first : nullptr, slot,
+                               road_slot, b.out))
+      return rc;
+    ISX_TRY(h, cudaEventRecord(h->ev_in_free[slot], h->s_tables));   // the inputs are read by the table build only
+    slot ^= 1;
+  }
+  h->host_slot = slot;
+  h->emit_join_pending = true;  // joined lazily: isx_flush / isx_synchronize / any result access
+  // the batch's results replace the last ones: the export reads its roads
+  h->last_batch = n;
+  if (b.roads) h->last_roads.assign(b.roads, b.roads + n);
+  else h->last_roads.clear();
+  h->last_roads_dev = b.d_roads;
   return ISX_OK;
 }
 
@@ -908,7 +1059,6 @@ int isx_finish(isx_handle h) {
   cudaFreeHost(h->h_stage_roads);
   h->h_stage_roads = nullptr;
   h->d_batch_roads = nullptr;
-  h->last_roads_device = false;
   h->last_roads_dev = nullptr;
   h->m_ground = nullptr;
   h->m_vhor = nullptr;
@@ -1114,18 +1264,16 @@ int isx_compute(isx_handle h, int pairwise, isx_section *sections, isx_frame_met
   if (int rc = no_batches_in_flight(h)) return rc;
   const int32_t *seg = d_segmentation_local ? d_segmentation_local : h->d_single_seg;
   if (int rc = begin_batch(h)) return rc;
-  h->direct_sections = device_view_of(sections);
-  const bool direct = h->direct_sections != nullptr;
-  const int erc = enqueue_chunk(h, pairwise != 0, 0, 1, h->d_single_disp, seg, &h->single_road, 0);
-  h->direct_sections = nullptr;
-  if (erc) return erc;
+  ResultDest out;
+  out.direct_sections = device_view_of(sections);
+  if (int rc = enqueue_chunk(h, pairwise != 0, 0, 1, h->d_single_disp, seg, &h->single_road, 0, -1, out)) return rc;
   ISX_TRY(h, cudaEventRecord(h->ev_in_free[0], h->s_tables));
   if (int rc = join_emit_stream(h)) return rc;
   h->last_batch = 1;
   h->last_roads.assign(1, h->single_road);
-  h->last_roads_device = false;
+  h->last_roads_dev = nullptr;
   if (int rc = wait_last_emission(h)) return rc;
-  if (int rc = deliver(h, h->rs[h->cur], 1, sections, nullptr, 0, nullptr, direct)) return rc;
+  if (int rc = deliver(h, h->rs[h->cur], 1, sections, nullptr, 0, nullptr, out.direct_sections != nullptr)) return rc;
   if (meta) {
     meta->rows = h->kp.rows; meta->cols = h->kp.cols; meta->realcols = h->kp.realcols;
     meta->max_sections = kMaxSections; meta->max_dis = h->kp.max_dis; meta->column_step = h->kp.column_step;
@@ -1166,27 +1314,12 @@ int isx_compute_batch_device(isx_handle h, int pairwise, int n, const float *d_d
   if (int rc = no_batches_in_flight(h)) return rc;
   if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
   if (!d_disparity || !d_segmentation || !roads) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  const size_t hw = (size_t)h->kp.rows * h->kp.cols, se = seg_elems(h);
-  int slot = h->host_slot;  // keeps alternating across batches (see enqueue_host_batch)
-  if (int rc = begin_batch(h)) return rc;
-  const int chunk = pairwise ? h->chunk : h->chunk_unary;
-  h->last_launch_frames = chunk;
-  for (int first = 0; first < n; first += chunk) {
-    const int cn = (n - first) < chunk ? (n - first) : chunk;
-    h->results_stay_on_device = true;
-    const int erc = enqueue_chunk(h, pairwise != 0, first, cn, d_disparity + first * hw, d_segmentation + first * se,
-                                  roads + first, slot);
-    h->results_stay_on_device = false;
-    if (erc) return erc;
-    ISX_TRY(h, cudaEventRecord(h->ev_in_free[slot], h->s_tables));
-    slot ^= 1;
-  }
-  h->host_slot = slot;
-  h->emit_join_pending = true;  // joined lazily: isx_flush / isx_synchronize / any result access
-  h->last_batch = n;
-  h->last_roads.assign(roads, roads + n);
-  h->last_roads_device = false;
-  return ISX_OK;
+  Batch b;
+  b.d_disparity = d_disparity;
+  b.d_segmentation = d_segmentation;
+  b.roads = roads;
+  b.out.stay_on_device = true;
+  return enqueue_batch(h, pairwise, n, b, /*caller_waits=*/false);
 }
 
 int isx_compute_batch_device_road(isx_handle h, isx_road_handle road, int pairwise, int n, const float *d_disparity,
@@ -1202,31 +1335,12 @@ int isx_compute_batch_device_road(isx_handle h, isx_road_handle road, int pairwi
   if (int rc = road_enqueue_batch(road, h->s_tables, n, d_disparity, fallback, d_estimates, d_roads, h->d_batch_roads,
                                   msg))
     return fail(h, rc, msg);
-  const size_t hw = (size_t)h->kp.rows * h->kp.cols, se = seg_elems(h);
-  int slot = h->host_slot;
-  if (int rc = begin_batch(h)) return rc;
-  const int chunk = pairwise ? h->chunk : h->chunk_unary;
-  h->last_launch_frames = chunk;
-  // the batch's results replace the last ones from here on: the export reads the device roads
-  h->last_batch = n;
-  h->last_roads.clear();
-  h->last_roads_device = true;
-  h->last_roads_dev = h->d_batch_roads;
-  for (int first = 0; first < n; first += chunk) {
-    const int cn = (n - first) < chunk ? (n - first) : chunk;
-    const int road_slot = stage_device_road_tables(h, h->d_batch_roads + first, cn, h->s_tables);
-    if (road_slot < 0) return road_slot;
-    h->results_stay_on_device = true;
-    const int erc = enqueue_chunk(h, pairwise != 0, first, cn, d_disparity + first * hw, d_segmentation + first * se,
-                                  nullptr, slot, road_slot);
-    h->results_stay_on_device = false;
-    if (erc) return erc;
-    ISX_TRY(h, cudaEventRecord(h->ev_in_free[slot], h->s_tables));
-    slot ^= 1;
-  }
-  h->host_slot = slot;
-  h->emit_join_pending = true;
-  return ISX_OK;
+  Batch b;
+  b.d_disparity = d_disparity;
+  b.d_segmentation = d_segmentation;
+  b.d_roads = h->d_batch_roads;
+  b.out.stay_on_device = true;
+  return enqueue_batch(h, pairwise, n, b, /*caller_waits=*/false);
 }
 
 int isx_flush(isx_handle h) {
@@ -1251,129 +1365,6 @@ int isx_fetch_batch_results(isx_handle h, int n, isx_section *sections, isx_inst
   return deliver(h, h->rs[h->cur], n, sections, instances, instances_capacity, instance_offsets);
 }
 
-// Host inputs of one batch: the reference's types (float disparity, int32 segmentation with its padding), or the
-// narrow forms of the isx_*_u16 entry points.
-struct HostInputs {
-  const float *disparity = nullptr;
-  const int32_t *segmentation = nullptr;
-  const uint16_t *disparity16 = nullptr;
-  float scale = 0.0f;
-  const int16_t *segmentation16 = nullptr;
-  bool narrow() const { return disparity16 != nullptr; }
-};
-
-static size_t narrow_seg_elems(const isx_context *c) {
-  const size_t used = (size_t)(c->kp.rows + kDownsample - 1) / kDownsample;
-  return (size_t)c->kp.realcols * c->kp.n_channels * (used < (size_t)c->kp.hs2 ? used : (size_t)c->kp.hs2);
-}
-
-static int ensure_narrow_staging(isx_handle h) {
-  if (h->d_in_disp16[0]) return ISX_OK;
-  const size_t hw = (size_t)h->kp.rows * h->kp.cols, ch = h->chunk;
-  for (int i = 0; i < 2; i++) {
-    ISX_TRY(h, dev_alloc(h, &h->d_in_disp16[i], ch * hw));
-    ISX_TRY(h, dev_alloc(h, &h->d_in_seg16[i], ch * narrow_seg_elems(h)));
-  }
-  return ISX_OK;
-}
-
-// The copy/kernel pipeline of one host batch: H2D on s_h2d, kernels on s_compute / s_emit; the results reach host
-// memory through pack_results_kernel (no D2H copies).  Blocks the caller only for the reuse of an input slot (two
-// chunks behind).
-// `caller_waits`: a synchronous call -- the kernels of the last chunk run with nothing beside them while the caller
-// waits, so the tail goes in quarter pieces like the head.
-// `hr`: estimate the roads on the device instead (then `roads` is null): the chunk's road step runs behind its images.
-static int enqueue_host_batch(isx_handle h, int pairwise, int n, const HostInputs &in, const isx_road *roads,
-                              bool caller_waits, const HostRoad *hr = nullptr) {
-  const size_t hw = (size_t)h->kp.rows * h->kp.cols, se = seg_elems(h), se16 = narrow_seg_elems(h);
-  if (in.narrow()) {
-    if (hw % 8 != 0) return fail(h, ISX_ERR_UNSUPPORTED, "the uint16 disparity path needs rows*cols to be a multiple of 8");
-    if (int rc = ensure_narrow_staging(h)) return rc;
-  }
-  if (int rc = begin_batch(h)) return rc;
-  // The slots keep alternating across batches, so that the first copy of a pipelined batch only waits for the
-  // second-to-last chunk of the batch before it.
-  int slot = h->host_slot;
-  int cn = 0;
-  const int chunk = pairwise ? h->chunk : h->chunk_unary;
-  h->last_launch_frames = chunk;
-  const bool pipeline_idle = h->submitted == h->waited;
-  for (int first = 0; first < n; first += cn) {
-    cn = (n - first) < chunk ? (n - first) : chunk;
-    // Nothing is running: no kernel hides the input copies, so the first `chunk` frames go in quarter pieces and the
-    // kernels of a piece run under the copy of the next (a synchronous 64-frame pairwise call: copy 13 ms + tables and
-    // DP of the last piece instead of copy + tables and DP of all 64 frames); likewise the last `chunk` frames of a
-    // call whose caller waits.  The shorter launches cost the DP a few per cent -- in between, and once the pipeline
-    // of a streaming caller is filled, launches are whole chunks.
-    const bool head = pipeline_idle && first < chunk, tail = caller_waits && n - first <= chunk;
-    if ((head || tail) && chunk >= 32) cn = cn < chunk / 4 ? cn : chunk / 4;
-    // H2D of this chunk on the copy stream, once the table build that last read this input slot is done (a
-    // device-side wait: the host thread runs ahead)
-    ISX_TRY(h, cudaStreamWaitEvent(h->s_h2d, h->ev_in_free[slot], 0));
-    auto mark_h2d = [&]() {
-      if (!h->profiling) return;
-      if (h->prof_h2d_used >= h->prof_h2d.size()) {
-        cudaEvent_t e;
-        cudaEventCreate(&e);
-        h->prof_h2d.push_back(e);
-      }
-      cudaEventRecord(h->prof_h2d[h->prof_h2d_used++], h->s_h2d);
-    };
-    mark_h2d();
-    int road_slot = -1;
-    if (!hr) {
-      road_slot = stage_road_tables(h, roads + first, cn, h->s_h2d);
-      if (road_slot < 0) return road_slot;
-    }
-    if (in.narrow()) {
-      ISX_TRY(h, cudaMemcpyAsync(h->d_in_disp16[slot], in.disparity16 + first * hw, sizeof(uint16_t) * hw * cn,
-                                 cudaMemcpyHostToDevice, h->s_h2d));
-      ISX_TRY(h, cudaMemcpyAsync(h->d_in_seg16[slot], in.segmentation16 + first * se16, sizeof(int16_t) * se16 * cn,
-                                 cudaMemcpyHostToDevice, h->s_h2d));
-    } else {
-      ISX_TRY(h, cudaMemcpyAsync(h->d_in_disp[slot], in.disparity + first * hw, sizeof(float) * hw * cn,
-                                 cudaMemcpyHostToDevice, h->s_h2d));
-      // Only the first rows/8 entries of every [rows_power2_segmentation] channel row are ever read
-      // (StixelsKernels.cu:393-405, 462-468 index v/8 with v < rows); the zero padding of FlipAndPad does not
-      // travel: a 2-D copy of the used part, the rest of the staging buffer stays zero from isx_initialize.
-      const size_t hs2 = (size_t)h->kp.hs2;
-      size_t used = (size_t)(h->kp.rows + kDownsample - 1) / kDownsample;
-      used = used < hs2 ? used : hs2;
-      ISX_TRY(h, cudaMemcpy2DAsync(h->d_in_seg[slot], hs2 * sizeof(int32_t), in.segmentation + first * se,
-                                   hs2 * sizeof(int32_t), used * sizeof(int32_t), (se / hs2) * cn,
-                                   cudaMemcpyHostToDevice, h->s_h2d));
-    }
-    mark_h2d();
-    ISX_TRY(h, cudaEventRecord(h->ev_in_ready[slot], h->s_h2d));
-    ISX_TRY(h, cudaStreamWaitEvent(h->s_tables, h->ev_in_ready[slot], 0));
-    if (in.narrow())
-      launch_widen_inputs(h->kp, h->d_in_disp16[slot], in.scale, h->d_in_seg16[slot], h->d_in_disp[slot],
-                          h->d_in_seg[slot], cn, h->s_tables);
-    if (hr) {
-      const isx_context::ResultSet &R = h->rs[h->cur];
-      road_slot = stage_estimated_road_tables(h, *hr, first == 0 ? hr->fallback : nullptr, cn, h->d_in_disp[slot],
-                                              R.m_est + first, R.m_roads + first);
-      if (road_slot < 0) return road_slot;
-    }
-    if (int rc = enqueue_chunk(h, pairwise != 0, first, cn, h->d_in_disp[slot], h->d_in_seg[slot],
-                               hr ? nullptr : roads + first, slot, road_slot))
-      return rc;
-    ISX_TRY(h, cudaEventRecord(h->ev_in_free[slot], h->s_tables));   // the inputs are read by the table build only
-    slot ^= 1;
-  }
-  h->host_slot = slot;
-  h->last_batch = n;
-  if (hr) {
-    h->last_roads.clear();
-    h->last_roads_device = true;
-    h->last_roads_dev = h->rs[h->cur].m_roads;
-  } else {
-    h->last_roads.assign(roads, roads + n);
-    h->last_roads_device = false;
-  }
-  return ISX_OK;
-}
-
 static int no_batches_in_flight(isx_handle h) {
   if (h->submitted != h->waited)
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "submitted batches are in flight: call isx_wait_batch_host first");
@@ -1387,35 +1378,31 @@ static int compute_batch_host(isx_handle h, int pairwise, int n, const HostInput
   if (int rc = no_batches_in_flight(h)) return rc;
   if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
   if (!roads) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  h->direct_sections = device_view_of(sections);
-  const bool direct = h->direct_sections != nullptr;
-  const int erc = enqueue_host_batch(h, pairwise, n, in, roads, /*caller_waits=*/true);
-  h->direct_sections = nullptr;
-  if (erc) return erc;
+  Batch b;
+  b.host = in;
+  b.roads = roads;
+  b.out.direct_sections = device_view_of(sections);
+  if (int rc = enqueue_batch(h, pairwise, n, b, /*caller_waits=*/true)) return rc;
   if (int rc = join_emit_stream(h)) return rc;
   if (int rc = wait_last_emission(h)) return rc;
-  return deliver(h, h->rs[h->cur], n, sections, instances, instances_capacity, instance_offsets, direct);
+  return deliver(h, h->rs[h->cur], n, sections, instances, instances_capacity, instance_offsets,
+                 b.out.direct_sections != nullptr);
 }
 
 int isx_compute_batch_host(isx_handle h, int pairwise, int n, const float *disparity, const int32_t *segmentation,
                            const isx_road *roads, isx_section *sections, isx_instance *instances,
                            int instances_capacity, int32_t *instance_offsets) {
   if (!disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  HostInputs in;
-  in.disparity = disparity;
-  in.segmentation = segmentation;
-  return compute_batch_host(h, pairwise, n, in, roads, sections, instances, instances_capacity, instance_offsets);
+  return compute_batch_host(h, pairwise, n, HostInputs(disparity, segmentation), roads, sections, instances,
+                            instances_capacity, instance_offsets);
 }
 
 int isx_compute_batch_host_u16(isx_handle h, int pairwise, int n, const uint16_t *disparity, float disparity_scale,
                                const int16_t *segmentation, const isx_road *roads, isx_section *sections,
                                isx_instance *instances, int instances_capacity, int32_t *instance_offsets) {
   if (!disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  HostInputs in;
-  in.disparity16 = disparity;
-  in.scale = disparity_scale;
-  in.segmentation16 = segmentation;
-  return compute_batch_host(h, pairwise, n, in, roads, sections, instances, instances_capacity, instance_offsets);
+  return compute_batch_host(h, pairwise, n, HostInputs(disparity, disparity_scale, segmentation), roads, sections,
+                            instances, instances_capacity, instance_offsets);
 }
 
 size_t isx_narrow_segmentation_elems(isx_handle h) { return (h && h->initialized) ? narrow_seg_elems(h) : 0; }
@@ -1450,13 +1437,18 @@ static int submit_batch_host(isx_handle h, int pairwise, int n, const HostInputs
   for (int i = 0; i < kResultSets; i++)
     if (!h->ev_batch_done[i]) ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_batch_done[i], cudaEventDisableTiming));
   h->cur = next;
-  h->direct_sections = device_view_of(sections);
-  const bool direct = h->direct_sections != nullptr;
-  const int erc = enqueue_host_batch(h, pairwise, n, in, roads, /*caller_waits=*/false, hr);
-  h->direct_sections = nullptr;
-  if (erc) return erc;
+  Batch b;
+  b.host = in;
+  b.roads = roads;
+  if (hr) {
+    b.estimate = *hr;
+    b.d_estimates = h->rs[next].m_est;
+    b.d_roads = h->rs[next].m_roads;
+  }
+  b.out.direct_sections = device_view_of(sections);
+  if (int rc = enqueue_batch(h, pairwise, n, b, /*caller_waits=*/false)) return rc;
   const int par = (int)(h->submitted % kResultSets);
-  h->batch_direct[par] = direct;
+  h->batch_direct[par] = b.out.direct_sections != nullptr;
   ISX_TRY(h, cudaEventRecord(h->ev_batch_done[par], h->s_emit));  // behind the packing of the last chunk
   h->batch_n[par] = n;
   h->batch_set[par] = h->cur;
@@ -1464,54 +1456,37 @@ static int submit_batch_host(isx_handle h, int pairwise, int n, const HostInputs
   h->batch_est[par] = hr ? estimates : nullptr;
   h->batch_roads[par] = hr ? roads_out : nullptr;
   h->submitted++;
-  h->emit_join_pending = true;  // isx_stream() itself has not been ordered behind the emission stream
   return ISX_OK;
 }
 
 int isx_submit_batch_host(isx_handle h, int pairwise, int n, const float *disparity, const int32_t *segmentation,
                           const isx_road *roads, isx_section *sections) {
   if (!disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  HostInputs in;
-  in.disparity = disparity;
-  in.segmentation = segmentation;
-  return submit_batch_host(h, pairwise, n, in, roads, sections);
+  return submit_batch_host(h, pairwise, n, HostInputs(disparity, segmentation), roads, sections);
 }
 
 int isx_submit_batch_host_u16(isx_handle h, int pairwise, int n, const uint16_t *disparity, float disparity_scale,
                               const int16_t *segmentation, const isx_road *roads, isx_section *sections) {
   if (!disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  HostInputs in;
-  in.disparity16 = disparity;
-  in.scale = disparity_scale;
-  in.segmentation16 = segmentation;
-  return submit_batch_host(h, pairwise, n, in, roads, sections);
+  return submit_batch_host(h, pairwise, n, HostInputs(disparity, disparity_scale, segmentation), roads, sections);
 }
 
 int isx_submit_batch_host_road(isx_handle h, isx_road_handle road, int pairwise, int n, const float *disparity,
                                const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
                                isx_road *roads_out, isx_section *sections) {
   if (!road || !disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  HostInputs in;
-  in.disparity = disparity;
-  in.segmentation = segmentation;
-  HostRoad hr;
-  hr.road = road;
-  hr.fallback = fallback;
-  return submit_batch_host(h, pairwise, n, in, nullptr, sections, &hr, estimates, roads_out);
+  const HostRoad hr{road, fallback};
+  return submit_batch_host(h, pairwise, n, HostInputs(disparity, segmentation), nullptr, sections, &hr, estimates,
+                           roads_out);
 }
 
 int isx_submit_batch_host_u16_road(isx_handle h, isx_road_handle road, int pairwise, int n, const uint16_t *disparity,
                                    float disparity_scale, const int16_t *segmentation, const isx_road *fallback,
                                    isx_road_estimate *estimates, isx_road *roads_out, isx_section *sections) {
   if (!road || !disparity || !segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  HostInputs in;
-  in.disparity16 = disparity;
-  in.scale = disparity_scale;
-  in.segmentation16 = segmentation;
-  HostRoad hr;
-  hr.road = road;
-  hr.fallback = fallback;
-  return submit_batch_host(h, pairwise, n, in, nullptr, sections, &hr, estimates, roads_out);
+  const HostRoad hr{road, fallback};
+  return submit_batch_host(h, pairwise, n, HostInputs(disparity, disparity_scale, segmentation), nullptr, sections,
+                           &hr, estimates, roads_out);
 }
 
 int isx_reserve_in_flight(isx_handle h, int batches) {
@@ -1619,7 +1594,7 @@ int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_res
   a.camera_center_x = m.camera_center_x;
   a.camera_center_y = m.camera_center_y;
   a.out = *out;
-  a.roads = h->last_roads_device ? h->last_roads_dev + first : nullptr;
+  a.roads = h->last_roads_dev ? h->last_roads_dev + first : nullptr;
   std::vector<float> alpha((size_t)n);
   std::vector<int> vhor((size_t)n);
   for (int f = 0; f < n && !a.roads; f++) {
@@ -1664,13 +1639,7 @@ int isx_read_tensor(isx_handle h, int tensor, int frame, void *host, size_t byte
   ISX_TRY(h, cudaStreamSynchronize(h->s_compute));
   const KParams &kp = h->kp;
   const size_t H = kp.rows, C = kp.realcols, D = kp.max_dis;
-  BatchBuffers b = h->buf;
-  {
-    const isx_context::ChunkSet &cs = h->sets[h->last_set];
-    b.ground = h->roads[h->last_road_slot].ground; b.vhor = h->roads[h->last_road_slot].vhor; b.stat = cs.stat;
-    b.records_b = cs.records_b; b.dp = cs.dp; b.pm = cs.pm;
-    b.joined = cs.joined; b.object_lut = cs.object_lut; b.col_flags = cs.col_flags;
-  }
+  const BatchBuffers b = chunk_buffers(h, h->last_set, h->last_road_slot);
   if (tensor == ISX_T_GROUND_TABLES) {
     ISX_TRY(h, cudaMemcpy(host, b.ground + (size_t)local * 3 * H, need, cudaMemcpyDeviceToHost));
   } else if (tensor == ISX_T_OBJ_COST_LUT) {
@@ -1816,14 +1785,9 @@ int pool_submit_batch_host_road(isx_handle h, isx_road_handle road, int pairwise
                                 const int32_t *segmentation, const isx_road *fallback, isx_road_estimate *estimates,
                                 isx_road *roads_out, isx_section *sections) {
   if (!road || !disparity || !segmentation || !fallback) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
-  HostInputs in;
-  in.disparity = disparity;
-  in.segmentation = segmentation;
-  HostRoad hr;
-  hr.road = road;
-  hr.fallback = fallback;
-  hr.carry = false;
-  return submit_batch_host(h, pairwise, n, in, nullptr, sections, &hr, estimates, roads_out);
+  const HostRoad hr{road, fallback, /*carry=*/false};
+  return submit_batch_host(h, pairwise, n, HostInputs(disparity, segmentation), nullptr, sections, &hr, estimates,
+                           roads_out);
 }
 
 int largest_chunk(isx_handle h) { return (h && h->initialized) ? std::max(h->chunk, h->chunk_unary) : 0; }
