@@ -14,7 +14,9 @@
 
 #include <algorithm>
 #include <cmath>
+#include <cstdint>
 #include <cstdlib>
+#include <cstring>
 #include <fstream>
 #include <iostream>
 #include <map>
@@ -156,31 +158,15 @@ public:
     // Corner points of every stixel in camera coordinates, 4 x (x, y, z) per stixel, clockwise
     // from the top-left corner (Stixels.cu:683-742).  Pure function of the result.
     std::vector<float> Get3DVertices(const StixelsData& d) {
-        if (cfg_.camera_center_x == -1 || cfg_.camera_center_y == -1)
-            throw std::invalid_argument("Camera parameters are not set.");
-        const float f = cfg_.focal, bf = cfg_.baseline * cfg_.focal;
-        const float cx = cfg_.camera_center_x, cy = cfg_.camera_center_y;
-        const int step = d.column_step;
+        check_camera(cfg_);
         std::vector<float> v;
         for (size_t i = 0; i < (size_t)d.realcols; i++) {
             for (size_t j = 0; j < (size_t)d.max_sections; j++) {
                 const Section& s = d.sections[i * d.max_sections + j];
                 if (s.type == -1) break;
-                const float xl = i * step, xr = xl + step;
-                const float yt = d.rows - s.vT - 1, yb = d.rows - s.vB;
-                float zt = 0.0, zb = 0.0;  // sky stays at depth 0
-                if (s.type == OBJECT) {
-                    zt = zb = bf / s.disparity;
-                } else if (s.type == GROUND) {
-                    zt = bf / (d.alpha_ground * (d.vhor - s.vT));
-                    zb = bf / (d.alpha_ground * (d.vhor - s.vB));
-                }
-                const float corner[4][3] = {{xl, yt, zt}, {xr, yt, zt}, {xr, yb, zb}, {xl, yb, zb}};
-                for (const auto& c : corner) {
-                    v.push_back(-c[2] / f * (cx - c[0]));
-                    v.push_back(-c[2] / f * (cy - c[1]));
-                    v.push_back(c[2]);
-                }
+                float c[12];
+                StixelVertices(cfg_, d, i, s, c);
+                v.insert(v.end(), c, c + 12);
             }
         }
         return v;
@@ -295,6 +281,75 @@ public:
         check(isx_export_batch_device(h_, first, n, &out));
     }
 
+    // Frames [first, first + n) of the last batch as objects, one record per (class, label) of GetInstanceStixels,
+    // into the caller's device buffers (isx_export_objects_device), asynchronous on isx_stream().
+    void ExportObjectsDevice(int first, int n, const isx_device_objects& out) {
+        check(isx_export_objects_device(h_, first, n, &out));
+    }
+
+    // The objects of one frame on the host, the definition isx_export_objects_device implements: one object per
+    // (class c in 11..18, label l >= 0) of `instances` (the frame's GetInstanceStixels map), ordered by class, then
+    // label; class c has 1 + (its largest label) objects.  Members are the stixels of the map with class c and label l.
+    // Float minima and maxima skip NaN and order -0.0 below +0.0; a field whose members are all NaN holds 0x7FC00000.
+    // `extents` (optional) receives 6 floats per object, min x, y, z then max x, y, z over the corners
+    // Get3DVertices computes for the members; like Get3DVertices it needs the camera centre.
+    std::vector<isx_object> GetInstanceObjects(const StixelsData& d, const InstanceMap& instances,
+                                               std::vector<float>* extents = nullptr) {
+        return GetInstanceObjects(cfg_, d, instances, extents);
+    }
+    // The same with the camera (focal, baseline, camera_center_x/y) of `camera`: needs no device.
+    static std::vector<isx_object> GetInstanceObjects(const StixelConfig& camera, const StixelsData& d,
+                                                      const InstanceMap& instances,
+                                                      std::vector<float>* extents = nullptr) {
+        if (extents) check_camera(camera);
+        const int first = ISX_FIRST_INSTANCE_CLASS, classes = ISX_INSTANCE_CLASSES;
+        int start[ISX_INSTANCE_CLASSES + 1] = {0};
+        for (const auto& e : instances) {
+            const int k = d.sections[(size_t)e.first.first * d.max_sections + e.first.second].semantic_class - first;
+            if (e.second >= 0 && k >= 0 && k < classes) start[k + 1] = std::max(start[k + 1], e.second + 1);
+        }
+        for (int k = 0; k < classes; k++) start[k + 1] += start[k];
+        float nan;
+        const uint32_t nan_bits = 0x7FC00000u;
+        std::memcpy(&nan, &nan_bits, sizeof nan);
+        std::vector<isx_object> out((size_t)start[classes]);
+        for (int k = 0; k < classes; k++)
+            for (int j = start[k]; j < start[k + 1]; j++)
+                out[(size_t)j] = isx_object{first + k, j - start[k], 0, 0, INT32_MAX, INT32_MIN, 0, INT32_MAX, 0,
+                                            INT32_MIN, nan, nan};
+        if (extents) extents->assign(out.size() * 6, nan);
+        for (const auto& e : instances) {
+            const size_t col = (size_t)e.first.first;
+            const Section& s = d.sections[col * d.max_sections + e.first.second];
+            const int k = s.semantic_class - first;
+            if (e.second < 0 || k < 0 || k >= classes) continue;
+            const size_t j = (size_t)(start[k] + e.second);
+            isx_object& o = out[j];
+            o.stixels += 1;
+            o.pixels += d.column_step * (s.vT - s.vB + 1);
+            o.col_min = std::min(o.col_min, (int32_t)col);
+            o.col_max = std::max(o.col_max, (int32_t)col);
+            o.y0 = std::min(o.y0, d.rows - 1 - s.vT);
+            o.y1 = std::max(o.y1, d.rows - 1 - s.vB);
+            fold_min(o.disparity_min, s.disparity);
+            fold_max(o.disparity_max, s.disparity);
+            if (extents) {
+                float c[12];
+                StixelVertices(camera, d, col, s, c);
+                float* x = extents->data() + j * 6;
+                for (int q = 0; q < 12; q++) {
+                    fold_min(x[q % 3], c[q]);
+                    fold_max(x[3 + q % 3], c[q]);
+                }
+            }
+        }
+        for (isx_object& o : out) {
+            o.x0 = o.col_min * d.column_step;
+            o.x1 = o.col_max * d.column_step + d.column_step - 1;
+        }
+        return out;
+    }
+
     isx_handle handle() { return h_; }  // for the other C entry points
 
 private:
@@ -333,6 +388,42 @@ private:
                 for (int32_t i = offs_[(size_t)f]; i < offs_[(size_t)f + 1]; i++)
                     (*instances)[(size_t)f][std::make_pair(inst_[(size_t)i].column, inst_[(size_t)i].index)] = inst_[(size_t)i].label;
         }
+    }
+
+    static void check_camera(const StixelConfig& c) {
+        if (c.camera_center_x == -1 || c.camera_center_y == -1)
+            throw std::invalid_argument("Camera parameters are not set.");
+    }
+    // The 4 corners (x, y, z) of stixel `s` of column i, clockwise from the top left (Stixels.cu:683-742), with the
+    // header's operation order: every operation rounded on its own.
+    static void StixelVertices(const StixelConfig& camera, const StixelsData& d, size_t i, const Section& s,
+                               float v[12]) {
+        const float f = camera.focal, bf = camera.baseline * camera.focal;
+        const float cx = camera.camera_center_x, cy = camera.camera_center_y;
+        const int step = d.column_step;
+        const float xl = i * step, xr = xl + step;
+        const float yt = d.rows - s.vT - 1, yb = d.rows - s.vB;
+        float zt = 0.0, zb = 0.0;  // sky stays at depth 0
+        if (s.type == OBJECT) {
+            zt = zb = bf / s.disparity;
+        } else if (s.type == GROUND) {
+            zt = bf / (d.alpha_ground * (d.vhor - s.vT));
+            zb = bf / (d.alpha_ground * (d.vhor - s.vB));
+        }
+        const float corner[4][3] = {{xl, yt, zt}, {xr, yt, zt}, {xr, yb, zb}, {xl, yb, zb}};
+        for (int k = 0; k < 4; k++) {
+            v[3 * k + 0] = -corner[k][2] / f * (cx - corner[k][0]);
+            v[3 * k + 1] = -corner[k][2] / f * (cy - corner[k][1]);
+            v[3 * k + 2] = corner[k][2];
+        }
+    }
+    // Minimum / maximum that skip NaN and order -0.0 below +0.0; `acc` starts as NaN (no value yet).
+    static bool below(float a, float b) { return a < b || (a == b && std::signbit(a) && !std::signbit(b)); }
+    static void fold_min(float& acc, float x) {
+        if (!std::isnan(x) && (std::isnan(acc) || below(x, acc))) acc = x;
+    }
+    static void fold_max(float& acc, float x) {
+        if (!std::isnan(x) && (std::isnan(acc) || below(acc, x))) acc = x;
     }
 
     static int device_from_env() {

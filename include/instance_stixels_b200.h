@@ -418,6 +418,44 @@ typedef struct isx_device_results { /* device pointers; NULL = not written (fram
 int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_results *out);
 
 /* ------------------------------------------------------------------------
+ * Device objects: the instances of frames [first, first + n) of the last batch (or of the last isx_compute: first = 0,
+ * n = 1) as one record per object in the caller's DEVICE buffers, for consumers that want objects, not stixels (a
+ * tracker, a planner, a message builder).  Frame f has one object per (semantic class c in 11..18, label l >= 0) of
+ * the map GetInstanceStixels returns for it; its members are the stixels of that map with class c and label l (noise,
+ * label -1, and stixels outside the map belong to no object).  Class c has 1 + (its largest label) objects in the frame.
+ * Objects are ordered by frame, then class, then label: those of frame f (0 = `first`) lie at
+ * [frame_offsets[f], frame_offsets[f+1]), those of class 11+k at [class_offsets[8f+k], class_offsets[8f+k+1]), and the
+ * object of (f, c, l) is class_offsets[8f + c-11] + l, which links the labels of isx_export_batch_device to objects.
+ * An object's box is the union of its members' rasteriser rectangles (isx_rasterize_batch_device).  extents[i] holds
+ * min x, y, z, then max x, y, z over the 4 corners of every member as Stixels::Get3DVertices computes them (needs
+ * camera_center_x/y).  Float minima and maxima skip NaN (a member over invalid pixels can have a NaN disparity) and
+ * order -0.0 below +0.0; a field whose members are all NaN holds 0x7FC00000.  Every field is order-independent, so
+ * the bytes are the same on every call.  `capacity` counts objects: a frame's objects (and extents) are written only
+ * if frame_offsets[f+1] <= capacity, nothing past it; the offsets are always complete.  Asynchronous on isx_stream();
+ * refusals (bad range, no frame_offsets, misaligned objects, negative capacity, extents without the camera centre,
+ * batches in flight) enqueue nothing.  Stixels::GetInstanceObjects (Stixels.hpp) computes the same on the host.
+ * ------------------------------------------------------------------------ */
+typedef struct isx_object {              /* 48 bytes */
+  int32_t semantic_class;                /* 11..18 */
+  int32_t label;                         /* DBSCAN label within the class (GetInstanceStixels), >= 0 */
+  int32_t stixels;                       /* number of members, >= 1 */
+  int32_t pixels;                        /* sum over the members of column_step * (vT - vB + 1) */
+  int32_t col_min, col_max;              /* stixel columns of the members */
+  int32_t x0, y0, x1, y1;                /* inclusive image box, top-left origin: x0 = col_min * column_step,
+                                            x1 = col_max * column_step + column_step - 1, y0 = min(rows-1-vT),
+                                            y1 = max(rows-1-vB) */
+  float disparity_min, disparity_max;    /* over the members' Section.disparity */
+} isx_object;
+typedef struct isx_device_objects { /* device pointers; NULL = not written (frame_offsets is required) */
+  isx_object *objects;              /* [capacity], 16-byte aligned */
+  int32_t *frame_offsets;           /* [n+1] */
+  int32_t *class_offsets;           /* [n*8+1] */
+  float *extents;                   /* [capacity][2][3] */
+  int32_t capacity, reserved;
+} isx_device_objects;               /* 40 bytes */
+int isx_export_objects_device(isx_handle h, int first, int n, const isx_device_objects *out);
+
+/* ------------------------------------------------------------------------
  * Road estimation (SURVEY.md 8f rank 1): the step in front of the stixel path.
  * Replaces `class RoadEstimation` (InstanceStixels/include/InstanceStixels/RoadEstimation.h:31-93,
  * src/RoadEstimation.cu:24-193, src/RoadEstimationKernels.cu:25-60) including its one third-party

@@ -37,7 +37,7 @@ EXPORTS = [
     # result images (SURVEY.md 8f rank 3)
     "isx_rasterize_batch_device",
     # device results
-    "isx_export_batch_device",
+    "isx_export_batch_device", "isx_export_objects_device",
     # road estimation (SURVEY.md 8f rank 1)
     "isx_road_create", "isx_road_destroy", "isx_road_initialize", "isx_road_finish", "isx_road_is_initialized",
     "isx_road_compute_host", "isx_road_compute_device", "isx_road_compute_batch_device", "isx_road_last_error",
@@ -95,15 +95,33 @@ class DeviceResults(C.Structure):
                 ("capacity", C.c_int32), ("reserved", C.c_int32)]
 
 
+class Object(C.Structure):
+    """isx_object: one instance of a frame, the summary of its member stixels."""
+    _fields_ = [(n, C.c_int32) for n in ("semantic_class", "label", "stixels", "pixels", "col_min", "col_max",
+                                         "x0", "y0", "x1", "y1")] + \
+               [("disparity_min", C.c_float), ("disparity_max", C.c_float)]
+
+
+class DeviceObjects(C.Structure):
+    """isx_device_objects: device pointers the object export writes (None = not written; frame_offsets is
+    required)."""
+    _fields_ = [("objects", C.c_void_p), ("frame_offsets", C.c_void_p), ("class_offsets", C.c_void_p),
+                ("extents", C.c_void_p), ("capacity", C.c_int32), ("reserved", C.c_int32)]
+
+
 # numpy views of isx_section (== Section, types.h:186-194) and isx_instance
 SECTION_DTYPE = np.dtype([("type", "<i4"), ("vB", "<i4"), ("vT", "<i4"), ("disparity", "<f4"),
                           ("semantic_class", "<i4"), ("cost", "<f4"), ("instance_meanx", "<f4"),
                           ("instance_meany", "<f4")])
 INSTANCE_DTYPE = np.dtype([("column", "<i4"), ("index", "<i4"), ("label", "<i4"), ("semantic_class", "<i4")])
+OBJECT_DTYPE = np.dtype([(n, "<i4") for n in ("semantic_class", "label", "stixels", "pixels", "col_min", "col_max",
+                                              "x0", "y0", "x1", "y1")] + [("disparity_min", "<f4"),
+                                                                           ("disparity_max", "<f4")])
 PACKED_FRAME_DTYPE = np.dtype([("section_offset", "<i4"), ("section_count", "<i4"), ("instance_offset", "<i4"),
                                ("instance_count", "<i4"), ("error", "<i4"), ("overflow", "<i4"),
                                ("reserved", "<i4", (2,))])
 assert SECTION_DTYPE.itemsize == 32 and INSTANCE_DTYPE.itemsize == 16 and PACKED_FRAME_DTYPE.itemsize == 32
+assert OBJECT_DTYPE.itemsize == 48
 
 ISX_OK = 0
 T_JOINED_DISPARITY, T_OBJECT_LUT, T_DISPARITY_PS, T_VALID_PS, T_GROUND_PS, T_SKY_PS, T_COST_TABLE, \
@@ -192,6 +210,7 @@ def _declare(lib):
     lib.isx_flip_and_pad_batch_device.argtypes = [H, i, C.c_void_p, i, i, C.c_void_p]
     lib.isx_rasterize_batch_device.argtypes = [H, i, i, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.isx_export_batch_device.argtypes = [H, i, i, C.POINTER(DeviceResults)]
+    lib.isx_export_objects_device.argtypes = [H, i, i, C.POINTER(DeviceObjects)]
     lib.isx_road_create.argtypes = [C.POINTER(H), i]
     lib.isx_road_destroy.argtypes = [H]
     lib.isx_road_destroy.restype = None

@@ -85,11 +85,37 @@ class DeviceRoads:
 
 
 @dataclass
+class DeviceObjects:
+    """isx_object records on the device (Stixels.ExportObjectsDevice): `data` is the int32 [capacity, 12] tensor, the
+    properties are its columns.  The objects of frame f are rows [frame_offsets[f], frame_offsets[f+1]); the object of
+    (frame f, class c, label l) is row class_offsets[8f + c - 11] + l.  `extents` is float32 [capacity, 2, 3] (min
+    x, y, z; max x, y, z) or None."""
+    data: Any
+    frame_offsets: Any
+    class_offsets: Any
+    extents: Any = None
+
+    semantic_class = property(lambda self: self.data[:, 0])
+    label = property(lambda self: self.data[:, 1])
+    stixels = property(lambda self: self.data[:, 2])
+    pixels = property(lambda self: self.data[:, 3])
+    col_min = property(lambda self: self.data[:, 4])
+    col_max = property(lambda self: self.data[:, 5])
+    x0 = property(lambda self: self.data[:, 6])
+    y0 = property(lambda self: self.data[:, 7])
+    x1 = property(lambda self: self.data[:, 8])
+    y1 = property(lambda self: self.data[:, 9])
+    disparity_min = property(lambda self: self.data[:, 10].view(_f32()))
+    disparity_max = property(lambda self: self.data[:, 11].view(_f32()))
+
+
+@dataclass
 class DeviceStixels:
     """Torch tensors of Stixels.ComputeBatchTensors (the isx_device_results layout).  `sections` is the int32
     [capacity, 8] view of the Sections; frame f owns rows [frame_offsets[f], frame_offsets[f+1]); `vertices` is
     [capacity, 4, 3] or None.  With road estimation on the device (road=), `road_estimates` holds what the
-    estimation returned for every frame and `roads` the road every frame was computed with."""
+    estimation returned for every frame and `roads` the road every frame was computed with.  With objects=True,
+    `objects` holds the instances of the batch as objects."""
     sections: Any
     frame_offsets: Any
     column_offsets: Any
@@ -98,6 +124,7 @@ class DeviceStixels:
     frame_errors: Any
     road_estimates: Optional[DeviceRoadEstimates] = None
     roads: Optional[DeviceRoads] = None
+    objects: Optional[DeviceObjects] = None
 
     # typed columns of `sections` (isx_section)
     @property
@@ -226,9 +253,20 @@ class Stixels:
                               vertices or None, frame_errors or None, capacity, 0)
         self._check(self._lib.isx_export_batch_device(self._h, first, n, C.byref(out)))
 
+    def ExportObjectsDevice(self, first: int, n: int, frame_offsets: int, objects: int = 0, class_offsets: int = 0,
+                            extents: int = 0, capacity: int = 0):
+        """Instances of frames [first, first+n) of the last batch as objects, one record per (class, label) of
+        GetInstanceStixels, into caller device buffers (raw pointers, 0 = not written): isx_object records, per-frame
+        and per-(frame, class) offsets and the 3D extents of every object; `capacity` counts objects.  Asynchronous
+        on stream()."""
+        out = L.DeviceObjects(objects or None, frame_offsets or None, class_offsets or None, extents or None,
+                              capacity, 0)
+        self._check(self._lib.isx_export_objects_device(self._h, first, n, C.byref(out)))
+
     def ComputeBatchTensors(self, pairwise: bool, disparity, roads: Optional[Sequence[dict]] = None,
                             segmentation=None, cnn=None, vertices: bool = False, capacity: Optional[int] = None,
-                            road: Optional["RoadEstimation"] = None, fallback: Optional[dict] = None) -> "DeviceStixels":
+                            road: Optional["RoadEstimation"] = None, fallback: Optional[dict] = None,
+                            objects: bool = False, object_capacity: Optional[int] = None) -> "DeviceStixels":
         """CUDA torch tensors in, torch tensors out, no host synchronisation: `disparity` float32 [n][rows][cols]
         and either `segmentation` int32 in the library layout [n][realcols][21][rows_power2_segmentation] or `cnn`
         float32 [n][21][rows/8][cols/8] (run through FlipAndPadBatchDevice).  The library's stream waits for the
@@ -236,7 +274,9 @@ class Stixels:
         to the worst case n * realcols * 200.
         The road of every frame: either `roads` (one dict per frame) or `road`, a RoadEstimation that estimates it
         on the device from the frame's disparity (ComputeBatchDeviceRoad; `fallback` as there).  With `road`, the
-        result also carries `road_estimates` and `roads`."""
+        result also carries `road_estimates` and `roads`.
+        objects=True: the result also carries `objects` (ExportObjectsDevice of the batch, with extents when
+        vertices=True); `object_capacity` defaults to the worst case n * realcols * 200."""
         import torch
         if (roads is None) == (road is None):
             raise InvalidArgument("pass exactly one of roads= and road=")
@@ -274,6 +314,13 @@ class Stixels:
             labels=torch.empty(cap, dtype=torch.int32, device=dev),
             vertices=torch.empty((cap, 4, 3), dtype=torch.float32, device=dev) if vertices else None,
             frame_errors=torch.empty(n, dtype=torch.int32, device=dev))
+        if objects:
+            ocap = n * C_ * self.GetMaxSections() if object_capacity is None else int(object_capacity)
+            out.objects = DeviceObjects(
+                data=torch.empty((ocap, 12), dtype=torch.int32, device=dev),
+                frame_offsets=torch.empty(n + 1, dtype=torch.int32, device=dev),
+                class_offsets=torch.empty(n * 8 + 1, dtype=torch.int32, device=dev),
+                extents=torch.empty((ocap, 2, 3), dtype=torch.float32, device=dev) if vertices else None)
         if road is not None:
             out.road_estimates = DeviceRoadEstimates(torch.empty((n, 7), dtype=torch.int32, device=dev))
             out.roads = DeviceRoads(torch.empty((n, 4), dtype=torch.int32, device=dev))
@@ -296,6 +343,11 @@ class Stixels:
                                column_offsets=out.column_offsets.data_ptr(), labels=out.labels.data_ptr(),
                                vertices=out.vertices.data_ptr() if vertices else 0,
                                frame_errors=out.frame_errors.data_ptr(), capacity=cap)
+        if objects:
+            ob = out.objects
+            self.ExportObjectsDevice(0, n, ob.frame_offsets.data_ptr(), objects=ob.data.data_ptr(),
+                                     class_offsets=ob.class_offsets.data_ptr(),
+                                     extents=ob.extents.data_ptr() if vertices else 0, capacity=ocap)
         done = torch.cuda.Event()
         done.record(ext)
         current.wait_event(done)

@@ -126,6 +126,7 @@ struct isx_context {
   int cur = 0;                                    // result set of the batch being enqueued / of the last batch
   int *d_raster_table = nullptr;                  // [max_batch][C][200] instance id per stixel (rasteriser)
   int *d_export_col = nullptr;                    // [max_batch][C] frame-relative column offsets (device export)
+  int *d_object_class = nullptr;                  // [max_batch*8+1] objects per (frame, class), then their prefix
   int inst_cap = 0;                               // instance records per frame of the device arrays: C * 200
   float *d_export_cost = nullptr;
   int *d_export_index = nullptr;
@@ -1005,6 +1006,7 @@ int isx_initialize(isx_handle h, int max_batch) {
   if (int rc = alloc_result_set(h, 0)) return rc;
   ISX_TRY(h, dev_alloc(h, &h->d_raster_table, MB * C * kMaxSections));
   ISX_TRY(h, dev_alloc(h, &h->d_export_col, MB * C));
+  ISX_TRY(h, dev_alloc(h, &h->d_object_class, MB * ISX_INSTANCE_CLASSES + 1));
   ISX_TRY(h, dev_alloc(h, &h->d_export_cost, C * H * 3));
   ISX_TRY(h, dev_alloc(h, &h->d_export_index, C * H * 3));
 
@@ -1602,6 +1604,40 @@ int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_res
     vhor[f] = h->kp.rows - h->last_roads[first + f].vhor - 1;   // isx_frame_meta.vhor (Stixels.cu:377)
   }
   launch_export_results(a, n, alpha.data(), vhor.data(), h->s_tables);
+  ISX_TRY(h, cudaGetLastError());
+  return ISX_OK;
+}
+
+// Like isx_export_batch_device: reads result set rs[cur] on s_tables.
+int isx_export_objects_device(isx_handle h, int first, int n, const isx_device_objects *out) {
+  if (int rc = check_ready(h)) return rc;
+  if (first < 0 || n < 1 || first + n > h->last_batch)
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "frames outside the last computed batch");
+  if (!out || !out->frame_offsets) return fail(h, ISX_ERR_INVALID_ARGUMENT, "frame_offsets is required");
+  if ((uintptr_t)out->objects % 16 != 0) return fail(h, ISX_ERR_INVALID_ARGUMENT, "objects must be 16-byte aligned");
+  if (out->capacity < 0) return fail(h, ISX_ERR_INVALID_ARGUMENT, "capacity must be >= 0");
+  const HostModel &m = h->model;
+  if (out->extents && (m.camera_center_x == -1 || m.camera_center_y == -1))
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "Camera parameters are not set.");  // Get3DVertices (Stixels.cu:685-687)
+  if (int rc = no_batches_in_flight(h)) return rc;
+  if (int rc = ensure_joined(h)) return rc;
+  const size_t C = h->kp.realcols;
+  const isx_context::ResultSet &R = h->rs[h->cur];
+  ObjectArgs a;
+  a.sections = R.d_sections + (size_t)first * C * kMaxSections;
+  a.inst = R.d_inst + (size_t)first * h->inst_cap;
+  a.inst_count = R.d_inst_count + first;
+  a.inst_cap = h->inst_cap;
+  a.class_start = h->d_object_class;
+  a.realcols = h->kp.realcols;
+  a.rows = h->kp.rows;
+  a.column_step = h->kp.column_step;
+  a.focal = m.focal;
+  a.bf = m.baseline * m.focal;
+  a.camera_center_x = m.camera_center_x;
+  a.camera_center_y = m.camera_center_y;
+  a.out = *out;
+  launch_export_objects(a, n, h->s_tables);
   ISX_TRY(h, cudaGetLastError());
   return ISX_OK;
 }

@@ -89,8 +89,10 @@ export_frame_scan_kernel(int *__restrict__ frame_offsets, int *__restrict__ colu
 // Stixels::Get3DVertices for one Section, in the header's operation order (xl = i * step, xr = xl + step,
 // yt = rows - vT - 1, yb = rows - vB; z = bf / disparity for objects, bf / (alpha_ground * (vhor - v)) for ground,
 // 0 for sky; then per corner -z / f * (c - x), -z / f * (c - y), z), with every operation rounded on its own.
-__device__ __forceinline__ void stixel_vertices(const isx_section &s, int col, const ExportArgs &a, float alpha,
-                                                int vhor, float *v) {
+// Args: ExportArgs or ObjectArgs (column_step, rows, bf, focal, camera_center_x/y).
+template <class Args>
+__device__ __forceinline__ void stixel_vertices(const isx_section &s, int col, const Args &a, float alpha, int vhor,
+                                                float *v) {
   const float xl = (float)(col * a.column_step), xr = __fadd_rn(xl, (float)a.column_step);
   const float yt = (float)(a.rows - s.vT - 1), yb = (float)(a.rows - s.vB);
   float zt = 0.0f, zb = 0.0f;
@@ -163,7 +165,149 @@ export_stixels_kernel(ExportArgs a, ExportFrames fr, int f0) {
   }
 }
 
+// ---- device objects (isx_export_objects_device): one record per (frame, class, label) of the instance records ----
+constexpr int kObjectThreads = 256;
+constexpr int kClasses = ISX_INSTANCE_CLASSES;
+constexpr int kKeyEmpty = 0x7fffffff;   // "no value" of a minimum: the key of no float but a NaN
+constexpr int kKeyEmptyMax = -kKeyEmpty - 1;
+
+// Order-preserving int key of a non-NaN float: signed comparison of the keys is the float order, with -0.0 below
+// +0.0.  The map is its own inverse.
+__device__ __forceinline__ int float_key(float x) {
+  const int b = __float_as_int(x);
+  return b >= 0 ? b : b ^ 0x7fffffff;
+}
+// key -> float bits; the empty key -> 0x7FC00000 (every member NaN)
+__device__ __forceinline__ int key_bits(int k, int empty) {
+  return k == empty ? 0x7fc00000 : (k >= 0 ? k : k ^ 0x7fffffff);
+}
+
+// One CTA per frame: objects of instance class 11+k = 1 + the largest label of the frame's records of that class, into
+// class_start[8f + k + 1].  The frame scan then makes class_start the exclusive prefix over (frame, class).
+__global__ void __launch_bounds__(kObjectThreads)
+object_count_kernel(const isx_instance *__restrict__ inst, const int *__restrict__ inst_count, int inst_cap,
+                    int *__restrict__ class_start) {
+  __shared__ int s_max[kClasses];
+  const int f = blockIdx.x, tid = threadIdx.x;
+  if (tid < kClasses) s_max[tid] = -1;
+  __syncthreads();
+  const int ni = min(inst_count[f], inst_cap);
+  const isx_instance *rec = inst + (size_t)f * inst_cap;
+  for (int i = tid; i < ni; i += kObjectThreads) {
+    const isx_instance r = rec[i];
+    const int k = r.semantic_class - ISX_FIRST_INSTANCE_CLASS;
+    if (r.label >= 0 && k >= 0 && k < kClasses) atomicMax(&s_max[k], r.label);
+  }
+  __syncthreads();
+  if (tid < kClasses) class_start[(size_t)f * kClasses + tid + 1] = s_max[tid] + 1;
+}
+
+// One CTA per frame.  Offsets are always written; the frame's objects and extents only if they all fit `capacity`.
+// Three passes over global memory, separated by CTA barriers: initialise the frame's records (minima at the empty key,
+// maxima at its negation), let every instance record fold its Section into its object with integer atomics (floats as
+// order-preserving keys, NaN skipped), then turn the keys back into floats and the column range into the image box.
+// Every update is a sum, a minimum or a maximum of integers, so the result does not depend on their order.
+__global__ void __launch_bounds__(kObjectThreads)
+export_objects_kernel(ObjectArgs a) {
+  __shared__ int s_start[kClasses + 1];
+  const int f = blockIdx.x, tid = threadIdx.x, last = gridDim.x - 1;
+  const isx_device_objects &o = a.out;
+  if (tid <= kClasses) {
+    const int v = a.class_start[(size_t)f * kClasses + tid];
+    s_start[tid] = v;
+    if (o.class_offsets && (tid < kClasses || f == last)) o.class_offsets[(size_t)f * kClasses + tid] = v;
+    if (tid == 0 || (tid == kClasses && f == last)) o.frame_offsets[f + tid / kClasses] = v;
+  }
+  __syncthreads();
+  const int lo = s_start[0], hi = s_start[kClasses];
+  int *obj = reinterpret_cast<int *>(o.objects);   // 12 words per object
+  int *ext = reinterpret_cast<int *>(o.extents);   // 6 words per object
+  if (hi > o.capacity || (!obj && !ext)) return;
+  for (int j = lo + tid; j < hi; j += kObjectThreads) {
+    int k = 0;
+    while (j >= s_start[k + 1]) k++;
+    if (obj) {
+      int4 *w = reinterpret_cast<int4 *>(obj + (size_t)j * 12);
+      w[0] = make_int4(ISX_FIRST_INSTANCE_CLASS + k, j - s_start[k], 0, 0);    // class, label, stixels, pixels
+      w[1] = make_int4(kKeyEmpty, kKeyEmptyMax, 0, kKeyEmpty);                 // col_min, col_max, x0, y0
+      w[2] = make_int4(0, kKeyEmptyMax, kKeyEmpty, kKeyEmptyMax);              // x1, y1, disparity_min, _max
+    }
+    if (ext)
+      for (int q = 0; q < 3; q++) {
+        ext[(size_t)j * 6 + q] = kKeyEmpty;
+        ext[(size_t)j * 6 + 3 + q] = kKeyEmptyMax;
+      }
+  }
+  __syncthreads();
+  const int ni = min(a.inst_count[f], a.inst_cap);
+  const isx_instance *rec = a.inst + (size_t)f * a.inst_cap;
+  for (int i = tid; i < ni; i += kObjectThreads) {
+    const isx_instance r = rec[i];
+    const int k = r.semantic_class - ISX_FIRST_INSTANCE_CLASS;
+    if (r.label < 0 || k < 0 || k >= kClasses) continue;
+    const size_t j = (size_t)(s_start[k] + r.label);
+    const isx_section s = a.sections[((size_t)f * a.realcols + r.column) * kMaxSections + r.index];
+    if (obj) {
+      int *w = obj + j * 12;
+      atomicAdd(w + 2, 1);
+      atomicAdd(w + 3, a.column_step * (s.vT - s.vB + 1));
+      atomicMin(w + 4, r.column);
+      atomicMax(w + 5, r.column);
+      atomicMin(w + 7, a.rows - 1 - s.vT);
+      atomicMax(w + 9, a.rows - 1 - s.vB);
+      if (!isnan(s.disparity)) {
+        const int key = float_key(s.disparity);
+        atomicMin(w + 10, key);
+        atomicMax(w + 11, key);
+      }
+    }
+    if (ext) {
+      float v[12];
+      stixel_vertices(s, r.column, a, 0.0f, 0, v);   // members are OBJECT stixels: no road enters
+      int mn[3] = {kKeyEmpty, kKeyEmpty, kKeyEmpty}, mx[3] = {kKeyEmptyMax, kKeyEmptyMax, kKeyEmptyMax};
+#pragma unroll
+      for (int c = 0; c < 12; c++) {
+        if (isnan(v[c])) continue;
+        const int key = float_key(v[c]);
+        mn[c % 3] = min(mn[c % 3], key);
+        mx[c % 3] = max(mx[c % 3], key);
+      }
+      int *e = ext + j * 6;
+#pragma unroll
+      for (int q = 0; q < 3; q++)
+        if (mn[q] != kKeyEmpty) {
+          atomicMin(e + q, mn[q]);
+          atomicMax(e + 3 + q, mx[q]);
+        }
+    }
+  }
+  __syncthreads();
+  // the atomics ran in L2: read their results past L1
+  for (int j = lo + tid; j < hi; j += kObjectThreads) {
+    if (obj) {
+      int *w = obj + (size_t)j * 12;
+      w[6] = __ldcg(w + 4) * a.column_step;
+      w[8] = __ldcg(w + 5) * a.column_step + a.column_step - 1;
+      w[10] = key_bits(__ldcg(w + 10), kKeyEmpty);
+      w[11] = key_bits(__ldcg(w + 11), kKeyEmptyMax);
+    }
+    if (ext)
+      for (int q = 0; q < 6; q++) {
+        int *e = ext + (size_t)j * 6 + q;
+        *e = key_bits(__ldcg(e), q < 3 ? kKeyEmpty : kKeyEmptyMax);
+      }
+  }
+}
+
 }  // namespace
+
+void launch_export_objects(const ObjectArgs &a, int nframes, cudaStream_t s) {
+  object_count_kernel<<<nframes, kObjectThreads, 0, s>>>(a.inst, a.inst_count, a.inst_cap, a.class_start);
+  // the frame scan over the n*8 counts in class_start[1..n*8]: class_start[i] = objects before (frame, class) i
+  export_frame_scan_kernel<<<1, kFrameScanThreads, 0, s>>>(a.class_start, nullptr, nframes * kClasses, 0);
+  export_objects_kernel<<<nframes, kObjectThreads, 0, s>>>(a);
+  g_launch_count += 3;
+}
 
 void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_ground, const int *vhor,
                            cudaStream_t s) {

@@ -113,6 +113,18 @@ struct ExportFrames {              // per-frame road scalars of one launch: alph
 };
 void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_ground, const int *vhor,
                            cudaStream_t s);
+// Device objects of a computed batch (export.cu): frames [0, n) of the arrays below, into the caller's buffers.
+struct ObjectArgs {
+  const isx_section *sections;   // [n][C][200] padded device results
+  const isx_instance *inst;      // [n][inst_cap]
+  const int *inst_count;         // [n]
+  int inst_cap;
+  int *class_start;              // [n*8+1] scratch: objects per (frame, class), then their exclusive prefix
+  int realcols, rows, column_step;
+  float focal, bf, camera_center_x, camera_center_y;   // bf = baseline * focal
+  isx_device_objects out;
+};
+void launch_export_objects(const ObjectArgs &a, int nframes, cudaStream_t s);
 // Road estimation in front of a device batch (road.cu, isx_compute_batch_device_road) or of a chunk of a host batch
 // (isx_submit_batch_host_road): the checks (nothing enqueued), then the Hough kernels, the device line selection and
 // the keep-last rule on the road handle's stream, ordered after and before `caller`.  d_roads [n]: the road every
