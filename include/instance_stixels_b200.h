@@ -172,9 +172,14 @@ int isx_set_model_parameters(isx_handle h, int column_step, int median_join, flo
 /* Stixels::Initialize (Stixels.cu:43-248): allocations + LUT precompute.
  * `max_batch` >= 1 is the number of frames one batched call may carry (the
  * reference has no batching; its Initialize is max_batch == 1).  Frames of
- * more than ISX_MAX_ROWS rows are refused with ISX_ERR_UNSUPPORTED. */
+ * more than ISX_MAX_ROWS rows are refused with ISX_ERR_UNSUPPORTED.  A failed
+ * call leaves the handle uninitialised, holding no device or pinned memory,
+ * and it may be initialised again (e.g. with a smaller max_batch). */
 int isx_initialize(isx_handle h, int max_batch);
-/* Stixels::Finish (Stixels.cu:250-283). */
+/* Stixels::Finish (Stixels.cu:250-283): waits for the device, then releases
+ * every allocation, stream and event of the handle, also with batches in
+ * flight.  The handle is left uninitialised, holding no device or pinned
+ * memory, and it may be initialised again. */
 int isx_finish(isx_handle h);
 /* Stixels::IsInitialized (Stixels.hpp:96). */
 int isx_is_initialized(isx_handle h);
@@ -480,7 +485,9 @@ typedef struct isx_road_estimate {
 
 int isx_road_create(isx_road_handle *out, int device);
 void isx_road_destroy(isx_road_handle h);
-/* RoadEstimation::Initialize (RoadEstimation.cu:32-84); max_batch sizes the batched entry point. */
+/* RoadEstimation::Initialize (RoadEstimation.cu:32-84); max_batch sizes the batched entry point.  An initialised
+ * handle is released first.  A failed call leaves the handle uninitialised, holding no device or pinned memory, and it
+ * may be initialised again. */
 int isx_road_initialize(isx_road_handle h, float camera_center_y, float baseline, float focal, int rows, int cols,
                         int max_dis, float road_vdisparity_threshold, int max_batch);
 int isx_road_finish(isx_road_handle h);        /* RoadEstimation::Finish (:86-94) */

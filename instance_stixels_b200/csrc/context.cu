@@ -16,23 +16,23 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
 
+#include "cuda_resources.h"
 #include "host_model.h"
 #include "kernels.h"
 
 namespace isx {
 
 static thread_local std::string g_last_error;
-constexpr int kStageSlots = 8;    // pinned staging buffers of the road tables (see isx_context::h_ground)
-constexpr int kRoadSlots = 4;     // device copies of a chunk's road tables (isx_context::roads)
+constexpr int kStageSlots = 8;    // pinned staging buffers of the road tables (see Initialized::h_ground)
+constexpr int kRoadSlots = 4;     // device copies of a chunk's road tables (Initialized::roads)
 constexpr int kResultSets = 4;    // result sets: up to kResultSets - 1 submitted batches in flight + the one waited last
 constexpr int kProfEvents = 9;    // profiling events per enqueued chunk (enqueue_chunk)
 constexpr int kTraceStamps = 11;  // time stamps per chunk of isx_get_chunk_trace
-
-static int fail(isx_context *ctx, int code, const std::string &msg);
 
 struct RoadKey {
   int vhor;
@@ -45,39 +45,33 @@ struct RoadKey {
   }
 };
 
-}  // namespace isx
+// Everything one isx_initialize acquires and everything that describes batches since then, up to the isx_finish
+// that releases it all.  isx_context::init is set only while the handle is initialised.
+struct Initialized {
+  explicit Initialized(int device) : res(device) {}
 
-struct isx_context {
-  int device = 0;
-  bool configured_parts[8] = {false, false, false, false, false, false, false, false};
-  bool initialized = false;
-  isx::HostModel model;
-  isx::KParams kp{};
+  KParams kp{};
   int max_batch = 0, chunk = 0;   // chunk: frames the intermediates hold = frames per pairwise launch
   int chunk_unary = 0;            // frames per unary launch
   int last_launch_frames = 0;     // of the last enqueued batch (isx_chunk_frames)
-  std::string last_error;
 
   // s_tables: join + table build (HBM-bound), s_compute: the DP (issue-bound), s_emit: backtracking, grouping, packing
   // (short, latency-bound).  The tables of chunk k+1 are built WHILE the DP of chunk k runs: their CTAs take the
   // places DP CTAs vacate (12 K registers against 16 K), so the memory-bound and the issue-bound kernel share the SMs.
-  cudaStream_t s_tables = nullptr, s_compute = nullptr, s_emit = nullptr, s_h2d = nullptr, s_d2h = nullptr;
+  cudaStream_t s_tables = nullptr, s_compute = nullptr, s_emit = nullptr, s_h2d = nullptr;
   cudaEvent_t ev_dp_done[2] = {nullptr, nullptr}, ev_emit_done[2] = {nullptr, nullptr};
   cudaEvent_t ev_tab_done[2] = {nullptr, nullptr};   // tables of the chunk in this set are complete
-  cudaEvent_t ev_user = nullptr;                     // the caller's work on isx_stream() before a device batch
   cudaEvent_t ev_in_ready[2] = {nullptr, nullptr}, ev_in_free[2] = {nullptr, nullptr};
-  cudaEvent_t ev_chunk_done = nullptr;
   // narrow host inputs (isx_*_u16): staging for the raw uint16 / int16 data, allocated on first use
   uint16_t *d_in_disp16[2] = {nullptr, nullptr};  // [chunk][H][W]
   int16_t *d_in_seg16[2] = {nullptr, nullptr};    // [chunk][C][21][ceil(H/8)]
 
   // device memory
-  std::vector<void *> allocations;
   float *d_in_disp[2] = {nullptr, nullptr};       // staging for host batches: [chunk][H][W]
   int32_t *d_in_seg[2] = {nullptr, nullptr};      // [chunk][seg_elems]
   float *d_single_disp = nullptr;                 // SetDisparityImage target (d_disparity_big)
   int32_t *d_single_seg = nullptr;                // SetSegmentation target
-  isx::BatchBuffers buf;                          // intermediates sized `chunk`, results sized `max_batch`
+  BatchBuffers buf;                               // intermediates sized `chunk`, results sized `max_batch`
   // Buffers the emission stream still reads while the compute stream works on the next chunk exist
   // twice; chunk k uses set k & 1.
   struct ChunkSet {
@@ -99,7 +93,7 @@ struct isx_context {
     float *ground = nullptr;
     int *vhor = nullptr;
     cudaEvent_t ev_free = nullptr;
-  } roads[isx::kRoadSlots];
+  } roads[kRoadSlots];
   unsigned long long road_next = 0;
   int last_road_slot = 0;
   bool overlap_tables = true;      // table build of chunk k+1 beside the DP of chunk k (ISX_OVERLAP_TABLES)
@@ -108,7 +102,6 @@ struct isx_context {
   // gets is packed by pack_results_kernel (emit.cu) straight into pinned host memory that is mapped into the
   // device address space (h_* = host address, m_* = the device's address of the same memory).
   struct ResultSet {
-    bool allocated = false;
     isx_section *d_sections = nullptr;            // [max_batch][C][200]
     int *d_nsections = nullptr;                   // [max_batch][C]
     isx_instance *d_inst = nullptr;               // [max_batch][inst_cap]
@@ -122,7 +115,7 @@ struct isx_context {
     // batches with estimated roads (isx_submit_batch_host_road), allocated on first use: mapped pinned [max_batch]
     isx_road_estimate *h_est = nullptr, *m_est = nullptr;   // what the estimation returned for every frame
     isx_road *h_roads = nullptr, *m_roads = nullptr;        // the road every frame was computed with
-  } rs[isx::kResultSets];
+  } rs[kResultSets];
   int cur = 0;                                    // result set of the batch being enqueued / of the last batch
   int *d_raster_table = nullptr;                  // [max_batch][C][200] instance id per stixel (rasteriser)
   int *d_export_col = nullptr;                    // [max_batch][C] frame-relative column offsets (device export)
@@ -136,18 +129,20 @@ struct isx_context {
   // that last read it, so that the enqueueing host thread may run several chunks ahead of the device
   float *h_ground = nullptr;                      // [kStageSlots][chunk][3][H]
   int *h_vhor = nullptr;                          // [kStageSlots][chunk]
-  cudaEvent_t ev_stage_done[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t ev_stage_done[kStageSlots] = {};
   unsigned long long stage_next = 0;
   // isx_submit_batch_host keeps up to kResultSets - 1 batches in flight: rs[cur] belongs to the batch submitted last;
   // a new batch takes the lowest set that is neither in flight nor the one handed out by the last wait (allocated on
   // first use: a caller with two batches in flight only ever touches three).  Indexed by ticket % kResultSets:
-  cudaEvent_t ev_batch_done[isx::kResultSets] = {};       // behind the packing of the batch's last chunk
-  int batch_n[isx::kResultSets] = {};                     // frames of the batch in flight with that ticket, 0 = none
-  int batch_set[isx::kResultSets] = {};                   // its result set
-  isx_section *batch_sections[isx::kResultSets] = {};     // the caller's padded array the wait expands into
-  isx_road_estimate *batch_est[isx::kResultSets] = {};    // the caller's arrays the wait fills (estimated roads)
-  isx_road *batch_roads[isx::kResultSets] = {};
-  bool batch_direct[isx::kResultSets] = {};               // ... or that the device has already filled (mapped memory)
+  struct InFlight {
+    cudaEvent_t done = nullptr;             // behind the packing of the batch's last chunk (created on first use)
+    int n = 0;                              // frames of the batch in flight with that ticket, 0 = none
+    int set = 0;                            // its result set
+    isx_section *sections = nullptr;        // the caller's padded array the wait expands into
+    bool direct = false;                    // ... or that the device has already filled (mapped memory)
+    isx_road_estimate *est = nullptr;       // the caller's arrays the wait fills (estimated roads)
+    isx_road *roads = nullptr;
+  } batches[kResultSets];
   int last_waited_set = -1;                           // result set of the batch waited for last (isx_wait_batch_packed)
   unsigned long long submitted = 0, waited = 0;       // tickets: batches [waited, submitted) are in flight
   unsigned long long dp_units_pairwise = 0;           // ... of which in pairwise mode (never pruned)
@@ -155,28 +150,25 @@ struct isx_context {
   int host_slot = 0;                                  // input slot / chunk set of the next host chunk (alternates across batches)
 
   // ground tables per road; also read by the host functions of isx_compute_batch_device_road (a driver thread)
-  std::map<isx::RoadKey, std::vector<float>> road_cache;
+  std::map<RoadKey, std::vector<float>> road_cache;
   std::mutex road_cache_mutex;
   isx_road *h_stage_roads = nullptr;  // [kStageSlots][chunk] pinned: the device-estimated roads of a staged chunk
   isx_road *d_batch_roads = nullptr;  // [max_batch] roads of the last isx_compute_batch_device_road batch
   // the roads of the last batch were estimated on the device: the export reads them here (d_batch_roads or
   // rs[cur].m_roads) instead of last_roads
   const isx_road *last_roads_dev = nullptr;
-  // device addresses of the pinned staging (h_ground, h_vhor, h_stage_roads), taken on the first host batch with
-  // estimated roads: its road step writes the roads there and pull_tables_kernel reads the tables from there
+  // device addresses of the pinned staging (h_ground, h_vhor, h_stage_roads): the road step of a host batch with
+  // estimated roads writes the roads there and pull_tables_kernel reads the tables from there
   float *m_ground = nullptr;
   int *m_vhor = nullptr;
   isx_road *m_stage_roads = nullptr;
-  isx_road single_road{0, 0.f, 0.f, 0.f};
-  bool single_has_road = false;
   int last_batch = 0;          // frames of the last batch (results valid for these)
   int last_chunk_first = 0;    // first frame whose intermediates are still in `buf`
   int last_chunk_n = 0;
   bool last_pairwise = false;
   std::vector<isx_road> last_roads;
 
-  // optional per-stage CUDA-event timing (isx_set_profiling)
-  bool profiling = false;
+  // per-stage CUDA-event timing (isx_set_profiling)
   std::vector<cudaEvent_t> prof_events;   // kStages+1 events per enqueued chunk
   size_t prof_used = 0;
   std::vector<cudaEvent_t> prof_h2d;      // host batches: begin / end of every chunk's input copies (copy stream)
@@ -185,6 +177,24 @@ struct isx_context {
   long stage_launches[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   // host time of the ground-table host functions of batches with estimated roads (a driver thread writes it)
   std::atomic<long long> host_fill_ns{0}, host_fill_calls{0};
+
+  // Owns every stream, event and allocation above.  Declared last, so destroyed first: its destructor synchronises
+  // the device before the road cache and its mutex go, and fill_stage_from_roads, which a driver thread runs on
+  // behalf of queued work and which reads this struct, must not outlive it.
+  CudaResources res;
+};
+
+}  // namespace isx
+
+struct isx_context {
+  int device = 0;
+  isx::HostModel model;
+  std::string last_error;
+  bool profiling = false;   // isx_set_profiling
+  // the road of isx_compute (SetRoadParameters, may be set before isx_initialize)
+  isx_road single_road{0, 0.f, 0.f, 0.f};
+  bool single_has_road = false;
+  std::unique_ptr<isx::Initialized> init;   // null: not initialised
 };
 
 namespace isx {
@@ -212,15 +222,17 @@ int fail_cuda(cudaError_t e, const char *expr, const char *file, int line) {
     }                                                                 \
   } while (0)
 
+// Device memory of `count` elements with a 256-byte tail, owned by I.res.
 template <typename T>
-static cudaError_t dev_alloc(isx_context *c, T **p, size_t count) {
-  void *q = nullptr;
-  cudaError_t e = cudaMalloc(&q, count * sizeof(T) + 256);
-  if (e == cudaSuccess) {
-    c->allocations.push_back(q);
-    *p = static_cast<T *>(q);
-  }
-  return e;
+static cudaError_t dev_alloc(Initialized &I, T **p, size_t count) {
+  return I.res.device(p, count * sizeof(T) + 256);
+}
+
+// Mapped pinned host memory of `count` elements (*h) and the device's address of it (*m), owned by I.res.
+template <typename T>
+static cudaError_t mapped_alloc(Initialized &I, T **h, T **m, size_t count) {
+  const cudaError_t e = I.res.host(h, sizeof(T) * count, cudaHostAllocMapped | cudaHostAllocPortable);
+  return e == cudaSuccess ? cudaHostGetDevicePointer(m, *h, 0) : e;
 }
 
 // Device bytes per frame of a chunk: both chunk sets, both input staging slots and the transition records of the
@@ -237,9 +249,7 @@ static size_t seg_elems(const isx_context *c) {
   return (size_t)c->model.rows_power2_seg * c->model.realcols * c->model.n_channels;
 }
 
-static void fill_kparams(isx_context *c) {
-  const HostModel &m = c->model;
-  KParams &k = c->kp;
+static void fill_kparams(const HostModel &m, KParams &k) {
   k.rows = m.rows;
   k.cols = m.cols;
   k.realcols = m.realcols;
@@ -335,41 +345,42 @@ struct Batch {
 };
 
 // The ground tables [3][H] of road `r` into `dst`.
-static void copy_road_tables(isx_context *c, const isx_road &r, float *dst) {
-  std::lock_guard<std::mutex> lock(c->road_cache_mutex);
+static void copy_road_tables(const HostModel &m, Initialized &I, const isx_road &r, float *dst) {
+  std::lock_guard<std::mutex> lock(I.road_cache_mutex);
   RoadKey key{r.vhor, r.camera_tilt, r.camera_height, r.alpha_ground};
-  auto it = c->road_cache.find(key);
-  if (it == c->road_cache.end()) {
-    if (c->road_cache.size() > 64) c->road_cache.clear();
-    std::vector<float> t((size_t)3 * c->model.rows);
-    c->model.ground_tables(r, t.data());
-    it = c->road_cache.emplace(key, std::move(t)).first;
+  auto it = I.road_cache.find(key);
+  if (it == I.road_cache.end()) {
+    if (I.road_cache.size() > 64) I.road_cache.clear();
+    std::vector<float> t((size_t)3 * m.rows);
+    m.ground_tables(r, t.data());
+    it = I.road_cache.emplace(key, std::move(t)).first;
   }
-  std::memcpy(dst, it->second.data(), sizeof(float) * 3 * c->model.rows);
+  std::memcpy(dst, it->second.data(), sizeof(float) * 3 * m.rows);
 }
 
 // The ground tables and flipped horizon rows of `n` roads into staging buffer `stage`.
-static void fill_stage(isx_context *c, int stage, const isx_road *roads, int n) {
-  const int H = c->kp.rows;
-  float *hg = c->h_ground + (size_t)stage * c->chunk * 3 * H;
-  int *hv = c->h_vhor + (size_t)stage * c->chunk;
+static void fill_stage(const HostModel &m, Initialized &I, int stage, const isx_road *roads, int n) {
+  const int H = I.kp.rows;
+  float *hg = I.h_ground + (size_t)stage * I.chunk * 3 * H;
+  int *hv = I.h_vhor + (size_t)stage * I.chunk;
   for (int i = 0; i < n; i++) {
-    copy_road_tables(c, roads[i], hg + (size_t)i * 3 * H);
+    copy_road_tables(m, I, roads[i], hg + (size_t)i * 3 * H);
     hv[i] = H - roads[i].vhor - 1;  // Stixels.cu:377
   }
 }
 
 // The staged road tables of `n` frames -> the next slot of the road ring, on `st`.  Returns the slot or an error.
 static int send_road_tables(isx_context *c, int stage, int n, cudaStream_t st) {
-  const int H = c->kp.rows;
-  const float *hg = c->h_ground + (size_t)stage * c->chunk * 3 * H;
-  const int *hv = c->h_vhor + (size_t)stage * c->chunk;
-  const int rslot = (int)(c->road_next++ % kRoadSlots);
-  const isx_context::RoadSlot &rd = c->roads[rslot];
+  Initialized &I = *c->init;
+  const int H = I.kp.rows;
+  const float *hg = I.h_ground + (size_t)stage * I.chunk * 3 * H;
+  const int *hv = I.h_vhor + (size_t)stage * I.chunk;
+  const int rslot = (int)(I.road_next++ % kRoadSlots);
+  const Initialized::RoadSlot &rd = I.roads[rslot];
   ISX_TRY(c, cudaStreamWaitEvent(st, rd.ev_free, 0));
   ISX_TRY(c, cudaMemcpyAsync(rd.ground, hg, sizeof(float) * 3 * H * n, cudaMemcpyHostToDevice, st));
   ISX_TRY(c, cudaMemcpyAsync(rd.vhor, hv, sizeof(int) * n, cudaMemcpyHostToDevice, st));
-  ISX_TRY(c, cudaEventRecord(c->ev_stage_done[stage], st));
+  ISX_TRY(c, cudaEventRecord(I.ev_stage_done[stage], st));
   return rslot;
 }
 
@@ -377,10 +388,10 @@ static int send_road_tables(isx_context *c, int stage, int n, cudaStream_t st) {
 // in the reference) go through a pinned staging buffer to the next slot of the road ring on stream `st`, behind the
 // emission that last read that slot (kRoadSlots chunks ago).  Returns the slot (>= 0) or an error (< 0).
 static int stage_road_tables(isx_context *c, const isx_road *roads, int n, cudaStream_t st) {
-  const int stage = (int)(c->stage_next++ % kStageSlots);
+  const int stage = (int)(c->init->stage_next++ % kStageSlots);
   // the copy that read this staging buffer kStageSlots chunks ago must be done (a never-recorded event is complete)
-  ISX_TRY(c, cudaEventSynchronize(c->ev_stage_done[stage]));
-  fill_stage(c, stage, roads, n);
+  ISX_TRY(c, cudaEventSynchronize(c->init->ev_stage_done[stage]));
+  fill_stage(c->model, *c->init, stage, roads, n);
   return send_road_tables(c, stage, n, st);
 }
 
@@ -390,8 +401,11 @@ static int stage_road_tables(isx_context *c, const isx_road *roads, int n, cudaS
 // of the chunk go to pinned memory, a host function fills the staging buffer from them (no CUDA calls; the ground
 // tables of a road are cached, and video frames mostly keep their road), and the usual copy takes it to the road ring.
 // The reuse of the staging buffer is ordered on the stream too, so the calling thread never waits.
+// The host function runs on a driver thread and reads the Initialized it was enqueued for: that struct is only
+// released after a device synchronise (CudaResources), so it outlives every such call.
 struct StageFill {
-  isx_context *c;
+  const HostModel *m;
+  Initialized *I;
   int stage, n;
   bool timed;   // isx_set_profiling at enqueue time: the host function's time goes to isx_get_road_fill_time
 };
@@ -399,21 +413,22 @@ struct StageFill {
 static void CUDART_CB fill_stage_from_roads(void *arg) {
   const StageFill p = *static_cast<StageFill *>(arg);
   delete static_cast<StageFill *>(arg);
-  isx_context *c = p.c;
+  Initialized &I = *p.I;
   const auto t0 = std::chrono::steady_clock::now();
-  fill_stage(c, p.stage, c->h_stage_roads + (size_t)p.stage * c->chunk, p.n);
+  fill_stage(*p.m, I, p.stage, I.h_stage_roads + (size_t)p.stage * I.chunk, p.n);
   if (p.timed) {
-    c->host_fill_ns += std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count();
-    c->host_fill_calls++;
+    I.host_fill_ns += std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count();
+    I.host_fill_calls++;
   }
 }
 
 static int stage_device_road_tables(isx_context *c, const isx_road *d_roads, int n, cudaStream_t st) {
-  const int stage = (int)(c->stage_next++ % kStageSlots);
-  ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_stage_done[stage], 0));
-  ISX_TRY(c, cudaMemcpyAsync(c->h_stage_roads + (size_t)stage * c->chunk, d_roads, sizeof(isx_road) * n,
+  Initialized &I = *c->init;
+  const int stage = (int)(I.stage_next++ % kStageSlots);
+  ISX_TRY(c, cudaStreamWaitEvent(st, I.ev_stage_done[stage], 0));
+  ISX_TRY(c, cudaMemcpyAsync(I.h_stage_roads + (size_t)stage * I.chunk, d_roads, sizeof(isx_road) * n,
                              cudaMemcpyDeviceToHost, st));
-  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{c, stage, n, c->profiling}));
+  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{&c->model, &I, stage, n, c->profiling}));
   return send_road_tables(c, stage, n, st);
 }
 
@@ -425,32 +440,33 @@ static int stage_device_road_tables(isx_context *c, const isx_road *d_roads, int
 // copy stream never waits for any of it, and the calling thread does not wait either.  Returns the ring slot or an
 // error.
 static int stage_estimated_road_tables(isx_context *c, const Batch &b, int first, int n, const float *d_disp) {
-  const int H = c->kp.rows;
-  cudaStream_t st = c->s_tables;
-  const int stage = (int)(c->stage_next++ % kStageSlots);
+  Initialized &I = *c->init;
+  const int H = I.kp.rows;
+  cudaStream_t st = I.s_tables;
+  const int stage = (int)(I.stage_next++ % kStageSlots);
   // the staging slot is free once the pull that last read it is done (the road stream is ordered behind st)
-  ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_stage_done[stage], 0));
+  ISX_TRY(c, cudaStreamWaitEvent(st, I.ev_stage_done[stage], 0));
   std::string msg;
   if (int rc = road_enqueue_batch(b.estimate.road, st, n, d_disp, first == 0 ? b.estimate.fallback : nullptr,
-                                  b.d_estimates + first, b.d_roads + first, c->m_stage_roads + (size_t)stage * c->chunk,
+                                  b.d_estimates + first, b.d_roads + first, I.m_stage_roads + (size_t)stage * I.chunk,
                                   msg, b.estimate.carry))
     return fail(c, rc, msg);
-  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{c, stage, n, c->profiling}));
-  const int rslot = (int)(c->road_next++ % kRoadSlots);
-  const isx_context::RoadSlot &rd = c->roads[rslot];
+  ISX_TRY(c, cudaLaunchHostFunc(st, fill_stage_from_roads, new StageFill{&c->model, &I, stage, n, c->profiling}));
+  const int rslot = (int)(I.road_next++ % kRoadSlots);
+  const Initialized::RoadSlot &rd = I.roads[rslot];
   ISX_TRY(c, cudaStreamWaitEvent(st, rd.ev_free, 0));
-  launch_pull_road_tables(c->m_ground + (size_t)stage * c->chunk * 3 * H, rd.ground, (size_t)n * 3 * H,
-                          c->m_vhor + (size_t)stage * c->chunk, rd.vhor, n, st);
+  launch_pull_road_tables(I.m_ground + (size_t)stage * I.chunk * 3 * H, rd.ground, (size_t)n * 3 * H,
+                          I.m_vhor + (size_t)stage * I.chunk, rd.vhor, n, st);
   ISX_TRY(c, cudaGetLastError());
-  ISX_TRY(c, cudaEventRecord(c->ev_stage_done[stage], st));
+  ISX_TRY(c, cudaEventRecord(I.ev_stage_done[stage], st));
   return rslot;
 }
 
 // The intermediates of the chunk in set `slot` with its road tables in slot `road_slot` of the road ring.
 static BatchBuffers chunk_buffers(const isx_context *c, int slot, int road_slot) {
-  const isx_context::ChunkSet &cs = c->sets[slot];
-  const isx_context::RoadSlot &rd = c->roads[road_slot];
-  BatchBuffers b = c->buf;
+  const Initialized::ChunkSet &cs = c->init->sets[slot];
+  const Initialized::RoadSlot &rd = c->init->roads[road_slot];
+  BatchBuffers b = c->init->buf;
   b.ground = rd.ground; b.vhor = rd.vhor; b.stat = cs.stat;
   b.records_b = cs.records_b; b.dp = cs.dp; b.pm = cs.pm;
   b.joined = cs.joined; b.object_lut = cs.object_lut; b.col_flags = cs.col_flags;
@@ -463,7 +479,7 @@ static void record_prof_event(isx_context *c, std::vector<cudaEvent_t> &pool, si
   if (!c->profiling) return;
   if (used >= pool.size()) {
     cudaEvent_t e;
-    cudaEventCreate(&e);
+    if (c->init->res.event(&e, cudaEventDefault) != cudaSuccess) return;
     pool.push_back(e);
   }
   cudaEventRecord(pool[used++], st);
@@ -480,27 +496,28 @@ static void record_prof_event(isx_context *c, std::vector<cudaEvent_t> &pool, si
 // measured with isx_get_chunk_trace).  Otherwise the given `roads` are staged here, behind the waits for the set.
 static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const float *d_disp, const int32_t *d_seg,
                          const isx_road *roads, int slot, int road_slot, const ResultDest &out) {
-  const KParams &kp = c->kp;
+  Initialized &I = *c->init;
+  const KParams &kp = I.kp;
   const int H = kp.rows, C = kp.realcols;
-  cudaStream_t st = c->s_tables, s = c->s_compute, se = c->s_emit;
+  cudaStream_t st = I.s_tables, s = I.s_compute, se = I.s_emit;
   // the emission of the chunk that used this set two chunks ago must be done with it (it follows that chunk's DP)
-  ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_emit_done[slot], 0));
+  ISX_TRY(c, cudaStreamWaitEvent(st, I.ev_emit_done[slot], 0));
   // ISX_OVERLAP_TABLES=0: the table build waits for the DP of the chunk before it (one kernel at a time on the SMs)
-  if (!c->overlap_tables) ISX_TRY(c, cudaStreamWaitEvent(st, c->ev_dp_done[slot ^ 1], 0));
+  if (!I.overlap_tables) ISX_TRY(c, cudaStreamWaitEvent(st, I.ev_dp_done[slot ^ 1], 0));
   if (road_slot < 0) {
     road_slot = stage_road_tables(c, roads, n, st);
     if (road_slot < 0) return road_slot;
   }
   BatchBuffers b = chunk_buffers(c, slot, road_slot);
   ISX_TRY(c, cudaMemsetAsync(b.error_flag, 0, sizeof(int) * n, st));  // the error words of THIS chunk's frames
-  isx_context::ResultSet &R = c->rs[c->cur];
+  Initialized::ResultSet &R = I.rs[I.cur];
   b.disparity = d_disp;
   b.segmentation = d_seg;
   b.sections = R.d_sections + (size_t)first * C * kMaxSections;
   b.n_sections = R.d_nsections + (size_t)first * C;
   // profiling events per chunk: 0 join | 1 frame tables | 2 column tables + LUT | 3 end (s_tables); 4 dp | 5 dp end
   //                             (s_compute); 6 backtrack + collect | 7 grouping + pack | 8 end (s_emit)
-  auto mark = [&](cudaStream_t st) { record_prof_event(c, c->prof_events, c->prof_used, st); };
+  auto mark = [&](cudaStream_t st) { record_prof_event(c, I.prof_events, I.prof_used, st); };
   mark(st);
   launch_join_columns(kp, b, n, st);
   mark(st);
@@ -508,21 +525,21 @@ static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const 
   mark(st);
   launch_column_tables(kp, b, n, st);
   mark(st);
-  ISX_TRY(c, cudaEventRecord(c->ev_tab_done[slot], st));
-  ISX_TRY(c, cudaStreamWaitEvent(s, c->ev_tab_done[slot], 0));
+  ISX_TRY(c, cudaEventRecord(I.ev_tab_done[slot], st));
+  ISX_TRY(c, cudaStreamWaitEvent(s, I.ev_tab_done[slot], 0));
   mark(s);
   launch_dp(kp, b, n, pairwise, s);
   {
     const unsigned long long nt = (unsigned long long)(H + 31) / 32;
-    c->dp_units_total += (unsigned long long)n * C * (nt * (nt + 1) / 2);
+    I.dp_units_total += (unsigned long long)n * C * (nt * (nt + 1) / 2);
     const char *ex = std::getenv("ISX_UNARY_EXHAUSTIVE");
     // the pruning kernels count on the device
     const bool walks_all = (pairwise && !pairwise_walk_used(n * C, b.qrows != nullptr)) || (!pairwise && ex && std::atoi(ex) != 0);
-    c->dp_units_pairwise += walks_all ? (unsigned long long)n * C * (nt * (nt + 1) / 2) : 0;
+    I.dp_units_pairwise += walks_all ? (unsigned long long)n * C * (nt * (nt + 1) / 2) : 0;
   }
   mark(s);
-  ISX_TRY(c, cudaEventRecord(c->ev_dp_done[slot], s));
-  ISX_TRY(c, cudaStreamWaitEvent(se, c->ev_dp_done[slot], 0));
+  ISX_TRY(c, cudaEventRecord(I.ev_dp_done[slot], s));
+  ISX_TRY(c, cudaStreamWaitEvent(se, I.ev_dp_done[slot], 0));
   mark(se);
   launch_emit(kp, b, n, pairwise, se);
   mark(se);
@@ -532,8 +549,8 @@ static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const 
     a.sections = b.sections; a.n_sections = b.n_sections;
     a.cand_count = b.cand_count; a.cand_idx = b.cand_idx; a.cand_label = b.cand_label;
     a.err = b.error_flag; a.col_offset = b.pack_offset;
-    a.inst_out = R.d_inst + (size_t)first * c->inst_cap; a.inst_count_out = R.d_inst_count + first;
-    a.inst_cap = c->inst_cap; a.cursors = R.d_cursors;
+    a.inst_out = R.d_inst + (size_t)first * I.inst_cap; a.inst_count_out = R.d_inst_count + first;
+    a.inst_cap = I.inst_cap; a.cursors = R.d_cursors;
     a.h_padded = out.direct_sections ? out.direct_sections + (size_t)first * C * kMaxSections : nullptr;
     a.h_sections = R.m_sections; a.h_sections_cap = out.stay_on_device ? 0 : R.sections_cap;
     a.h_inst = R.m_inst; a.h_inst_cap = out.stay_on_device ? 0 : R.inst_cap;
@@ -541,14 +558,14 @@ static int enqueue_chunk(isx_context *c, bool pairwise, int first, int n, const 
     launch_pack(kp, a, n, se);
   }
   mark(se);
-  ISX_TRY(c, cudaEventRecord(c->ev_emit_done[slot], se));
-  ISX_TRY(c, cudaEventRecord(c->roads[road_slot].ev_free, se));
+  ISX_TRY(c, cudaEventRecord(I.ev_emit_done[slot], se));
+  ISX_TRY(c, cudaEventRecord(I.roads[road_slot].ev_free, se));
   ISX_TRY(c, cudaGetLastError());
-  c->last_chunk_first = first;
-  c->last_chunk_n = n;
-  c->last_pairwise = pairwise;
-  c->last_set = slot;
-  c->last_road_slot = road_slot;
+  I.last_chunk_first = first;
+  I.last_chunk_n = n;
+  I.last_pairwise = pairwise;
+  I.last_set = slot;
+  I.last_road_slot = road_slot;
   return ISX_OK;
 }
 
@@ -571,22 +588,22 @@ static isx_section *device_view_of(isx_section *sections) {
 // Every batch starts its packed result arrays from the front (ordered on the emission stream behind the packing of
 // whatever batch used this result set before).
 static int begin_batch(isx_context *c) {
-  ISX_TRY(c, cudaMemsetAsync(c->rs[c->cur].d_cursors, 0, 2 * sizeof(int), c->s_emit));
+  ISX_TRY(c, cudaMemsetAsync(c->init->rs[c->init->cur].d_cursors, 0, 2 * sizeof(int), c->init->s_emit));
   return ISX_OK;
 }
 
 // The result arrays of one batch: padded device arrays + packed arrays in mapped pinned host memory.
-static int alloc_result_set(isx_context *c, int i) {
-  isx_context::ResultSet &R = c->rs[i];
-  if (R.allocated) return ISX_OK;
-  const size_t C = c->kp.realcols, MB = c->max_batch;
-  ISX_TRY(c, dev_alloc(c, &R.d_sections, MB * C * kMaxSections));
+static int alloc_result_set(isx_context *c, Initialized &I, int i) {
+  Initialized::ResultSet &R = I.rs[i];
+  if (R.m_frames) return ISX_OK;   // set last below: the set is complete
+  const size_t C = I.kp.realcols, MB = I.max_batch;
+  ISX_TRY(c, dev_alloc(I, &R.d_sections, MB * C * kMaxSections));
   // entries after a column's terminator are never written: start them from zero
   ISX_TRY(c, cudaMemset(R.d_sections, 0, MB * C * kMaxSections * sizeof(isx_section)));
-  ISX_TRY(c, dev_alloc(c, &R.d_nsections, MB * C));
-  ISX_TRY(c, dev_alloc(c, &R.d_inst, MB * (size_t)c->inst_cap));
-  ISX_TRY(c, dev_alloc(c, &R.d_inst_count, MB));
-  ISX_TRY(c, dev_alloc(c, &R.d_cursors, 2));
+  ISX_TRY(c, dev_alloc(I, &R.d_nsections, MB * C));
+  ISX_TRY(c, dev_alloc(I, &R.d_inst, MB * (size_t)I.inst_cap));
+  ISX_TRY(c, dev_alloc(I, &R.d_inst_count, MB));
+  ISX_TRY(c, dev_alloc(I, &R.d_cursors, 2));
   ISX_TRY(c, cudaMemset(R.d_cursors, 0, 2 * sizeof(int)));
   // Packed arrays: sized for `budget` stixels per column on average over a batch (the pairwise model yields about
   // ten per column on street scenes, the unary model with its 1/n prior sixty to seventy; the capacity of the
@@ -594,76 +611,50 @@ static int alloc_result_set(isx_context *c, int i) {
   // Frames taller than 1024 rows have proportionally more stixels per column (synthetic unary frames: 80 at 1280
   // rows, 129 at 2047): the budget grows with the rows there, up to the capacity of 200.
   size_t budget = 100;
-  if (c->kp.rows > kShortRows) budget = ((size_t)c->kp.rows * 100 + kShortRows - 1) / kShortRows;
+  if (I.kp.rows > kShortRows) budget = ((size_t)I.kp.rows * 100 + kShortRows - 1) / kShortRows;
   if (const char *e = std::getenv("ISX_PACK_BUDGET")) budget = std::atoi(e) > 0 ? (size_t)std::atoi(e) : budget;
   budget = budget < (size_t)kMaxSections ? budget : (size_t)kMaxSections;
   R.sections_cap = R.inst_cap = (int)(MB * C * budget);
-  const unsigned flags = cudaHostAllocMapped | cudaHostAllocPortable;
-  ISX_TRY(c, cudaHostAlloc(&R.h_sections, sizeof(isx_section) * (size_t)R.sections_cap, flags));
-  ISX_TRY(c, cudaHostAlloc(&R.h_inst, sizeof(isx_instance) * (size_t)R.inst_cap, flags));
-  ISX_TRY(c, cudaHostAlloc(&R.h_counts, sizeof(int) * MB * C, flags));
-  ISX_TRY(c, cudaHostAlloc(&R.h_frames, sizeof(isx_packed_frame) * MB, flags));
-  ISX_TRY(c, cudaHostGetDevicePointer(&R.m_sections, R.h_sections, 0));
-  ISX_TRY(c, cudaHostGetDevicePointer(&R.m_inst, R.h_inst, 0));
-  ISX_TRY(c, cudaHostGetDevicePointer(&R.m_counts, R.h_counts, 0));
-  ISX_TRY(c, cudaHostGetDevicePointer(&R.m_frames, R.h_frames, 0));
+  ISX_TRY(c, mapped_alloc(I, &R.h_sections, &R.m_sections, (size_t)R.sections_cap));
+  ISX_TRY(c, mapped_alloc(I, &R.h_inst, &R.m_inst, (size_t)R.inst_cap));
+  ISX_TRY(c, mapped_alloc(I, &R.h_counts, &R.m_counts, MB * C));
+  ISX_TRY(c, mapped_alloc(I, &R.h_frames, &R.m_frames, MB));
   std::memset(R.h_frames, 0, sizeof(isx_packed_frame) * MB);
-  R.allocated = true;
-  return ISX_OK;
-}
-
-// The estimates and roads of a batch with estimated roads (mapped pinned, written by resolve_kernel), and the device
-// addresses of the staging its road steps write and read.
-static int alloc_road_results(isx_context *c, int i) {
-  isx_context::ResultSet &R = c->rs[i];
-  const size_t MB = c->max_batch;
-  const unsigned flags = cudaHostAllocMapped | cudaHostAllocPortable;
-  if (!R.h_est) {
-    ISX_TRY(c, cudaHostAlloc(&R.h_est, sizeof(isx_road_estimate) * MB, flags));
-    ISX_TRY(c, cudaHostGetDevicePointer(&R.m_est, R.h_est, 0));
-  }
-  if (!R.h_roads) {
-    ISX_TRY(c, cudaHostAlloc(&R.h_roads, sizeof(isx_road) * MB, flags));
-    ISX_TRY(c, cudaHostGetDevicePointer(&R.m_roads, R.h_roads, 0));
-  }
-  if (!c->m_ground) {
-    ISX_TRY(c, cudaHostGetDevicePointer(&c->m_ground, c->h_ground, 0));
-    ISX_TRY(c, cudaHostGetDevicePointer(&c->m_vhor, c->h_vhor, 0));
-    ISX_TRY(c, cudaHostGetDevicePointer(&c->m_stage_roads, c->h_stage_roads, 0));
-  }
   return ISX_OK;
 }
 
 // Results of every enqueued chunk become visible to work ordered after this on isx_stream() (the table stream: the
 // first stream of the pipeline, where a caller's producers of device inputs and consumers of results run).
 static int join_emit_stream(isx_context *c) {
-  ISX_TRY(c, cudaStreamWaitEvent(c->s_tables, c->ev_emit_done[c->last_set], 0));
-  c->emit_join_pending = false;
+  ISX_TRY(c, cudaStreamWaitEvent(c->init->s_tables, c->init->ev_emit_done[c->init->last_set], 0));
+  c->init->emit_join_pending = false;
   return ISX_OK;
 }
 // isx_compute_batch_device leaves the join to whoever touches the results next (or to isx_flush), so that the
 // first kernels of a following batch do not wait for the emission tail of this one.
-static int ensure_joined(isx_context *c) { return c->emit_join_pending ? join_emit_stream(c) : ISX_OK; }
+static int ensure_joined(isx_context *c) { return c->init->emit_join_pending ? join_emit_stream(c) : ISX_OK; }
 
 static int check_ready(isx_context *c) {
   if (!c) return fail(nullptr, ISX_ERR_INVALID_ARGUMENT, "null handle");
-  if (!c->initialized) return fail(c, ISX_ERR_NOT_INITIALIZED, "Initialize() has not been called");
+  if (!c->init) return fail(c, ISX_ERR_NOT_INITIALIZED, "Initialize() has not been called");
   cudaError_t e = cudaSetDevice(c->device);
   if (e != cudaSuccess) return fail(c, ISX_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
   return ISX_OK;
 }
 
 static size_t narrow_seg_elems(const isx_context *c) {
-  const size_t used = (size_t)(c->kp.rows + kDownsample - 1) / kDownsample;
-  return (size_t)c->kp.realcols * c->kp.n_channels * (used < (size_t)c->kp.hs2 ? used : (size_t)c->kp.hs2);
+  Initialized &I = *c->init;
+  const size_t used = (size_t)(I.kp.rows + kDownsample - 1) / kDownsample;
+  return (size_t)I.kp.realcols * I.kp.n_channels * (used < (size_t)I.kp.hs2 ? used : (size_t)I.kp.hs2);
 }
 
 static int ensure_narrow_staging(isx_handle h) {
-  if (h->d_in_disp16[0]) return ISX_OK;
-  const size_t hw = (size_t)h->kp.rows * h->kp.cols, ch = h->chunk;
+  Initialized &I = *h->init;
+  if (I.d_in_seg16[1]) return ISX_OK;
+  const size_t hw = (size_t)I.kp.rows * I.kp.cols, ch = I.chunk;
   for (int i = 0; i < 2; i++) {
-    ISX_TRY(h, dev_alloc(h, &h->d_in_disp16[i], ch * hw));
-    ISX_TRY(h, dev_alloc(h, &h->d_in_seg16[i], ch * narrow_seg_elems(h)));
+    ISX_TRY(h, dev_alloc(I, &I.d_in_disp16[i], ch * hw));
+    ISX_TRY(h, dev_alloc(I, &I.d_in_seg16[i], ch * narrow_seg_elems(h)));
   }
   return ISX_OK;
 }
@@ -674,9 +665,10 @@ static int ensure_narrow_staging(isx_handle h) {
 // `caller_waits`: a synchronous host call -- the kernels of the last chunk run with nothing beside them while the
 // caller waits, so the tail goes in quarter pieces like the head.
 static int enqueue_batch(isx_handle h, int pairwise, int n, const Batch &b, bool caller_waits) {
+  Initialized &I = *h->init;
   const HostInputs &in = b.host;
   const bool host = b.d_disparity == nullptr;
-  const size_t hw = (size_t)h->kp.rows * h->kp.cols, se = seg_elems(h), se16 = narrow_seg_elems(h);
+  const size_t hw = (size_t)I.kp.rows * I.kp.cols, se = seg_elems(h), se16 = narrow_seg_elems(h);
   if (in.narrow()) {
     if (hw % 8 != 0) return fail(h, ISX_ERR_UNSUPPORTED, "the uint16 disparity path needs rows*cols to be a multiple of 8");
     if (int rc = ensure_narrow_staging(h)) return rc;
@@ -684,11 +676,11 @@ static int enqueue_batch(isx_handle h, int pairwise, int n, const Batch &b, bool
   if (int rc = begin_batch(h)) return rc;
   // The slots keep alternating across batches, so that the first copy of a pipelined batch only waits for the
   // second-to-last chunk of the batch before it.
-  int slot = h->host_slot;
+  int slot = I.host_slot;
   int cn = 0;
-  const int chunk = pairwise ? h->chunk : h->chunk_unary;
-  h->last_launch_frames = chunk;
-  const bool pipeline_idle = h->submitted == h->waited;
+  const int chunk = pairwise ? I.chunk : I.chunk_unary;
+  I.last_launch_frames = chunk;
+  const bool pipeline_idle = I.submitted == I.waited;
   for (int first = 0; first < n; first += cn) {
     cn = (n - first) < chunk ? (n - first) : chunk;
     // Where each road source is staged is part of its timing: given roads go in front of a host chunk's images (on
@@ -707,60 +699,60 @@ static int enqueue_batch(isx_handle h, int pairwise, int n, const Batch &b, bool
       if ((head || tail) && chunk >= 32) cn = cn < chunk / 4 ? cn : chunk / 4;
       // H2D of this chunk on the copy stream, once the table build that last read this input slot is done (a
       // device-side wait: the host thread runs ahead)
-      ISX_TRY(h, cudaStreamWaitEvent(h->s_h2d, h->ev_in_free[slot], 0));
-      record_prof_event(h, h->prof_h2d, h->prof_h2d_used, h->s_h2d);
+      ISX_TRY(h, cudaStreamWaitEvent(I.s_h2d, I.ev_in_free[slot], 0));
+      record_prof_event(h, I.prof_h2d, I.prof_h2d_used, I.s_h2d);
       if (b.roads) {
-        road_slot = stage_road_tables(h, b.roads + first, cn, h->s_h2d);
+        road_slot = stage_road_tables(h, b.roads + first, cn, I.s_h2d);
         if (road_slot < 0) return road_slot;
       }
       if (in.narrow()) {
-        ISX_TRY(h, cudaMemcpyAsync(h->d_in_disp16[slot], in.disparity16 + first * hw, sizeof(uint16_t) * hw * cn,
-                                   cudaMemcpyHostToDevice, h->s_h2d));
-        ISX_TRY(h, cudaMemcpyAsync(h->d_in_seg16[slot], in.segmentation16 + first * se16, sizeof(int16_t) * se16 * cn,
-                                   cudaMemcpyHostToDevice, h->s_h2d));
+        ISX_TRY(h, cudaMemcpyAsync(I.d_in_disp16[slot], in.disparity16 + first * hw, sizeof(uint16_t) * hw * cn,
+                                   cudaMemcpyHostToDevice, I.s_h2d));
+        ISX_TRY(h, cudaMemcpyAsync(I.d_in_seg16[slot], in.segmentation16 + first * se16, sizeof(int16_t) * se16 * cn,
+                                   cudaMemcpyHostToDevice, I.s_h2d));
       } else {
-        ISX_TRY(h, cudaMemcpyAsync(h->d_in_disp[slot], in.disparity + first * hw, sizeof(float) * hw * cn,
-                                   cudaMemcpyHostToDevice, h->s_h2d));
+        ISX_TRY(h, cudaMemcpyAsync(I.d_in_disp[slot], in.disparity + first * hw, sizeof(float) * hw * cn,
+                                   cudaMemcpyHostToDevice, I.s_h2d));
         // Only the first rows/8 entries of every [rows_power2_segmentation] channel row are ever read
         // (StixelsKernels.cu:393-405, 462-468 index v/8 with v < rows); the zero padding of FlipAndPad does not
         // travel: a 2-D copy of the used part, the rest of the staging buffer stays zero from isx_initialize.
-        const size_t hs2 = (size_t)h->kp.hs2;
-        size_t used = (size_t)(h->kp.rows + kDownsample - 1) / kDownsample;
+        const size_t hs2 = (size_t)I.kp.hs2;
+        size_t used = (size_t)(I.kp.rows + kDownsample - 1) / kDownsample;
         used = used < hs2 ? used : hs2;
-        ISX_TRY(h, cudaMemcpy2DAsync(h->d_in_seg[slot], hs2 * sizeof(int32_t), in.segmentation + first * se,
+        ISX_TRY(h, cudaMemcpy2DAsync(I.d_in_seg[slot], hs2 * sizeof(int32_t), in.segmentation + first * se,
                                      hs2 * sizeof(int32_t), used * sizeof(int32_t), (se / hs2) * cn,
-                                     cudaMemcpyHostToDevice, h->s_h2d));
+                                     cudaMemcpyHostToDevice, I.s_h2d));
       }
-      record_prof_event(h, h->prof_h2d, h->prof_h2d_used, h->s_h2d);
-      ISX_TRY(h, cudaEventRecord(h->ev_in_ready[slot], h->s_h2d));
-      ISX_TRY(h, cudaStreamWaitEvent(h->s_tables, h->ev_in_ready[slot], 0));
+      record_prof_event(h, I.prof_h2d, I.prof_h2d_used, I.s_h2d);
+      ISX_TRY(h, cudaEventRecord(I.ev_in_ready[slot], I.s_h2d));
+      ISX_TRY(h, cudaStreamWaitEvent(I.s_tables, I.ev_in_ready[slot], 0));
       if (in.narrow())
-        launch_widen_inputs(h->kp, h->d_in_disp16[slot], in.scale, h->d_in_seg16[slot], h->d_in_disp[slot],
-                            h->d_in_seg[slot], cn, h->s_tables);
-      d_disp = h->d_in_disp[slot];
-      d_seg = h->d_in_seg[slot];
+        launch_widen_inputs(I.kp, I.d_in_disp16[slot], in.scale, I.d_in_seg16[slot], I.d_in_disp[slot],
+                            I.d_in_seg[slot], cn, I.s_tables);
+      d_disp = I.d_in_disp[slot];
+      d_seg = I.d_in_seg[slot];
     } else {
       d_disp = b.d_disparity + first * hw;
       d_seg = b.d_segmentation + first * se;
     }
     if (!b.roads) {
       road_slot = b.estimate.road ? stage_estimated_road_tables(h, b, first, cn, d_disp)
-                                  : stage_device_road_tables(h, b.d_roads + first, cn, h->s_tables);
+                                  : stage_device_road_tables(h, b.d_roads + first, cn, I.s_tables);
       if (road_slot < 0) return road_slot;
     }
     if (int rc = enqueue_chunk(h, pairwise != 0, first, cn, d_disp, d_seg, b.roads ? b.roads + first : nullptr, slot,
                                road_slot, b.out))
       return rc;
-    ISX_TRY(h, cudaEventRecord(h->ev_in_free[slot], h->s_tables));   // the inputs are read by the table build only
+    ISX_TRY(h, cudaEventRecord(I.ev_in_free[slot], I.s_tables));   // the inputs are read by the table build only
     slot ^= 1;
   }
-  h->host_slot = slot;
-  h->emit_join_pending = true;  // joined lazily: isx_flush / isx_synchronize / any result access
+  I.host_slot = slot;
+  I.emit_join_pending = true;  // joined lazily: isx_flush / isx_synchronize / any result access
   // the batch's results replace the last ones: the export reads its roads
-  h->last_batch = n;
-  if (b.roads) h->last_roads.assign(b.roads, b.roads + n);
-  else h->last_roads.clear();
-  h->last_roads_dev = b.d_roads;
+  I.last_batch = n;
+  if (b.roads) I.last_roads.assign(b.roads, b.roads + n);
+  else I.last_roads.clear();
+  I.last_roads_dev = b.d_roads;
   return ISX_OK;
 }
 
@@ -807,12 +799,7 @@ int isx_create(isx_handle *out, int device) {
   return ISX_OK;
 }
 
-int isx_destroy(isx_handle h) {
-  if (!h) return ISX_OK;
-  if (h->initialized) isx_finish(h);
-  delete h;
-  return ISX_OK;
-}
+int isx_destroy(isx_handle h) { delete h; return ISX_OK; }
 
 int isx_set_config(isx_handle h, const isx_config *cfg) {
   if (!h || !cfg) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
@@ -840,8 +827,9 @@ int isx_set_segmentation_parameters(isx_handle h, int classes, int instance_chan
 int isx_set_clustering_parameters(isx_handle h, float eps, int min_pts, int size_filter) {
   if (!h) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null handle");
   h->model.eps = eps; h->model.min_pts = min_pts; h->model.size_filter = size_filter;
-  if (h->initialized) {  // the reference writes these straight into m_params (Stixels.cu:395-400)
-    h->kp.eps_cluster = eps; h->kp.min_pts = min_pts; h->kp.size_filter = size_filter;
+  if (h->init) {  // the reference writes these straight into m_params (Stixels.cu:395-400)
+    KParams &kp = h->init->kp;
+    kp.eps_cluster = eps; kp.min_pts = min_pts; kp.size_filter = size_filter;
   }
   return ISX_OK;
 }
@@ -890,7 +878,7 @@ int isx_set_model_parameters(isx_handle h, int column_step, int median_join, flo
 
 int isx_initialize(isx_handle h, int max_batch) {
   if (!h) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null handle");
-  if (h->initialized) return fail(h, ISX_ERR_INVALID_ARGUMENT, "already initialized: call Finish() first");
+  if (h->init) return fail(h, ISX_ERR_INVALID_ARGUMENT, "already initialized: call Finish() first");
   if (max_batch < 1) return fail(h, ISX_ERR_INVALID_ARGUMENT, "max_batch must be >= 1");
   HostModel &m = h->model;
   if (m.rows <= 0 || m.cols <= 0 || m.max_dis <= 0 || m.column_step <= 0)
@@ -904,11 +892,14 @@ int isx_initialize(isx_handle h, int max_batch) {
   if (m.column_step > 16) return fail(h, ISX_ERR_UNSUPPORTED, "column_step > 16 is not supported");
   ISX_TRY(h, cudaSetDevice(h->device));
   m.derive();
-  fill_kparams(h);
-  const KParams &kp = h->kp;
+  // Built here and moved onto the handle only on success: every early return releases what was acquired.
+  auto init = std::make_unique<Initialized>(h->device);
+  Initialized &I = *init;
+  fill_kparams(m, I.kp);
+  const KParams &kp = I.kp;
   const size_t H = kp.rows, W = kp.cols, C = kp.realcols, D = kp.max_dis;
   if (C == 0) return fail(h, ISX_ERR_INVALID_ARGUMENT, "no stixel columns");
-  h->max_batch = max_batch;
+  I.max_batch = max_batch;
   // Frames per launch.  Every DP launch ends with a partly filled wave, so few large launches beat many small
   // ones; but the copies of a host batch only overlap kernels of OTHER chunks.  Measured (B200, 64-frame batches,
   // frames/s resident | end to end): unary 16 / 32 / 64 frames per launch = 7095 | 4614, 7999 | 4628, 8083 | 4525;
@@ -926,13 +917,13 @@ int isx_initialize(isx_handle h, int max_batch) {
     chunk_unary = chunk < 32 ? chunk : 32;
   }
   if (const char *e = std::getenv("ISX_CHUNK")) chunk = chunk_unary = std::atoi(e) > 0 ? std::atoi(e) : chunk;
-  h->chunk = chunk < max_batch ? chunk : max_batch;
-  h->chunk_unary = chunk_unary < h->chunk ? chunk_unary : h->chunk;
-  h->last_launch_frames = h->chunk_unary;
-  h->kp.lut_cols = h->chunk * (int)C;
-  const size_t ch = h->chunk, MB = max_batch;
+  I.chunk = chunk < max_batch ? chunk : max_batch;
+  I.chunk_unary = chunk_unary < I.chunk ? chunk_unary : I.chunk;
+  I.last_launch_frames = I.chunk_unary;
+  I.kp.lut_cols = I.chunk * (int)C;
+  const size_t ch = I.chunk, MB = max_batch;
   const size_t cap = C * kMaxSections;
-  h->inst_cap = (int)cap;  // every stixel of a frame can be an instance stixel (the reference sizes 8 x this)
+  I.inst_cap = (int)cap;  // every stixel of a frame can be an instance stixel (the reference sizes 8 x this)
 
   {
     // The emission stream's short kernels should not queue behind the DP's thousands of CTAs: highest priority.
@@ -944,74 +935,69 @@ int isx_initialize(isx_handle h, int max_batch) {
     int prio_mid = prio_lo;
     if (const char *e = std::getenv("ISX_TABLES_PRIO"))   // A/B runs: 1 = between the DP and the emission kernels
       prio_mid = (std::atoi(e) != 0 && prio_hi < prio_lo - 1) ? prio_hi + 1 : prio_lo;
-    ISX_TRY(h, cudaStreamCreateWithPriority(&h->s_compute, cudaStreamNonBlocking, prio_lo));
-    ISX_TRY(h, cudaStreamCreateWithPriority(&h->s_tables, cudaStreamNonBlocking, prio_mid));
-    ISX_TRY(h, cudaStreamCreateWithPriority(&h->s_emit, cudaStreamNonBlocking, prio_hi));
+    ISX_TRY(h, I.res.stream(&I.s_compute, prio_lo));
+    ISX_TRY(h, I.res.stream(&I.s_tables, prio_mid));
+    ISX_TRY(h, I.res.stream(&I.s_emit, prio_hi));
   }
-  ISX_TRY(h, cudaStreamCreateWithFlags(&h->s_h2d, cudaStreamNonBlocking));
-  ISX_TRY(h, cudaStreamCreateWithFlags(&h->s_d2h, cudaStreamNonBlocking));
+  ISX_TRY(h, I.res.stream(&I.s_h2d));
   for (int i = 0; i < 2; i++) {
-    ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_in_ready[i], cudaEventDisableTiming));
-    ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_in_free[i], cudaEventDisableTiming));
-    ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_dp_done[i], cudaEventDisableTiming));
-    ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_emit_done[i], cudaEventDisableTiming));
-    ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_tab_done[i], cudaEventDisableTiming));
+    ISX_TRY(h, I.res.event(&I.ev_in_ready[i]));
+    ISX_TRY(h, I.res.event(&I.ev_in_free[i]));
+    ISX_TRY(h, I.res.event(&I.ev_dp_done[i]));
+    ISX_TRY(h, I.res.event(&I.ev_emit_done[i]));
+    ISX_TRY(h, I.res.event(&I.ev_tab_done[i]));
   }
-  ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_chunk_done, cudaEventDisableTiming));
-  ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_user, cudaEventDisableTiming));
 
-  BatchBuffers &b = h->buf;
+  BatchBuffers &b = I.buf;
   for (int i = 0; i < kRoadSlots; i++) {
-    ISX_TRY(h, dev_alloc(h, &h->roads[i].ground, ch * 3 * H));
-    ISX_TRY(h, dev_alloc(h, &h->roads[i].vhor, ch));
-    ISX_TRY(h, cudaEventCreateWithFlags(&h->roads[i].ev_free, cudaEventDisableTiming));
+    ISX_TRY(h, dev_alloc(I, &I.roads[i].ground, ch * 3 * H));
+    ISX_TRY(h, dev_alloc(I, &I.roads[i].vhor, ch));
+    ISX_TRY(h, I.res.event(&I.roads[i].ev_free));
   }
-  h->road_next = 0;
   for (int i = 0; i < 2; i++) {
-    ISX_TRY(h, dev_alloc(h, &h->d_in_disp[i], ch * H * W));
-    ISX_TRY(h, dev_alloc(h, &h->d_in_seg[i], ch * seg_elems(h)));
-    ISX_TRY(h, cudaMemset(h->d_in_seg[i], 0, ch * seg_elems(h) * sizeof(int32_t)));
+    ISX_TRY(h, dev_alloc(I, &I.d_in_disp[i], ch * H * W));
+    ISX_TRY(h, dev_alloc(I, &I.d_in_seg[i], ch * seg_elems(h)));
+    ISX_TRY(h, cudaMemset(I.d_in_seg[i], 0, ch * seg_elems(h) * sizeof(int32_t)));
   }
-  ISX_TRY(h, dev_alloc(h, &h->d_single_disp, H * W));
-  ISX_TRY(h, dev_alloc(h, &h->d_single_seg, seg_elems(h)));
+  ISX_TRY(h, dev_alloc(I, &I.d_single_disp, H * W));
+  ISX_TRY(h, dev_alloc(I, &I.d_single_seg, seg_elems(h)));
   for (int i = 0; i < 2; i++) {
-    isx_context::ChunkSet &cs = h->sets[i];
-    ISX_TRY(h, dev_alloc(h, &cs.stat, ch * H * kStatWords));
-    ISX_TRY(h, dev_alloc(h, &cs.records_b, ch * C * kRecBWords * (size_t)kp.rec_stride));
+    Initialized::ChunkSet &cs = I.sets[i];
+    ISX_TRY(h, dev_alloc(I, &cs.stat, ch * H * kStatWords));
+    ISX_TRY(h, dev_alloc(I, &cs.records_b, ch * C * kRecBWords * (size_t)kp.rec_stride));
     ISX_TRY(h, cudaMemset(cs.records_b, 0, ch * C * kRecBWords * (size_t)kp.rec_stride * sizeof(uint32_t)));
-    ISX_TRY(h, dev_alloc(h, &cs.pm, ch * C * H));
+    ISX_TRY(h, dev_alloc(I, &cs.pm, ch * C * H));
     ISX_TRY(h, cudaMemset(cs.pm, 0, ch * C * H * sizeof(float)));
-    ISX_TRY(h, dev_alloc(h, &cs.dp, ch * C * H));
-    ISX_TRY(h, dev_alloc(h, &cs.err, ch));
-    ISX_TRY(h, dev_alloc(h, &cs.joined, ch * C * H));
-    ISX_TRY(h, dev_alloc(h, &cs.object_lut, lut_buffer_bytes(ch * C, D * (size_t)kp.lut_stride * 4) / 4));
-    ISX_TRY(h, dev_alloc(h, &cs.col_flags, ch * C));
+    ISX_TRY(h, dev_alloc(I, &cs.dp, ch * C * H));
+    ISX_TRY(h, dev_alloc(I, &cs.err, ch));
+    ISX_TRY(h, dev_alloc(I, &cs.joined, ch * C * H));
+    ISX_TRY(h, dev_alloc(I, &cs.object_lut, lut_buffer_bytes(ch * C, D * (size_t)kp.lut_stride * 4) / 4));
+    ISX_TRY(h, dev_alloc(I, &cs.col_flags, ch * C));
     ISX_TRY(h, cudaMemset(cs.col_flags, 0, ch * C * sizeof(int)));
   }
-  ISX_TRY(h, dev_alloc(h, &b.cand_count, ch * kInstanceClasses));
-  ISX_TRY(h, dev_alloc(h, &b.cand_offset, ch * (C + 1) * kInstanceClasses));
-  ISX_TRY(h, dev_alloc(h, &b.cand_xy, ch * kInstanceClasses * cap));
-  ISX_TRY(h, dev_alloc(h, &b.cand_idx, ch * kInstanceClasses * cap));
-  ISX_TRY(h, dev_alloc(h, &b.cand_core, ch * kInstanceClasses * cap));
-  ISX_TRY(h, dev_alloc(h, &b.cand_label, ch * kInstanceClasses * cap));
-  ISX_TRY(h, dev_alloc(h, &b.cand_scratch, ch * kInstanceClasses * cap));
-  ISX_TRY(h, dev_alloc(h, &b.pack_offset, ch * (C + 1)));
-  ISX_TRY(h, dev_alloc(h, &b.dp_units, 1));
+  ISX_TRY(h, dev_alloc(I, &b.cand_count, ch * kInstanceClasses));
+  ISX_TRY(h, dev_alloc(I, &b.cand_offset, ch * (C + 1) * kInstanceClasses));
+  ISX_TRY(h, dev_alloc(I, &b.cand_xy, ch * kInstanceClasses * cap));
+  ISX_TRY(h, dev_alloc(I, &b.cand_idx, ch * kInstanceClasses * cap));
+  ISX_TRY(h, dev_alloc(I, &b.cand_core, ch * kInstanceClasses * cap));
+  ISX_TRY(h, dev_alloc(I, &b.cand_label, ch * kInstanceClasses * cap));
+  ISX_TRY(h, dev_alloc(I, &b.cand_scratch, ch * kInstanceClasses * cap));
+  ISX_TRY(h, dev_alloc(I, &b.pack_offset, ch * (C + 1)));
+  ISX_TRY(h, dev_alloc(I, &b.dp_units, 1));
   if (pairwise_walk_enabled()) {
-    ISX_TRY(h, dev_alloc(h, &b.qrows, ch * C * (size_t)kp.rec_stride * kDynWords));
+    ISX_TRY(h, dev_alloc(I, &b.qrows, ch * C * (size_t)kp.rec_stride * kDynWords));
     ISX_TRY(h, cudaMemset(b.qrows, 0, ch * C * (size_t)kp.rec_stride * kDynWords * sizeof(float)));
   }
   ISX_TRY(h, cudaMemset(b.dp_units, 0, sizeof(unsigned long long)));
-  h->cur = 0;
-  if (int rc = alloc_result_set(h, 0)) return rc;
-  ISX_TRY(h, dev_alloc(h, &h->d_raster_table, MB * C * kMaxSections));
-  ISX_TRY(h, dev_alloc(h, &h->d_export_col, MB * C));
-  ISX_TRY(h, dev_alloc(h, &h->d_object_class, MB * ISX_INSTANCE_CLASSES + 1));
-  ISX_TRY(h, dev_alloc(h, &h->d_export_cost, C * H * 3));
-  ISX_TRY(h, dev_alloc(h, &h->d_export_index, C * H * 3));
+  if (int rc = alloc_result_set(h, I, 0)) return rc;
+  ISX_TRY(h, dev_alloc(I, &I.d_raster_table, MB * C * kMaxSections));
+  ISX_TRY(h, dev_alloc(I, &I.d_export_col, MB * C));
+  ISX_TRY(h, dev_alloc(I, &I.d_object_class, MB * ISX_INSTANCE_CLASSES + 1));
+  ISX_TRY(h, dev_alloc(I, &I.d_export_cost, C * H * 3));
+  ISX_TRY(h, dev_alloc(I, &I.d_export_index, C * H * 3));
 
   float *d_tmp = nullptr;
-  ISX_TRY(h, dev_alloc(h, &d_tmp, D * D));
+  ISX_TRY(h, dev_alloc(I, &d_tmp, D * D));
   ISX_TRY(h, cudaMemcpy(d_tmp, m.obj_cost_lut.data(), sizeof(float) * D * D, cudaMemcpyHostToDevice));
   b.obj_cost_lut = d_tmp;
   {
@@ -1022,138 +1008,71 @@ int isx_initialize(isx_handle h, int max_batch) {
       for (size_t dis = 0; dis < D; dis++) t[dis * Dp + fn] = m.obj_cost_lut[fn * D + dis];
     // object_lut_kernel addresses the table with 32-bit arithmetic on one upper address word: keep it inside one
     // 4 GB window (room for two copies; the second cannot straddle if the first does)
-    ISX_TRY(h, dev_alloc(h, &d_tmp, 2 * D * Dp));
+    ISX_TRY(h, dev_alloc(I, &d_tmp, 2 * D * Dp));
     const unsigned long long a0 = (unsigned long long)d_tmp, bytes = sizeof(float) * D * Dp;
     if (((a0 ^ (a0 + bytes - 1)) >> 32) != 0) d_tmp += D * Dp;
     ISX_TRY(h, cudaMemcpy(d_tmp, t.data(), bytes, cudaMemcpyHostToDevice));
     b.obj_cost_lut_t = d_tmp;
   }
-  ISX_TRY(h, dev_alloc(h, &d_tmp, D));
+  ISX_TRY(h, dev_alloc(I, &d_tmp, D));
   ISX_TRY(h, cudaMemcpy(d_tmp, m.object_disparity_range.data(), sizeof(float) * D, cudaMemcpyHostToDevice));
   b.object_disparity_range = d_tmp;
-  ISX_TRY(h, dev_alloc(h, &d_tmp, H + 1));
+  ISX_TRY(h, dev_alloc(I, &d_tmp, H + 1));
   ISX_TRY(h, cudaMemcpy(d_tmp, m.inverse_height.data(), sizeof(float) * (H + 1), cudaMemcpyHostToDevice));
   b.inverse_height = d_tmp;
 
-  ISX_TRY(h, cudaMallocHost(&h->h_ground, sizeof(float) * kStageSlots * ch * 3 * H));
-  ISX_TRY(h, cudaMallocHost(&h->h_vhor, sizeof(int) * kStageSlots * ch));
-  ISX_TRY(h, cudaMallocHost(&h->h_stage_roads, sizeof(isx_road) * kStageSlots * ch));
-  ISX_TRY(h, dev_alloc(h, &h->d_batch_roads, MB));
-  for (int i = 0; i < kStageSlots; i++) ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_stage_done[i], cudaEventDisableTiming));
-  h->stage_next = 0;
-  h->road_cache.clear();
-  h->overlap_tables = true;
-  if (const char *e = std::getenv("ISX_OVERLAP_TABLES")) h->overlap_tables = std::atoi(e) != 0;
-  h->initialized = true;
-  h->last_batch = 0;
+  ISX_TRY(h, mapped_alloc(I, &I.h_ground, &I.m_ground, kStageSlots * ch * 3 * H));
+  ISX_TRY(h, mapped_alloc(I, &I.h_vhor, &I.m_vhor, kStageSlots * ch));
+  ISX_TRY(h, mapped_alloc(I, &I.h_stage_roads, &I.m_stage_roads, kStageSlots * ch));
+  ISX_TRY(h, dev_alloc(I, &I.d_batch_roads, MB));
+  for (int i = 0; i < kStageSlots; i++) ISX_TRY(h, I.res.event(&I.ev_stage_done[i]));
+  if (const char *e = std::getenv("ISX_OVERLAP_TABLES")) I.overlap_tables = std::atoi(e) != 0;
+  h->init = std::move(init);
   return ISX_OK;
 }
 
 int isx_finish(isx_handle h) {
   if (!h) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null handle");
-  if (!h->initialized) return ISX_OK;
-  cudaSetDevice(h->device);
-  cudaDeviceSynchronize();
-  for (void *p : h->allocations) cudaFree(p);
-  h->allocations.clear();
-  cudaFreeHost(h->h_ground);
-  cudaFreeHost(h->h_vhor);
-  cudaFreeHost(h->h_stage_roads);
-  h->h_stage_roads = nullptr;
-  h->d_batch_roads = nullptr;
-  h->last_roads_dev = nullptr;
-  h->m_ground = nullptr;
-  h->m_vhor = nullptr;
-  h->m_stage_roads = nullptr;
-  for (int i = 0; i < kStageSlots; i++) {
-    if (h->ev_stage_done[i]) cudaEventDestroy(h->ev_stage_done[i]);
-    h->ev_stage_done[i] = nullptr;
-  }
-  for (int i = 0; i < kRoadSlots; i++) {
-    if (h->roads[i].ev_free) cudaEventDestroy(h->roads[i].ev_free);
-    h->roads[i] = isx_context::RoadSlot();
-  }
-  for (int i = 0; i < kResultSets; i++) {
-    isx_context::ResultSet &R = h->rs[i];
-    if (R.allocated) {
-      cudaFreeHost(R.h_sections);
-      cudaFreeHost(R.h_inst);
-      cudaFreeHost(R.h_counts);
-      cudaFreeHost(R.h_frames);
-    }
-    if (R.h_est) cudaFreeHost(R.h_est);
-    if (R.h_roads) cudaFreeHost(R.h_roads);
-    R = isx_context::ResultSet();
-    if (h->ev_batch_done[i]) cudaEventDestroy(h->ev_batch_done[i]);
-    h->ev_batch_done[i] = nullptr;
-    h->batch_sections[i] = nullptr;
-    h->batch_est[i] = nullptr;
-    h->batch_roads[i] = nullptr;
-    h->batch_n[i] = 0;
-  }
-  for (int i = 0; i < 2; i++) {
-    h->d_in_disp16[i] = nullptr;
-    h->d_in_seg16[i] = nullptr;
-  }
-  h->cur = 0;
-  h->submitted = h->waited = 0;
-  h->last_waited_set = -1;
-  h->host_slot = 0;
-  h->dp_units_total = h->dp_units_pairwise = 0;
-  h->emit_join_pending = false;
-  for (int i = 0; i < 2; i++) {
-    cudaEventDestroy(h->ev_in_ready[i]);
-    cudaEventDestroy(h->ev_in_free[i]);
-    cudaEventDestroy(h->ev_dp_done[i]);
-    cudaEventDestroy(h->ev_emit_done[i]);
-    cudaEventDestroy(h->ev_tab_done[i]);
-  }
-  cudaEventDestroy(h->ev_chunk_done);
-  cudaEventDestroy(h->ev_user);
-  cudaStreamDestroy(h->s_tables);
-  cudaStreamDestroy(h->s_compute);
-  cudaStreamDestroy(h->s_emit);
-  cudaStreamDestroy(h->s_h2d);
-  cudaStreamDestroy(h->s_d2h);
-  h->buf = BatchBuffers();
-  h->initialized = false;
+  h->init.reset();
   return ISX_OK;
 }
 
-int isx_is_initialized(isx_handle h) { return h && h->initialized; }
-int isx_real_cols(isx_handle h) { return h ? (h->initialized ? h->kp.realcols : 0) : 0; }
+int isx_is_initialized(isx_handle h) { return h && h->init; }
+int isx_real_cols(isx_handle h) { return h ? (h->init ? h->init->kp.realcols : 0) : 0; }
 int isx_max_sections(isx_handle h) { (void)h; return kMaxSections; }
-size_t isx_segmentation_elems(isx_handle h) { return (h && h->initialized) ? seg_elems(h) : 0; }
+size_t isx_segmentation_elems(isx_handle h) { return (h && h->init) ? seg_elems(h) : 0; }
 
 int isx_set_disparity_image(isx_handle h, const float *host, size_t n) {
   if (int rc = check_ready(h)) return rc;
-  if (!host || n != (size_t)h->kp.rows * h->kp.cols)
+  Initialized &I = *h->init;
+  if (!host || n != (size_t)I.kp.rows * I.kp.cols)
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "disparity image must hold rows*cols floats");
-  ISX_TRY(h, cudaMemcpyAsync(h->d_single_disp, host, n * sizeof(float), cudaMemcpyHostToDevice, h->s_tables));
+  ISX_TRY(h, cudaMemcpyAsync(I.d_single_disp, host, n * sizeof(float), cudaMemcpyHostToDevice, I.s_tables));
   return ISX_OK;
 }
 
 float *isx_input_disparity_device(isx_handle h) {
-  if (!h || !h->initialized) return nullptr;
+  if (!h || !h->init) return nullptr;
   // the caller hands the pointer to its own kernels (RoadEstimation::Compute(pixel_t *d_im), RoadEstimation.cu:107):
   // the image SetDisparityImage is still copying must have arrived
   cudaSetDevice(h->device);
-  cudaStreamSynchronize(h->s_tables);
-  return h->d_single_disp;
+  cudaStreamSynchronize(h->init->s_tables);
+  return h->init->d_single_disp;
 }
 
 int isx_set_segmentation(isx_handle h, const int32_t *host, size_t n) {
   if (int rc = check_ready(h)) return rc;
   if (!host || n != seg_elems(h))
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "segmentation must hold realcols*channels*rows_power2_segmentation ints");
-  ISX_TRY(h, cudaMemcpyAsync(h->d_single_seg, host, n * sizeof(int32_t), cudaMemcpyHostToDevice, h->s_tables));
+  ISX_TRY(h, cudaMemcpyAsync(h->init->d_single_seg, host, n * sizeof(int32_t), cudaMemcpyHostToDevice,
+                             h->init->s_tables));
   return ISX_OK;
 }
 
 // FlipAndPad on the device (ingest.cu).  The CNN grid is [channels][rows/8][cols/8]; width_margin must be 0 and
 // column_step must divide 8, as in every configuration the reference ships.
 static int check_cnn_grid(isx_handle h, int cnn_rows, int cnn_cols) {
-  const KParams &kp = h->kp;
+  const KParams &kp = h->init->kp;
   if (kp.width_margin != 0 || kp.column_step < 1 || kDownsample % kp.column_step != 0)
     return fail(h, ISX_ERR_UNSUPPORTED, "segmentation ingest needs width_margin == 0 and column_step dividing 8");
   if (cnn_rows != kp.rows / kDownsample || cnn_cols * (kDownsample / kp.column_step) != kp.realcols)
@@ -1165,7 +1084,7 @@ int isx_set_segmentation_from_cnn_device(isx_handle h, const float *d_cnn, int c
   if (int rc = check_ready(h)) return rc;
   if (!d_cnn) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
   if (int rc = check_cnn_grid(h, cnn_rows, cnn_cols)) return rc;
-  launch_flip_and_pad(h->kp, d_cnn, h->d_single_seg, 1, cnn_rows, cnn_cols, h->s_tables);
+  launch_flip_and_pad(h->init->kp, d_cnn, h->init->d_single_seg, 1, cnn_rows, cnn_cols, h->init->s_tables);
   ISX_TRY(h, cudaGetLastError());
   return ISX_OK;
 }
@@ -1175,7 +1094,7 @@ int isx_flip_and_pad_batch_device(isx_handle h, int n, const float *d_cnn, int c
   if (int rc = check_ready(h)) return rc;
   if (!d_cnn || !d_segmentation || n < 1) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument or empty batch");
   if (int rc = check_cnn_grid(h, cnn_rows, cnn_cols)) return rc;
-  launch_flip_and_pad(h->kp, d_cnn, d_segmentation, n, cnn_rows, cnn_cols, h->s_tables);
+  launch_flip_and_pad(h->init->kp, d_cnn, d_segmentation, n, cnn_rows, cnn_cols, h->init->s_tables);
   ISX_TRY(h, cudaGetLastError());
   return ISX_OK;
 }
@@ -1195,10 +1114,10 @@ static int no_batches_in_flight(isx_handle h);
 // frame after frame.  Everything comes from pinned host memory the device has already written (the caller has
 // waited for the emission stream); only a frame that did not fit the packed arrays costs a device -> host copy.
 // Returns the first per-frame error AFTER delivering what there is.
-static int deliver(isx_handle h, isx_context::ResultSet &R, int n, isx_section *sections, isx_instance *instances,
+static int deliver(isx_handle h, Initialized::ResultSet &R, int n, isx_section *sections, isx_instance *instances,
                    int instances_capacity, int32_t *instance_offsets, bool direct = false) {
   if (direct) sections = nullptr;   // the device has written the caller's array itself
-  const size_t C = h->kp.realcols;
+  const size_t C = h->init->kp.realcols;
   int rc = ISX_OK;
   int total = 0;
   for (int f = 0; f < n; f++) {
@@ -1241,8 +1160,8 @@ static int deliver(isx_handle h, isx_context::ResultSet &R, int n, isx_section *
       const int take = d.instance_count < room ? d.instance_count : (room > 0 ? room : 0);
       if (take > 0) {
         if (d.overflow & 2)
-          ISX_TRY(h, cudaMemcpy(instances + total, R.d_inst + (size_t)f * h->inst_cap, sizeof(isx_instance) * take,
-                                cudaMemcpyDeviceToHost));
+          ISX_TRY(h, cudaMemcpy(instances + total, R.d_inst + (size_t)f * h->init->inst_cap,
+                                sizeof(isx_instance) * take, cudaMemcpyDeviceToHost));
         else
           std::memcpy(instances + total, R.h_inst + d.instance_offset, sizeof(isx_instance) * (size_t)take);
       }
@@ -1255,32 +1174,33 @@ static int deliver(isx_handle h, isx_context::ResultSet &R, int n, isx_section *
 
 // Waits until the results of the last enqueued batch are in host memory.
 static int wait_last_emission(isx_handle h) {
-  ISX_TRY(h, cudaEventSynchronize(h->ev_emit_done[h->last_set]));
+  ISX_TRY(h, cudaEventSynchronize(h->init->ev_emit_done[h->init->last_set]));
   return ISX_OK;
 }
 
 int isx_compute(isx_handle h, int pairwise, isx_section *sections, isx_frame_meta *meta,
                 const int32_t *d_segmentation_local) {
   if (int rc = check_ready(h)) return rc;
+  Initialized &I = *h->init;
   if (!h->single_has_road) return fail(h, ISX_ERR_INVALID_ARGUMENT, "SetRoadParameters has not been called");
   if (int rc = no_batches_in_flight(h)) return rc;
-  const int32_t *seg = d_segmentation_local ? d_segmentation_local : h->d_single_seg;
+  const int32_t *seg = d_segmentation_local ? d_segmentation_local : I.d_single_seg;
   if (int rc = begin_batch(h)) return rc;
   ResultDest out;
   out.direct_sections = device_view_of(sections);
-  if (int rc = enqueue_chunk(h, pairwise != 0, 0, 1, h->d_single_disp, seg, &h->single_road, 0, -1, out)) return rc;
-  ISX_TRY(h, cudaEventRecord(h->ev_in_free[0], h->s_tables));
+  if (int rc = enqueue_chunk(h, pairwise != 0, 0, 1, I.d_single_disp, seg, &h->single_road, 0, -1, out)) return rc;
+  ISX_TRY(h, cudaEventRecord(I.ev_in_free[0], I.s_tables));
   if (int rc = join_emit_stream(h)) return rc;
-  h->last_batch = 1;
-  h->last_roads.assign(1, h->single_road);
-  h->last_roads_dev = nullptr;
+  I.last_batch = 1;
+  I.last_roads.assign(1, h->single_road);
+  I.last_roads_dev = nullptr;
   if (int rc = wait_last_emission(h)) return rc;
-  if (int rc = deliver(h, h->rs[h->cur], 1, sections, nullptr, 0, nullptr, out.direct_sections != nullptr)) return rc;
+  if (int rc = deliver(h, I.rs[I.cur], 1, sections, nullptr, 0, nullptr, out.direct_sections != nullptr)) return rc;
   if (meta) {
-    meta->rows = h->kp.rows; meta->cols = h->kp.cols; meta->realcols = h->kp.realcols;
-    meta->max_sections = kMaxSections; meta->max_dis = h->kp.max_dis; meta->column_step = h->kp.column_step;
-    meta->semantic_classes = h->kp.n_classes; meta->alpha_ground = h->single_road.alpha_ground;
-    meta->vhor = h->kp.rows - h->single_road.vhor - 1;
+    meta->rows = I.kp.rows; meta->cols = I.kp.cols; meta->realcols = I.kp.realcols;
+    meta->max_sections = kMaxSections; meta->max_dis = I.kp.max_dis; meta->column_step = I.kp.column_step;
+    meta->semantic_classes = I.kp.n_classes; meta->alpha_ground = h->single_road.alpha_ground;
+    meta->vhor = I.kp.rows - h->single_road.vhor - 1;
   }
   return ISX_OK;
 }
@@ -1301,11 +1221,11 @@ int isx_dbscan_fit_host(int device, const float *xy, int n, float eps, int min_p
 
 int isx_get_instance_stixels(isx_handle h, isx_instance *out, int capacity, int *n) {
   if (int rc = check_ready(h)) return rc;
-  if (h->last_batch < 1) return fail(h, ISX_ERR_INVALID_ARGUMENT, "Compute has not been called");
+  if (h->init->last_batch < 1) return fail(h, ISX_ERR_INVALID_ARGUMENT, "Compute has not been called");
   if (int rc = no_batches_in_flight(h)) return rc;
   if (int rc = wait_last_emission(h)) return rc;
   int32_t offs[2] = {0, 0};
-  if (int rc = deliver(h, h->rs[h->cur], 1, nullptr, out, out ? capacity : 0, offs)) return rc;
+  if (int rc = deliver(h, h->init->rs[h->init->cur], 1, nullptr, out, out ? capacity : 0, offs)) return rc;
   if (n) *n = offs[1];
   return ISX_OK;
 }
@@ -1314,7 +1234,7 @@ int isx_compute_batch_device(isx_handle h, int pairwise, int n, const float *d_d
                              const int32_t *d_segmentation, const isx_road *roads) {
   if (int rc = check_ready(h)) return rc;
   if (int rc = no_batches_in_flight(h)) return rc;
-  if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
+  if (n < 1 || n > h->init->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
   if (!d_disparity || !d_segmentation || !roads) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
   Batch b;
   b.d_disparity = d_disparity;
@@ -1328,19 +1248,20 @@ int isx_compute_batch_device_road(isx_handle h, isx_road_handle road, int pairwi
                                   const int32_t *d_segmentation, const isx_road *fallback,
                                   isx_road_estimate *d_estimates, isx_road *d_roads) {
   if (int rc = check_ready(h)) return rc;
+  Initialized &I = *h->init;
   if (int rc = no_batches_in_flight(h)) return rc;
-  if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
+  if (n < 1 || n > I.max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
   if (!road || !d_disparity || !d_segmentation) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
   std::string msg;
-  if (int rc = road_check_batch(road, h->device, h->kp.rows, h->kp.cols, h->kp.max_dis, n, fallback != nullptr, msg))
+  if (int rc = road_check_batch(road, h->device, I.kp.rows, I.kp.cols, I.kp.max_dis, n, fallback != nullptr, msg))
     return fail(h, rc, msg);
-  if (int rc = road_enqueue_batch(road, h->s_tables, n, d_disparity, fallback, d_estimates, d_roads, h->d_batch_roads,
+  if (int rc = road_enqueue_batch(road, I.s_tables, n, d_disparity, fallback, d_estimates, d_roads, I.d_batch_roads,
                                   msg))
     return fail(h, rc, msg);
   Batch b;
   b.d_disparity = d_disparity;
   b.d_segmentation = d_segmentation;
-  b.d_roads = h->d_batch_roads;
+  b.d_roads = I.d_batch_roads;
   b.out.stay_on_device = true;
   return enqueue_batch(h, pairwise, n, b, /*caller_waits=*/false);
 }
@@ -1353,22 +1274,22 @@ int isx_flush(isx_handle h) {
 int isx_synchronize(isx_handle h) {
   if (int rc = check_ready(h)) return rc;
   if (int rc = ensure_joined(h)) return rc;
-  ISX_TRY(h, cudaStreamSynchronize(h->s_tables));
+  ISX_TRY(h, cudaStreamSynchronize(h->init->s_tables));
   return ISX_OK;
 }
 
 int isx_fetch_batch_results(isx_handle h, int n, isx_section *sections, isx_instance *instances,
                             int instances_capacity, int32_t *instance_offsets) {
   if (int rc = check_ready(h)) return rc;
-  if (n < 1 || n > h->last_batch) return fail(h, ISX_ERR_INVALID_ARGUMENT, "no results for that many frames");
+  if (n < 1 || n > h->init->last_batch) return fail(h, ISX_ERR_INVALID_ARGUMENT, "no results for that many frames");
   if (int rc = no_batches_in_flight(h)) return rc;
   if (int rc = ensure_joined(h)) return rc;
   if (int rc = wait_last_emission(h)) return rc;
-  return deliver(h, h->rs[h->cur], n, sections, instances, instances_capacity, instance_offsets);
+  return deliver(h, h->init->rs[h->init->cur], n, sections, instances, instances_capacity, instance_offsets);
 }
 
 static int no_batches_in_flight(isx_handle h) {
-  if (h->submitted != h->waited)
+  if (h->init->submitted != h->init->waited)
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "submitted batches are in flight: call isx_wait_batch_host first");
   return ISX_OK;
 }
@@ -1378,7 +1299,7 @@ static int compute_batch_host(isx_handle h, int pairwise, int n, const HostInput
                               int32_t *instance_offsets) {
   if (int rc = check_ready(h)) return rc;
   if (int rc = no_batches_in_flight(h)) return rc;
-  if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
+  if (n < 1 || n > h->init->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
   if (!roads) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
   Batch b;
   b.host = in;
@@ -1387,7 +1308,7 @@ static int compute_batch_host(isx_handle h, int pairwise, int n, const HostInput
   if (int rc = enqueue_batch(h, pairwise, n, b, /*caller_waits=*/true)) return rc;
   if (int rc = join_emit_stream(h)) return rc;
   if (int rc = wait_last_emission(h)) return rc;
-  return deliver(h, h->rs[h->cur], n, sections, instances, instances_capacity, instance_offsets,
+  return deliver(h, h->init->rs[h->init->cur], n, sections, instances, instances_capacity, instance_offsets,
                  b.out.direct_sections != nullptr);
 }
 
@@ -1407,57 +1328,59 @@ int isx_compute_batch_host_u16(isx_handle h, int pairwise, int n, const uint16_t
                             instances, instances_capacity, instance_offsets);
 }
 
-size_t isx_narrow_segmentation_elems(isx_handle h) { return (h && h->initialized) ? narrow_seg_elems(h) : 0; }
+size_t isx_narrow_segmentation_elems(isx_handle h) { return (h && h->init) ? narrow_seg_elems(h) : 0; }
 
 static int submit_batch_host(isx_handle h, int pairwise, int n, const HostInputs &in, const isx_road *roads,
                              isx_section *sections, const HostRoad *hr = nullptr, isx_road_estimate *estimates = nullptr,
                              isx_road *roads_out = nullptr) {
   if (int rc = check_ready(h)) return rc;
-  if (n < 1 || n > h->max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
+  Initialized &I = *h->init;
+  if (n < 1 || n > I.max_batch) return fail(h, ISX_ERR_CAPACITY, "batch size exceeds isx_initialize(max_batch)");
   if (!roads && !hr) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null argument");
   if (hr) {
     // the road step runs per chunk: the road handle must hold the largest chunk the batch is cut into
-    const int chunk = pairwise ? h->chunk : h->chunk_unary;
+    const int chunk = pairwise ? I.chunk : I.chunk_unary;
     std::string msg;
-    if (int rc = road_check_batch(hr->road, h->device, h->kp.rows, h->kp.cols, h->kp.max_dis, n < chunk ? n : chunk,
+    if (int rc = road_check_batch(hr->road, h->device, I.kp.rows, I.kp.cols, I.kp.max_dis, n < chunk ? n : chunk,
                                   hr->fallback != nullptr, msg))
       return fail(h, rc, msg);
   }
-  if (h->submitted - h->waited >= (unsigned long long)(kResultSets - 1))
+  if (I.submitted - I.waited >= (unsigned long long)(kResultSets - 1))
     return fail(h, ISX_ERR_CAPACITY, "three batches are already in flight: call isx_wait_batch_host first");
   int next = 0;
   {
     bool busy[kResultSets] = {};
-    for (unsigned long long t = h->waited; t < h->submitted; t++) busy[h->batch_set[t % kResultSets]] = true;
-    if (h->last_waited_set >= 0) busy[h->last_waited_set] = true;  // its packed arrays may still be read
+    for (unsigned long long t = I.waited; t < I.submitted; t++) busy[I.batches[t % kResultSets].set] = true;
+    if (I.last_waited_set >= 0) busy[I.last_waited_set] = true;  // its packed arrays may still be read
     while (busy[next]) next++;
   }
-  if (int rc = alloc_result_set(h, next)) return rc;
-  if (hr) {
-    if (int rc = alloc_road_results(h, next)) return rc;
+  if (int rc = alloc_result_set(h, I, next)) return rc;
+  Initialized::ResultSet &R = I.rs[next];
+  if (hr && !R.m_roads) {
+    ISX_TRY(h, mapped_alloc(I, &R.h_est, &R.m_est, I.max_batch));
+    ISX_TRY(h, mapped_alloc(I, &R.h_roads, &R.m_roads, I.max_batch));
   }
-  for (int i = 0; i < kResultSets; i++)
-    if (!h->ev_batch_done[i]) ISX_TRY(h, cudaEventCreateWithFlags(&h->ev_batch_done[i], cudaEventDisableTiming));
-  h->cur = next;
+  Initialized::InFlight &t = I.batches[I.submitted % kResultSets];
+  if (!t.done) ISX_TRY(h, I.res.event(&t.done));
+  I.cur = next;
   Batch b;
   b.host = in;
   b.roads = roads;
   if (hr) {
     b.estimate = *hr;
-    b.d_estimates = h->rs[next].m_est;
-    b.d_roads = h->rs[next].m_roads;
+    b.d_estimates = R.m_est;
+    b.d_roads = R.m_roads;
   }
   b.out.direct_sections = device_view_of(sections);
   if (int rc = enqueue_batch(h, pairwise, n, b, /*caller_waits=*/false)) return rc;
-  const int par = (int)(h->submitted % kResultSets);
-  h->batch_direct[par] = b.out.direct_sections != nullptr;
-  ISX_TRY(h, cudaEventRecord(h->ev_batch_done[par], h->s_emit));  // behind the packing of the last chunk
-  h->batch_n[par] = n;
-  h->batch_set[par] = h->cur;
-  h->batch_sections[par] = sections;
-  h->batch_est[par] = hr ? estimates : nullptr;
-  h->batch_roads[par] = hr ? roads_out : nullptr;
-  h->submitted++;
+  ISX_TRY(h, cudaEventRecord(t.done, I.s_emit));  // behind the packing of the last chunk
+  t.n = n;
+  t.set = I.cur;
+  t.sections = sections;
+  t.direct = b.out.direct_sections != nullptr;
+  t.est = hr ? estimates : nullptr;
+  t.roads = hr ? roads_out : nullptr;
+  I.submitted++;
   return ISX_OK;
 }
 
@@ -1497,67 +1420,70 @@ int isx_reserve_in_flight(isx_handle h, int batches) {
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "isx_reserve_in_flight: between one and three batches");
   cudaSetDevice(h->device);
   for (int i = 0; i <= batches && i < kResultSets; i++)
-    if (int rc = alloc_result_set(h, i)) return rc;
+    if (int rc = alloc_result_set(h, *h->init, i)) return rc;
   return ISX_OK;
 }
 
 // Waits for the oldest batch in flight; returns its ticket slot (>= 0) or an error (< 0).
 static int wait_oldest(isx_handle h) {
   if (int rc = check_ready(h)) return rc;
-  if (h->submitted == h->waited) return fail(h, ISX_ERR_INVALID_ARGUMENT, "no submitted batch is in flight");
-  const int par = (int)(h->waited % kResultSets);
-  ISX_TRY(h, cudaEventSynchronize(h->ev_batch_done[par]));
-  h->last_waited_set = h->batch_set[par];
-  h->waited++;
-  const isx_context::ResultSet &R = h->rs[h->batch_set[par]];
-  const size_t n = (size_t)h->batch_n[par];
-  if (h->batch_est[par]) std::memcpy(h->batch_est[par], R.h_est, sizeof(isx_road_estimate) * n);
-  if (h->batch_roads[par]) std::memcpy(h->batch_roads[par], R.h_roads, sizeof(isx_road) * n);
-  h->batch_est[par] = nullptr;
-  h->batch_roads[par] = nullptr;
+  Initialized &I = *h->init;
+  if (I.submitted == I.waited) return fail(h, ISX_ERR_INVALID_ARGUMENT, "no submitted batch is in flight");
+  const int par = (int)(I.waited % kResultSets);
+  Initialized::InFlight &t = I.batches[par];
+  ISX_TRY(h, cudaEventSynchronize(t.done));
+  I.last_waited_set = t.set;
+  I.waited++;
+  const Initialized::ResultSet &R = I.rs[t.set];
+  if (t.est) std::memcpy(t.est, R.h_est, sizeof(isx_road_estimate) * (size_t)t.n);
+  if (t.roads) std::memcpy(t.roads, R.h_roads, sizeof(isx_road) * (size_t)t.n);
+  t.est = nullptr;
+  t.roads = nullptr;
   return par;
 }
 
 int isx_wait_batch_host(isx_handle h, isx_instance *instances, int instances_capacity, int32_t *instance_offsets) {
   const int par = wait_oldest(h);
   if (par < 0) return par;
-  const int n = h->batch_n[par];
-  h->batch_n[par] = 0;
-  return deliver(h, h->rs[h->batch_set[par]], n, h->batch_sections[par], instances, instances_capacity,
-                 instance_offsets, h->batch_direct[par]);
+  Initialized::InFlight &t = h->init->batches[par];
+  const int n = t.n;
+  t.n = 0;
+  return deliver(h, h->init->rs[t.set], n, t.sections, instances, instances_capacity, instance_offsets, t.direct);
 }
 
 int isx_wait_batch_packed(isx_handle h, const isx_section **sections, const int32_t **counts,
                           const isx_instance **instances, const isx_packed_frame **frames, int *n) {
   const int par = wait_oldest(h);
   if (par < 0) return par;
-  const isx_context::ResultSet &R = h->rs[h->batch_set[par]];
+  Initialized::InFlight &t = h->init->batches[par];
+  const Initialized::ResultSet &R = h->init->rs[t.set];
   if (sections) *sections = R.h_sections;
   if (counts) *counts = R.h_counts;
   if (instances) *instances = R.h_inst;
   if (frames) *frames = R.h_frames;
-  if (n) *n = h->batch_n[par];
+  if (n) *n = t.n;
   int rc = ISX_OK;
-  for (int f = 0; f < h->batch_n[par] && rc == ISX_OK; f++) {
+  for (int f = 0; f < t.n && rc == ISX_OK; f++) {
     if (R.h_frames[f].error & kErrOffsetRange) rc = fail(h, ISX_ERR_UNSUPPORTED, "instance offsets out of range in a frame of the batch");
     else if (R.h_frames[f].error) rc = fail(h, ISX_ERR_CAPACITY, "a column produced >= 200 stixels (MAX_STIXELS_PER_COLUMN)");
   }
-  h->batch_n[par] = 0;
+  t.n = 0;
   return rc;
 }
 
 int isx_rasterize_batch_device(isx_handle h, int first, int n, uint8_t *d_label_ids, int32_t *d_instance_ids,
                                float *d_disparity) {
   if (int rc = check_ready(h)) return rc;
-  if (first < 0 || n < 1 || first + n > h->last_batch)
+  Initialized &I = *h->init;
+  if (first < 0 || n < 1 || first + n > I.last_batch)
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "frames outside the last computed batch");
   if (!d_label_ids && !d_instance_ids && !d_disparity) return fail(h, ISX_ERR_INVALID_ARGUMENT, "no output image");
   if (int rc = ensure_joined(h)) return rc;
-  const size_t C = h->kp.realcols;
-  const isx_context::ResultSet &R = h->rs[h->cur];
-  launch_rasterize(h->kp, R.d_sections + (size_t)first * C * kMaxSections, R.d_nsections + (size_t)first * C,
-                   R.d_inst + (size_t)first * h->inst_cap, R.d_inst_count + first, h->inst_cap,
-                   h->d_raster_table, n, d_label_ids, d_instance_ids, d_disparity, h->s_tables);
+  const size_t C = I.kp.realcols;
+  const Initialized::ResultSet &R = I.rs[I.cur];
+  launch_rasterize(I.kp, R.d_sections + (size_t)first * C * kMaxSections, R.d_nsections + (size_t)first * C,
+                   R.d_inst + (size_t)first * I.inst_cap, R.d_inst_count + first, I.inst_cap,
+                   I.d_raster_table, n, d_label_ids, d_instance_ids, d_disparity, I.s_tables);
   ISX_TRY(h, cudaGetLastError());
   return ISX_OK;
 }
@@ -1567,7 +1493,8 @@ int isx_rasterize_batch_device(isx_handle h, int first, int n, uint8_t *d_label_
 // so it starts after whatever was enqueued here.
 int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_results *out) {
   if (int rc = check_ready(h)) return rc;
-  if (first < 0 || n < 1 || first + n > h->last_batch)
+  Initialized &I = *h->init;
+  if (first < 0 || n < 1 || first + n > I.last_batch)
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "frames outside the last computed batch");
   if (!out || !out->frame_offsets) return fail(h, ISX_ERR_INVALID_ARGUMENT, "frame_offsets is required");
   if ((uintptr_t)out->sections % 16 != 0)
@@ -1578,32 +1505,32 @@ int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_res
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "Camera parameters are not set.");  // Get3DVertices (Stixels.cu:685-687)
   if (int rc = no_batches_in_flight(h)) return rc;
   if (int rc = ensure_joined(h)) return rc;
-  const size_t C = h->kp.realcols;
-  const isx_context::ResultSet &R = h->rs[h->cur];
+  const size_t C = I.kp.realcols;
+  const Initialized::ResultSet &R = I.rs[I.cur];
   ExportArgs a;
   a.sections = R.d_sections + (size_t)first * C * kMaxSections;
   a.n_sections = R.d_nsections + (size_t)first * C;
-  a.inst = R.d_inst + (size_t)first * h->inst_cap;
+  a.inst = R.d_inst + (size_t)first * I.inst_cap;
   a.inst_count = R.d_inst_count + first;
-  a.inst_cap = h->inst_cap;
+  a.inst_cap = I.inst_cap;
   a.frames = R.m_frames + first;
-  a.col_local = h->d_export_col;
-  a.realcols = h->kp.realcols;
-  a.rows = h->kp.rows;
-  a.column_step = h->kp.column_step;
+  a.col_local = I.d_export_col;
+  a.realcols = I.kp.realcols;
+  a.rows = I.kp.rows;
+  a.column_step = I.kp.column_step;
   a.focal = m.focal;
   a.bf = m.baseline * m.focal;
   a.camera_center_x = m.camera_center_x;
   a.camera_center_y = m.camera_center_y;
   a.out = *out;
-  a.roads = h->last_roads_dev ? h->last_roads_dev + first : nullptr;
+  a.roads = I.last_roads_dev ? I.last_roads_dev + first : nullptr;
   std::vector<float> alpha((size_t)n);
   std::vector<int> vhor((size_t)n);
   for (int f = 0; f < n && !a.roads; f++) {
-    alpha[f] = h->last_roads[first + f].alpha_ground;
-    vhor[f] = h->kp.rows - h->last_roads[first + f].vhor - 1;   // isx_frame_meta.vhor (Stixels.cu:377)
+    alpha[f] = I.last_roads[first + f].alpha_ground;
+    vhor[f] = I.kp.rows - I.last_roads[first + f].vhor - 1;   // isx_frame_meta.vhor (Stixels.cu:377)
   }
-  launch_export_results(a, n, alpha.data(), vhor.data(), h->s_tables);
+  launch_export_results(a, n, alpha.data(), vhor.data(), I.s_tables);
   ISX_TRY(h, cudaGetLastError());
   return ISX_OK;
 }
@@ -1611,7 +1538,8 @@ int isx_export_batch_device(isx_handle h, int first, int n, const isx_device_res
 // Like isx_export_batch_device: reads result set rs[cur] on s_tables.
 int isx_export_objects_device(isx_handle h, int first, int n, const isx_device_objects *out) {
   if (int rc = check_ready(h)) return rc;
-  if (first < 0 || n < 1 || first + n > h->last_batch)
+  Initialized &I = *h->init;
+  if (first < 0 || n < 1 || first + n > I.last_batch)
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "frames outside the last computed batch");
   if (!out || !out->frame_offsets) return fail(h, ISX_ERR_INVALID_ARGUMENT, "frame_offsets is required");
   if ((uintptr_t)out->objects % 16 != 0) return fail(h, ISX_ERR_INVALID_ARGUMENT, "objects must be 16-byte aligned");
@@ -1621,32 +1549,32 @@ int isx_export_objects_device(isx_handle h, int first, int n, const isx_device_o
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "Camera parameters are not set.");  // Get3DVertices (Stixels.cu:685-687)
   if (int rc = no_batches_in_flight(h)) return rc;
   if (int rc = ensure_joined(h)) return rc;
-  const size_t C = h->kp.realcols;
-  const isx_context::ResultSet &R = h->rs[h->cur];
+  const size_t C = I.kp.realcols;
+  const Initialized::ResultSet &R = I.rs[I.cur];
   ObjectArgs a;
   a.sections = R.d_sections + (size_t)first * C * kMaxSections;
-  a.inst = R.d_inst + (size_t)first * h->inst_cap;
+  a.inst = R.d_inst + (size_t)first * I.inst_cap;
   a.inst_count = R.d_inst_count + first;
-  a.inst_cap = h->inst_cap;
-  a.class_start = h->d_object_class;
-  a.realcols = h->kp.realcols;
-  a.rows = h->kp.rows;
-  a.column_step = h->kp.column_step;
+  a.inst_cap = I.inst_cap;
+  a.class_start = I.d_object_class;
+  a.realcols = I.kp.realcols;
+  a.rows = I.kp.rows;
+  a.column_step = I.kp.column_step;
   a.focal = m.focal;
   a.bf = m.baseline * m.focal;
   a.camera_center_x = m.camera_center_x;
   a.camera_center_y = m.camera_center_y;
   a.out = *out;
-  launch_export_objects(a, n, h->s_tables);
+  launch_export_objects(a, n, I.s_tables);
   ISX_TRY(h, cudaGetLastError());
   return ISX_OK;
 }
 
-uint64_t isx_stream(isx_handle h) { return (h && h->initialized) ? (uint64_t)(uintptr_t)h->s_tables : 0; }
+uint64_t isx_stream(isx_handle h) { return (h && h->init) ? (uint64_t)(uintptr_t)h->init->s_tables : 0; }
 
 size_t isx_tensor_elems(isx_handle h, int tensor) {
-  if (!h || !h->initialized) return 0;
-  const size_t H = h->kp.rows, C = h->kp.realcols, D = h->kp.max_dis;
+  if (!h || !h->init) return 0;
+  const size_t H = h->init->kp.rows, C = h->init->kp.realcols, D = h->init->kp.max_dis;
   switch (tensor) {
     case ISX_T_JOINED_DISPARITY: return C * H;
     case ISX_T_OBJECT_LUT: return C * D * (H + 1);
@@ -1665,17 +1593,18 @@ size_t isx_tensor_elems(isx_handle h, int tensor) {
 
 int isx_read_tensor(isx_handle h, int tensor, int frame, void *host, size_t bytes) {
   if (int rc = check_ready(h)) return rc;
+  Initialized &I = *h->init;
   const size_t need = isx_tensor_elems(h, tensor) * 4;
   if (need == 0 || !host || bytes < need) return fail(h, ISX_ERR_INVALID_ARGUMENT, "bad tensor id or buffer too small");
-  const int local = frame - h->last_chunk_first;
-  if (local < 0 || local >= h->last_chunk_n)
+  const int local = frame - I.last_chunk_first;
+  if (local < 0 || local >= I.last_chunk_n)
     return fail(h, ISX_ERR_INVALID_ARGUMENT, "intermediates are only kept for the last chunk of the last batch");
   if (int rc = ensure_joined(h)) return rc;
-  ISX_TRY(h, cudaStreamSynchronize(h->s_tables));
-  ISX_TRY(h, cudaStreamSynchronize(h->s_compute));
-  const KParams &kp = h->kp;
+  ISX_TRY(h, cudaStreamSynchronize(I.s_tables));
+  ISX_TRY(h, cudaStreamSynchronize(I.s_compute));
+  const KParams &kp = I.kp;
   const size_t H = kp.rows, C = kp.realcols, D = kp.max_dis;
-  const BatchBuffers b = chunk_buffers(h, h->last_set, h->last_road_slot);
+  const BatchBuffers b = chunk_buffers(h, I.last_set, I.last_road_slot);
   if (tensor == ISX_T_GROUND_TABLES) {
     ISX_TRY(h, cudaMemcpy(host, b.ground + (size_t)local * 3 * H, need, cudaMemcpyDeviceToHost));
   } else if (tensor == ISX_T_OBJ_COST_LUT) {
@@ -1705,9 +1634,9 @@ int isx_read_tensor(isx_handle h, int tensor, int frame, void *host, size_t byte
                               b.records_b + (((size_t)local * C + col) * kp.rec_stride) * kRecBWords + word,
                               (size_t)kRecBWords * 4, 4, H + 1, cudaMemcpyDeviceToHost));
   } else {
-    launch_export_tables(kp, b, local, h->last_pairwise, h->d_export_cost, h->d_export_index, h->s_compute);
-    ISX_TRY(h, cudaStreamSynchronize(h->s_compute));
-    ISX_TRY(h, cudaMemcpy(host, tensor == ISX_T_COST_TABLE ? (void *)h->d_export_cost : (void *)h->d_export_index,
+    launch_export_tables(kp, b, local, I.last_pairwise, I.d_export_cost, I.d_export_index, I.s_compute);
+    ISX_TRY(h, cudaStreamSynchronize(I.s_compute));
+    ISX_TRY(h, cudaMemcpy(host, tensor == ISX_T_COST_TABLE ? (void *)I.d_export_cost : (void *)I.d_export_index,
                           need, cudaMemcpyDeviceToHost));
   }
   return ISX_OK;
@@ -1733,42 +1662,43 @@ int isx_set_profiling(isx_handle h, int enable) {
 
 int isx_get_stage_times(isx_handle h, double *ms, long *chunks, int n_stages, int reset) {
   if (int rc = check_ready(h)) return rc;
-  ISX_TRY(h, cudaStreamSynchronize(h->s_tables));
-  ISX_TRY(h, cudaStreamSynchronize(h->s_compute));
-  ISX_TRY(h, cudaStreamSynchronize(h->s_emit));
+  Initialized &I = *h->init;
+  ISX_TRY(h, cudaStreamSynchronize(I.s_tables));
+  ISX_TRY(h, cudaStreamSynchronize(I.s_compute));
+  ISX_TRY(h, cudaStreamSynchronize(I.s_emit));
   // 9 events per chunk (enqueue_chunk): stages 0..2 = events i..i+1 on s_tables, stage 3 = events 4..5 on s_compute,
   // stages 4, 5 = events 6..8 on s_emit.  The table build of a chunk overlaps the DP of the chunk before it, so the
   // stage times of a stream of chunks add up to more than the wall time.
   const int per = kProfEvents;
-  for (size_t base = 0; base + per <= h->prof_used; base += per) {
+  for (size_t base = 0; base + per <= I.prof_used; base += per) {
     for (int i = 0; i < 6; i++) {
       const int e0 = i < 3 ? i : i + 1;
       float t = 0.f;
-      if (cudaEventElapsedTime(&t, h->prof_events[base + e0], h->prof_events[base + e0 + 1]) == cudaSuccess) {
-        h->stage_ms[i] += t;
-        h->stage_launches[i]++;
+      if (cudaEventElapsedTime(&t, I.prof_events[base + e0], I.prof_events[base + e0 + 1]) == cudaSuccess) {
+        I.stage_ms[i] += t;
+        I.stage_launches[i]++;
       }
     }
   }
-  h->prof_used = 0;
-  h->prof_h2d_used = 0;
+  I.prof_used = 0;
+  I.prof_h2d_used = 0;
   for (int i = 0; i < n_stages && i < 6; i++) {
-    if (ms) ms[i] = h->stage_ms[i];
-    if (chunks) chunks[i] = h->stage_launches[i];
+    if (ms) ms[i] = I.stage_ms[i];
+    if (chunks) chunks[i] = I.stage_launches[i];
   }
   if (reset)
-    for (int i = 0; i < 8; i++) { h->stage_ms[i] = 0; h->stage_launches[i] = 0; }
+    for (int i = 0; i < 8; i++) { I.stage_ms[i] = 0; I.stage_launches[i] = 0; }
   return ISX_OK;
 }
 
 int isx_get_road_fill_time(isx_handle h, double *ms, long *calls, int reset) {
   if (int rc = check_ready(h)) return rc;
-  ISX_TRY(h, cudaStreamSynchronize(h->s_tables));
-  if (ms) *ms = (double)h->host_fill_ns.load() * 1e-6;
-  if (calls) *calls = (long)h->host_fill_calls.load();
+  ISX_TRY(h, cudaStreamSynchronize(h->init->s_tables));
+  if (ms) *ms = (double)h->init->host_fill_ns.load() * 1e-6;
+  if (calls) *calls = (long)h->init->host_fill_calls.load();
   if (reset) {
-    h->host_fill_ns = 0;
-    h->host_fill_calls = 0;
+    h->init->host_fill_ns = 0;
+    h->init->host_fill_calls = 0;
   }
   return ISX_OK;
 }
@@ -1779,37 +1709,38 @@ int isx_get_road_fill_time(isx_handle h, double *ms, long *calls, int reset) {
 // Returns the number of chunks written; call before isx_get_stage_times (which consumes the events).
 int isx_get_chunk_trace(isx_handle h, double *ms, int max_chunks) {
   if (int rc = check_ready(h)) return rc;
-  ISX_TRY(h, cudaStreamSynchronize(h->s_tables));
-  ISX_TRY(h, cudaStreamSynchronize(h->s_compute));
-  ISX_TRY(h, cudaStreamSynchronize(h->s_emit));
-  ISX_TRY(h, cudaStreamSynchronize(h->s_h2d));
-  const size_t chunks = std::min(h->prof_used / kProfEvents, h->prof_h2d_used / 2);
+  Initialized &I = *h->init;
+  ISX_TRY(h, cudaStreamSynchronize(I.s_tables));
+  ISX_TRY(h, cudaStreamSynchronize(I.s_compute));
+  ISX_TRY(h, cudaStreamSynchronize(I.s_emit));
+  ISX_TRY(h, cudaStreamSynchronize(I.s_h2d));
+  const size_t chunks = std::min(I.prof_used / kProfEvents, I.prof_h2d_used / 2);
   int n = 0;
   if (chunks == 0) return 0;
-  cudaEvent_t t0 = h->prof_h2d[0];
+  cudaEvent_t t0 = I.prof_h2d[0];
   for (size_t c = 0; c < chunks && n < max_chunks; c++, n++) {
     for (int i = 0; i < kTraceStamps; i++) {
-      cudaEvent_t e = i < 2 ? h->prof_h2d[2 * c + i] : h->prof_events[kProfEvents * c + (i - 2)];
+      cudaEvent_t e = i < 2 ? I.prof_h2d[2 * c + i] : I.prof_events[kProfEvents * c + (i - 2)];
       float t = 0.f;
       cudaEventElapsedTime(&t, t0, e);
       ms[(size_t)n * kTraceStamps + i] = t;
     }
   }
-  h->prof_h2d_used = 0;
+  I.prof_h2d_used = 0;
   return n;
 }
 
 int isx_get_dp_units(isx_handle h, unsigned long long *evaluated, unsigned long long *total) {
   if (int rc = check_ready(h)) return rc;
   unsigned long long dev = 0;
-  ISX_TRY(h, cudaStreamSynchronize(h->s_compute));
-  ISX_TRY(h, cudaMemcpy(&dev, h->buf.dp_units, sizeof dev, cudaMemcpyDeviceToHost));
-  if (evaluated) *evaluated = dev + h->dp_units_pairwise;
-  if (total) *total = h->dp_units_total;
+  ISX_TRY(h, cudaStreamSynchronize(h->init->s_compute));
+  ISX_TRY(h, cudaMemcpy(&dev, h->init->buf.dp_units, sizeof dev, cudaMemcpyDeviceToHost));
+  if (evaluated) *evaluated = dev + h->init->dp_units_pairwise;
+  if (total) *total = h->init->dp_units_total;
   return ISX_OK;
 }
-int isx_chunk_frames(isx_handle h) { return (h && h->initialized) ? h->last_launch_frames : 0; }
-int isx_instance_capacity(isx_handle h) { return (h && h->initialized) ? h->inst_cap : 0; }
+int isx_chunk_frames(isx_handle h) { return (h && h->init) ? h->init->last_launch_frames : 0; }
+int isx_instance_capacity(isx_handle h) { return (h && h->init) ? h->init->inst_cap : 0; }
 
 }  // extern "C"
 
@@ -1826,6 +1757,6 @@ int pool_submit_batch_host_road(isx_handle h, isx_road_handle road, int pairwise
                            roads_out);
 }
 
-int largest_chunk(isx_handle h) { return (h && h->initialized) ? std::max(h->chunk, h->chunk_unary) : 0; }
+int largest_chunk(isx_handle h) { return (h && h->init) ? std::max(h->init->chunk, h->init->chunk_unary) : 0; }
 
 }  // namespace isx

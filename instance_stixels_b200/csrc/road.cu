@@ -26,9 +26,11 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
+#include <memory>
 #include <string>
 #include <vector>
 
+#include "cuda_resources.h"
 #include "kernels.h"
 
 namespace isx {
@@ -208,16 +210,10 @@ pull_tables_kernel(const float *__restrict__ src_ground, float *__restrict__ dst
 }
 
 }  // namespace
-}  // namespace isx
 
-struct isx_road_estimator {
-  int device = 0;
-  bool initialized = false;
-  float cy = 0, baseline = 0, focal = 0, threshold = 0.2f;
-  int rows = 0, cols = 0, max_dis = 0, max_batch = 1;
-  int numangle = 0, numrho = 0;
-  float theta_step = 0;
-  float min_pitch = 0, max_pitch = 0;
+// Everything one isx_road_initialize acquires, and the state of the device selection since then.
+struct InitializedRoad {
+  explicit InitializedRoad(int device) : res(device) {}
   cudaStream_t stream = nullptr;
   float *d_disparity = nullptr;  // staging for host images
   int *d_vdisp = nullptr, *d_counters = nullptr;  // counters: [3][max_batch] maximum | n_points | n_cand
@@ -227,7 +223,6 @@ struct isx_road_estimator {
   float *d_tab = nullptr;  // sin | cos
   int *h_counters = nullptr;
   int2 *h_cand = nullptr;
-  int last_n = 0;
   // device selection (isx_compute_batch_device_road): the estimate of every Hough cell [numangle][numrho], uploaded on
   // first use; the selected key per frame; the keep-last state (cell of the last accepted estimate, -1 = seed)
   isx_road_estimate *d_cells = nullptr;
@@ -237,6 +232,20 @@ struct isx_road_estimator {
   bool has_seed = false;
   isx_road seed{0, 0.f, 0.f, 0.f};
   cudaEvent_t ev_in = nullptr, ev_done = nullptr;   // hand-off from / back to the stixel handle's stream
+  CudaResources res;   // owns every stream, event and allocation above
+};
+
+}  // namespace isx
+
+struct isx_road_estimator {
+  int device = 0;
+  float cy = 0, baseline = 0, focal = 0, threshold = 0.2f;
+  int rows = 0, cols = 0, max_dis = 0, max_batch = 1;
+  int numangle = 0, numrho = 0;
+  float theta_step = 0;
+  float min_pitch = 0, max_pitch = 0;
+  int last_n = 0;
+  std::unique_ptr<isx::InitializedRoad> init;   // null: not initialised
   std::string last_error;
 };
 
@@ -253,21 +262,6 @@ int road_fail(isx_road_estimator *h, int code, const std::string &msg) {
     if (_e != cudaSuccess)                                                                       \
       return road_fail(h, ISX_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));    \
   } while (0)
-
-void road_free(isx_road_estimator *h) {
-  cudaFree(h->d_disparity); cudaFree(h->d_vdisp); cudaFree(h->d_counters); cudaFree(h->d_binary);
-  cudaFree(h->d_points); cudaFree(h->d_cand); cudaFree(h->d_accum); cudaFree(h->d_tab);
-  cudaFree(h->d_cells); cudaFree(h->d_sel); cudaFree(h->d_state);
-  cudaFreeHost(h->h_counters); cudaFreeHost(h->h_cand);
-  if (h->stream) cudaStreamDestroy(h->stream);
-  if (h->ev_in) cudaEventDestroy(h->ev_in);
-  if (h->ev_done) cudaEventDestroy(h->ev_done);
-  h->d_disparity = nullptr; h->d_vdisp = nullptr; h->d_counters = nullptr; h->d_binary = nullptr;
-  h->d_points = nullptr; h->d_cand = nullptr; h->d_accum = nullptr; h->d_tab = nullptr;
-  h->d_cells = nullptr; h->d_sel = nullptr; h->d_state = nullptr; h->cells_ready = false; h->has_seed = false;
-  h->h_counters = nullptr; h->h_cand = nullptr; h->stream = nullptr; h->ev_in = nullptr; h->ev_done = nullptr;
-  h->initialized = false;
-}
 
 // RoadEstimation::ComputeCameraProperties (RoadEstimation.cu:172-193), same float expressions and libm calls.
 void camera_properties(const isx_road_estimator *h, float rho, float theta, float &horizon, float &pitch,
@@ -298,26 +292,27 @@ void cell_estimate(const isx_road_estimator *h, int nidx, int r, isx_road_estima
 
 int road_run(isx_road_estimator *h, int n, const float *d_disparity, isx_road_estimate *out) {
   using namespace isx;
+  isx::InitializedRoad &I = *h->init;
   const int rows = h->rows, cols = h->cols, D = h->max_dis, total = rows * D;
   const int B = h->max_batch;
-  cudaStream_t s = h->stream;
-  ROAD_TRY(h, cudaMemsetAsync(h->d_counters, 0, sizeof(int) * 3 * B, s));
-  vdisp_kernel<<<dim3(rows, n), 256, D * sizeof(int), s>>>(d_disparity, h->d_vdisp, h->d_counters, rows, cols, D);
-  binarize_kernel<<<dim3((total + 255) / 256, n), 256, 0, s>>>(h->d_vdisp, h->d_counters, h->d_binary, h->d_points,
-                                                               h->d_counters + B, h->threshold, rows, D);
+  cudaStream_t s = I.stream;
+  ROAD_TRY(h, cudaMemsetAsync(I.d_counters, 0, sizeof(int) * 3 * B, s));
+  vdisp_kernel<<<dim3(rows, n), 256, D * sizeof(int), s>>>(d_disparity, I.d_vdisp, I.d_counters, rows, cols, D);
+  binarize_kernel<<<dim3((total + 255) / 256, n), 256, 0, s>>>(I.d_vdisp, I.d_counters, I.d_binary, I.d_points,
+                                                               I.d_counters + B, h->threshold, rows, D);
   hough_kernel<<<dim3(h->numangle, n), 256, (h->numrho + 2) * sizeof(int), s>>>(
-      h->d_points, h->d_counters + B, h->d_tab, h->d_tab + h->numangle, h->d_accum, h->numangle, h->numrho, total);
+      I.d_points, I.d_counters + B, I.d_tab, I.d_tab + h->numangle, I.d_accum, h->numangle, h->numrho, total);
   maxima_kernel<<<dim3((h->numangle * h->numrho + 255) / 256, n), 256, 0, s>>>(
-      h->d_accum, h->d_cand, h->d_counters + 2 * B, h->numangle, h->numrho, kHoughThreshold, kMaxCandidates);
+      I.d_accum, I.d_cand, I.d_counters + 2 * B, h->numangle, h->numrho, kHoughThreshold, kMaxCandidates);
   g_launch_count += 4;
   ROAD_TRY(h, cudaGetLastError());
-  ROAD_TRY(h, cudaMemcpyAsync(h->h_counters, h->d_counters, sizeof(int) * 3 * B, cudaMemcpyDeviceToHost, s));
+  ROAD_TRY(h, cudaMemcpyAsync(I.h_counters, I.d_counters, sizeof(int) * 3 * B, cudaMemcpyDeviceToHost, s));
   ROAD_TRY(h, cudaStreamSynchronize(s));
   // only the used part of every frame's candidate array travels
   int most = 0;
-  for (int f = 0; f < n; f++) most = std::max(most, std::min(h->h_counters[2 * B + f], kMaxCandidates));
+  for (int f = 0; f < n; f++) most = std::max(most, std::min(I.h_counters[2 * B + f], kMaxCandidates));
   if (most > 0) {
-    ROAD_TRY(h, cudaMemcpy2DAsync(h->h_cand, sizeof(int2) * kMaxCandidates, h->d_cand, sizeof(int2) * kMaxCandidates,
+    ROAD_TRY(h, cudaMemcpy2DAsync(I.h_cand, sizeof(int2) * kMaxCandidates, I.d_cand, sizeof(int2) * kMaxCandidates,
                                   sizeof(int2) * most, n, cudaMemcpyDeviceToHost, s));
     ROAD_TRY(h, cudaStreamSynchronize(s));
   }
@@ -326,9 +321,9 @@ int road_run(isx_road_estimator *h, int n, const float *d_disparity, isx_road_es
   for (int f = 0; f < n; f++) {
     isx_road_estimate &e = out[f];
     e = isx_road_estimate{0, 0, 0.f, 0.f, 0.f, 0.f, 0.f};
-    const int nc = h->h_counters[2 * B + f];
+    const int nc = I.h_counters[2 * B + f];
     if (nc > kMaxCandidates) return road_fail(h, ISX_ERR_CAPACITY, "more Hough line candidates than the buffer holds");
-    int2 *c = h->h_cand + (size_t)f * kMaxCandidates;
+    int2 *c = I.h_cand + (size_t)f * kMaxCandidates;
     // hough_cmp_gt: votes descending, accumulator index ascending
     std::sort(c, c + nc, [](const int2 &a, const int2 &b) { return a.y > b.y || (a.y == b.y && a.x < b.x); });
     for (int k = 0; k < nc; k++) {
@@ -357,22 +352,18 @@ int isx_road_create(isx_road_handle *out, int device) {
   return ISX_OK;
 }
 
-void isx_road_destroy(isx_road_handle h) {
-  if (!h) return;
-  if (h->initialized) { cudaSetDevice(h->device); road_free(h); }
-  delete h;
-}
+void isx_road_destroy(isx_road_handle h) { delete h; }
 
 const char *isx_road_last_error(isx_road_handle h) { return h ? h->last_error.c_str() : g_road_error.c_str(); }
-int isx_road_is_initialized(isx_road_handle h) { return h && h->initialized; }
+int isx_road_is_initialized(isx_road_handle h) { return h && h->init; }
 
 int isx_road_initialize(isx_road_handle h, float camera_center_y, float baseline, float focal, int rows, int cols,
                         int max_dis, float road_vdisparity_threshold, int max_batch) {
   if (!h) return road_fail(h, ISX_ERR_INVALID_ARGUMENT, "null handle");
   if (rows < 1 || cols < 1 || max_dis < 1 || max_batch < 1)
     return road_fail(h, ISX_ERR_INVALID_ARGUMENT, "rows, cols, max_dis and max_batch must be positive");
+  h->init.reset();
   ROAD_TRY(h, cudaSetDevice(h->device));
-  if (h->initialized) road_free(h);
   h->cy = camera_center_y; h->baseline = baseline; h->focal = focal; h->threshold = road_vdisparity_threshold;
   h->rows = rows; h->cols = cols; h->max_dis = max_dis; h->max_batch = max_batch;
   // RoadEstimation.cu:47-58
@@ -397,41 +388,44 @@ int isx_road_initialize(isx_road_handle h, float camera_center_y, float baseline
     }
   }
   const size_t B = max_batch, total = (size_t)rows * max_dis;
-  ROAD_TRY(h, cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
-  ROAD_TRY(h, cudaMalloc(&h->d_disparity, sizeof(float) * rows * cols));
-  ROAD_TRY(h, cudaMalloc(&h->d_vdisp, sizeof(int) * B * total));
-  ROAD_TRY(h, cudaMalloc(&h->d_counters, sizeof(int) * 3 * B));
-  ROAD_TRY(h, cudaMalloc(&h->d_binary, B * total));
-  ROAD_TRY(h, cudaMalloc(&h->d_points, sizeof(int2) * B * total));
-  ROAD_TRY(h, cudaMalloc(&h->d_cand, sizeof(int2) * B * isx::kMaxCandidates));
+  // built here and kept only on success: an early return releases what was acquired
+  auto init = std::make_unique<isx::InitializedRoad>(h->device);
+  isx::InitializedRoad &I = *init;
+  ROAD_TRY(h, I.res.stream(&I.stream));
+  ROAD_TRY(h, I.res.device(&I.d_disparity, sizeof(float) * rows * cols));
+  ROAD_TRY(h, I.res.device(&I.d_vdisp, sizeof(int) * B * total));
+  ROAD_TRY(h, I.res.device(&I.d_counters, sizeof(int) * 3 * B));
+  ROAD_TRY(h, I.res.device(&I.d_binary, B * total));
+  ROAD_TRY(h, I.res.device(&I.d_points, sizeof(int2) * B * total));
+  ROAD_TRY(h, I.res.device(&I.d_cand, sizeof(int2) * B * isx::kMaxCandidates));
   const size_t acc = (size_t)(numangle + 2) * (h->numrho + 2);
-  ROAD_TRY(h, cudaMalloc(&h->d_accum, sizeof(int) * B * acc));
-  ROAD_TRY(h, cudaMemset(h->d_accum, 0, sizeof(int) * B * acc));  // border rows n = 0 and numangle + 1 stay zero
-  ROAD_TRY(h, cudaMalloc(&h->d_tab, sizeof(float) * 2 * numangle));
-  ROAD_TRY(h, cudaMemcpy(h->d_tab, tab.data(), sizeof(float) * 2 * numangle, cudaMemcpyHostToDevice));
-  ROAD_TRY(h, cudaMallocHost(&h->h_counters, sizeof(int) * 3 * B));
-  ROAD_TRY(h, cudaMallocHost(&h->h_cand, sizeof(int2) * B * isx::kMaxCandidates));
-  ROAD_TRY(h, cudaMalloc(&h->d_cells, sizeof(isx_road_estimate) * numangle * h->numrho));
-  ROAD_TRY(h, cudaMalloc(&h->d_sel, sizeof(unsigned long long) * B));
-  ROAD_TRY(h, cudaMalloc(&h->d_state, sizeof(int)));
-  ROAD_TRY(h, cudaEventCreateWithFlags(&h->ev_in, cudaEventDisableTiming));
-  ROAD_TRY(h, cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming));
+  ROAD_TRY(h, I.res.device(&I.d_accum, sizeof(int) * B * acc));
+  ROAD_TRY(h, cudaMemset(I.d_accum, 0, sizeof(int) * B * acc));  // border rows n = 0 and numangle + 1 stay zero
+  ROAD_TRY(h, I.res.device(&I.d_tab, sizeof(float) * 2 * numangle));
+  ROAD_TRY(h, cudaMemcpy(I.d_tab, tab.data(), sizeof(float) * 2 * numangle, cudaMemcpyHostToDevice));
+  ROAD_TRY(h, I.res.host(&I.h_counters, sizeof(int) * 3 * B));
+  ROAD_TRY(h, I.res.host(&I.h_cand, sizeof(int2) * B * isx::kMaxCandidates));
+  ROAD_TRY(h, I.res.device(&I.d_cells, sizeof(isx_road_estimate) * numangle * h->numrho));
+  ROAD_TRY(h, I.res.device(&I.d_sel, sizeof(unsigned long long) * B));
+  ROAD_TRY(h, I.res.device(&I.d_state, sizeof(int)));
+  ROAD_TRY(h, I.res.event(&I.ev_in));
+  ROAD_TRY(h, I.res.event(&I.ev_done));
   if ((h->numrho + 2) * sizeof(int) > 48 * 1024)
     ROAD_TRY(h, cudaFuncSetAttribute(isx::hough_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)((h->numrho + 2) * sizeof(int))));
-  h->initialized = true;
+  h->init = std::move(init);
   return ISX_OK;
 }
 
 int isx_road_finish(isx_road_handle h) {
   if (!h) return road_fail(h, ISX_ERR_INVALID_ARGUMENT, "null handle");
-  if (h->initialized) { cudaSetDevice(h->device); road_free(h); }
+  h->init.reset();
   return ISX_OK;
 }
 
 static int road_ready(isx_road_handle h) {
   if (!h) return road_fail(h, ISX_ERR_INVALID_ARGUMENT, "null handle");
-  if (!h->initialized) return road_fail(h, ISX_ERR_NOT_INITIALIZED, "Initialize() has not been called");
+  if (!h->init) return road_fail(h, ISX_ERR_NOT_INITIALIZED, "Initialize() has not been called");
   cudaError_t e = cudaSetDevice(h->device);
   if (e != cudaSuccess) return road_fail(h, ISX_ERR_CUDA, cudaGetErrorString(e));
   return ISX_OK;
@@ -441,8 +435,9 @@ int isx_road_compute_host(isx_road_handle h, const float *disparity, size_t n_pi
   if (int rc = road_ready(h)) return rc;
   if (!disparity || !out || n_pixels != (size_t)h->rows * h->cols)
     return road_fail(h, ISX_ERR_INVALID_ARGUMENT, "disparity image must hold rows * cols pixels");
-  ROAD_TRY(h, cudaMemcpyAsync(h->d_disparity, disparity, sizeof(float) * n_pixels, cudaMemcpyHostToDevice, h->stream));
-  return road_run(h, 1, h->d_disparity, out);
+  ROAD_TRY(h, cudaMemcpyAsync(h->init->d_disparity, disparity, sizeof(float) * n_pixels, cudaMemcpyHostToDevice,
+                              h->init->stream));
+  return road_run(h, 1, h->init->d_disparity, out);
 }
 
 int isx_road_compute_device(isx_road_handle h, const float *d_disparity, isx_road_estimate *out) {
@@ -459,7 +454,7 @@ int isx_road_compute_batch_device(isx_road_handle h, int n, const float *d_dispa
 }
 
 size_t isx_road_tensor_bytes(isx_road_handle h, int tensor) {
-  if (!h || !h->initialized) return 0;
+  if (!h || !h->init) return 0;
   const size_t total = (size_t)h->rows * h->max_dis;
   switch (tensor) {
     case 0: return total * sizeof(int);
@@ -474,10 +469,11 @@ int isx_road_read_tensor(isx_road_handle h, int tensor, int frame, void *host, s
   const size_t need = isx_road_tensor_bytes(h, tensor);
   if (need == 0 || !host || bytes < need || frame < 0 || frame >= h->last_n)
     return road_fail(h, ISX_ERR_INVALID_ARGUMENT, "bad tensor id, frame or buffer");
-  const char *src = tensor == 0 ? (const char *)h->d_vdisp : tensor == 1 ? (const char *)h->d_binary : (const char *)h->d_accum;
+  const char *src = tensor == 0 ? (const char *)h->init->d_vdisp
+                    : tensor == 1 ? (const char *)h->init->d_binary : (const char *)h->init->d_accum;
   // isx_compute_batch_device_road leaves its work queued on the road stream, which does not synchronise with the
   // legacy stream of cudaMemcpy
-  ROAD_TRY(h, cudaStreamSynchronize(h->stream));
+  ROAD_TRY(h, cudaStreamSynchronize(h->init->stream));
   ROAD_TRY(h, cudaMemcpy(host, src + need * frame, need, cudaMemcpyDeviceToHost));
   return ISX_OK;
 }
@@ -488,12 +484,12 @@ namespace isx {
 
 int road_check_batch(isx_road_handle h, int device, int rows, int cols, int max_dis, int n, bool has_fallback,
                      std::string &msg) {
-  if (!h || !h->initialized) return msg = "the road handle is not initialised", ISX_ERR_INVALID_ARGUMENT;
+  if (!h || !h->init) return msg = "the road handle is not initialised", ISX_ERR_INVALID_ARGUMENT;
   if (h->device != device) return msg = "the road handle computes on another device", ISX_ERR_INVALID_ARGUMENT;
   if (h->rows != rows || h->cols != cols || h->max_dis != max_dis)
     return msg = "the road handle was initialised for other rows, cols or max_dis", ISX_ERR_INVALID_ARGUMENT;
   if (n > h->max_batch) return msg = "batch size exceeds isx_road_initialize(max_batch)", ISX_ERR_CAPACITY;
-  if (!has_fallback && !h->has_seed)
+  if (!has_fallback && !h->init->has_seed)
     return msg = "no fallback road: the road handle has no state to continue from", ISX_ERR_INVALID_ARGUMENT;
   return ISX_OK;
 }
@@ -511,40 +507,41 @@ int road_enqueue_batch(isx_road_handle h, cudaStream_t caller, int n, const floa
   };
 #define ROAD_ENQ(expr) \
   if (int _rc = cuda((expr), #expr)) return _rc
-  if (!h->cells_ready) {
+  isx::InitializedRoad &I = *h->init;
+  if (!I.cells_ready) {
     // once per handle: the estimate of every Hough cell, by the code of the host walk (road_run)
     std::vector<isx_road_estimate> cells((size_t)h->numangle * h->numrho);
     for (int a = 0; a < h->numangle; a++)
       for (int r = 0; r < h->numrho; r++) cell_estimate(h, a, r, cells[(size_t)a * h->numrho + r]);
     // pageable source: returns once the driver has staged it, without waiting for other streams
-    ROAD_ENQ(cudaMemcpyAsync(h->d_cells, cells.data(), sizeof(isx_road_estimate) * cells.size(),
-                             cudaMemcpyHostToDevice, h->stream));
-    h->cells_ready = true;
+    ROAD_ENQ(cudaMemcpyAsync(I.d_cells, cells.data(), sizeof(isx_road_estimate) * cells.size(),
+                             cudaMemcpyHostToDevice, I.stream));
+    I.cells_ready = true;
   }
   if (fallback) {
-    h->seed = *fallback;
-    h->has_seed = true;
+    I.seed = *fallback;
+    I.has_seed = true;
   }
   const int rows = h->rows, cols = h->cols, D = h->max_dis, total = rows * D;
   const int B = h->max_batch;
-  cudaStream_t s = h->stream;
-  ROAD_ENQ(cudaEventRecord(h->ev_in, caller));
-  ROAD_ENQ(cudaStreamWaitEvent(s, h->ev_in, 0));
-  ROAD_ENQ(cudaMemsetAsync(h->d_counters, 0, sizeof(int) * 3 * B, s));
-  ROAD_ENQ(cudaMemsetAsync(h->d_sel, 0, sizeof(unsigned long long) * n, s));
-  vdisp_kernel<<<dim3(rows, n), 256, D * sizeof(int), s>>>(d_disparity, h->d_vdisp, h->d_counters, rows, cols, D);
-  binarize_kernel<<<dim3((total + 255) / 256, n), 256, 0, s>>>(h->d_vdisp, h->d_counters, h->d_binary, h->d_points,
-                                                               h->d_counters + B, h->threshold, rows, D);
+  cudaStream_t s = I.stream;
+  ROAD_ENQ(cudaEventRecord(I.ev_in, caller));
+  ROAD_ENQ(cudaStreamWaitEvent(s, I.ev_in, 0));
+  ROAD_ENQ(cudaMemsetAsync(I.d_counters, 0, sizeof(int) * 3 * B, s));
+  ROAD_ENQ(cudaMemsetAsync(I.d_sel, 0, sizeof(unsigned long long) * n, s));
+  vdisp_kernel<<<dim3(rows, n), 256, D * sizeof(int), s>>>(d_disparity, I.d_vdisp, I.d_counters, rows, cols, D);
+  binarize_kernel<<<dim3((total + 255) / 256, n), 256, 0, s>>>(I.d_vdisp, I.d_counters, I.d_binary, I.d_points,
+                                                               I.d_counters + B, h->threshold, rows, D);
   hough_kernel<<<dim3(h->numangle, n), 256, (h->numrho + 2) * sizeof(int), s>>>(
-      h->d_points, h->d_counters + B, h->d_tab, h->d_tab + h->numangle, h->d_accum, h->numangle, h->numrho, total);
-  select_kernel<<<dim3((h->numangle * h->numrho + 255) / 256, n), 256, 0, s>>>(h->d_accum, h->d_cells, h->d_sel,
+      I.d_points, I.d_counters + B, I.d_tab, I.d_tab + h->numangle, I.d_accum, h->numangle, h->numrho, total);
+  select_kernel<<<dim3((h->numangle * h->numrho + 255) / 256, n), 256, 0, s>>>(I.d_accum, I.d_cells, I.d_sel,
                                                                                h->numangle, h->numrho, kHoughThreshold);
-  resolve_kernel<<<1, 32, 0, s>>>(h->d_sel, h->d_cells, h->d_state, fallback ? 1 : 0, carry ? 1 : 0, h->seed, n,
+  resolve_kernel<<<1, 32, 0, s>>>(I.d_sel, I.d_cells, I.d_state, fallback ? 1 : 0, carry ? 1 : 0, I.seed, n,
                                   d_estimates, d_roads_out, d_roads);
   g_launch_count += 5;
   ROAD_ENQ(cudaGetLastError());
-  ROAD_ENQ(cudaEventRecord(h->ev_done, s));
-  ROAD_ENQ(cudaStreamWaitEvent(caller, h->ev_done, 0));
+  ROAD_ENQ(cudaEventRecord(I.ev_done, s));
+  ROAD_ENQ(cudaStreamWaitEvent(caller, I.ev_done, 0));
 #undef ROAD_ENQ
   h->last_n = n;
   return ISX_OK;
