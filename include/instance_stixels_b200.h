@@ -461,6 +461,69 @@ typedef struct isx_device_objects { /* device pointers; NULL = not written (fram
 int isx_export_objects_device(isx_handle h, int first, int n, const isx_device_objects *out);
 
 /* ------------------------------------------------------------------------
+ * Object tracking: one persistent id per object of a frame stream, on the device.  The DBSCAN labels of the objects
+ * are numbered per frame in column order, so they say nothing about identity; a tracker links the objects of
+ * consecutive frames by their image boxes and gives each chain one int64 id.  The definition (ObjectTracker.hpp states
+ * it on the host, HostObjectTracker): for every frame, each class c in 11..18 on its own,
+ *   1. candidates: every (live track t of class c, object o of class c) whose inclusive boxes overlap (I > 0,
+ *      U = area(t) + area(o) - I), with 1000 * I >= iou_min_permille * U in int64, and whose disparity ranges pass
+ *      the gate !(o.min > t.max + margin) && !(t.min > o.max + margin), each sum one round-to-nearest float add with
+ *      subnormals kept; the gate also passes when any of the four bounds is NaN;
+ *   2. greedy association: candidates by IoU descending (I1 * U2 against I2 * U1 in int64), then track id ascending,
+ *      then object label ascending; a pair is taken when neither its track nor its object is taken yet;
+ *   3. a matched track takes the object's box and disparity range, hits + 1, misses = 0; the object gets its id and hits;
+ *   4. an unmatched track gets misses + 1 and is removed when misses > max_age; its id never returns;
+ *   5. unmatched objects become tracks (hits 1) in label order while the class holds fewer than max_tracks live tracks;
+ *      an object left over gets id -1, hits 0 and sets ISX_TRACK_UNMATCHED in its frame's flags.
+ * Ids come from one counter per tracker, from 0, in record order within a frame (class, then label).  A frame whose
+ * records were not written (frame_offsets[f+1] > capacity, the export's rule) sets ISX_TRACK_NOT_WRITTEN and counts as
+ * a frame without objects: every track ages.  Exact while every box side stays below 2^15 pixels.  No motion model,
+ * no optimal (Hungarian) assignment, no 3D association, no re-identification.
+ * ------------------------------------------------------------------------ */
+#define ISX_TRACK_MAX_TRACKS 1024  /* largest max_tracks the device tracker holds per class */
+#define ISX_TRACK_MAX_FRAMES 4096  /* frames per isx_tracker_update_device call */
+#define ISX_TRACK_UNMATCHED 1      /* frame flag: an object was left without a track (its class was full) */
+#define ISX_TRACK_NOT_WRITTEN 2    /* frame flag: the frame's records were not written (capacity) */
+typedef struct isx_track_params {  /* 16 bytes */
+  int32_t iou_min_permille;        /* 1..1000, default 300 */
+  int32_t max_age;                 /* frames a track survives without a match, >= 0, default 2 */
+  float disparity_margin;          /* >= 0, not NaN, default 2.0; +inf turns the gate off */
+  int32_t max_tracks;              /* live tracks per class, 1..ISX_TRACK_MAX_TRACKS, default 1024 */
+} isx_track_params;
+typedef struct isx_track {         /* 48 bytes */
+  int64_t id;
+  int32_t semantic_class;
+  int32_t hits;                    /* frames in which the track was matched, its birth included */
+  int32_t misses;                  /* consecutive frames without a match */
+  int32_t x0, y0, x1, y1;          /* box and disparity range of the last matched object */
+  float disparity_min, disparity_max;
+  int32_t reserved;
+} isx_track;
+typedef struct isx_tracker *isx_tracker_handle;
+void isx_track_params_init(isx_track_params *p);
+/* params == NULL: the defaults.  Refused: ISX_ERR_INVALID_ARGUMENT for values outside the ranges above,
+ * ISX_ERR_UNSUPPORTED for max_tracks > ISX_TRACK_MAX_TRACKS. */
+int isx_tracker_create(isx_tracker_handle *out, int device, const isx_track_params *params);
+/* Waits for the updates in flight, then releases the tracker. */
+int isx_tracker_destroy(isx_tracker_handle t);
+/* Empties the tracker and restarts ids at 0, in order after the previous update; asynchronous. */
+int isx_tracker_reset(isx_tracker_handle t);
+/* The n frames of `in` (what isx_export_objects_device filled, capacity included) are the next n frames of the
+ * sequence.  Outputs are aligned with in->objects: d_track_ids [capacity] (8-byte aligned) and d_hits [capacity] get
+ * the id and hits of every object of the written frames, nothing else; d_frame_flags [n] the ISX_TRACK_* flags of
+ * every frame.  d_hits and d_frame_flags may be NULL.  Asynchronous on `stream` (a cudaStream_t, e.g. isx_stream(h)
+ * after the export); the host never waits, object counts are read on the device.  Every update waits for the previous
+ * update of the tracker, so calls on different streams are applied in call order.  in->class_offsets is required.
+ * Refusals enqueue nothing and leave the state alone: n outside 1..ISX_TRACK_MAX_FRAMES, null or misaligned
+ * pointers, pointers to host memory or to another device, negative capacity. */
+int isx_tracker_update_device(isx_tracker_handle t, uint64_t stream, int n, const isx_device_objects *in,
+                              int64_t *d_track_ids, int32_t *d_hits, int32_t *d_frame_flags);
+/* For tests: waits for the updates in flight and writes up to `capacity` live tracks ordered by id; *n = live tracks,
+ * *next_id = the id the next new track gets (either may be NULL). */
+int isx_tracker_read_state(isx_tracker_handle t, isx_track *host, int capacity, int *n, int64_t *next_id);
+const char *isx_tracker_last_error(isx_tracker_handle t); /* t may be NULL: last global error */
+
+/* ------------------------------------------------------------------------
  * Road estimation (SURVEY.md 8f rank 1): the step in front of the stixel path.
  * Replaces `class RoadEstimation` (InstanceStixels/include/InstanceStixels/RoadEstimation.h:31-93,
  * src/RoadEstimation.cu:24-193, src/RoadEstimationKernels.cu:25-60) including its one third-party

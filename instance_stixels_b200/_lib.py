@@ -47,6 +47,9 @@ EXPORTS = [
     # host batches and the frame pool with road estimation inside the pipeline
     "isx_submit_batch_host_road", "isx_submit_batch_host_u16_road", "isx_pool_compute_host_road",
     "isx_get_road_fill_time",
+    # object tracking on the device
+    "isx_track_params_init", "isx_tracker_create", "isx_tracker_destroy", "isx_tracker_reset",
+    "isx_tracker_update_device", "isx_tracker_read_state", "isx_tracker_last_error",
 ]
 
 
@@ -109,6 +112,12 @@ class DeviceObjects(C.Structure):
                 ("extents", C.c_void_p), ("capacity", C.c_int32), ("reserved", C.c_int32)]
 
 
+class TrackParams(C.Structure):
+    """isx_track_params: the tracker's association and lifetime parameters (isx_track_params_init: defaults)."""
+    _fields_ = [("iou_min_permille", C.c_int32), ("max_age", C.c_int32), ("disparity_margin", C.c_float),
+                ("max_tracks", C.c_int32)]
+
+
 # numpy views of isx_section (== Section, types.h:186-194) and isx_instance
 SECTION_DTYPE = np.dtype([("type", "<i4"), ("vB", "<i4"), ("vT", "<i4"), ("disparity", "<f4"),
                           ("semantic_class", "<i4"), ("cost", "<f4"), ("instance_meanx", "<f4"),
@@ -121,7 +130,10 @@ PACKED_FRAME_DTYPE = np.dtype([("section_offset", "<i4"), ("section_count", "<i4
                                ("instance_count", "<i4"), ("error", "<i4"), ("overflow", "<i4"),
                                ("reserved", "<i4", (2,))])
 assert SECTION_DTYPE.itemsize == 32 and INSTANCE_DTYPE.itemsize == 16 and PACKED_FRAME_DTYPE.itemsize == 32
-assert OBJECT_DTYPE.itemsize == 48
+TRACK_DTYPE = np.dtype([("id", "<i8")] + [(n, "<i4") for n in ("semantic_class", "hits", "misses", "x0", "y0", "x1",
+                                                                   "y1")] +
+                       [("disparity_min", "<f4"), ("disparity_max", "<f4"), ("reserved", "<i4")])
+assert OBJECT_DTYPE.itemsize == 48 and TRACK_DTYPE.itemsize == 48
 
 ISX_OK = 0
 T_JOINED_DISPARITY, T_OBJECT_LUT, T_DISPARITY_PS, T_VALID_PS, T_GROUND_PS, T_SKY_PS, T_COST_TABLE, \
@@ -232,6 +244,16 @@ def _declare(lib):
     lib.isx_submit_batch_host_u16_road.argtypes = [H, H, i, i, C.c_void_p, f, C.c_void_p, C.POINTER(Road), C.c_void_p,
                                                    C.c_void_p, C.c_void_p]
     lib.isx_get_road_fill_time.argtypes = [H, C.POINTER(C.c_double), C.POINTER(C.c_long), i]
+    lib.isx_track_params_init.argtypes = [C.POINTER(TrackParams)]
+    lib.isx_track_params_init.restype = None
+    lib.isx_tracker_create.argtypes = [C.POINTER(H), i, C.POINTER(TrackParams)]
+    lib.isx_tracker_destroy.argtypes = [H]
+    lib.isx_tracker_reset.argtypes = [H]
+    lib.isx_tracker_update_device.argtypes = [H, C.c_uint64, i, C.POINTER(DeviceObjects), C.c_void_p, C.c_void_p,
+                                              C.c_void_p]
+    lib.isx_tracker_read_state.argtypes = [H, C.c_void_p, i, C.POINTER(i), C.POINTER(C.c_int64)]
+    lib.isx_tracker_last_error.argtypes = [H]
+    lib.isx_tracker_last_error.restype = C.c_char_p
     lib.isx_pool_compute_host_road.argtypes = [H, i, i, C.c_void_p, C.c_void_p, C.POINTER(Road), C.c_void_p,
                                                C.c_void_p, C.c_void_p, C.c_void_p, i, C.c_void_p]
 

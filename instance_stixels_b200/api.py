@@ -89,11 +89,16 @@ class DeviceObjects:
     """isx_object records on the device (Stixels.ExportObjectsDevice): `data` is the int32 [capacity, 12] tensor, the
     properties are its columns.  The objects of frame f are rows [frame_offsets[f], frame_offsets[f+1]); the object of
     (frame f, class c, label l) is row class_offsets[8f + c - 11] + l.  `extents` is float32 [capacity, 2, 3] (min
-    x, y, z; max x, y, z) or None."""
+    x, y, z; max x, y, z) or None.  With a tracker (ComputeBatchTensors(tracker=)), `track_ids` int64 [capacity] and
+    `track_hits` int32 [capacity] hold the persistent id and hits of every object, `track_flags` int32 [n] the
+    ISX_TRACK_* flags of every frame (ObjectTracker.update)."""
     data: Any
     frame_offsets: Any
     class_offsets: Any
     extents: Any = None
+    track_ids: Any = None
+    track_hits: Any = None
+    track_flags: Any = None
 
     semantic_class = property(lambda self: self.data[:, 0])
     label = property(lambda self: self.data[:, 1])
@@ -266,7 +271,8 @@ class Stixels:
     def ComputeBatchTensors(self, pairwise: bool, disparity, roads: Optional[Sequence[dict]] = None,
                             segmentation=None, cnn=None, vertices: bool = False, capacity: Optional[int] = None,
                             road: Optional["RoadEstimation"] = None, fallback: Optional[dict] = None,
-                            objects: bool = False, object_capacity: Optional[int] = None) -> "DeviceStixels":
+                            objects: bool = False, object_capacity: Optional[int] = None,
+                            tracker: Optional["ObjectTracker"] = None) -> "DeviceStixels":
         """CUDA torch tensors in, torch tensors out, no host synchronisation: `disparity` float32 [n][rows][cols]
         and either `segmentation` int32 in the library layout [n][realcols][21][rows_power2_segmentation] or `cnn`
         float32 [n][21][rows/8][cols/8] (run through FlipAndPadBatchDevice).  The library's stream waits for the
@@ -276,8 +282,14 @@ class Stixels:
         on the device from the frame's disparity (ComputeBatchDeviceRoad; `fallback` as there).  With `road`, the
         result also carries `road_estimates` and `roads`.
         objects=True: the result also carries `objects` (ExportObjectsDevice of the batch, with extents when
-        vertices=True); `object_capacity` defaults to the worst case n * realcols * 200."""
+        vertices=True); `object_capacity` defaults to the worst case n * realcols * 200.
+        tracker=ObjectTracker (with objects=True): the n frames are the tracker's next frames; `objects` also carries
+        `track_ids`, `track_hits` and `track_flags` (ObjectTracker.update), in stream order after the export."""
         import torch
+        if tracker is not None and not objects:
+            raise InvalidArgument("tracker= needs objects=True")
+        if tracker is not None and tracker._device != self._device:
+            raise InvalidArgument(f"the tracker tracks on cuda:{tracker._device}, the handle computes on cuda:{self._device}")
         if (roads is None) == (road is None):
             raise InvalidArgument("pass exactly one of roads= and road=")
         if fallback is not None and road is None:
@@ -321,6 +333,10 @@ class Stixels:
                 frame_offsets=torch.empty(n + 1, dtype=torch.int32, device=dev),
                 class_offsets=torch.empty(n * 8 + 1, dtype=torch.int32, device=dev),
                 extents=torch.empty((ocap, 2, 3), dtype=torch.float32, device=dev) if vertices else None)
+            if tracker is not None:
+                out.objects.track_ids = torch.empty(ocap, dtype=torch.int64, device=dev)
+                out.objects.track_hits = torch.empty(ocap, dtype=torch.int32, device=dev)
+                out.objects.track_flags = torch.empty(n, dtype=torch.int32, device=dev)
         if road is not None:
             out.road_estimates = DeviceRoadEstimates(torch.empty((n, 7), dtype=torch.int32, device=dev))
             out.roads = DeviceRoads(torch.empty((n, 4), dtype=torch.int32, device=dev))
@@ -348,6 +364,8 @@ class Stixels:
             self.ExportObjectsDevice(0, n, ob.frame_offsets.data_ptr(), objects=ob.data.data_ptr(),
                                      class_offsets=ob.class_offsets.data_ptr(),
                                      extents=ob.extents.data_ptr() if vertices else 0, capacity=ocap)
+            if tracker is not None:
+                tracker._enqueue(self.stream(), n, ob, ob.track_ids, ob.track_hits, ob.track_flags)
         done = torch.cuda.Event()
         done.record(ext)
         current.wait_event(done)
@@ -746,6 +764,84 @@ class RoadEstimation:
         if tensor == 1:
             return out.reshape(rows, max_dis)
         return out.view(np.int32).reshape(-1, 2 * (rows + max_dis) + 3)
+
+
+class ObjectTracker:
+    """Persistent ids for the objects of a frame stream, on the device (isx_tracker_*; the definition is
+    HostObjectTracker in include/InstanceStixels/ObjectTracker.hpp).  Keyword parameters: iou_min_permille (300),
+    max_age (2), disparity_margin (2.0), max_tracks (1024)."""
+
+    def __init__(self, device: int = 0, **params):
+        self._lib = L.load()
+        p = L.TrackParams()
+        self._lib.isx_track_params_init(C.byref(p))
+        names = {n for n, _ in L.TrackParams._fields_}
+        for k, v in params.items():
+            if k not in names:
+                raise InvalidArgument(f"unknown tracker parameter {k!r}")
+            setattr(p, k, v)
+        self._h = C.c_void_p()
+        rc = self._lib.isx_tracker_create(C.byref(self._h), device, C.byref(p))
+        if rc != L.ISX_OK:
+            self._h = None
+            self._raise(rc)
+        self._device = device
+        self.params = {n: getattr(p, n) for n in names}
+
+    def _raise(self, rc):
+        msg = self._lib.isx_tracker_last_error(self._h).decode()
+        raise (InvalidArgument if rc == -1 else StixelsError)(f"{msg} ({rc})")
+
+    def _check(self, rc):
+        if rc != L.ISX_OK:
+            self._raise(rc)
+
+    def __del__(self):
+        try:
+            if self._h:
+                self._lib.isx_tracker_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def _enqueue(self, stream: int, n: int, objects: DeviceObjects, track_ids, hits, flags):
+        ob = L.DeviceObjects(objects.data.data_ptr(), objects.frame_offsets.data_ptr(),
+                             objects.class_offsets.data_ptr(), None, int(objects.data.shape[0]), 0)
+        self._check(self._lib.isx_tracker_update_device(self._h, stream, n, C.byref(ob), track_ids.data_ptr(),
+                                                        hits.data_ptr() if hits is not None else None,
+                                                        flags.data_ptr() if flags is not None else None))
+
+    def update(self, objects: DeviceObjects, n: int):
+        """The n frames of `objects` (Stixels.ComputeBatchTensors(objects=True)) as the tracker's next frames, on the
+        current torch stream, without a host synchronisation.  Returns (track_ids int64 [capacity], hits int32
+        [capacity], frame_flags int32 [n]) aligned with objects.data; entries of unwritten frames are not written."""
+        import torch
+        dev = objects.data.device
+        if dev.type != "cuda" or dev.index != self._device:
+            raise InvalidArgument(f"the objects are on {dev}, the tracker tracks on cuda:{self._device}")
+        cap = int(objects.data.shape[0])
+        ids = torch.empty(cap, dtype=torch.int64, device=dev)
+        hits = torch.empty(cap, dtype=torch.int32, device=dev)
+        flags = torch.empty(n, dtype=torch.int32, device=dev)
+        self._enqueue(torch.cuda.current_stream(dev).cuda_stream, n, objects, ids, hits, flags)
+        return ids, hits, flags
+
+    def reset(self):
+        """Empty the tracker and restart ids at 0 (ordered after the previous update)."""
+        self._check(self._lib.isx_tracker_reset(self._h))
+
+    def state(self):
+        """Waits for the updates in flight: (live tracks as a TRACK_DTYPE array ordered by id, next id)."""
+        n, nxt = C.c_int(0), C.c_int64(0)
+        self._check(self._lib.isx_tracker_read_state(self._h, None, 0, C.byref(n), None))
+        out = np.zeros(n.value, dtype=L.TRACK_DTYPE)
+        self._check(self._lib.isx_tracker_read_state(self._h, out.ctypes.data if n.value else None, n.value,
+                                                     C.byref(n), C.byref(nxt)))
+        return out, nxt.value
+
+    def handle(self):
+        """The isx_tracker_handle, for the C entry points."""
+        return self._h
 
 
 def dbscan_fit(xy: np.ndarray, eps: float, min_pts: int, core_candidates: np.ndarray, device: int = 0) -> np.ndarray:

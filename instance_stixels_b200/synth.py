@@ -63,12 +63,59 @@ def make_frame(index: int, rows: int = 1024, cols: int = 2048, column_step: int 
                max_dis: int = 128, vhor: int | None = None) -> Frame:
     """Frame `index` of the synthetic stream (seed = SEED0 + index)."""
     rng = np.random.Generator(np.random.PCG64(SEED0 + index))
+    vhor, alpha = _horizon(rows, vhor)
+    return _render(rng, _rectangles(rng, rows, cols, vhor), rows, cols, column_step, max_dis, vhor, alpha)
+
+
+def make_moving_batch(n: int, start: int = 0, rows: int = 1024, cols: int = 2048, column_step: int = 8,
+                      max_dis: int = 128, seed: int = 0):
+    """A moving scene: the rectangles of scene `seed`, each shifted sideways by its own 1..4 pixels per frame (bouncing
+    off the image borders), over the same road.  Frames start..start+n-1 as make_batch returns them; the noise and the
+    CNN output of frame i are drawn afresh (seed and i)."""
+    rng = np.random.Generator(np.random.PCG64([SEED0, seed]))
+    vhor, alpha = _horizon(rows, None)
+    rects = _rectangles(rng, rows, cols, vhor)
+    speed = rng.integers(1, 5, size=len(rects)) * rng.choice([-1, 1], size=len(rects))
+    frames = []
+    for i in range(start, start + n):
+        moved = []
+        for (base, top, x0, rw, c), v in zip(rects, speed):
+            span = cols - rw
+            x = (x0 + i * int(v)) % (2 * span)          # bounce between 0 and cols - rw
+            moved.append((base, top, x if x <= span else 2 * span - x, rw, c))
+        frame_rng = np.random.Generator(np.random.PCG64([SEED0, seed, i]))
+        frames.append(_render(frame_rng, moved, rows, cols, column_step, max_dis, vhor, alpha))
+    return (np.stack([f.disparity for f in frames]), np.stack([f.segmentation for f in frames]),
+            [f.road for f in frames])
+
+
+def _horizon(rows: int, vhor: int | None):
+    if vhor is None:
+        vhor = int(round(ROAD_PARAMS["vhor"] * rows / 1024.0))
+    alpha = ROAD_PARAMS["alpha_ground"] * 1024.0 / rows  # keep bottom-row disparity ~110 < max_dis - epsilon
+    return vhor, alpha
+
+
+def _rectangles(rng, rows: int, cols: int, vhor: int):
+    """6..14 object rectangles (base row, top row, x0, width, class)."""
+    H, W = rows, cols
+    n_rect = int(rng.integers(6, 15))
+    rects = []
+    for _ in range(n_rect):
+        rw = int(rng.integers(max(8, 40 * W // 2048), max(9, 400 * W // 2048) + 1))
+        rh = int(rng.integers(max(8, 60 * H // 1024), max(9, 500 * H // 1024) + 1))
+        x0 = int(rng.integers(0, W - rw))
+        base = int(rng.integers(vhor + max(2, 20 * H // 1024), H))  # image row of the base
+        top = max(0, base - rh)
+        c = int(OBJECT_CLASSES[int(rng.integers(0, len(OBJECT_CLASSES)))])
+        rects.append((base, top, x0, rw, c))
+    return rects
+
+
+def _render(rng, rects, rows: int, cols: int, column_step: int, max_dis: int, vhor: int, alpha: float) -> Frame:
     H, W, w = rows, cols, column_step
     Hs, C = H // 8, W // w
     Hs2 = rows_power2_segmentation(H)
-    if vhor is None:
-        vhor = int(round(ROAD_PARAMS["vhor"] * H / 1024.0))
-    alpha = ROAD_PARAMS["alpha_ground"] * 1024.0 / H  # keep bottom-row disparity ~110 < max_dis - epsilon
 
     y = np.arange(H, dtype=np.float32)[:, None]
     disp = np.where(y > vhor, alpha * (y - vhor), 0.0).astype(np.float32)
@@ -82,16 +129,6 @@ def make_frame(index: int, rows: int = 1024, cols: int = 2048, column_step: int 
     cx = np.full((H, W), np.nan, dtype=np.float32)
     cy = np.full((H, W), np.nan, dtype=np.float32)
 
-    n_rect = int(rng.integers(6, 15))
-    rects = []
-    for _ in range(n_rect):
-        rw = int(rng.integers(max(8, 40 * W // 2048), max(9, 400 * W // 2048) + 1))
-        rh = int(rng.integers(max(8, 60 * H // 1024), max(9, 500 * H // 1024) + 1))
-        x0 = int(rng.integers(0, W - rw))
-        base = int(rng.integers(vhor + max(2, 20 * H // 1024), H))  # image row of the base
-        top = max(0, base - rh)
-        c = int(OBJECT_CLASSES[int(rng.integers(0, len(OBJECT_CLASSES)))])
-        rects.append((base, top, x0, rw, c))
     # far objects first so nearer ones (larger base row) occlude them
     for base, top, x0, rw, c in sorted(rects):
         d = alpha * (base - vhor)
