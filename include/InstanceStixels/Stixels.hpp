@@ -350,6 +350,81 @@ public:
         return out;
     }
 
+    // Frames [first, first + n) of the last batch as bird's-eye-view grids, [n][nz][nx] cells, into the caller's
+    // device buffer (isx_bev_grid_device), asynchronous on isx_stream().
+    void BevGridDevice(int first, int n, const isx_bev_params& params, isx_bev_cell* d_cells) {
+        check(isx_bev_grid_device(h_, first, n, &params, d_cells));
+    }
+
+    // The bird's-eye-view grid of one frame on the host, the definition isx_bev_grid_device implements (the header
+    // states it in full): [nz][nx] cells, row-major, iz growing forward.  An OBJECT stixel marks the cells of its row
+    // a = (z - z_min) / cell between its corners xl and xr; a cell's occupant is the stixel with the smallest z, ties
+    // to the smallest frame-local index.  A cell without an occupant is free when the image row and column of its
+    // centre show a GROUND stixel, else unknown.  Every operation is one binary32 operation rounded to nearest, so a
+    // build that contracts a * b + c into an FMA computes something else (the tests build with -ffp-contract=off).
+    // Needs the camera centre, like Get3DVertices; the road is the frame's alpha_ground and (flipped) vhor.
+    std::vector<isx_bev_cell> GetBevGrid(const StixelsData& d, const isx_bev_params& p) {
+        return GetBevGrid(cfg_, d, p);
+    }
+    // The same with the camera (focal, baseline, camera_center_x/y) of `camera`: needs no device.
+    static std::vector<isx_bev_cell> GetBevGrid(const StixelConfig& camera, const StixelsData& d,
+                                                const isx_bev_params& p) {
+        check_camera(camera);
+        if (!(std::isfinite(p.cell) && p.cell >= 1e-3f && p.cell <= 1e3f) || p.nx < 1 || p.nx > ISX_BEV_MAX_SIDE ||
+            p.nz < 1 || p.nz > ISX_BEV_MAX_SIDE || !(std::isfinite(p.x_min) && std::fabs(p.x_min) <= 1e5f) ||
+            !(std::isfinite(p.z_min) && std::fabs(p.z_min) <= 1e5f) || p.reserved != 0)
+            throw std::invalid_argument("BEV parameters out of range");
+        const size_t nx = (size_t)p.nx;
+        std::vector<isx_bev_cell> out((size_t)p.nz * nx, isx_bev_cell{-1, ISX_BEV_UNKNOWN});
+        std::vector<float> nearest(out.size());
+        int32_t i = 0;   // frame-local index: column 0 first, each column top to bottom
+        for (size_t col = 0; col < (size_t)d.realcols; col++) {
+            for (size_t j = 0; j < (size_t)d.max_sections; j++, i++) {
+                const Section& s = d.sections[col * d.max_sections + j];
+                if (s.type == -1) break;
+                if (s.type != OBJECT) continue;
+                float v[12];
+                StixelVertices(camera, d, col, s, v);
+                const float z = v[2], a = (z - p.z_min) / p.cell;
+                if (!(a >= 0 && a < p.nz)) continue;
+                const float l = (v[0] - p.x_min) / p.cell, r = (v[3] - p.x_min) / p.cell;
+                if (!(r >= 0 && l < p.nx)) continue;
+                const int ix0 = l < 0 ? 0 : (int)l, ix1 = r >= p.nx ? p.nx - 1 : (int)r;
+                for (int ix = ix0; ix <= ix1; ix++) {
+                    const size_t k = (size_t)(int)a * nx + ix;
+                    if (out[k].stixel < 0 || z < nearest[k]) {
+                        out[k] = isx_bev_cell{i, ISX_BEV_OCCUPIED};
+                        nearest[k] = z;
+                    }
+                }
+            }
+        }
+        const float bf = camera.baseline * camera.focal;
+        for (int iz = 0; iz < p.nz; iz++)
+            for (int ix = 0; ix < p.nx; ix++) {
+                isx_bev_cell& cell = out[(size_t)iz * nx + ix];
+                if (cell.stixel >= 0) continue;
+                const float xc = p.x_min + ((float)ix + 0.5f) * p.cell;
+                const float zc = p.z_min + ((float)iz + 0.5f) * p.cell;
+                if (!(zc > 0)) continue;
+                const float u = camera.camera_center_x + camera.focal * (xc / zc);
+                if (!(u >= 0 && u < d.realcols * d.column_step)) continue;
+                const size_t c = (size_t)((int)u / d.column_step);
+                const float t = bf / (d.alpha_ground * zc), vf = (float)d.vhor - t;
+                if (!(t > 0 && vf >= 0 && vf < d.rows)) continue;
+                const int v = (int)vf;
+                for (size_t j = 0; j < (size_t)d.max_sections; j++) {   // top to bottom: the first with vB <= v
+                    const Section& s = d.sections[c * d.max_sections + j];
+                    if (s.type == -1) break;
+                    if (s.vB <= v) {
+                        if (v <= s.vT && s.type == GROUND) cell.state = ISX_BEV_FREE;
+                        break;
+                    }
+                }
+            }
+        return out;
+    }
+
     isx_handle handle() { return h_; }  // for the other C entry points
 
 private:

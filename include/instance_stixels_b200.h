@@ -524,6 +524,51 @@ int isx_tracker_read_state(isx_tracker_handle t, isx_track *host, int capacity, 
 const char *isx_tracker_last_error(isx_tracker_handle t); /* t may be NULL: last global error */
 
 /* ------------------------------------------------------------------------
+ * Bird's-eye-view grid: the stixels of frames [first, first + n) of the last batch (or of the last isx_compute:
+ * first = 0, n = 1) projected onto a grid on the ground plane, in the caller's DEVICE buffer, for planners that want
+ * free space and obstacles, not stixels.  The grid lies on the camera's x (right) / z (forward) plane, in metres:
+ * cell (iz, ix) covers x in [x_min + ix*cell, x_min + (ix+1)*cell) and z in [z_min + iz*cell, z_min + (iz+1)*cell);
+ * d_cells is [n][nz][nx], row-major, iz growing forward.  The road of a frame is the one the export uses
+ * (alpha_ground and the flipped horizon vhor = rows - road.vhor - 1); bf = baseline * focal, one float product.
+ *   Occupied: every OBJECT stixel of the frame, with frame-local index i (its position in isx_export_batch_device's
+ *   order: column 0 first, each column top to bottom), takes its corners as Get3DVertices computes them (xl = v[0],
+ *   xr = v[3], z = v[2]).  a = (z - z_min) / cell; the stixel counts only if a >= 0 && a < nz (a NaN never counts),
+ *   iz = (int)a.  l = (xl - x_min) / cell, r = (xr - x_min) / cell; the stixel is skipped unless r >= 0 && l < nx,
+ *   else it marks every ix from (l < 0 ? 0 : (int)l) to (r >= nx ? nx-1 : (int)r), both included.  A cell's occupant
+ *   is the stixel with the smallest z (-0.0 equal to +0.0), ties to the smallest i.
+ *   Free: a cell without an occupant, with centre xc = x_min + ((float)ix + 0.5f)*cell, zc = z_min + ((float)iz +
+ *   0.5f)*cell, is free iff zc > 0; u = cx + focal*(xc/zc) has u >= 0 && u < realcols*column_step, column
+ *   c = (int)u / column_step; t = bf / (alpha_ground*zc) and vf = (float)vhor - t have t > 0 && vf >= 0 && vf < rows,
+ *   row v = (int)vf; and the stixel of column c with vB <= v <= vT is GROUND.
+ *   Every other cell is unknown: ground hidden behind an object, sky, cells outside the field of view or below the
+ *   image, every cell of a frame with alpha_ground <= 0.
+ * Every operation is one IEEE binary32 operation rounded to nearest with subnormals kept (the corners are the
+ * export's vertices).  Every field is an order-independent minimum, so the bytes are the same on every call.  The
+ * occupant's index reaches everything else through the exports of the same frames: its Section and vertices are
+ * sections[frame_offsets[f] + stixel], its instance label labels[...], its object (label >= 0, class 11..18)
+ * class_offsets[8f + class - 11] + label, and that object's id track_ids[object].  Needs camera_center_x/y.
+ * Asynchronous on isx_stream(); refusals (frames outside the batch, null or non-8-byte-aligned d_cells, parameters
+ * outside the ranges below, no camera centre, batches in flight) enqueue nothing.  Stixels::GetBevGrid (Stixels.hpp)
+ * computes the same on the host.
+ * ------------------------------------------------------------------------ */
+#define ISX_BEV_UNKNOWN 0
+#define ISX_BEV_FREE 1
+#define ISX_BEV_OCCUPIED 2
+#define ISX_BEV_MAX_SIDE 4096       /* largest nx and nz */
+typedef struct isx_bev_params {     /* 24 bytes */
+  float x_min, z_min;               /* grid origin in metres: finite, magnitude <= 1e5; default -20, 0 */
+  float cell;                       /* cell side in metres, finite, in [1e-3, 1e3]; default 0.2 */
+  int32_t nx, nz;                   /* cells across and forward, 1..ISX_BEV_MAX_SIDE; default 200 x 300 (40 m x 60 m) */
+  int32_t reserved;                 /* 0 */
+} isx_bev_params;
+typedef struct isx_bev_cell {       /* 8 bytes */
+  int32_t stixel;                   /* the occupant's frame-local index, -1 if none */
+  int32_t state;                    /* ISX_BEV_UNKNOWN, ISX_BEV_FREE or ISX_BEV_OCCUPIED */
+} isx_bev_cell;
+void isx_bev_params_init(isx_bev_params *p);
+int isx_bev_grid_device(isx_handle h, int first, int n, const isx_bev_params *p, isx_bev_cell *d_cells);
+
+/* ------------------------------------------------------------------------
  * Road estimation (SURVEY.md 8f rank 1): the step in front of the stixel path.
  * Replaces `class RoadEstimation` (InstanceStixels/include/InstanceStixels/RoadEstimation.h:31-93,
  * src/RoadEstimation.cu:24-193, src/RoadEstimationKernels.cu:25-60) including its one third-party

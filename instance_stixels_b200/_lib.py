@@ -50,6 +50,8 @@ EXPORTS = [
     # object tracking on the device
     "isx_track_params_init", "isx_tracker_create", "isx_tracker_destroy", "isx_tracker_reset",
     "isx_tracker_update_device", "isx_tracker_read_state", "isx_tracker_last_error",
+    # bird's-eye-view grid on the device
+    "isx_bev_params_init", "isx_bev_grid_device",
 ]
 
 
@@ -117,6 +119,20 @@ class TrackParams(C.Structure):
     _fields_ = [("iou_min_permille", C.c_int32), ("max_age", C.c_int32), ("disparity_margin", C.c_float),
                 ("max_tracks", C.c_int32)]
 
+
+class BevParams(C.Structure):
+    """isx_bev_params: the grid on the ground plane (isx_bev_params_init: defaults, 200 x 300 cells of 0.2 m)."""
+    _fields_ = [("x_min", C.c_float), ("z_min", C.c_float), ("cell", C.c_float), ("nx", C.c_int32),
+                ("nz", C.c_int32), ("reserved", C.c_int32)]
+
+
+class BevCell(C.Structure):
+    """isx_bev_cell: the occupant's frame-local stixel index (-1 = none) and the ISX_BEV_* state."""
+    _fields_ = [("stixel", C.c_int32), ("state", C.c_int32)]
+
+
+BEV_UNKNOWN, BEV_FREE, BEV_OCCUPIED = 0, 1, 2
+BEV_MAX_SIDE = 4096
 
 # numpy views of isx_section (== Section, types.h:186-194) and isx_instance
 SECTION_DTYPE = np.dtype([("type", "<i4"), ("vB", "<i4"), ("vT", "<i4"), ("disparity", "<f4"),
@@ -254,6 +270,9 @@ def _declare(lib):
     lib.isx_tracker_read_state.argtypes = [H, C.c_void_p, i, C.POINTER(i), C.POINTER(C.c_int64)]
     lib.isx_tracker_last_error.argtypes = [H]
     lib.isx_tracker_last_error.restype = C.c_char_p
+    lib.isx_bev_params_init.argtypes = [C.POINTER(BevParams)]
+    lib.isx_bev_params_init.restype = None
+    lib.isx_bev_grid_device.argtypes = [H, i, i, C.POINTER(BevParams), C.c_void_p]
     lib.isx_pool_compute_host_road.argtypes = [H, i, i, C.c_void_p, C.c_void_p, C.POINTER(Road), C.c_void_p,
                                                C.c_void_p, C.c_void_p, C.c_void_p, i, C.c_void_p]
 

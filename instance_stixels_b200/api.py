@@ -37,6 +37,20 @@ def StixelConfig(**fields) -> L.Config:
     return cfg
 
 
+def BevParams(**fields) -> L.BevParams:
+    """isx_bev_params with the library's defaults (isx_bev_params_init: x_min -20, z_min 0, cell 0.2 m, nx 200,
+    nz 300) + overrides."""
+    lib = L.load()
+    p = L.BevParams()
+    lib.isx_bev_params_init(C.byref(p))
+    names = {n for n, _ in L.BevParams._fields_}
+    for k, v in fields.items():
+        if k not in names:
+            raise InvalidArgument(f"BevParams has no field {k!r}")
+        setattr(p, k, v)
+    return p
+
+
 def _roads(roads: Sequence[dict]):
     arr = (L.Road * len(roads))()
     for i, r in enumerate(roads):
@@ -115,12 +129,24 @@ class DeviceObjects:
 
 
 @dataclass
+class DeviceBev:
+    """Bird's-eye-view grids on the device (Stixels.BevGridDevice): `cells` is the int32 [n, nz, nx, 2] tensor of
+    isx_bev_cell records, `stixel` the occupant's frame-local index (-1 = none; row frame_offsets[f] + stixel of the
+    stixel export), `state` BEV_UNKNOWN / BEV_FREE / BEV_OCCUPIED.  `params` is the isx_bev_params of the grid."""
+    cells: Any
+    params: Any
+
+    stixel = property(lambda self: self.cells[..., 0])
+    state = property(lambda self: self.cells[..., 1])
+
+
+@dataclass
 class DeviceStixels:
     """Torch tensors of Stixels.ComputeBatchTensors (the isx_device_results layout).  `sections` is the int32
     [capacity, 8] view of the Sections; frame f owns rows [frame_offsets[f], frame_offsets[f+1]); `vertices` is
     [capacity, 4, 3] or None.  With road estimation on the device (road=), `road_estimates` holds what the
     estimation returned for every frame and `roads` the road every frame was computed with.  With objects=True,
-    `objects` holds the instances of the batch as objects."""
+    `objects` holds the instances of the batch as objects.  With bev=, `bev` holds its bird's-eye-view grids."""
     sections: Any
     frame_offsets: Any
     column_offsets: Any
@@ -130,6 +156,7 @@ class DeviceStixels:
     road_estimates: Optional[DeviceRoadEstimates] = None
     roads: Optional[DeviceRoads] = None
     objects: Optional[DeviceObjects] = None
+    bev: Optional[DeviceBev] = None
 
     # typed columns of `sections` (isx_section)
     @property
@@ -268,11 +295,18 @@ class Stixels:
                               capacity, 0)
         self._check(self._lib.isx_export_objects_device(self._h, first, n, C.byref(out)))
 
+    def BevGridDevice(self, first: int, n: int, params: L.BevParams, d_cells: int):
+        """Stixels of frames [first, first+n) of the last batch projected onto bird's-eye-view grids (`params`, see
+        BevParams) in a caller device buffer of n * nz * nx isx_bev_cell records (raw pointer, 8-byte aligned): free,
+        occupied (with the nearest OBJECT stixel's frame-local index) and unknown cells.  Asynchronous on stream()."""
+        self._check(self._lib.isx_bev_grid_device(self._h, first, n, C.byref(params), d_cells or None))
+
     def ComputeBatchTensors(self, pairwise: bool, disparity, roads: Optional[Sequence[dict]] = None,
                             segmentation=None, cnn=None, vertices: bool = False, capacity: Optional[int] = None,
                             road: Optional["RoadEstimation"] = None, fallback: Optional[dict] = None,
                             objects: bool = False, object_capacity: Optional[int] = None,
-                            tracker: Optional["ObjectTracker"] = None) -> "DeviceStixels":
+                            tracker: Optional["ObjectTracker"] = None,
+                            bev: Optional[L.BevParams] = None) -> "DeviceStixels":
         """CUDA torch tensors in, torch tensors out, no host synchronisation: `disparity` float32 [n][rows][cols]
         and either `segmentation` int32 in the library layout [n][realcols][21][rows_power2_segmentation] or `cnn`
         float32 [n][21][rows/8][cols/8] (run through FlipAndPadBatchDevice).  The library's stream waits for the
@@ -284,7 +318,8 @@ class Stixels:
         objects=True: the result also carries `objects` (ExportObjectsDevice of the batch, with extents when
         vertices=True); `object_capacity` defaults to the worst case n * realcols * 200.
         tracker=ObjectTracker (with objects=True): the n frames are the tracker's next frames; `objects` also carries
-        `track_ids`, `track_hits` and `track_flags` (ObjectTracker.update), in stream order after the export."""
+        `track_ids`, `track_hits` and `track_flags` (ObjectTracker.update), in stream order after the export.
+        bev=BevParams(...): the result also carries `bev`, the bird's-eye-view grid of every frame (BevGridDevice)."""
         import torch
         if tracker is not None and not objects:
             raise InvalidArgument("tracker= needs objects=True")
@@ -337,6 +372,11 @@ class Stixels:
                 out.objects.track_ids = torch.empty(ocap, dtype=torch.int64, device=dev)
                 out.objects.track_hits = torch.empty(ocap, dtype=torch.int32, device=dev)
                 out.objects.track_flags = torch.empty(n, dtype=torch.int32, device=dev)
+        if bev is not None:
+            if not (1 <= bev.nx <= L.BEV_MAX_SIDE and 1 <= bev.nz <= L.BEV_MAX_SIDE):
+                raise InvalidArgument("bev: nx and nz must be in 1..4096")
+            out.bev = DeviceBev(torch.empty((n, bev.nz, bev.nx, 2), dtype=torch.int32, device=dev),
+                                L.BevParams(bev.x_min, bev.z_min, bev.cell, bev.nx, bev.nz, bev.reserved))
         if road is not None:
             out.road_estimates = DeviceRoadEstimates(torch.empty((n, 7), dtype=torch.int32, device=dev))
             out.roads = DeviceRoads(torch.empty((n, 4), dtype=torch.int32, device=dev))
@@ -348,27 +388,32 @@ class Stixels:
         ext.wait_event(ready)
         for t in inputs:
             t.record_stream(ext)   # read on the library's stream: not reused before that work is done
-        if cnn is not None:
-            self.FlipAndPadBatchDevice(n, cnn.data_ptr(), cnn.shape[2], cnn.shape[3], segmentation.data_ptr())
-        if road is None:
-            self.ComputeBatchDevice(pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), roads)
-        else:
-            self.ComputeBatchDeviceRoad(road, pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), fallback,
-                                        out.road_estimates.data.data_ptr(), out.roads.data.data_ptr())
-        self.ExportBatchDevice(0, n, out.frame_offsets.data_ptr(), sections=out.sections.data_ptr(),
-                               column_offsets=out.column_offsets.data_ptr(), labels=out.labels.data_ptr(),
-                               vertices=out.vertices.data_ptr() if vertices else 0,
-                               frame_errors=out.frame_errors.data_ptr(), capacity=cap)
-        if objects:
-            ob = out.objects
-            self.ExportObjectsDevice(0, n, ob.frame_offsets.data_ptr(), objects=ob.data.data_ptr(),
-                                     class_offsets=ob.class_offsets.data_ptr(),
-                                     extents=ob.extents.data_ptr() if vertices else 0, capacity=ocap)
-            if tracker is not None:
-                tracker._enqueue(self.stream(), n, ob, ob.track_ids, ob.track_hits, ob.track_flags)
-        done = torch.cuda.Event()
-        done.record(ext)
-        current.wait_event(done)
+        try:
+            if cnn is not None:
+                self.FlipAndPadBatchDevice(n, cnn.data_ptr(), cnn.shape[2], cnn.shape[3], segmentation.data_ptr())
+            if road is None:
+                self.ComputeBatchDevice(pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), roads)
+            else:
+                self.ComputeBatchDeviceRoad(road, pairwise, n, disparity.data_ptr(), segmentation.data_ptr(), fallback,
+                                            out.road_estimates.data.data_ptr(), out.roads.data.data_ptr())
+            self.ExportBatchDevice(0, n, out.frame_offsets.data_ptr(), sections=out.sections.data_ptr(),
+                                   column_offsets=out.column_offsets.data_ptr(), labels=out.labels.data_ptr(),
+                                   vertices=out.vertices.data_ptr() if vertices else 0,
+                                   frame_errors=out.frame_errors.data_ptr(), capacity=cap)
+            if objects:
+                ob = out.objects
+                self.ExportObjectsDevice(0, n, ob.frame_offsets.data_ptr(), objects=ob.data.data_ptr(),
+                                         class_offsets=ob.class_offsets.data_ptr(),
+                                         extents=ob.extents.data_ptr() if vertices else 0, capacity=ocap)
+                if tracker is not None:
+                    tracker._enqueue(self.stream(), n, ob, ob.track_ids, ob.track_hits, ob.track_flags)
+            if bev is not None:
+                self.BevGridDevice(0, n, out.bev.params, out.bev.cells.data_ptr())
+        finally:
+            # also after a refusal: the outputs are not released before the work already enqueued is done
+            done = torch.cuda.Event()
+            done.record(ext)
+            current.wait_event(done)
         return out
 
     def SetRoadParameters(self, vhor: int, camera_tilt: float, camera_height: float, alpha_ground: float):

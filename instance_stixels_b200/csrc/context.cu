@@ -12,6 +12,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -120,6 +121,7 @@ struct Initialized {
   int *d_raster_table = nullptr;                  // [max_batch][C][200] instance id per stixel (rasteriser)
   int *d_export_col = nullptr;                    // [max_batch][C] frame-relative column offsets (device export)
   int *d_object_class = nullptr;                  // [max_batch*8+1] objects per (frame, class), then their prefix
+  int *d_bev_frames = nullptr;                    // [max_batch+1] stixels per frame (the BEV grid's column scan)
   int inst_cap = 0;                               // instance records per frame of the device arrays: C * 200
   float *d_export_cost = nullptr;
   int *d_export_index = nullptr;
@@ -993,6 +995,7 @@ int isx_initialize(isx_handle h, int max_batch) {
   ISX_TRY(h, dev_alloc(I, &I.d_raster_table, MB * C * kMaxSections));
   ISX_TRY(h, dev_alloc(I, &I.d_export_col, MB * C));
   ISX_TRY(h, dev_alloc(I, &I.d_object_class, MB * ISX_INSTANCE_CLASSES + 1));
+  ISX_TRY(h, dev_alloc(I, &I.d_bev_frames, MB + 1));
   ISX_TRY(h, dev_alloc(I, &I.d_export_cost, C * H * 3));
   ISX_TRY(h, dev_alloc(I, &I.d_export_index, C * H * 3));
 
@@ -1566,6 +1569,60 @@ int isx_export_objects_device(isx_handle h, int first, int n, const isx_device_o
   a.camera_center_y = m.camera_center_y;
   a.out = *out;
   launch_export_objects(a, n, I.s_tables);
+  ISX_TRY(h, cudaGetLastError());
+  return ISX_OK;
+}
+
+void isx_bev_params_init(isx_bev_params *p) {
+  if (p) *p = isx_bev_params{-20.0f, 0.0f, 0.2f, 200, 300, 0};
+}
+
+// Like isx_export_batch_device: reads result set rs[cur] on s_tables, with the export's roads.
+int isx_bev_grid_device(isx_handle h, int first, int n, const isx_bev_params *p, isx_bev_cell *d_cells) {
+  if (int rc = check_ready(h)) return rc;
+  Initialized &I = *h->init;
+  if (first < 0 || n < 1 || first + n > I.last_batch)
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "frames outside the last computed batch");
+  if (!d_cells || (uintptr_t)d_cells % 8 != 0)
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "d_cells must be a non-null 8-byte aligned device pointer");
+  if (!p) return fail(h, ISX_ERR_INVALID_ARGUMENT, "null BEV parameters");
+  if (!(std::isfinite(p->cell) && p->cell >= 1e-3f && p->cell <= 1e3f))
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "cell must be finite and in [1e-3, 1e3] metres");
+  if (p->nx < 1 || p->nx > ISX_BEV_MAX_SIDE || p->nz < 1 || p->nz > ISX_BEV_MAX_SIDE)
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "nx and nz must be in 1..ISX_BEV_MAX_SIDE");
+  if (!(std::isfinite(p->x_min) && std::isfinite(p->z_min) && std::fabs(p->x_min) <= 1e5f &&
+        std::fabs(p->z_min) <= 1e5f))
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "x_min and z_min must be finite with magnitude <= 1e5");
+  if (p->reserved != 0) return fail(h, ISX_ERR_INVALID_ARGUMENT, "reserved must be 0");
+  const HostModel &m = h->model;
+  if (m.camera_center_x == -1 || m.camera_center_y == -1)
+    return fail(h, ISX_ERR_INVALID_ARGUMENT, "Camera parameters are not set.");  // Get3DVertices (Stixels.cu:685-687)
+  if (int rc = no_batches_in_flight(h)) return rc;
+  if (int rc = ensure_joined(h)) return rc;
+  const size_t C = I.kp.realcols;
+  const Initialized::ResultSet &R = I.rs[I.cur];
+  BevArgs a;
+  a.sections = R.d_sections + (size_t)first * C * kMaxSections;
+  a.n_sections = R.d_nsections + (size_t)first * C;
+  a.col_local = I.d_export_col;
+  a.frame_totals = I.d_bev_frames;
+  a.realcols = I.kp.realcols;
+  a.rows = I.kp.rows;
+  a.column_step = I.kp.column_step;
+  a.focal = m.focal;
+  a.bf = m.baseline * m.focal;
+  a.camera_center_x = m.camera_center_x;
+  a.camera_center_y = m.camera_center_y;
+  a.roads = I.last_roads_dev ? I.last_roads_dev + first : nullptr;
+  a.p = *p;
+  a.cells = d_cells;
+  std::vector<float> alpha((size_t)n);
+  std::vector<int> vhor((size_t)n);
+  for (int f = 0; f < n && !a.roads; f++) {
+    alpha[f] = I.last_roads[first + f].alpha_ground;
+    vhor[f] = I.kp.rows - I.last_roads[first + f].vhor - 1;   // isx_frame_meta.vhor (Stixels.cu:377)
+  }
+  launch_bev_grid(a, n, alpha.data(), vhor.data(), I.s_tables);
   ISX_TRY(h, cudaGetLastError());
   return ISX_OK;
 }

@@ -3,10 +3,11 @@
 // [frame_offsets[f], frame_offsets[f+1]), column 0 first, each column top to bottom (the order of
 // isx_wait_batch_packed and of Stixels::Get3DVertices); column c of frame f starts at column_offsets[f*C + c].
 // Per stixel there is an instance label (the map GetInstanceStixels returns, -2 for stixels outside it) and the
-// four corner points Get3DVertices computes (Stixels.hpp, Stixels.cu:683-742).
+// four corner points Get3DVertices computes (Stixels.hpp, Stixels.cu:683-742, vertices.cuh).
 // Unlike pack_results_kernel, which places frames with atomicAdd, every position follows from the scans: the bytes
 // are the same from run to run.
 #include "kernels.h"
+#include "vertices.cuh"
 
 namespace isx {
 namespace {
@@ -83,32 +84,6 @@ export_frame_scan_kernel(int *__restrict__ frame_offsets, int *__restrict__ colu
   if (tid == 0) {
     frame_offsets[0] = 0;
     if (column_offsets) column_offsets[(size_t)n * C] = s_running;
-  }
-}
-
-// Stixels::Get3DVertices for one Section, in the header's operation order (xl = i * step, xr = xl + step,
-// yt = rows - vT - 1, yb = rows - vB; z = bf / disparity for objects, bf / (alpha_ground * (vhor - v)) for ground,
-// 0 for sky; then per corner -z / f * (c - x), -z / f * (c - y), z), with every operation rounded on its own.
-// Args: ExportArgs or ObjectArgs (column_step, rows, bf, focal, camera_center_x/y).
-template <class Args>
-__device__ __forceinline__ void stixel_vertices(const isx_section &s, int col, const Args &a, float alpha, int vhor,
-                                                float *v) {
-  const float xl = (float)(col * a.column_step), xr = __fadd_rn(xl, (float)a.column_step);
-  const float yt = (float)(a.rows - s.vT - 1), yb = (float)(a.rows - s.vB);
-  float zt = 0.0f, zb = 0.0f;
-  if (s.type == OBJECT) {
-    zt = zb = __fdiv_rn(a.bf, s.disparity);
-  } else if (s.type == GROUND) {
-    zt = __fdiv_rn(a.bf, __fmul_rn(alpha, (float)(vhor - s.vT)));
-    zb = __fdiv_rn(a.bf, __fmul_rn(alpha, (float)(vhor - s.vB)));
-  }
-  const float cx[4] = {xl, xr, xr, xl}, cy[4] = {yt, yt, yb, yb}, cz[4] = {zt, zt, zb, zb};
-#pragma unroll
-  for (int k = 0; k < 4; k++) {
-    const float q = __fdiv_rn(-cz[k], a.focal);
-    v[3 * k + 0] = __fmul_rn(q, __fsub_rn(a.camera_center_x, cx[k]));
-    v[3 * k + 1] = __fmul_rn(q, __fsub_rn(a.camera_center_y, cy[k]));
-    v[3 * k + 2] = cz[k];
   }
 }
 
@@ -307,6 +282,12 @@ void launch_export_objects(const ObjectArgs &a, int nframes, cudaStream_t s) {
   export_frame_scan_kernel<<<1, kFrameScanThreads, 0, s>>>(a.class_start, nullptr, nframes * kClasses, 0);
   export_objects_kernel<<<nframes, kObjectThreads, 0, s>>>(a);
   g_launch_count += 3;
+}
+
+void launch_export_column_scan(const int *n_sections, int realcols, int *col_local, int *frame_totals, int nframes,
+                               cudaStream_t s) {
+  export_column_scan_kernel<<<nframes, kExportThreads, 0, s>>>(n_sections, realcols, col_local, frame_totals);
+  g_launch_count++;
 }
 
 void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_ground, const int *vhor,

@@ -113,6 +113,9 @@ struct ExportFrames {              // per-frame road scalars of one launch: alph
 };
 void launch_export_results(const ExportArgs &a, int nframes, const float *alpha_ground, const int *vhor,
                            cudaStream_t s);
+// The export's column scan alone: col_local [n][C] as above, the stixels of frame f into frame_totals[f + 1].
+void launch_export_column_scan(const int *n_sections, int realcols, int *col_local, int *frame_totals, int nframes,
+                               cudaStream_t s);
 // Device objects of a computed batch (export.cu): frames [0, n) of the arrays below, into the caller's buffers.
 struct ObjectArgs {
   const isx_section *sections;   // [n][C][200] padded device results
@@ -125,6 +128,19 @@ struct ObjectArgs {
   isx_device_objects out;
 };
 void launch_export_objects(const ObjectArgs &a, int nframes, cudaStream_t s);
+// Bird's-eye-view grid of a computed batch (bev.cu): frames [0, n) of the arrays below, into the caller's cells.
+struct BevArgs {
+  const isx_section *sections;   // [n][C][200] padded device results
+  const int *n_sections;         // [n][C]
+  int *col_local;                // [n][C] scratch: column offsets relative to the frame (the export's column scan)
+  int *frame_totals;             // [n+1] scratch: stixels per frame (written by the scan, not read)
+  int realcols, rows, column_step;
+  float focal, bf, camera_center_x, camera_center_y;   // bf = baseline * focal
+  const isx_road *roads;         // [n] device roads (batches that estimated them) or null: ExportFrames then
+  isx_bev_params p;
+  isx_bev_cell *cells;           // [n][nz][nx], 8-byte aligned
+};
+void launch_bev_grid(const BevArgs &a, int nframes, const float *alpha_ground, const int *vhor, cudaStream_t s);
 // Road estimation in front of a device batch (road.cu, isx_compute_batch_device_road) or of a chunk of a host batch
 // (isx_submit_batch_host_road): the checks (nothing enqueued), then the Hough kernels, the device line selection and
 // the keep-last rule on the road handle's stream, ordered after and before `caller`.  d_roads [n]: the road every
